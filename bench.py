@@ -24,16 +24,32 @@ facades (YOLODetector.detect -> DeepSORT.update), timed the reference's way (fra
 --config crowded (configs[4]): 300 persons per frame per stream: ReID batch 300 per stream and a 300 x 300
 association per stream through TrackingPipeline (planted person boxes riding on the moving texture; the detector still
 runs and is timed).
+
+--dump-outputs DIR (--config streams64): after the timed steps, rank 0 writes what TrackingPipeline.step returned in the
+last timed step as DIR/out_tracks.npy (float64 [S, T, 6]: x1, y1, x2, y2, id, class), DIR/out_conf.npy (float32 [S, T])
+and DIR/out_count.npy (float64 [S]).  Rows at or past a stream's count hold no track and are written as zeros.  The
+inputs depend only on the arguments, so two builds run with the same arguments can be compared file for file.
+
+--steps sets the number of timed steps of --config streams64 and crowded and of --impl reference.  --config clip
+times the whole clip (and 128 device-resident steps), --config sweep fixed iteration counts per batch size.
+
+The benchmark writes nothing into the repository, so it also runs from a read-only checkout: the seeded weight blobs go
+to $AICAM_BLOB_DIR when it is set, else to a temporary directory removed at exit (regenerating them takes a few
+seconds, outside every timed region).
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True  # nothing into the tree, not even __pycache__ for the modules build() never imported
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -202,6 +218,18 @@ def pin_rank(local, world):
         pass
 
 
+def dump_outputs(directory, out_tracks, out_conf, out_count):
+    """Host copies of one step's track tables -> DIR/<name>.npy; rows past each stream's count are zeroed (they are
+    left over from earlier steps, not part of the result)."""
+    import numpy as np
+    tracks, conf, count = (t.cpu().numpy() for t in (out_tracks, out_conf, out_count))
+    valid = np.arange(tracks.shape[1])[None, :] < count[:, None]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "out_tracks.npy"), np.where(valid[..., None], tracks, 0).astype(np.float64))
+    np.save(os.path.join(directory, "out_conf.npy"), np.where(valid, conf, 0).astype(np.float32))
+    np.save(os.path.join(directory, "out_count.npy"), count.astype(np.float64))
+
+
 def conv_roofline(lib, _lib, one_step, crops_of_step, flops_of, prof_steps=6):
     """Event-instrumented pass over the tcgen05 convolution kernels: (TFLOP/s, ms per step, launches per step, crops)."""
     lib.aicam_profile_enable(1)
@@ -341,6 +369,8 @@ def run_streams(args):
     torch.cuda.synchronize(dev)
     total_ms = ev[0].elapsed_time(ev[-1])
     per_step = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
+    if args.dump_outputs and rank == 0:  # the buffers TrackingPipeline.step returns (and the graphs write into)
+        dump_outputs(args.dump_outputs, pipe.tracker.out_tracks, pipe.tracker.out_conf, pipe.tracker.out_count)
     sync_all()
     launches_eager = launches_counted
     gpu_launches = (lib.aicam_launch_count() - launches0) if graphs is None else launches_eager * args.steps
@@ -733,6 +763,13 @@ def run_crowded(args):
     emit(line)
 
 
+def positive_int(text):
+    value = int(text)
+    if value < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % value)
+    return value
+
+
 def main():
     global _RESULT
     sys.stdout.flush()
@@ -740,7 +777,9 @@ def main():
     os.dup2(2, 1)  # stdout carries exactly one JSON line
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=positive_int, default=40,
+                    help="timed steps of --config streams64 / crowded and of --impl reference; --config clip times the "
+                         "whole clip and --config sweep fixed iteration counts per batch size")
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="aicam", choices=["aicam", "reference"])
     ap.add_argument("--config", default="streams64", choices=["streams64", "clip", "sweep", "crowded"])
@@ -750,7 +789,14 @@ def main():
     ap.add_argument("--max-batch", type=int, default=256)
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's track tables as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "aicam" or args.config != "streams64"):
+        ap.error("--dump-outputs is implemented for --impl aicam --config streams64")
+    if "AICAM_BLOB_DIR" not in os.environ:
+        blob_dir = tempfile.mkdtemp(prefix="aicam-bench-blobs-")
+        atexit.register(shutil.rmtree, blob_dir, True)
+        os.environ["AICAM_BLOB_DIR"] = blob_dir
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

@@ -16,7 +16,8 @@ from oracle import ref_bridge  # noqa: E402
 
 def reference_visualization():
     if not ref_bridge.available():
-        pytest.skip("oracle/_ref (snapshot of the reference) is not built")
+        pytest.skip("needs oracle/_ref, a snapshot of the original AI-Camera sources (python oracle/build_ref.py "
+                    "<checkout of the original project>); no recorded output of its drawing functions replaces it")
     ref_bridge.import_reference()
     import src.utils.visualization as rv
     rv.config.CLASS_COLORS = dict(config.CLASS_COLORS)  # (the reference draws its colours at random at import)

@@ -1,6 +1,9 @@
-"""The REAL reference tracker (oracle/_ref, snapshotted from /root/reference by oracle/build_ref.py at build
-time; it travels to the GPU box) against the oracle restatement (CPU) and against the device tracker (GPU), on
-fresh seeds - the golden fixtures pin the same thing on recorded seeds only."""
+"""The REAL reference tracker against the oracle restatement (CPU) and against the device tracker (GPU), on fresh
+seeds - the golden fixtures pin the same thing on recorded seeds only.
+
+The reference runs from oracle/_ref, a snapshot of the original AI-Camera sources that ``python oracle/build_ref.py
+<checkout of the original project>`` makes.  The sources are not part of this repository and no output of the
+reference on these seeds is stored, so without the snapshot these tests skip."""
 import numpy as np
 import pytest
 
@@ -11,7 +14,8 @@ from scenarios import make_scenario
 def _ref():
     from oracle import ref_bridge
     if not ref_bridge.available():
-        pytest.skip("oracle/_ref is not built (python oracle/build_ref.py needs /root/reference)")
+        pytest.skip("needs oracle/_ref, a snapshot of the original AI-Camera sources (python oracle/build_ref.py "
+                    "<checkout of the original project>); no recorded output replaces it")
     return ref_bridge
 
 
