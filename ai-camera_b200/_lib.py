@@ -45,6 +45,11 @@ class NmsParams(C.Structure):
                 ("max_candidates", C.c_int), ("frame_h", C.c_int), ("frame_w", C.c_int)]
 
 
+class FrameDesc(C.Structure):
+    _fields_ = [("data", C.c_void_p), ("chroma", C.c_void_p), ("h", C.c_int), ("w", C.c_int), ("pitch", C.c_int),
+                ("kind", C.c_int)]
+
+
 class TrackerConfig(C.Structure):
     _fields_ = [("n_streams", C.c_int), ("max_tracks", C.c_int), ("max_dets", C.c_int),
                 ("feature_dim", C.c_int), ("max_cosine_distance", C.c_double),
@@ -102,6 +107,13 @@ SIGNATURES = {
     "aicam_preprocess": (_I, [_P, _I, _I, _I, _I, _P, _P]),
     "aicam_preprocess_nv12": (_I, [_P, _I, _I, _I, _I, _P, _P]),
     "aicam_nv12_to_bgr": (_I, [_P, _I, _I, _I, _P, _P]),
+    "aicam_frame_table_create": (_I, [_I, _I, _I, _I, C.POINTER(_P)]),
+    "aicam_frame_table_destroy": (None, [_P]),
+    "aicam_frame_table_set": (_I, [_P, C.POINTER(FrameDesc), _I, _P]),
+    "aicam_preprocess_table": (_I, [_P, _I, _P, _P]),
+    "aicam_yolo_detect_table": (_I, [_P, _P, _I, _P, C.POINTER(NmsParams), _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
+    "aicam_reid_crops_table": (_I, [_P, _P, _P, _P, _P, _I, C.c_float, C.c_uint64, C.c_uint64, _I, _I, _P, _P, _P, _P,
+                                    _P, _P, _P]),
     "aicam_decode_nms": (_I, [_P, _I, _I, _I, C.POINTER(NmsParams), _P, _P, _P, _P, _P, _P,
                               C.c_size_t, _P]),
     "aicam_decode_nms_workspace": (C.c_size_t, [_I, _I, C.POINTER(NmsParams)]),

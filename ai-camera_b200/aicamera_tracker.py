@@ -107,7 +107,8 @@ def run_single_stream(frames: Iterable[np.ndarray], detector, tracker, on_frame=
 def run_batched(sources: List[Iterable[np.ndarray]], pipeline, on_step=None, max_steps=0, stats_out=None) -> LoopStats:
     """N streams, one ``TrackingPipeline.step`` per time step.  Frames are read on the host (cv2), staged in two
     pinned buffers and uploaded on a copy stream while the previous step computes; per-stream frame order is kept.
-    Stops when the first source ends.  Time per step = wall time from "frames of the step are on the host" to
+    Sources of different frame shapes get per-stream pinned and device buffers (two each) and the step takes the list
+    of device frames.  Stops when the first source ends.  Time per step = wall time from "frames of the step are on the host" to
     "track tables are on the host" (the detect + update span of the reference loop)."""
     dev = pipeline.device
     its = [iter(s) for s in sources]
@@ -129,15 +130,23 @@ def run_batched(sources: List[Iterable[np.ndarray]], pipeline, on_step=None, max
                 return stats
             batch.append(f)
         if host is None:
-            shape = (S,) + tuple(batch[0].shape)
-            host = [torch.empty(shape, dtype=torch.uint8).pin_memory() for _ in range(2)]
-            dev_buf = [torch.empty(shape, dtype=torch.uint8, device=dev) for _ in range(2)]
+            shapes = [tuple(f.shape) for f in batch]
+            if all(sh == shapes[0] for sh in shapes):
+                host = [torch.empty((S,) + shapes[0], dtype=torch.uint8).pin_memory() for _ in range(2)]
+                dev_buf = [torch.empty((S,) + shapes[0], dtype=torch.uint8, device=dev) for _ in range(2)]
+            else:  # one buffer per stream: the step takes the list of frames
+                host = [[torch.empty(sh, dtype=torch.uint8).pin_memory() for sh in shapes] for _ in range(2)]
+                dev_buf = [[torch.empty(sh, dtype=torch.uint8, device=dev) for sh in shapes] for _ in range(2)]
         h = host[step & 1]
         for s, f in enumerate(batch):
             h[s].numpy()[...] = f
         t0 = time.time()
         d = dev_buf[step & 1]
-        d.copy_(h, non_blocking=True)
+        if isinstance(d, list):
+            for ds, hs in zip(d, h):
+                ds.copy_(hs, non_blocking=True)
+        else:
+            d.copy_(h, non_blocking=True)
         ot, oc, on = pipeline.step(d)
         out_host[0].copy_(ot, non_blocking=True)
         out_host[1].copy_(oc, non_blocking=True)

@@ -16,6 +16,7 @@
 // (~score bits, anchor) in shared memory, (2) all threads fill the suppression bit matrix
 // mask[i][j/32] for j > i, (3) one warp scans it, keeping its "removed" bitmap in registers.
 #include "common.cuh"
+#include "frame_table.cuh"
 
 namespace aicam {
 
@@ -120,6 +121,7 @@ struct NmsArgs {
   int* out_labels;
   int* keep_index;
   uint32_t* mask_ws;     // [batch][max_cand][max_cand/32]
+  const FrameRec* recs;  // frame table: per-frame un-letterboxing (pad_w .. frame_h above unused); null: one geometry
 };
 
 __device__ __forceinline__ bool iou_gt(const float4& a, const float4& b, float thr) {
@@ -222,6 +224,11 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(const NmsArgs p) {
   __syncthreads();
   const int kept = s_kept;
   const long long ob = static_cast<long long>(b) * p.topk;
+  float pad_w = p.pad_w, pad_h = p.pad_h, ratio = p.ratio, frame_w = p.frame_w, frame_h = p.frame_h;
+  if (p.recs) {
+    const FrameRec& g = p.recs[b];
+    pad_w = g.pad_w; pad_h = g.pad_h; ratio = g.ratio; frame_w = static_cast<float>(g.w); frame_h = static_cast<float>(g.h);
+  }
   for (int r = tid; r < p.topk; r += NMS_THREADS) {
     float4 bx = make_float4(0.f, 0.f, 0.f, 0.f), bo = bx;
     float sc = 0.f;
@@ -233,10 +240,10 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(const NmsArgs p) {
       ki = static_cast<int>(keys[i] & 0xffffffffu);
       sc = __uint_as_float(~static_cast<uint32_t>(keys[i] >> 32));
       // scale_bboxes (image_processing.py:162-181): subtract pad, divide by ratio, clip
-      bo.x = fminf(fmaxf(__fdiv_rn(bx.x - p.pad_w, p.ratio), 0.0f), p.frame_w);
-      bo.y = fminf(fmaxf(__fdiv_rn(bx.y - p.pad_h, p.ratio), 0.0f), p.frame_h);
-      bo.z = fminf(fmaxf(__fdiv_rn(bx.z - p.pad_w, p.ratio), 0.0f), p.frame_w);
-      bo.w = fminf(fmaxf(__fdiv_rn(bx.w - p.pad_h, p.ratio), 0.0f), p.frame_h);
+      bo.x = fminf(fmaxf(__fdiv_rn(bx.x - pad_w, ratio), 0.0f), frame_w);
+      bo.y = fminf(fmaxf(__fdiv_rn(bx.y - pad_h, ratio), 0.0f), frame_h);
+      bo.z = fminf(fmaxf(__fdiv_rn(bx.z - pad_w, ratio), 0.0f), frame_w);
+      bo.w = fminf(fmaxf(__fdiv_rn(bx.w - pad_h, ratio), 0.0f), frame_h);
     }
     reinterpret_cast<float4*>(p.boxes_lb)[ob + r] = bx;
     if (p.boxes_orig) reinterpret_cast<float4*>(p.boxes_orig)[ob + r] = bo;
@@ -265,7 +272,7 @@ size_t mask_bytes(int batch, const aicam_nms_params* p) {
 
 int launch_nms(const float* boxes, const float* scores, const int* labels, int batch, int anchors,
                const aicam_nms_params* p, int* num_dets, float* boxes_lb, float* boxes_orig, float* out_scores,
-               int* out_labels, int* keep_index, uint32_t* mask_ws, cudaStream_t stream) {
+               int* out_labels, int* keep_index, uint32_t* mask_ws, cudaStream_t stream, const FrameRec* recs) {
   NmsArgs a;
   a.boxes = boxes; a.scores = scores; a.labels = labels; a.anchors = anchors;
   a.score_thr = p->score_thr; a.iou_thr = p->iou_thr; a.topk = p->topk; a.max_cand = p->max_candidates;
@@ -274,7 +281,8 @@ int launch_nms(const float* boxes, const float* scores, const int* labels, int b
   if (p->frame_h > 0 && p->frame_w > 0) letterbox_geometry(p->frame_h, p->frame_w, &r, &nh, &nw, &dw, &dh, &top, &left);
   a.pad_w = static_cast<float>(dw); a.pad_h = static_cast<float>(dh); a.ratio = static_cast<float>(r);
   a.frame_w = static_cast<float>(p->frame_w); a.frame_h = static_cast<float>(p->frame_h);
-  a.num_dets = num_dets; a.boxes_lb = boxes_lb; a.boxes_orig = (p->frame_h > 0 && p->frame_w > 0) ? boxes_orig : nullptr;
+  a.num_dets = num_dets; a.boxes_lb = boxes_lb; a.boxes_orig = (recs || (p->frame_h > 0 && p->frame_w > 0)) ? boxes_orig : nullptr;
+  a.recs = recs;
   a.out_scores = out_scores; a.out_labels = out_labels; a.keep_index = keep_index; a.mask_ws = mask_ws;
   if (int rc = ensure_dynamic_smem(nms_kernel, NMS_SMEM)) return rc;
   nms_kernel<<<batch, NMS_THREADS, NMS_SMEM, stream>>>(a);
@@ -283,6 +291,37 @@ int launch_nms(const float* boxes, const float* scores, const int* labels, int b
 }
 
 }  // namespace
+
+// aicam_nms / aicam_decode_nms; recs: per-frame un-letterboxing from a frame table (aicam_yolo_detect_table), or null
+int nms_impl(const float* boxes, const float* scores, const int32_t* labels, int batch, int anchors, const aicam_nms_params* p,
+             int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* out_scores, int32_t* out_labels, int32_t* keep_index,
+             void* workspace, size_t workspace_bytes, void* stream, const FrameRec* recs) {
+  if (int rc = check_params(p, anchors)) return rc;
+  if (!boxes || !scores || !labels || !num_dets || !boxes_lb || !out_scores || !out_labels || batch < 0)
+    return fail(AICAM_ERR_INVALID_ARG, "nms: null argument");
+  if (batch == 0) return AICAM_OK;
+  if (!workspace || workspace_bytes < mask_bytes(batch, p)) return fail(AICAM_ERR_CAPACITY, "nms: workspace too small");
+  return launch_nms(boxes, scores, labels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, out_scores, out_labels,
+                    keep_index, static_cast<uint32_t*>(workspace), static_cast<cudaStream_t>(stream), recs);
+}
+
+int decode_nms_impl(const float* head, int batch, int anchors, int nc, const aicam_nms_params* p, int32_t* num_dets,
+                    float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
+                    size_t workspace_bytes, void* stream, const FrameRec* recs) {
+  if (int rc = check_params(p, anchors)) return rc;
+  if (batch == 0) return AICAM_OK;
+  if (!workspace || workspace_bytes < aicam_decode_nms_workspace(batch, anchors, p))
+    return fail(AICAM_ERR_CAPACITY, "decode_nms: workspace too small");
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  float* dboxes = reinterpret_cast<float*>(ws);
+  float* dscores = reinterpret_cast<float*>(ws + static_cast<size_t>(batch) * anchors * 16);
+  int* dlabels = reinterpret_cast<int*>(ws + static_cast<size_t>(batch) * anchors * 20);
+  uint32_t* mask = reinterpret_cast<uint32_t*>(ws + (dense_bytes(batch, anchors) + 255) / 256 * 256);
+  if (int rc = aicam_decode(head, batch, anchors, nc, dboxes, dscores, dlabels, stream)) return rc;
+  return launch_nms(dboxes, dscores, dlabels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, scores, labels, nullptr,
+                    mask, static_cast<cudaStream_t>(stream), recs);
+}
+
 }  // namespace aicam
 
 using namespace aicam;
@@ -311,30 +350,15 @@ int aicam_decode(const float* head, int batch, int anchors, int nc, float* boxes
 int aicam_nms(const float* boxes, const float* scores, const int32_t* labels, int batch, int anchors,
               const aicam_nms_params* p, int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* out_scores,
               int32_t* out_labels, int32_t* keep_index, void* workspace, size_t workspace_bytes, void* stream) {
-  if (int rc = check_params(p, anchors)) return rc;
-  if (!boxes || !scores || !labels || !num_dets || !boxes_lb || !out_scores || !out_labels || batch < 0)
-    return fail(AICAM_ERR_INVALID_ARG, "nms: null argument");
-  if (batch == 0) return AICAM_OK;
-  if (!workspace || workspace_bytes < mask_bytes(batch, p)) return fail(AICAM_ERR_CAPACITY, "nms: workspace too small");
-  return launch_nms(boxes, scores, labels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, out_scores, out_labels,
-                    keep_index, static_cast<uint32_t*>(workspace), static_cast<cudaStream_t>(stream));
+  return nms_impl(boxes, scores, labels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, out_scores, out_labels, keep_index,
+                  workspace, workspace_bytes, stream, nullptr);
 }
 
 int aicam_decode_nms(const float* head, int batch, int anchors, int nc, const aicam_nms_params* p, int32_t* num_dets,
                      float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
                      size_t workspace_bytes, void* stream) {
-  if (int rc = check_params(p, anchors)) return rc;
-  if (batch == 0) return AICAM_OK;
-  if (!workspace || workspace_bytes < aicam_decode_nms_workspace(batch, anchors, p))
-    return fail(AICAM_ERR_CAPACITY, "decode_nms: workspace too small");
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  float* dboxes = reinterpret_cast<float*>(ws);
-  float* dscores = reinterpret_cast<float*>(ws + static_cast<size_t>(batch) * anchors * 16);
-  int* dlabels = reinterpret_cast<int*>(ws + static_cast<size_t>(batch) * anchors * 20);
-  uint32_t* mask = reinterpret_cast<uint32_t*>(ws + (dense_bytes(batch, anchors) + 255) / 256 * 256);
-  if (int rc = aicam_decode(head, batch, anchors, nc, dboxes, dscores, dlabels, stream)) return rc;
-  return launch_nms(dboxes, dscores, dlabels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, scores, labels, nullptr,
-                    mask, static_cast<cudaStream_t>(stream));
+  return decode_nms_impl(head, batch, anchors, nc, p, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
+                         stream, nullptr);
 }
 
 }  // extern "C"

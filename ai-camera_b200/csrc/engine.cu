@@ -18,12 +18,19 @@
 
 #include "conv_chain.cuh"
 #include "conv_tc.cuh"
+#include "frame_table.cuh"
 #include "layers.cuh"
 #include "stem_pool.cuh"
 
 namespace aicam {
 
 bool profile_enabled();
+int nms_impl(const float* boxes, const float* scores, const int32_t* labels, int batch, int anchors, const aicam_nms_params* p,
+             int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* out_scores, int32_t* out_labels, int32_t* keep_index,
+             void* workspace, size_t workspace_bytes, void* stream, const FrameRec* recs);
+int decode_nms_impl(const float* head, int batch, int anchors, int nc, const aicam_nms_params* p, int32_t* num_dets,
+                    float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
+                    size_t workspace_bytes, void* stream, const FrameRec* recs);
 
 namespace {
 
@@ -868,9 +875,10 @@ int aicam_engine_fused_decode(const aicam_engine* e) {
   return (nc % 16 == 0 && nc <= 80 && e->num_anchors == 8400) ? 1 : 0;  // one n-tile of whole 16-column groups per branch
 }
 
-int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch, const aicam_nms_params* p, float* head,
-                      int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
-                      size_t workspace_bytes, void* stream) {
+// aicam_yolo_detect[_table]; recs: the frame table's records (per-frame un-letterboxing), or null
+static int yolo_detect_impl(aicam_engine* e, const void* in, int in_is_s2d, int batch, const aicam_nms_params* p, float* head,
+                            int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
+                            size_t workspace_bytes, void* stream, const FrameRec* recs) {
   if (!e || e->kind != AICAM_KIND_YOLOV8) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect: not a yolov8 engine");
   if (batch < 0 || batch > e->max_batch) return fail(AICAM_ERR_CAPACITY, "yolo_detect: batch exceeds max_batch");
   if (in_is_s2d < 0 || in_is_s2d > 2) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect: in_is_s2d must be 0, 1 or 2");
@@ -881,8 +889,8 @@ int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch,
   if (!aicam_engine_fused_decode(e)) {
     if (!head) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect: this engine needs the fp32 head tensor (no fused decode)");
     if (int rc = run_ops(e, in, batch, head, static_cast<cudaStream_t>(stream), nullptr, in_is_s2d)) return rc;
-    return aicam_decode_nms(head, batch, anchors, nc, p, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
-                            stream);
+    return decode_nms_impl(head, batch, anchors, nc, p, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
+                           stream, recs);
   }
   const size_t need = aicam_decode_nms_workspace(batch, anchors, p);
   if (need == 0 || !workspace || workspace_bytes < need) return fail(AICAM_ERR_CAPACITY, "yolo_detect: workspace too small");
@@ -895,8 +903,23 @@ int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch,
   dec.labels = reinterpret_cast<int*>(ws + static_cast<size_t>(batch) * anchors * 20);
   uint8_t* mask = ws + (dense + 255) / 256 * 256;
   if (int rc = run_ops(e, in, batch, nullptr, static_cast<cudaStream_t>(stream), nullptr, in_is_s2d, &dec)) return rc;
-  return aicam_nms(dec.boxes, dec.scores, dec.labels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, scores, labels, nullptr,
-                   mask, workspace_bytes - static_cast<size_t>(mask - ws), stream);
+  return nms_impl(dec.boxes, dec.scores, dec.labels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, scores, labels, nullptr,
+                  mask, workspace_bytes - static_cast<size_t>(mask - ws), stream, recs);
+}
+
+int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch, const aicam_nms_params* p, float* head,
+                      int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  return yolo_detect_impl(e, in, in_is_s2d, batch, p, head, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
+                          stream, nullptr);
+}
+
+int aicam_yolo_detect_table(aicam_engine* e, const void* in, int in_is_s2d, const aicam_frame_table* t, const aicam_nms_params* p,
+                            float* head, int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  if (!t) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect_table: null frame table");
+  return yolo_detect_impl(e, in, in_is_s2d, t->n, p, head, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
+                          stream, t->recs());
 }
 
 int aicam_yolo_forward_s2d(aicam_engine* e, const void* in_s2d16, int batch, float* head, void* stream) {

@@ -50,4 +50,29 @@ struct FrameSrc<1> {
   }
 };
 
+// Frames of a frame table (frame_table.cuh): rows `pitch` bytes apart, the NV12 chroma plane anywhere.
+//   SRC 2  BGR, row y at f + y * pitch
+//   SRC 3  NV12, luma row y at f + y * pitch, chroma row y / 2 at c + (y / 2) * pitch
+template <>
+struct FrameSrc<2> {
+  const uint8_t* f;
+  int pitch;
+  __device__ __forceinline__ void pix(int y, int x, int (&v)[3]) const {
+    const uint8_t* s = f + static_cast<long long>(y) * pitch + x * 3;
+    v[0] = __ldg(s); v[1] = __ldg(s + 1); v[2] = __ldg(s + 2);
+  }
+};
+
+template <>
+struct FrameSrc<3> {
+  const uint8_t* f;
+  const uint8_t* c;
+  int pitch;
+  __device__ __forceinline__ void pix(int y, int x, int (&v)[3]) const {
+    const int yy = __ldg(f + static_cast<long long>(y) * pitch + x);
+    const uint8_t* cp = c + static_cast<long long>(y >> 1) * pitch + (x & ~1);
+    yuv_to_bgr_601(yy, __ldg(cp), __ldg(cp + 1), v);
+  }
+};
+
 }  // namespace aicam

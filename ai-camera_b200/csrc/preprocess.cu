@@ -26,6 +26,7 @@
 
 #include "common.cuh"
 #include "frame_src.cuh"
+#include "frame_table.cuh"
 #include "tc_ptx.cuh"
 
 namespace aicam {
@@ -131,6 +132,17 @@ int get_geometry(int h, int w, Geometry* out) {
   return AICAM_OK;
 }
 
+}  // namespace
+
+int k1_geometry(int h, int w, int* decimate, int* mode, int* new_h, int* new_w, int* top, int* left, const int** tab) {
+  Geometry g;
+  if (int rc = get_geometry(h, w, &g)) return rc;
+  *decimate = g.decimate; *mode = g.mode; *new_h = g.new_h; *new_w = g.new_w; *top = g.top; *left = g.left; *tab = g.tab;
+  return AICAM_OK;
+}
+
+namespace {
+
 constexpr int PIX = 4;  // output pixels per thread (consecutive x)
 
 // float(v) / 255.0f, correctly rounded, for an integer 0 <= v <= 255: q = v * RN(1/255), one exact remainder, one
@@ -144,18 +156,10 @@ __device__ __forceinline__ float byte_to_unit(int v) {
   return fmaf(fmaf(-255.0f, q, a), rcp, q);
 }
 
-template <int FORMAT, int SRC>
-__global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restrict__ frames, int h, int w, int mode,
-                                                         int new_h, int new_w, int top, int left,
-                                                         const int* __restrict__ tab, void* __restrict__ out,
-                                                         long long total) {
-  const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-  if (idx >= total) return;
-  const int xg = static_cast<int>(idx % (S / PIX));
-  long long t = idx / (S / PIX);
-  const int y = static_cast<int>(t % S);
-  const int n = static_cast<int>(t / S);
-  const FrameSrc<SRC> src{frames + n * FrameSrc<SRC>::frame_bytes(h, w), h, w};
+// Output pixels 4 xg .. 4 xg + 3 of row y of frame n, read from `src` through the frame's letterbox geometry.
+template <int FORMAT, typename Src>
+__device__ __forceinline__ void preprocess_pixels(const Src& src, int mode, int new_h, int new_w, int top, int left,
+                                                  const int* __restrict__ tab, void* __restrict__ out, int n, int y, int xg) {
   const int dy = y - top;
   const bool row_in = dy >= 0 && dy < new_h;
   const int* tx = tab;
@@ -242,6 +246,42 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restri
   }
 }
 
+template <int FORMAT, int SRC>
+__global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restrict__ frames, int h, int w, int mode,
+                                                         int new_h, int new_w, int top, int left,
+                                                         const int* __restrict__ tab, void* __restrict__ out,
+                                                         long long total) {
+  const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+  if (idx >= total) return;
+  const int xg = static_cast<int>(idx % (S / PIX));
+  long long t = idx / (S / PIX);
+  const int y = static_cast<int>(t % S);
+  const int n = static_cast<int>(t / S);
+  const FrameSrc<SRC> src{frames + n * FrameSrc<SRC>::frame_bytes(h, w), h, w};
+  preprocess_pixels<FORMAT>(src, mode, new_h, new_w, top, left, tab, out, n, y, xg);
+}
+
+// The per-pixel path over a frame table: the frames of the table's per-pixel list (frame_table.cuh), any size, pitch and
+// kind.  The grid is sized from the table's capacity and walks the list with a grid-stride loop; the list's length is read
+// on the device, so a captured launch stays valid when the table is set to other frames.
+template <int FORMAT>
+__global__ void __launch_bounds__(256) preprocess_table_kernel(const int* __restrict__ counts, const int* __restrict__ list,
+                                                               const FrameRec* __restrict__ recs, void* __restrict__ out) {
+  const long long total = static_cast<long long>(counts[2]) * S * (S / PIX);
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int xg = static_cast<int>(idx % (S / PIX));
+    const long long t = idx / (S / PIX);
+    const int y = static_cast<int>(t % S);
+    const int n = list[t / S];
+    const FrameRec& r = recs[n];
+    if (r.kind == 0)
+      preprocess_pixels<FORMAT>(FrameSrc<2>{r.data, r.pitch}, r.mode, r.new_h, r.new_w, r.top, r.left, r.tab, out, n, y, xg);
+    else
+      preprocess_pixels<FORMAT>(FrameSrc<3>{r.data, r.chroma, r.pitch}, r.mode, r.new_h, r.new_w, r.top, r.left, r.tab, out, n, y, xg);
+  }
+}
+
 // Row-staged fast path for pure decimation (Geometry::decimate).  Persistent CTAs, each walking output-row PAIRS
 // (y, y + 1 with y even: the two rows of a space-to-depth block row); the touched source rows of a pair are brought into
 // a K1_STAGES-deep shared-memory ring by bulk copies (cp.async.bulk, completion counted on an mbarrier) issued by one
@@ -250,47 +290,98 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restri
 // Each thread then picks the bytes of its four pixels of both rows from shared memory and writes 64 contiguous bytes
 // (format 2: two whole 2x2 blocks) or 32 per row (format 1).  Rows of the letterbox border issue no loads.
 constexpr int K1_STAGES = 4;
-template <int FORMAT, int SRC>
+
+// The frame an output-row pair of the row-staged path belongs to, and where its source rows are.
+struct PairFrame {
+  const uint8_t* data;    // BGR rows / NV12 luma rows, `pitch` bytes apart
+  const uint8_t* chroma;  // NV12 chroma rows, `pitch` bytes apart
+  int pitch, w, nv12, new_h, new_w, top, left, n;
+  const int* tab;
+};
+
+// TABLE: the pairs are those of the frames on the table's row-staged list (frame_table.cuh), each with its own geometry, and
+// the count is read on the device; the frame arguments are then unused and a ring stage holds two rows of stage_row bytes.
+// Each CTA then walks one contiguous, even-aligned run of pairs, so that its frame - and the geometry it loads from the table,
+// three dependent loads - changes at most a few times per CTA instead of at every pair.
+template <int FORMAT, int SRC, bool TABLE = false>
 __global__ void __launch_bounds__(S / PIX) preprocess_pairs_kernel(const uint8_t* __restrict__ frames, int h, int w, int new_h,
                                                                    int new_w, int top, int left, const int* __restrict__ tab,
-                                                                   void* __restrict__ out, int n_pairs, int stages) {
+                                                                   void* __restrict__ out, int n_pairs, int stages,
+                                                                   const int* __restrict__ t_counts = nullptr,
+                                                                   const int* __restrict__ t_list = nullptr,
+                                                                   const FrameRec* __restrict__ t_recs = nullptr,
+                                                                   int stage_row = 0) {
   extern __shared__ __align__(128) uint8_t sm_rows[];
   __shared__ __align__(8) uint64_t full_bar[K1_STAGES];
-  const int row_bytes = SRC == 0 ? w * 3 : 2 * w;  // one staged source row: BGR, or the luma row followed by its chroma row
+  const int row_bytes = TABLE ? stage_row : (SRC == 0 ? w * 3 : 2 * w);  // one staged source row: BGR, or the luma row followed by its chroma row
   const int stage_bytes = 2 * row_bytes;
+  if (TABLE) n_pairs = t_counts[1] * (S / 2);
   const int tid = threadIdx.x;
   if (tid == 0) {
     for (int k = 0; k < stages; ++k) ptx::mbar_init(smem_u32(&full_bar[k]), 1);
     ptx::mbar_init_fence();
   }
   __syncthreads();
-  const int* ty = tab + 4 * new_w;
+  auto frame_of = [&](int pair) -> PairFrame {
+    PairFrame g;
+    if (TABLE) {
+      g.n = t_list[pair / (S / 2)];
+      const FrameRec& r = t_recs[g.n];
+      g.data = r.data; g.chroma = r.chroma; g.pitch = r.pitch; g.w = r.w; g.nv12 = r.kind;
+      g.new_h = r.new_h; g.new_w = r.new_w; g.top = r.top; g.left = r.left; g.tab = r.tab;
+    } else {
+      g.n = pair / (S / 2);
+      g.data = frames + g.n * FrameSrc<SRC>::frame_bytes(h, w);
+      g.chroma = g.data + static_cast<long long>(h) * w;
+      g.pitch = SRC == 0 ? 3 * w : w; g.w = w; g.nv12 = SRC;
+      g.new_h = new_h; g.new_w = new_w; g.top = top; g.left = left; g.tab = tab;
+    }
+    return g;
+  };
+  // Over a table the geometry of a pair's frame is reloaded only when the frame changes (list position k); on the uniform
+  // path it is arithmetic.  One copy for thread 0's refills (which run ahead), one for the pair being computed.
+  PairFrame ig, g;
+  int ik = -1, gk = -1;
   auto issue = [&](int pair, int stage) {  // thread 0: the source rows of one output-row pair -> ring stage
-    const int n = pair / (S / 2), y0 = (pair - n * (S / 2)) * 2;
+    if (!TABLE || pair / (S / 2) != ik) {
+      ik = pair / (S / 2);
+      ig = frame_of(pair);
+    }
+    const int y0 = (pair - (pair / (S / 2)) * (S / 2)) * 2;
+    const int* ty = ig.tab + 4 * ig.new_w;
     const uint32_t bar = smem_u32(&full_bar[stage]);
+    const int fetch = ig.nv12 ? 2 * ig.w : 3 * ig.w;
     int sy[2];
     uint32_t bytes = 0;
+#pragma unroll
     for (int r = 0; r < 2; ++r) {
-      const int dy = y0 + r - top;
-      sy[r] = (dy >= 0 && dy < new_h) ? __ldg(ty + dy) : -1;
-      if (sy[r] >= 0) bytes += row_bytes;
+      const int dy = y0 + r - ig.top;
+      sy[r] = (dy >= 0 && dy < ig.new_h) ? __ldg(ty + dy) : -1;
+      if (sy[r] >= 0) bytes += fetch;
     }
     ptx::mbar_arrive_expect_tx(bar, bytes);  // (a border pair completes the phase with no bytes)
+#pragma unroll
     for (int r = 0; r < 2; ++r) {
       if (sy[r] < 0) continue;
       const uint32_t dst = smem_u32(sm_rows + static_cast<size_t>(stage) * stage_bytes + r * row_bytes);
-      if (SRC == 0) {
-        ptx::bulk_g2s(dst, frames + (static_cast<long long>(n) * h + sy[r]) * w * 3, row_bytes, bar);
+      if (!ig.nv12) {
+        ptx::bulk_g2s(dst, ig.data + static_cast<long long>(sy[r]) * ig.pitch, fetch, bar);
       } else {
-        const uint8_t* fr = frames + n * FrameSrc<1>::frame_bytes(h, w);
-        ptx::bulk_g2s(dst, fr + static_cast<long long>(sy[r]) * w, w, bar);
-        ptx::bulk_g2s(dst + w, fr + static_cast<long long>(h) * w + static_cast<long long>(sy[r] >> 1) * w, w, bar);
+        ptx::bulk_g2s(dst, ig.data + static_cast<long long>(sy[r]) * ig.pitch, ig.w, bar);
+        ptx::bulk_g2s(dst + ig.w, ig.chroma + static_cast<long long>(sy[r] >> 1) * ig.pitch, ig.w, bar);
       }
     }
   };
   // k-th item of this CTA: output-row pairs are handed out two at a time (n_pairs is even), so the four rows of a 4x4 pixel block
   // (format 3: the two 64-byte halves of a 128-byte block) are written by the same threads in consecutive iterations
+  long long run_begin = 0, run_end = 0;  // TABLE: this CTA's pairs (run lengths even: pair parity = item parity)
+  if (TABLE) {
+    const int run = (n_pairs + 2 * static_cast<int>(gridDim.x) - 1) / (2 * static_cast<int>(gridDim.x)) * 2;
+    run_begin = static_cast<long long>(blockIdx.x) * run;
+    run_end = min(static_cast<long long>(n_pairs), run_begin + run);
+  }
   auto pair_of = [&](int k) -> long long {
+    if (TABLE) return run_begin + k < run_end ? run_begin + k : n_pairs;
     return 2 * (blockIdx.x + static_cast<long long>(k >> 1) * gridDim.x) + (k & 1);
   };
   if (tid == 0)
@@ -298,39 +389,52 @@ __global__ void __launch_bounds__(S / PIX) preprocess_pairs_kernel(const uint8_t
       const long long pair = pair_of(k);
       if (pair < n_pairs) issue(static_cast<int>(pair), k);
     }
-  // the four source columns of this thread never change
+  // the four source columns of this thread (for one geometry: fixed on the uniform path, per frame over a table)
   const int xg = tid;
   int sx[PIX];
+  if (!TABLE) {
 #pragma unroll
-  for (int p = 0; p < PIX; ++p) {
-    const int dx = xg * PIX + p - left;
-    sx[p] = (dx >= 0 && dx < new_w) ? __ldg(tab + dx) : -1;
+    for (int p = 0; p < PIX; ++p) {
+      const int dx = xg * PIX + p - left;
+      sx[p] = (dx >= 0 && dx < new_w) ? __ldg(tab + dx) : -1;
+    }
   }
   for (int it = 0;; ++it) {
     const long long pair_l = pair_of(it);
     if (pair_l >= n_pairs) break;
     const int pair = static_cast<int>(pair_l);
     const int stage = it % stages;
-    const int n = pair / (S / 2), y0 = (pair - n * (S / 2)) * 2;
+    if (!TABLE || pair / (S / 2) != gk) {
+      gk = pair / (S / 2);
+      g = frame_of(pair);
+      if (TABLE) {
+#pragma unroll
+        for (int p = 0; p < PIX; ++p) {
+          const int dx = xg * PIX + p - g.left;
+          sx[p] = (dx >= 0 && dx < g.new_w) ? __ldg(g.tab + dx) : -1;
+        }
+      }
+    }
+    const int n = g.n, y0 = (pair - (pair / (S / 2)) * (S / 2)) * 2;
     ptx::mbar_wait(smem_u32(&full_bar[stage]), (it / stages) & 1);
     uint4 q[2][2];
     float pl[2][PIX][3];
 #pragma unroll
     for (int r = 0; r < 2; ++r) {
-      const int dy = y0 + r - top;
-      const bool row_in = dy >= 0 && dy < new_h;
+      const int dy = y0 + r - g.top;
+      const bool row_in = dy >= 0 && dy < g.new_h;
       const uint8_t* srow = sm_rows + static_cast<size_t>(stage) * stage_bytes + r * row_bytes;
       float rgb[PIX][3];
 #pragma unroll
       for (int p = 0; p < PIX; ++p) {
         int v0 = 114, v1 = 114, v2 = 114;  // BGR pad colour (image_processing.py:10)
         if (row_in && sx[p] >= 0) {
-          if (SRC == 0) {
+          if (!g.nv12) {
             const uint8_t* sp = srow + sx[p] * 3;
             v0 = sp[0]; v1 = sp[1]; v2 = sp[2];
           } else {
             int bgr[3];
-            yuv_to_bgr_601(srow[sx[p]], srow[w + (sx[p] & ~1)], srow[w + (sx[p] & ~1) + 1], bgr);
+            yuv_to_bgr_601(srow[sx[p]], srow[g.w + (sx[p] & ~1)], srow[g.w + (sx[p] & ~1) + 1], bgr);
             v0 = bgr[0]; v1 = bgr[1]; v2 = bgr[2];
           }
         }
@@ -435,6 +539,41 @@ int aicam_preprocess_nv12(const uint8_t* frames_nv12, int batch, int h, int w, i
   return preprocess_impl<1>(frames_nv12, batch, h, w, format, out, stream);
 }
 
+int aicam_preprocess_table(const aicam_frame_table* t, int format, void* out, void* stream) {
+  if (!t || !out) return fail(AICAM_ERR_INVALID_ARG, "preprocess_table: null argument");
+  if (format < 0 || format > 3) return fail(AICAM_ERR_INVALID_ARG, "preprocess_table: format must be 0, 1, 2 or 3");
+  const int n = t->n;
+  if (n == 0) return AICAM_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // Row-staged path: the ring is sized from the table's width bound, the grid from n; the kernel reads how many frames take it.
+  const size_t stage_bytes = 2 * static_cast<size_t>(t->stage_row());
+  if (t->ring_fits()) {  // (the condition under which aicam_frame_table_set puts frames on this path)
+    int stages = K1_STAGES * stage_bytes <= K1_SMEM_LIMIT / 2 ? K1_STAGES : 2;
+    if (format == 3) stages = 2;  // as aicam_preprocess
+    const size_t smem = stages * stage_bytes + (format == 3 ? K1_BLOCK_ROW_IMAGE : 0);
+    auto kernel = format == 0 ? preprocess_pairs_kernel<0, 0, true>
+                              : (format == 1 ? preprocess_pairs_kernel<1, 0, true>
+                                             : (format == 2 ? preprocess_pairs_kernel<2, 0, true> : preprocess_pairs_kernel<3, 0, true>));
+    if (smem > 48 * 1024) {
+      if (int rc = ensure_dynamic_smem(kernel, K1_SMEM_LIMIT)) return rc;
+    }
+    const int per_sm = static_cast<int>(std::max<size_t>(1, std::min<size_t>(8, K1_SMEM_LIMIT / (smem + 1024))));
+    const unsigned grid = static_cast<unsigned>(std::min<long long>(static_cast<long long>(n) * (S / 4), static_cast<long long>(current_num_sms()) * per_sm));
+    kernel<<<grid, S / PIX, smem, st>>>(nullptr, 0, 0, 0, 0, 0, 0, nullptr, out, 0, stages, t->counts(), t->lists(), t->recs(),
+                                        t->stage_row());
+    count_launch();
+    if (int rc = last_launch("preprocess_pairs_kernel (table)")) return rc;
+  }
+  // Per-pixel path for every other frame.
+  auto kernel = format == 0 ? preprocess_table_kernel<0>
+                            : (format == 1 ? preprocess_table_kernel<1> : (format == 2 ? preprocess_table_kernel<2> : preprocess_table_kernel<3>));
+  const long long total = static_cast<long long>(n) * S * (S / PIX);
+  const unsigned blocks = static_cast<unsigned>(std::min<long long>((total + 255) / 256, static_cast<long long>(current_num_sms()) * 8));
+  kernel<<<blocks, 256, 0, st>>>(t->counts(), t->lists() + t->capacity, t->recs(), out);
+  count_launch();
+  return last_launch("preprocess_table_kernel");
+}
+
 }  // extern "C"
 
 namespace aicam {
@@ -469,7 +608,8 @@ int preprocess_impl(const uint8_t* frames, int batch, int h, int w, int format, 
     int per_sm = static_cast<int>(std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024))));
     if (env_ctas > 0) per_sm = std::min(per_sm, env_ctas);
     const unsigned grid = static_cast<unsigned>(std::min<long long>(n_pairs / 2, static_cast<long long>(current_num_sms()) * per_sm));
-    kernel<<<grid, S / PIX, smem, st>>>(frames, h, w, g.new_h, g.new_w, g.top, g.left, g.tab, out, n_pairs, stages);
+    kernel<<<grid, S / PIX, smem, st>>>(frames, h, w, g.new_h, g.new_w, g.top, g.left, g.tab, out, n_pairs, stages, nullptr, nullptr,
+                                        nullptr, 0);
     count_launch();
     return last_launch("preprocess_pairs_kernel");
   }

@@ -15,6 +15,7 @@
 // HBM-bound: reads ~crop bytes, writes 128*64*8 B (NHWC4 bf16) or 128*64*16 B (NHWC8, what the fused ReID stem reads) per crop.
 #include "common.cuh"
 #include "frame_src.cuh"
+#include "frame_table.cuh"
 
 namespace aicam {
 
@@ -32,7 +33,8 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
                                                       unsigned long long mask_lo, unsigned long long mask_hi,
                                                       int max_crops, int* __restrict__ det_index,
                                                       int* __restrict__ det_count, int* __restrict__ crop_slot,
-                                                      int* __restrict__ crop_rect, int* __restrict__ crop_count) {
+                                                      int* __restrict__ crop_rect, int* __restrict__ crop_count,
+                                                      const FrameRec* __restrict__ recs) {  // frame table: per-frame (w, h); or null
   __shared__ int s_scan[32];  // valid crops per frame of the current group of 32 frames, then their exclusive scan
   __shared__ int s_base;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -41,6 +43,7 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
   __syncthreads();
   for (int b0 = 0; b0 < batch; b0 += 32) {
     const int b = b0 + warp;
+    const int fw = recs && b < batch ? recs[b].w : w, fh = recs && b < batch ? recs[b].h : h;
     int nvalid = 0, nkeep = 0;
     if (b < batch) {
       const int n = min(num_dets[b], stride_k);
@@ -55,7 +58,7 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
           if (keep) {
             const float4 bx = reinterpret_cast<const float4*>(boxes)[fo + i];
             const int x1 = max(0, static_cast<int>(bx.x)), y1 = max(0, static_cast<int>(bx.y));
-            const int x2 = min(w, static_cast<int>(bx.z)), y2 = min(h, static_cast<int>(bx.w));
+            const int x2 = min(fw, static_cast<int>(bx.z)), y2 = min(fh, static_cast<int>(bx.w));
             ok = x1 < x2 && y1 < y2;
           }
         }
@@ -98,8 +101,8 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
           crop_rect[slot * 5 + 0] = b;
           crop_rect[slot * 5 + 1] = max(0, static_cast<int>(bx.x));
           crop_rect[slot * 5 + 2] = max(0, static_cast<int>(bx.y));
-          crop_rect[slot * 5 + 3] = min(w, static_cast<int>(bx.z));
-          crop_rect[slot * 5 + 4] = min(h, static_cast<int>(bx.w));
+          crop_rect[slot * 5 + 3] = min(fw, static_cast<int>(bx.z));
+          crop_rect[slot * 5 + 4] = min(fh, static_cast<int>(bx.w));
         } else {
           crop_slot[fo + k] = -1;
         }
@@ -204,20 +207,27 @@ constexpr int CROP_STAGE_W = 168;
 constexpr int CROP_SEG = CROP_STAGE_W * 3 + 16;  // bytes of one staged segment (BGR row; NV12: luma + chroma halves)
 constexpr int CROP_WARPS = 8;
 
+// Row addresses of the frame sources (frame_src.cuh) for the staged path: BGR / luma row y, and the chroma row of row y.
+__device__ __forceinline__ const uint8_t* src_row(const FrameSrc<0>& s, int y) { return s.f + static_cast<long long>(y) * s.w * 3; }
+__device__ __forceinline__ const uint8_t* src_row(const FrameSrc<1>& s, int y) { return s.f + static_cast<long long>(y) * s.w; }
+__device__ __forceinline__ const uint8_t* src_row(const FrameSrc<2>& s, int y) { return s.f + static_cast<long long>(y) * s.pitch; }
+__device__ __forceinline__ const uint8_t* src_row(const FrameSrc<3>& s, int y) { return s.f + static_cast<long long>(y) * s.pitch; }
+__device__ __forceinline__ const uint8_t* src_crow(const FrameSrc<0>& s, int y) { return nullptr; }
+__device__ __forceinline__ const uint8_t* src_crow(const FrameSrc<1>& s, int y) {
+  return s.f + static_cast<long long>(s.h) * s.w + static_cast<long long>(y >> 1) * s.w;
+}
+__device__ __forceinline__ const uint8_t* src_crow(const FrameSrc<2>& s, int y) { return nullptr; }
+__device__ __forceinline__ const uint8_t* src_crow(const FrameSrc<3>& s, int y) { return s.c + static_cast<long long>(y >> 1) * s.pitch; }
+
 // (Staging: the aligned 32-bit words that cover a byte segment [p, p + n) are loaded with coalesced __ldg, WPP words per lane, and
-//  written to 4-byte aligned shared memory; shift = p & 3 is where the segment starts there.  The frame batch is a multiple of
-//  4 bytes long and 4-byte aligned (checked by the caller), so no word crosses its end.)
+//  written to 4-byte aligned shared memory; shift = p & 3 is where the segment starts there.  The caller passes frame_words only
+//  when no such word crosses the end of the frame's planes.)
+// One crop (slot) of the rectangle (x1, y1, cw, ch) of `src`; tx / ty / seg: the CTA's shared memory.
 template <int FORMAT, int SRC>
-__global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __restrict__ frames, int batch, int h, int w,
-                                                               const int* __restrict__ crop_rect,
-                                                               const int* __restrict__ crop_count, void* __restrict__ out) {
-  const int slot = blockIdx.x;
-  if (slot >= *crop_count) return;
-  __shared__ int tx[4][RW];
-  __shared__ int ty[4][RH];
-  __shared__ __align__(16) uint8_t seg[CROP_WARPS][2][CROP_SEG];
-  const int b = crop_rect[slot * 5], x1 = crop_rect[slot * 5 + 1], y1 = crop_rect[slot * 5 + 2];
-  const int cw = crop_rect[slot * 5 + 3] - x1, ch = crop_rect[slot * 5 + 4] - y1;
+__device__ __forceinline__ void crop_body(const FrameSrc<SRC>& src, bool frame_words, int x1, int y1, int cw, int ch,
+                                          int (&tx)[4][RW], int (&ty)[4][RH], uint8_t (&seg)[CROP_WARPS][2][CROP_SEG],
+                                          void* __restrict__ out, int slot) {
+  constexpr bool NV = (SRC & 1) != 0;
   const int mode = (cw == RW && ch == RH) ? 2 : ((cw == 2 * RW && ch == 2 * RH) ? 1 : 0);
   {
     const int t = threadIdx.x;
@@ -231,9 +241,7 @@ __global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __
     }
   }
   __syncthreads();
-  const FrameSrc<SRC> src{frames + b * FrameSrc<SRC>::frame_bytes(h, w), h, w};
-  const bool staged = cw <= CROP_STAGE_W && (reinterpret_cast<uintptr_t>(frames) & 3) == 0 &&
-                      ((static_cast<long long>(batch) * FrameSrc<SRC>::frame_bytes(h, w)) & 3) == 0;
+  const bool staged = cw <= CROP_STAGE_W && frame_words;
   if (!staged) {
     for (int p = threadIdx.x; p < RH * RW; p += blockDim.x) {
       const int oy = p / RW, ox = p - oy * RW;
@@ -254,7 +262,7 @@ __global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __
   // have been written to shared memory, so their memory round trip overlaps the interpolation of row i (a row used to cost one
   // exposed round trip, 16 of them in series per warp).  Measured per 1 024 crops, filter + crops: 95 -> 71 us (NV12 114 -> 95);
   // two rows ahead measured no better (73 us).  One pass per row: staged segments are at most 128 (BGR) / 64 (NV12) words.
-  constexpr int NSEG = SRC == 0 ? 2 : 4, WPP = SRC == 0 ? 4 : 2;
+  constexpr int NSEG = NV ? 4 : 2, WPP = NV ? 2 : 4;
   struct RowFetch {
     uint32_t v[NSEG][WPP];
     int nwords[NSEG], shift[NSEG];
@@ -266,14 +274,13 @@ __global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __
     const bool need[2] = {mode != 0 || b0 != 0, mode == 1 || (mode == 0 && b1 != 0)};
     const uint8_t* ps[NSEG];
     int ns[NSEG];
-    if (SRC == 0) {
-      ps[0] = src.f + (static_cast<long long>(sy[0]) * w + x1) * 3; ps[1] = src.f + (static_cast<long long>(sy[1]) * w + x1) * 3;
+    if (!NV) {
+      ps[0] = src_row(src, sy[0]) + x1 * 3; ps[1] = src_row(src, sy[1]) + x1 * 3;
       ns[0] = need[0] ? cw * 3 : 0; ns[1] = need[1] ? cw * 3 : 0;
     } else {  // luma segments, then the chroma pairs of columns x1 & ~1 .. (even start: U first)
-      const uint8_t* chroma = src.f + static_cast<long long>(h) * w + (x1 & ~1);
       const int cn = ((x1 + cw + 1) & ~1) - (x1 & ~1);
-      ps[0] = src.f + static_cast<long long>(sy[0]) * w + x1; ps[1] = src.f + static_cast<long long>(sy[1]) * w + x1;
-      ps[NSEG - 2] = chroma + static_cast<long long>(sy[0] >> 1) * w; ps[NSEG - 1] = chroma + static_cast<long long>(sy[1] >> 1) * w;
+      ps[0] = src_row(src, sy[0]) + x1; ps[1] = src_row(src, sy[1]) + x1;
+      ps[NSEG - 2] = src_crow(src, sy[0]) + (x1 & ~1); ps[NSEG - 1] = src_crow(src, sy[1]) + (x1 & ~1);
       ns[0] = need[0] ? cw : 0; ns[1] = need[1] ? cw : 0; ns[NSEG - 2] = need[0] ? cn : 0; ns[NSEG - 1] = need[1] ? cn : 0;
     }
 #pragma unroll
@@ -293,7 +300,7 @@ __global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __
   for (int oy = warp; oy < RH; oy += CROP_WARPS) {
     const int b0 = ty[2][oy], b1 = ty[3][oy];
     int shift[2] = {cur.shift[0], cur.shift[1]}, cshift[2] = {0, 0};
-    if (SRC != 0) { cshift[0] = cur.shift[NSEG - 2]; cshift[1] = cur.shift[NSEG - 1]; }
+    if (NV) { cshift[0] = cur.shift[NSEG - 2]; cshift[1] = cur.shift[NSEG - 1]; }
     __syncwarp();  // the previous row's taps have been read
     {
       uint8_t* const ds[4] = {seg[warp][0], seg[warp][1], seg[warp][0] + CROP_SEG / 2, seg[warp][1] + CROP_SEG / 2};
@@ -313,7 +320,7 @@ __global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __
       const int sx[2] = {lsx[k][0], lsx[k][1]};
       crop_pixel<FORMAT>(mode, la[k][0], la[k][1], b0, b1,
                          [&](int r, int i, int (&v)[3]) {
-                           if (SRC == 0) {
+                           if (!NV) {
                              const uint8_t* q = seg[warp][r] + shift[r] + sx[i] * 3;
                              v[0] = q[0]; v[1] = q[1]; v[2] = q[2];
                            } else {
@@ -324,6 +331,43 @@ __global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __
                          out, slot, oy * RW + ox);
     }
   }
+}
+
+
+template <int FORMAT, int SRC>
+__global__ void __launch_bounds__(32 * CROP_WARPS) crop_kernel(const uint8_t* __restrict__ frames, int batch, int h, int w,
+                                                               const int* __restrict__ crop_rect,
+                                                               const int* __restrict__ crop_count, void* __restrict__ out) {
+  const int slot = blockIdx.x;
+  if (slot >= *crop_count) return;
+  __shared__ int tx[4][RW];
+  __shared__ int ty[4][RH];
+  __shared__ __align__(16) uint8_t seg[CROP_WARPS][2][CROP_SEG];
+  const int b = crop_rect[slot * 5], x1 = crop_rect[slot * 5 + 1], y1 = crop_rect[slot * 5 + 2];
+  const int cw = crop_rect[slot * 5 + 3] - x1, ch = crop_rect[slot * 5 + 4] - y1;
+  // the frame batch is a multiple of 4 bytes long and 4-byte aligned: no word crosses its end
+  const bool words = (reinterpret_cast<uintptr_t>(frames) & 3) == 0 && ((static_cast<long long>(batch) * FrameSrc<SRC>::frame_bytes(h, w)) & 3) == 0;
+  crop_body<FORMAT>(FrameSrc<SRC>{frames + b * FrameSrc<SRC>::frame_bytes(h, w), h, w}, words, x1, y1, cw, ch, tx, ty, seg, out, slot);
+}
+
+// The crops over a frame table: each crop reads its frame's record (any size, pitch, BGR or NV12).  Whole words are loaded
+// only from frames whose planes allow it (FrameRec::crop_staged); a crop at the last row of a separately allocated frame
+// would otherwise read past the allocation.
+template <int FORMAT>
+__global__ void __launch_bounds__(32 * CROP_WARPS) crop_table_kernel(const FrameRec* __restrict__ recs, const int* __restrict__ crop_rect,
+                                                                     const int* __restrict__ crop_count, void* __restrict__ out) {
+  const int slot = blockIdx.x;
+  if (slot >= *crop_count) return;
+  __shared__ int tx[4][RW];
+  __shared__ int ty[4][RH];
+  __shared__ __align__(16) uint8_t seg[CROP_WARPS][2][CROP_SEG];
+  const int b = crop_rect[slot * 5], x1 = crop_rect[slot * 5 + 1], y1 = crop_rect[slot * 5 + 2];
+  const int cw = crop_rect[slot * 5 + 3] - x1, ch = crop_rect[slot * 5 + 4] - y1;
+  const FrameRec& r = recs[b];
+  if (r.kind == 0)
+    crop_body<FORMAT>(FrameSrc<2>{r.data, r.pitch}, r.crop_staged != 0, x1, y1, cw, ch, tx, ty, seg, out, slot);
+  else
+    crop_body<FORMAT>(FrameSrc<3>{r.data, r.chroma, r.pitch}, r.crop_staged != 0, x1, y1, cw, ch, tx, ty, seg, out, slot);
 }
 
 }  // namespace
@@ -347,7 +391,7 @@ int reid_crops_impl(const uint8_t* frames, int batch, int h, int w, const float*
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   filter_kernel<<<1, 1024, 0, st>>>(boxes, scores, labels, num_dets, batch, stride_k, h, w, min_confidence,
                                     class_mask_lo, class_mask_hi, max_crops, det_index, det_count, crop_slot, crop_rect,
-                                    crop_count);
+                                    crop_count, nullptr);
   count_launch();
   if (int rc = last_launch("filter_kernel")) return rc;
   if (max_crops == 0 || !frames || !crops) return AICAM_OK;  // filter only
@@ -380,6 +424,31 @@ extern "C" int aicam_reid_crops_nv12(const uint8_t* frames_nv12, int batch, int 
   if (h % 2 || w % 2) return fail(AICAM_ERR_INVALID_ARG, "reid_crops_nv12: NV12 frames have even height and width");
   return reid_crops_impl<1>(frames_nv12, batch, h, w, boxes, scores, labels, num_dets, stride_k, min_confidence, class_mask_lo,
                             class_mask_hi, format, max_crops, det_index, det_count, crop_slot, crop_rect, crops, crop_count, stream);
+}
+
+extern "C" int aicam_reid_crops_table(const aicam_frame_table* t, const float* boxes, const float* scores, const int32_t* labels,
+                                      const int32_t* num_dets, int stride_k, float min_confidence, uint64_t class_mask_lo,
+                                      uint64_t class_mask_hi, int format, int max_crops, int32_t* det_index, int32_t* det_count,
+                                      int32_t* crop_slot, int32_t* crop_rect, void* crops, int32_t* crop_count, void* stream) {
+  if (!t || !boxes || !scores || !labels || !num_dets || !det_index || !det_count || !crop_slot || !crop_rect || !crop_count)
+    return fail(AICAM_ERR_INVALID_ARG, "reid_crops_table: null argument");
+  if (stride_k <= 0 || max_crops < 0 || (format < 0 || format > 2))
+    return fail(AICAM_ERR_INVALID_ARG, "reid_crops_table: bad shape arguments");
+  if (reinterpret_cast<uintptr_t>(boxes) % 16) return fail(AICAM_ERR_INVALID_ARG, "reid_crops_table: boxes must be 16-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  filter_kernel<<<1, 1024, 0, st>>>(boxes, scores, labels, num_dets, t->n, stride_k, 0, 0, min_confidence, class_mask_lo,
+                                    class_mask_hi, max_crops, det_index, det_count, crop_slot, crop_rect, crop_count, t->recs());
+  count_launch();
+  if (int rc = last_launch("filter_kernel (table)")) return rc;
+  if (max_crops == 0 || !crops) return AICAM_OK;  // filter only
+  if (format == 0)
+    crop_table_kernel<0><<<max_crops, 32 * CROP_WARPS, 0, st>>>(t->recs(), crop_rect, crop_count, crops);
+  else if (format == 1)
+    crop_table_kernel<1><<<max_crops, 32 * CROP_WARPS, 0, st>>>(t->recs(), crop_rect, crop_count, crops);
+  else
+    crop_table_kernel<2><<<max_crops, 32 * CROP_WARPS, 0, st>>>(t->recs(), crop_rect, crop_count, crops);
+  count_launch();
+  return last_launch("crop_table_kernel");
 }
 
 // NV12 -> packed BGR (cv2.cvtColor(.., COLOR_YUV2BGR_NV12)): the frames the NV12 entry points see, as the reference's

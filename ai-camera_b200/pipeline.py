@@ -8,7 +8,7 @@ buffers.  ``YOLODetector`` / ``DeepSORT`` (the reference-shaped facades) are thi
 wrappers around ``BatchDetector`` / ``BatchTracker``.
 """
 import ctypes as C
-from typing import Optional, Tuple
+from typing import Optional, Sequence, Tuple, Union
 
 import torch
 
@@ -27,12 +27,76 @@ def frame_geometry(frames: torch.Tensor):
     raise _lib.AicamError(-1, "frames must be [n, H, W, 3] (BGR) or [n, H*3/2, W] (NV12)")
 
 
+def is_frame_list(frames) -> bool:
+    return isinstance(frames, (list, tuple))
+
+
+class FrameTable:
+    """Owner of an ``aicam_frame_table``: per-stream frames of any size, row pitch and surface format for one batched
+    step.  ``set(frames)`` takes a list of uint8 CUDA tensors, each ``[H, W, 3]`` BGR or ``[H*3/2, W]`` NV12, whose rows
+    are contiguous (a view into a larger surface is fine: its row stride is the pitch).  The library may read every
+    plane as rows * pitch bytes, so a view's last row must be followed by the rest of its pitch inside the same storage."""
+
+    def __init__(self, device, capacity: int, max_frame_hw=(2160, 3840)):
+        self.lib = _lib.load()
+        self.device = torch.device(device)
+        self.capacity, self.max_frame_hw = int(capacity), tuple(max_frame_hw)
+        self._h = C.c_void_p()
+        _lib.check(self.lib.aicam_frame_table_create(self.device.index or 0, self.capacity, self.max_frame_hw[0],
+                                                     self.max_frame_hw[1], C.byref(self._h)))
+        self._descs = (_lib.FrameDesc * self.capacity)()
+        self.n = 0
+        self.frames = []
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h:
+            self.lib.aicam_frame_table_destroy(h)
+            self._h = None
+
+    @staticmethod
+    def describe(frame: torch.Tensor):
+        """(h, w, pitch, kind) of one frame; kind 0 BGR, 1 NV12."""
+        if frame.dtype != torch.uint8 or not frame.is_cuda:
+            raise _lib.AicamError(-1, "frames must be uint8 CUDA tensors")
+        if frame.dim() == 3 and frame.shape[2] == 3 and frame.stride(2) == 1 and frame.stride(1) == 3:
+            return frame.shape[0], frame.shape[1], frame.stride(0), 0
+        if frame.dim() == 2 and frame.shape[0] % 3 == 0 and frame.stride(1) == 1:
+            return frame.shape[0] * 2 // 3, frame.shape[1], frame.stride(0), 1
+        raise _lib.AicamError(-1, "each frame must be [H, W, 3] (BGR) or [H*3/2, W] (NV12) with contiguous rows")
+
+    def set(self, frames: Sequence[torch.Tensor]):
+        n = len(frames)
+        if n > self.capacity:
+            raise _lib.AicamError(-4, "%d frames exceed the frame table's capacity %d" % (n, self.capacity))
+        for i, f in enumerate(frames):
+            if f.device != self.device:
+                raise _lib.AicamError(-1, "frame %d is not on %s" % (i, self.device))
+            h, w, pitch, kind = self.describe(f)
+            if f.storage_offset() + f.shape[0] * pitch > f.untyped_storage().nbytes():
+                raise _lib.AicamError(-1, "frame %d: its %d rows of %d bytes (the pitch) run past the end of its storage"
+                                      % (i, f.shape[0], pitch))
+            d = self._descs[i]
+            d.data, d.h, d.w, d.pitch, d.kind = f.data_ptr(), h, w, pitch, kind
+            d.chroma = f.data_ptr() + h * pitch if kind == 1 else None
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_frame_table_set(self._h, self._descs, n, _lib.stream_ptr(self.device)))
+        self.n = n
+        self.frames = list(frames)  # kept alive while work that reads the table may be in flight
+
+    @property
+    def handle(self):
+        return self._h
+
+
 class BatchDetector:
     """K1-K4 + detect() post-processing for ``batch`` frames of one size."""
 
     def __init__(self, engine_path, batch: int, device=None, conf_threshold=config.YOLO_CONF_THRESHOLD,
                  nms_threshold=config.YOLO_NMS_THRESHOLD, topk=config.YOLO_TOPK,
-                 max_candidates=config.YOLO_MAX_CANDIDATES):
+                 max_candidates=config.YOLO_MAX_CANDIDATES, max_frame_hw=(2160, 3840)):
+        self.max_frame_hw = tuple(max_frame_hw)
+        self.frame_table = None  # created on the first list of frames
         self.engine = TRTEngine(engine_path, device, max_batch=batch, topk=topk,
                                 score_threshold=min(conf_threshold, config.YOLO_CONF_THRESHOLD),
                                 nms_threshold=nms_threshold, max_candidates=max_candidates)
@@ -52,11 +116,17 @@ class BatchDetector:
         # 0: NHWC4 input (aicam_preprocess format 1), 1: 2x2 pixel blocks (format 2), 2: 4x4 pixel blocks (format 3, yolov8n)
         self._s2d = int(self.lib.aicam_engine_accepts_s2d(e.handle))
 
-    def detect(self, frames: torch.Tensor):
+    def detect(self, frames):
         """frames: uint8 cuda [n<=batch, H, W, 3] BGR, or [n, H*3/2, W] NV12 (Y plane + interleaved UV plane, the
-        surface format of hardware decoders: half the bytes).  Returns device tensors (num_dets [n],
+        surface format of hardware decoders: half the bytes), or a list of n such frames ([H_s, W_s, 3] / [H_s*3/2, W_s])
+        of any sizes and kinds.  Returns device tensors (num_dets [n],
         boxes [n,topk,4] in frame pixels, scores [n,topk], labels [n,topk]); views of internal
         buffers, valid until the next call; asynchronous on the current stream."""
+        if is_frame_list(frames):
+            if self.frame_table is None:
+                self.frame_table = FrameTable(self.device, self.batch, self.max_frame_hw)
+            self.frame_table.set(frames)
+            return self.detect_table(self.frame_table)
         n, h, w, nv12 = frame_geometry(frames)
         pre = self.lib.aicam_preprocess_nv12 if nv12 else self.lib.aicam_preprocess
         if n > self.batch:
@@ -74,9 +144,26 @@ class BatchDetector:
                 _lib.ptr(e._ws), e._ws.numel(), st))
         return self.num_dets[:n], self.boxes[:n], self.scores[:n], self.labels[:n]
 
-    def launches_per_step(self):
-        # K1 + network + NMS (+ the decode kernel when the engine cannot decode inside its Detect-head epilogues)
-        return 1 + self.engine.launches_per_forward() + (1 if self.engine.fused_decode else 2)
+    def detect_table(self, table: FrameTable):
+        """detect() on the frames a FrameTable holds (each un-letterboxed with its own size); capturable."""
+        n = table.n
+        if n > self.batch:
+            raise _lib.AicamError(-4, "detect: %d frames exceed the detector's batch %d" % (n, self.batch))
+        e, st = self.engine, _lib.stream_ptr(self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_preprocess_table(table.handle, 1 + self._s2d, _lib.ptr(e._nhwc), st))
+            _lib.check(self.lib.aicam_yolo_detect_table(
+                e.handle, _lib.ptr(e._nhwc), self._s2d, table.handle, C.byref(self._nms),
+                _lib.ptr(e._head) if e._head is not None else None, _lib.ptr(self.num_dets),
+                _lib.ptr(self.boxes_lb), _lib.ptr(self.boxes), _lib.ptr(self.scores), _lib.ptr(self.labels),
+                _lib.ptr(e._ws), e._ws.numel(), st))
+        return self.num_dets[:n], self.boxes[:n], self.scores[:n], self.labels[:n]
+
+    def launches_per_step(self, frame_list=False):
+        # K1 + network + NMS (+ the decode kernel when the engine cannot decode inside its Detect-head epilogues); over a frame
+        # table K1 is two launches (row-staged and per-pixel), both made whatever the frame sizes
+        k1 = 2 if frame_list else 1
+        return k1 + self.engine.launches_per_forward() + (1 if self.engine.fused_decode else 2)
 
 
 class BatchTracker:
@@ -86,7 +173,10 @@ class BatchTracker:
                  max_tracks: int = 256, max_crops: Optional[int] = None,
                  max_cosine_distance=config.DEEPSORT_MAX_DIST, nn_budget=config.DEEPSORT_NN_BUDGET,
                  max_iou_distance=config.DEEPSORT_MAX_IOU_DISTANCE, max_age=config.DEEPSORT_MAX_AGE,
-                 n_init=config.DEEPSORT_N_INIT, min_detection_confidence=config.DEEPSORT_MIN_CONFIDENCE):
+                 n_init=config.DEEPSORT_N_INIT, min_detection_confidence=config.DEEPSORT_MIN_CONFIDENCE,
+                 max_frame_hw=(2160, 3840)):
+        self.max_frame_hw = tuple(max_frame_hw)
+        self.frame_table = None  # created on the first list of frames
         self.max_crops = int(max_crops if max_crops is not None else min(n_streams * max_dets, 4096))
         self.reid = TRTEngine(reid_engine_path, device, max_batch=self.max_crops)
         if self.reid.kind != _lib.KIND_REID:
@@ -135,9 +225,15 @@ class BatchTracker:
         self.crop_count.zero_()
 
     def update(self, frames, num_dets, boxes, scores, labels):
-        """One frame per stream.  frames uint8 cuda [S,H,W,3] BGR or [S,H*3/2,W] NV12; detections as BatchDetector
+        """One frame per stream.  frames uint8 cuda [S,H,W,3] BGR or [S,H*3/2,W] NV12, or a list of S frames of any
+        sizes and kinds (see BatchDetector.detect); detections as BatchDetector
         returns them ([S], [S,K,4], [S,K], [S,K]).  Returns device (out_tracks [S,T,6] int32 =
         x1,y1,x2,y2,id,class, out_conf [S,T], out_count [S]); asynchronous."""
+        if is_frame_list(frames):
+            if self.frame_table is None:
+                self.frame_table = FrameTable(self.device, self.S, self.max_frame_hw)
+            self.frame_table.set(frames)
+            return self.update_table(self.frame_table, num_dets, boxes, scores, labels)
         S, h, w, nv12 = frame_geometry(frames)
         crops_fn = self.lib.aicam_reid_crops_nv12 if nv12 else self.lib.aicam_reid_crops
         if S != self.S or boxes.shape[1] != self.K:
@@ -150,6 +246,23 @@ class BatchTracker:
                 _lib.ptr(self.det_index),
                 _lib.ptr(self.det_count), _lib.ptr(self.crop_slot), _lib.ptr(self.crop_rect), _lib.ptr(self.crops),
                 _lib.ptr(self.crop_count), st))
+        return self._reid_and_step(boxes, scores, labels)
+
+    def update_table(self, table: FrameTable, num_dets, boxes, scores, labels):
+        """update() on the frames a FrameTable holds (one per stream); capturable."""
+        if table.n != self.S or boxes.shape[1] != self.K:
+            raise _lib.AicamError(-4, "update: expected %d streams x %d detections" % (self.S, self.K))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_reid_crops_table(
+                table.handle, _lib.ptr(boxes), _lib.ptr(scores), _lib.ptr(labels), _lib.ptr(num_dets),
+                self.K, self.min_conf, self._mask[0], self._mask[1], 2 if self._nhwc8 else 1, self.max_crops,
+                _lib.ptr(self.det_index), _lib.ptr(self.det_count), _lib.ptr(self.crop_slot), _lib.ptr(self.crop_rect),
+                _lib.ptr(self.crops), _lib.ptr(self.crop_count), _lib.stream_ptr(self.device)))
+        return self._reid_and_step(boxes, scores, labels)
+
+    def _reid_and_step(self, boxes, scores, labels):
+        st = _lib.stream_ptr(self.device)
+        with torch.cuda.device(self.device):
             fwd = self.lib.aicam_reid_forward_nhwc8 if self._nhwc8 else self.lib.aicam_reid_forward
             _lib.check(fwd(self.reid.handle, _lib.ptr(self.crops), self.max_crops, _lib.ptr(self.crop_count),
                            _lib.ptr(self.feats), st))
@@ -185,13 +298,14 @@ class BatchTracker:
 
 
 class TrackingPipeline:
-    """detect + track for ``n_streams`` streams of one frame size; one call per time step."""
+    """detect + track for ``n_streams`` streams; one call per time step.  A step takes one stacked tensor of frames of
+    one size, or a list with one frame per stream of any sizes (up to ``max_frame_hw``), pitches and kinds (BGR / NV12)."""
 
     def __init__(self, yolo_engine_path, reid_engine_path, n_streams: int, device=None, max_tracks: int = 256,
                  max_crops: Optional[int] = None, conf_threshold=config.YOLO_CONF_THRESHOLD, topk=config.YOLO_TOPK,
-                 max_candidates=config.YOLO_MAX_CANDIDATES, **tracker_kw):
+                 max_candidates=config.YOLO_MAX_CANDIDATES, max_frame_hw=(2160, 3840), **tracker_kw):
         self.detector = BatchDetector(yolo_engine_path, n_streams, device, conf_threshold=conf_threshold, topk=topk,
-                                      max_candidates=max_candidates)
+                                      max_candidates=max_candidates, max_frame_hw=max_frame_hw)
         # detect() drops detections below conf_threshold before update() sees them (yolo_detector.py:131); on the
         # device that filter and DeepSORT's own (deepsort_tracker.py:88-95) are one comparison
         tracker_kw.setdefault("min_detection_confidence", max(config.DEEPSORT_MIN_CONFIDENCE, conf_threshold))
@@ -199,10 +313,22 @@ class TrackingPipeline:
                                     max_tracks=max_tracks, max_crops=max_crops, **tracker_kw)
         self.device = self.detector.device
         self.n_streams = n_streams
+        # the frames of a list step: set once, read by the detector and the tracker
+        self.frame_table = FrameTable(self.device, n_streams, max_frame_hw)
 
-    def step(self, frames: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    def step(self, frames: Union[torch.Tensor, Sequence[torch.Tensor]]) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        if is_frame_list(frames):
+            self.frame_table.set(frames)
+            return self.step_table()
         num, boxes, scores, labels = self.detector.detect(frames)
         return self.tracker.update(frames, num, boxes, scores, labels)
 
-    def launches_per_step(self):
-        return self.detector.launches_per_step() + self.tracker.launches_per_step()
+    def step_table(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """One step over the frames ``frame_table`` holds.  Launches depend only on the stream count and the size
+        bound, so a captured step_table() stays valid when ``frame_table.set`` changes the frames between replays."""
+        num, boxes, scores, labels = self.detector.detect_table(self.frame_table)
+        return self.tracker.update_table(self.frame_table, num, boxes, scores, labels)
+
+    def launches_per_step(self, frame_list=False):
+        """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True)."""
+        return self.detector.launches_per_step(frame_list) + self.tracker.launches_per_step()

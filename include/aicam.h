@@ -219,6 +219,42 @@ int aicam_nv12_to_bgr(const uint8_t* frames_nv12, int batch, int h, int w, uint8
                       void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Frame table: one descriptor per stream, so that one batched step can take frames of different sizes, row pitches and
+ * surface formats (a camera fleet mixes 4K, 1080p, 720p and 540p; decoders hand out one pitched surface per stream).
+ * The table entry points below (aicam_preprocess_table, aicam_yolo_detect_table, aicam_reid_crops_table) take the
+ * batch from the table; frame n of the batch is descriptor n of the last aicam_frame_table_set.
+ *   data   : BGR: h rows of 3w bytes, `pitch` bytes apart;  NV12: the luma plane, h rows of w bytes, `pitch` apart
+ *   chroma : NV12: the interleaved U, V plane, h/2 rows of w bytes, `pitch` apart (any allocation);  NULL for BGR
+ *   kind   : 0 BGR, 1 NV12 (one table may mix them)
+ * The caller guarantees that `data` spans h * pitch bytes and `chroma` (h/2) * pitch bytes, and that the frames stay
+ * valid while work that reads the table is in flight.
+ * aicam_frame_table_create: capacity = the most frames one set may hold; (max_h, max_w) = the largest frame size it may
+ *   hold.  The launch configuration of every table entry point depends only on the count of the last set and on this
+ *   bound, never on the frame sizes, and the kernels read everything else from the table on the device: a step
+ *   captured into a CUDA graph stays valid when aicam_frame_table_set changes pointers, pitches, kinds and sizes
+ *   (within the bound, same count) between replays.
+ * aicam_frame_table_set: validates every descriptor on the host and launches nothing on error: null plane pointer,
+ *   h or w <= 0, a kind other than 0 / 1, odd NV12 sizes, pitch < row bytes (AICAM_ERR_INVALID_ARG); n > capacity or a
+ *   frame beyond the bound (AICAM_ERR_CAPACITY).  It resolves each frame's letterbox geometry (the first sight of a
+ *   frame size allocates and uploads its coefficient table, as aicam_preprocess does), then copies the records to the
+ *   device with one asynchronous copy on `stream` from pinned staging (two buffers used alternately; a set waits for
+ *   the copy out of the buffer it reuses).  Not capturable; everything that reads the table is. */
+typedef struct aicam_frame_table aicam_frame_table;
+typedef struct {
+  const uint8_t* data;
+  const uint8_t* chroma;
+  int h, w, pitch;
+  int kind;
+} aicam_frame_desc;
+int aicam_frame_table_create(int device, int capacity, int max_h, int max_w, aicam_frame_table** out);
+void aicam_frame_table_destroy(aicam_frame_table* t);
+int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* host_descs, int n, void* stream);
+/* aicam_preprocess / aicam_preprocess_nv12 over a frame table (formats 0-3): frame n's slice of `out` equals the uniform
+ * entry on that frame alone.  Frames whose geometry is a pure decimation (1080p) and whose planes, pitch and row bytes
+ * are multiples of 16 take the row-staged path, all others the per-pixel path: at most one launch each. */
+int aicam_preprocess_table(const aicam_frame_table* t, int format, void* out, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Detection post-processing: the decode + NMS the reference's engine embeds (it returns
  * num_dets/bboxes/scores/labels, yolo_detector.py:49-54,108-112) and the part of
  * YOLODetector.detect after the engine (yolo_detector.py:107-149, scale_bboxes
@@ -259,6 +295,12 @@ int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch,
                       float* head, int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores,
                       int32_t* labels, void* workspace, size_t workspace_bytes, void* stream);
 int aicam_engine_fused_decode(const aicam_engine* e);
+/* aicam_yolo_detect over a frame table (in = aicam_preprocess_table output): the batch is the table's count, and
+ * boxes_orig un-letterboxes each frame with its own ratio, pad and size (p->frame_h / frame_w are ignored).  Frame n's
+ * results equal aicam_yolo_detect with batch 1 on that frame. */
+int aicam_yolo_detect_table(aicam_engine* e, const void* in, int in_is_s2d, const aicam_frame_table* t,
+                            const aicam_nms_params* p, float* head, int32_t* num_dets, float* boxes_lb, float* boxes_orig,
+                            float* scores, int32_t* labels, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * ReID crops: replaces DeepSORT.update steps 1-2 (class/confidence filter,
@@ -292,6 +334,13 @@ int aicam_reid_crops_nv12(const uint8_t* frames_nv12, int batch, int h, int w, c
                           uint64_t class_mask_hi, int format, int max_crops, int32_t* det_index,
                           int32_t* det_count, int32_t* crop_slot, int32_t* crop_rect, void* crops,
                           int32_t* crop_count, void* stream);
+/* The same over a frame table (any mix of sizes, pitches, BGR and NV12): the batch is the table's count, boxes are
+ * clamped to each frame's own size, crop_rect's frame index is the table index.  A crop loads whole 32-bit words of its
+ * rows only when its frame's planes are 4-byte aligned and h * pitch ((h/2) * pitch) is a multiple of 4. */
+int aicam_reid_crops_table(const aicam_frame_table* t, const float* boxes, const float* scores, const int32_t* labels,
+                           const int32_t* num_dets, int stride_k, float min_confidence, uint64_t class_mask_lo,
+                           uint64_t class_mask_hi, int format, int max_crops, int32_t* det_index, int32_t* det_count,
+                           int32_t* crop_slot, int32_t* crop_rect, void* crops, int32_t* crop_count, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Tracker: replaces TrackerCore / Track / KalmanFilter / matching / linear_assignment
