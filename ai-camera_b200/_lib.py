@@ -110,6 +110,8 @@ SIGNATURES = {
     "aicam_frame_table_create": (_I, [_I, _I, _I, _I, C.POINTER(_P)]),
     "aicam_frame_table_destroy": (None, [_P]),
     "aicam_frame_table_set": (_I, [_P, C.POINTER(FrameDesc), _I, _P]),
+    "aicam_frame_table_set_present": (_I, [_P, C.POINTER(FrameDesc), _P, _I, _P]),
+    "aicam_frame_table_present": (_P, [_P]),
     "aicam_preprocess_table": (_I, [_P, _I, _P, _P]),
     "aicam_yolo_detect_table": (_I, [_P, _P, _I, _P, C.POINTER(NmsParams), _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
     "aicam_reid_crops_table": (_I, [_P, _P, _P, _P, _P, _I, C.c_float, C.c_uint64, C.c_uint64, _I, _I, _P, _P, _P, _P,
@@ -127,7 +129,9 @@ SIGNATURES = {
     "aicam_tracker_create": (_I, [C.POINTER(TrackerConfig), C.POINTER(_P)]),
     "aicam_tracker_destroy": (None, [_P]),
     "aicam_tracker_reset": (_I, [_P, _P]),
+    "aicam_tracker_reset_streams": (_I, [_P, _P, _P]),
     "aicam_tracker_step": (_I, [_P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "aicam_tracker_step_present": (_I, [_P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "aicam_tracker_cost_probe": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "aicam_tracker_snapshot": (_I, [_P, _I, _P, _P, _I]),
     "aicam_tracker_overflow": (_I, [_P, _P]),

@@ -17,6 +17,9 @@ Differences, all in the direction of the hardware:
     labels, status panel on a device copy of the frame the detector already uploaded) and only then copied back for
     ``cv2.VideoWriter`` (this image has no NVENC: the encode stays on the host); next to it the track tuples of every
     frame go to ``<stem>.tracks.jsonl``.  Batched mode writes videos only with ``--save_video`` (one per stream).
+  * batched mode stops when its first input ends; ``--run_all_inputs`` (new) runs every input to its end instead: inputs
+    beyond ``--streams`` wait for a slot whose input has ended, an ended slot without a waiting input is absent from
+    the steps, track lines carry the input's name and ``--save_video`` writes one file per input.
 """
 import argparse
 import json
@@ -52,6 +55,10 @@ def parse_arguments(argv=None) -> argparse.Namespace:
                         help="Batched mode: number of streams per step (inputs are cycled to fill it). 0 = one "
                              "reference-shaped single-stream loop per input.")
     parser.add_argument("--max_frames", type=int, default=0, help="Stop after this many frames per stream (0 = all).")
+    parser.add_argument("--run_all_inputs", action="store_true",
+                        help="Batched mode: run every input to its end, whatever its length; inputs beyond --streams wait "
+                             "for a free stream slot (a slot whose input has ended takes the next one with a fresh "
+                             "tracker). Track lines carry the input's name and --save_video writes one file per input.")
     args = parser.parse_args(argv)
     if args.device == "cpu":
         parser.error("this build has no CPU path (the reference's TensorRT engines do not run on CPU either)")
@@ -104,16 +111,29 @@ def run_single_stream(frames: Iterable[np.ndarray], detector, tracker, on_frame=
     return stats
 
 
-def run_batched(sources: List[Iterable[np.ndarray]], pipeline, on_step=None, max_steps=0, stats_out=None) -> LoopStats:
+def run_batched(sources: List[Iterable[np.ndarray]], pipeline, on_step=None, max_steps=0, stats_out=None, until="first",
+                refill: Optional[Iterable[Iterable[np.ndarray]]] = None, on_refill=None) -> LoopStats:
     """N streams, one ``TrackingPipeline.step`` per time step.  Frames are read on the host (cv2), staged in two
     pinned buffers and uploaded on a copy stream while the previous step computes; per-stream frame order is kept.
     Sources of different frame shapes get per-stream pinned and device buffers (two each) and the step takes the list
-    of device frames.  Stops when the first source ends.  Time per step = wall time from "frames of the step are on the host" to
-    "track tables are on the host" (the detect + update span of the reference loop)."""
+    of device frames.  Time per step = wall time from "frames of the step are on the host" to "track tables are on the
+    host" (the detect + update span of the reference loop).
+
+    until="first" (default): stop when the first source ends.  until="all": a source that has ended is absent from
+    the steps that follow (None in ``batch`` for ``on_step``; it uploads nothing and its tracks are left as they are)
+    and the loop ends when every source has ended.  refill: an iterable of further sources; a slot whose source ends
+    takes the next one, after ``pipeline.reset_streams([slot])`` gave it a fresh tracker, and ``on_refill(slot, k)`` is
+    told that it now holds refill source k (0-based).  With until="all" or a refill, every step takes the list of
+    per-stream frames, and a slot's buffers are reallocated when its new source has another frame shape."""
+    if until not in ("first", "all"):
+        raise ValueError("until must be 'first' or 'all'")
     dev = pipeline.device
     its = [iter(s) for s in sources]
     S = pipeline.n_streams
     assert len(its) == S
+    refill = iter(refill) if refill is not None else None
+    n_refills = 0
+    per_slot = until == "all" or refill is not None
     stats = LoopStats()
     if stats_out is not None:
         stats_out.append(stats)
@@ -121,14 +141,32 @@ def run_batched(sources: List[Iterable[np.ndarray]], pipeline, on_step=None, max
     T = pipeline.tracker.T
     out_host = [torch.empty((S, T, 6), dtype=torch.int32).pin_memory(), torch.empty((S, T), dtype=torch.float32).pin_memory(),
                 torch.empty(S, dtype=torch.int32).pin_memory()]
+    if per_slot:  # per slot and buffer parity: (pinned, device) staging of the slot's current frame shape
+        host = [[None] * S for _ in range(2)]
+        dev_buf = [[None] * S for _ in range(2)]
     step = 0
     while not max_steps or step < max_steps:
         batch = []
-        for it in its:
-            f = next(it, None)
-            if f is None:
-                return stats
+        for s in range(S):
+            f = None
+            while its[s] is not None:
+                f = next(its[s], None)
+                if f is not None:
+                    break
+                nxt = next(refill, None) if refill is not None else None
+                if nxt is None:
+                    if until == "first":
+                        return stats
+                    its[s] = None  # ended: absent from now on
+                else:
+                    its[s] = iter(nxt)
+                    pipeline.reset_streams([s])
+                    if on_refill is not None:
+                        on_refill(s, n_refills)
+                    n_refills += 1
             batch.append(f)
+        if per_slot and all(f is None for f in batch):
+            return stats
         if host is None:
             shapes = [tuple(f.shape) for f in batch]
             if all(sh == shapes[0] for sh in shapes):
@@ -138,11 +176,24 @@ def run_batched(sources: List[Iterable[np.ndarray]], pipeline, on_step=None, max
                 host = [[torch.empty(sh, dtype=torch.uint8).pin_memory() for sh in shapes] for _ in range(2)]
                 dev_buf = [[torch.empty(sh, dtype=torch.uint8, device=dev) for sh in shapes] for _ in range(2)]
         h = host[step & 1]
-        for s, f in enumerate(batch):
-            h[s].numpy()[...] = f
-        t0 = time.time()
         d = dev_buf[step & 1]
-        if isinstance(d, list):
+        if per_slot:
+            for s, f in enumerate(batch):
+                if f is not None and (h[s] is None or tuple(h[s].shape) != tuple(f.shape)):
+                    h[s] = torch.empty(f.shape, dtype=torch.uint8).pin_memory()
+                    d[s] = torch.empty(f.shape, dtype=torch.uint8, device=dev)
+        for s, f in enumerate(batch):
+            if f is not None:
+                h[s].numpy()[...] = f
+        t0 = time.time()
+        if per_slot:
+            frames_dev = []
+            for s, f in enumerate(batch):
+                if f is not None:
+                    d[s].copy_(h[s], non_blocking=True)
+                frames_dev.append(d[s] if f is not None else None)
+            d = frames_dev
+        elif isinstance(d, list):
             for ds, hs in zip(d, h):
                 ds.copy_(hs, non_blocking=True)
         else:
@@ -239,6 +290,10 @@ def main(argv=None):
             print("Initializing the batched pipeline (%d streams)..." % args.streams)
             pipe = TrackingPipeline(args.yolo_engine, args.reid_engine, args.streams, device,
                                     conf_threshold=args.conf_thresh)
+            if args.run_all_inputs:
+                stats, frames = _run_all_inputs(args, pipe, sources_spec, writer, out_dir if writer else None,
+                                                stem if writer else None, videos, device)
+                return _summary(args, stats, frames)
             srcs = [video_frames(sources_spec[s % len(sources_spec)], args.max_frames) for s in range(args.streams)]
 
             if writer and args.save_video:
@@ -292,6 +347,10 @@ def main(argv=None):
             writer.close()
         for v in videos:
             v.close()
+    return _summary(args, stats, frames)
+
+
+def _summary(args, stats, frames):
     print("\n--- Processing Summary ---")
     print(f"Total frames processed: {frames}")
     print(f"Total time: {stats.total_s:.2f} seconds")
@@ -299,6 +358,52 @@ def main(argv=None):
     print("Latency per %s: p50 %.2f ms, p99 %.2f ms" % ("step" if args.streams > 0 else "frame", stats.percentile(50),
                                                         stats.percentile(99)))
     return 0
+
+
+def _run_all_inputs(args, pipe, inputs, writer, out_dir, stem, videos, device):
+    """--streams N --run_all_inputs: the first N inputs start in slots 0..N-1, the others wait for a slot whose input
+    has ended; every input runs to its end (an ended slot without a waiting input is absent from the steps).  Returns
+    (stats, frames processed)."""
+    N = args.streams
+    names = [Path(p).name if isinstance(p, str) else "webcam_%s" % p for p in inputs]
+    slot_input = [i if i < len(inputs) else None for i in range(N)]
+    frame_idx = [0] * N
+    srcs = [video_frames(inputs[i], args.max_frames) if i < len(inputs) else iter(()) for i in range(N)]
+    refill = (video_frames(p, args.max_frames) for p in inputs[N:])
+    if writer and args.save_video:
+        videos.extend(AnnotatedWriter(out_dir / ("%s_in%02d_%s.mp4" % (stem, i, Path(n).stem)), device)
+                      for i, n in enumerate(names))
+    dev_frames = {}
+    pipe_step = pipe.step
+
+    def step_and_keep(frames_dev, *a, **k):  # (the step's device frames, for the overlay)
+        dev_frames["f"] = frames_dev
+        return pipe_step(frames_dev, *a, **k)
+    pipe.step = step_and_keep
+    stats_ref, counted = [], [0]
+
+    def on_refill(slot, k):
+        slot_input[slot] = N + k
+        frame_idx[slot] = 0
+
+    def on_step(step, batch, table):
+        tabs = [t.numpy() for t in table] if writer else None
+        for s, f in enumerate(batch):
+            if f is None:
+                continue
+            counted[0] += 1
+            if writer:
+                i = slot_input[s]
+                rows = tracks_to_rows(tabs, s)
+                writer.write(json.dumps({"frame": frame_idx[s], "stream": s, "input": names[i], "tracks": rows}) + "\n")
+                if videos:
+                    fps = stats_ref[0].fps() * N if stats_ref else 0.0
+                    videos[i].write(dev_frames["f"][s], rows, ["AICamera: YOLOv8 + DeepSORT", f"Input: {names[i]}", "FPS: %.2f" % fps])
+            frame_idx[s] += 1
+        if (step + 1) % 100 == 0:
+            print(f"Processed {step + 1} steps.")
+    stats = run_batched(srcs, pipe, on_step, stats_out=stats_ref, until="all", refill=refill, on_refill=on_refill)
+    return stats, counted[0]
 
 
 if __name__ == "__main__":

@@ -54,6 +54,7 @@ struct TfArgs {
   int min_dets;             // streams with at most this many detections are left to the row kernel
   const int* n_tracks; const int* order; const int* state; const int* gal_count;
   const int* det_count; const int* crop_slot; int stride_k;
+  const int* present;       // [S] 0: the stream is absent this step (no work), or null
   float* app_cost;          // [S][T][D] by (slot, det)
 };
 
@@ -117,7 +118,7 @@ __global__ void __launch_bounds__(TF_THREADS, 1) appearance_tf32_kernel(const __
   for (int w = threadIdx.x; w < TF_MAX_STREAMS / 32; w += TF_THREADS) crowded[w] = 0;
   __syncthreads();
   for (int s = threadIdx.x; s < a.S; s += TF_THREADS)
-    if (min(__ldg(a.det_count + s), a.D) > a.min_dets) {
+    if ((!a.present || __ldg(a.present + s)) && min(__ldg(a.det_count + s), a.D) > a.min_dets) {
       atomicOr(&crowded[s >> 5], 1u << (s & 31));
       s_any = 1;
     }
@@ -296,13 +297,13 @@ void appearance_tf32_destroy(AppearanceTf32* p) { delete p; }
 
 int launch_appearance_tf32(const AppearanceTf32* p, int S, int T, int D, int F, int G, int min_dets, const int* n_tracks,
                            const int* order, const int* state, const int* gal_count, const int* det_count, const int* crop_slot,
-                           int stride_k, float* app_cost, cudaStream_t stream) {
+                           int stride_k, const int* present, float* app_cost, cudaStream_t stream) {
   TfArgs a;
   a.S = S; a.T = T; a.D = D; a.F = F; a.G = G;
   a.m_tiles = (D + TF_M - 1) / TF_M;
   a.min_dets = min_dets;
   a.n_tracks = n_tracks; a.order = order; a.state = state; a.gal_count = gal_count;
-  a.det_count = det_count; a.crop_slot = crop_slot; a.stride_k = stride_k; a.app_cost = app_cost;
+  a.det_count = det_count; a.crop_slot = crop_slot; a.stride_k = stride_k; a.present = present; a.app_cost = app_cost;
   if (int rc = ensure_dynamic_smem(appearance_tf32_kernel, TF_SMEM)) return rc;
   const long long total = static_cast<long long>(S) * T * a.m_tiles;
   const int sms = current_num_sms();

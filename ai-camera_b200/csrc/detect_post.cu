@@ -121,7 +121,8 @@ struct NmsArgs {
   int* out_labels;
   int* keep_index;
   uint32_t* mask_ws;     // [batch][max_cand][max_cand/32]
-  const FrameRec* recs;  // frame table: per-frame un-letterboxing (pad_w .. frame_h above unused); null: one geometry
+  const FrameRec* recs;  // frame table: per-frame un-letterboxing (pad_w .. frame_h above unused) and packed slot; null: one
+                         // geometry, frame b at b
 };
 
 __device__ __forceinline__ bool iou_gt(const float4& a, const float4& b, float thr) {
@@ -143,7 +144,22 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(const NmsArgs p) {
   int* keep = clab + MAX_CAND;                                                         // MAX_CAND x 4
   __shared__ int s_count, s_kept;
   const int b = blockIdx.x, tid = threadIdx.x;
-  const float* scores = p.scores + static_cast<long long>(b) * p.anchors;
+  // frame table: CTA b is table entry b, whose network outputs sit at its packed slot; an absent entry (slot -1) reports no
+  // detections and a zeroed row (the whole CTA leaves before the first barrier)
+  const int slot = p.recs ? p.recs[b].slot : b;
+  if (slot < 0) {
+    const long long ob = static_cast<long long>(b) * p.topk;
+    for (int r = tid; r < p.topk; r += NMS_THREADS) {
+      reinterpret_cast<float4*>(p.boxes_lb)[ob + r] = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (p.boxes_orig) reinterpret_cast<float4*>(p.boxes_orig)[ob + r] = make_float4(0.f, 0.f, 0.f, 0.f);
+      p.out_scores[ob + r] = 0.f;
+      p.out_labels[ob + r] = 0;
+      if (p.keep_index) p.keep_index[ob + r] = -1;
+    }
+    if (tid == 0) p.num_dets[b] = 0;
+    return;
+  }
+  const float* scores = p.scores + static_cast<long long>(slot) * p.anchors;
   if (tid == 0) { s_count = 0; s_kept = 0; }
   __syncthreads();
   for (int a = tid; a < p.anchors; a += NMS_THREADS) {
@@ -173,8 +189,8 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(const NmsArgs p) {
     }
   }
   const int n = min(count, p.max_cand);
-  const float4* gboxes = reinterpret_cast<const float4*>(p.boxes) + static_cast<long long>(b) * p.anchors;
-  const int* glabels = p.labels + static_cast<long long>(b) * p.anchors;
+  const float4* gboxes = reinterpret_cast<const float4*>(p.boxes) + static_cast<long long>(slot) * p.anchors;
+  const int* glabels = p.labels + static_cast<long long>(slot) * p.anchors;
   for (int i = tid; i < n; i += NMS_THREADS) {
     const int a = static_cast<int>(keys[i] & 0xffffffffu);
     cbox[i] = __ldg(gboxes + a);

@@ -510,7 +510,7 @@ int run_ops(aicam_engine* e, const void* input, int batch, void* output, cudaStr
   const void* input_s2d = input;
   if (e->s2d_in >= 0 && !input_is_s2d) {
     __nv_bfloat16* dst = e->buffers[e->s2d_in].ptr;
-    if (int rc = launch_space_to_depth(static_cast<const __nv_bfloat16*>(input), batch, e->in_h, e->in_w, 4, dst, stream)) return rc;
+    if (int rc = launch_space_to_depth(static_cast<const __nv_bfloat16*>(input), batch, e->in_h, e->in_w, 4, dst, stream, n_dev)) return rc;
     input_s2d = dst;
   } else if (e->s2d_in < 0 && input_is_s2d && e->kind == AICAM_KIND_YOLOV8) {
     return fail(AICAM_ERR_UNSUPPORTED, "engine: this engine was built without the space-to-depth stem");
@@ -648,7 +648,7 @@ int run_ops(aicam_engine* e, const void* input, int batch, void* output, cudaStr
       case Op::UPSAMPLE:
         geom(op.out, 0, &op_, &os, &oc);
         rc = launch_upsample2x(ip, is, ic, op.in.coff, batch, op.h, op.w, op.c, const_cast<__nv_bfloat16*>(op_), os,
-                               oc, op.out.coff, stream);
+                               oc, op.out.coff, stream, n_dev);
         break;
       case Op::STEMPOOL: {
         geom(op.out, 0, &op_, &os, &oc);
@@ -875,10 +875,11 @@ int aicam_engine_fused_decode(const aicam_engine* e) {
   return (nc % 16 == 0 && nc <= 80 && e->num_anchors == 8400) ? 1 : 0;  // one n-tile of whole 16-column groups per branch
 }
 
-// aicam_yolo_detect[_table]; recs: the frame table's records (per-frame un-letterboxing), or null
+// aicam_yolo_detect[_table]; recs: the frame table's records (per-frame un-letterboxing and packed slot), or null;
+// n_dev: the table's device count of present frames, which the network runs over (packed to the front of `in`), or null
 static int yolo_detect_impl(aicam_engine* e, const void* in, int in_is_s2d, int batch, const aicam_nms_params* p, float* head,
                             int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
-                            size_t workspace_bytes, void* stream, const FrameRec* recs) {
+                            size_t workspace_bytes, void* stream, const FrameRec* recs, const int* n_dev) {
   if (!e || e->kind != AICAM_KIND_YOLOV8) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect: not a yolov8 engine");
   if (batch < 0 || batch > e->max_batch) return fail(AICAM_ERR_CAPACITY, "yolo_detect: batch exceeds max_batch");
   if (in_is_s2d < 0 || in_is_s2d > 2) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect: in_is_s2d must be 0, 1 or 2");
@@ -888,7 +889,7 @@ static int yolo_detect_impl(aicam_engine* e, const void* in, int in_is_s2d, int 
   if (batch == 0) return AICAM_OK;
   if (!aicam_engine_fused_decode(e)) {
     if (!head) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect: this engine needs the fp32 head tensor (no fused decode)");
-    if (int rc = run_ops(e, in, batch, head, static_cast<cudaStream_t>(stream), nullptr, in_is_s2d)) return rc;
+    if (int rc = run_ops(e, in, batch, head, static_cast<cudaStream_t>(stream), n_dev, in_is_s2d)) return rc;
     return decode_nms_impl(head, batch, anchors, nc, p, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
                            stream, recs);
   }
@@ -902,7 +903,7 @@ static int yolo_detect_impl(aicam_engine* e, const void* in, int in_is_s2d, int 
   dec.scores = reinterpret_cast<float*>(ws + static_cast<size_t>(batch) * anchors * 16);
   dec.labels = reinterpret_cast<int*>(ws + static_cast<size_t>(batch) * anchors * 20);
   uint8_t* mask = ws + (dense + 255) / 256 * 256;
-  if (int rc = run_ops(e, in, batch, nullptr, static_cast<cudaStream_t>(stream), nullptr, in_is_s2d, &dec)) return rc;
+  if (int rc = run_ops(e, in, batch, nullptr, static_cast<cudaStream_t>(stream), n_dev, in_is_s2d, &dec)) return rc;
   return nms_impl(dec.boxes, dec.scores, dec.labels, batch, anchors, p, num_dets, boxes_lb, boxes_orig, scores, labels, nullptr,
                   mask, workspace_bytes - static_cast<size_t>(mask - ws), stream, recs);
 }
@@ -911,7 +912,7 @@ int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch,
                       int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores, int32_t* labels, void* workspace,
                       size_t workspace_bytes, void* stream) {
   return yolo_detect_impl(e, in, in_is_s2d, batch, p, head, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
-                          stream, nullptr);
+                          stream, nullptr, nullptr);
 }
 
 int aicam_yolo_detect_table(aicam_engine* e, const void* in, int in_is_s2d, const aicam_frame_table* t, const aicam_nms_params* p,
@@ -919,7 +920,7 @@ int aicam_yolo_detect_table(aicam_engine* e, const void* in, int in_is_s2d, cons
                             void* workspace, size_t workspace_bytes, void* stream) {
   if (!t) return fail(AICAM_ERR_INVALID_ARG, "yolo_detect_table: null frame table");
   return yolo_detect_impl(e, in, in_is_s2d, t->n, p, head, num_dets, boxes_lb, boxes_orig, scores, labels, workspace, workspace_bytes,
-                          stream, t->recs());
+                          stream, t->recs(), t->counts() + 3);
 }
 
 int aicam_yolo_forward_s2d(aicam_engine* e, const void* in_s2d16, int batch, float* head, void* stream) {

@@ -2,10 +2,14 @@
 // (aicam_preprocess_table, aicam_yolo_detect_table, aicam_reid_crops_table) read on the device, so that one batched step
 // can take frames of different sizes, pitches and surface formats.
 //
-// Device block layout (one cudaMemcpyAsync per aicam_frame_table_set):
-//   int  counts[4]           n, frames on the row-staged K1 path, frames on the per-pixel K1 path, 0
-//   int  lists[2][capacity]  table indices of the frames of each K1 path, in table order
+// Device block layout (one cudaMemcpyAsync per aicam_frame_table_set[_present]):
+//   int  counts[4]           n, frames on the row-staged K1 path, frames on the per-pixel K1 path, present frames
+//   int  lists[2][capacity]  table indices of the present frames of each K1 path, in table order
+//   int  present[capacity]   1: frame i is present, 0: absent (and every entry at or past n)
 //   FrameRec recs[capacity]
+// The present frames are packed to the front of the network batch: present frame i takes slot p(i), the number of present
+// frames before it, and the network runs over counts[3] images, a count it reads on the device.  Only the copy of a set
+// writes the block, so kernels that read the count before their grid dependency resolves see the step's value.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -23,6 +27,7 @@ struct FrameRec {
   // the un-letterboxing of detect() (scale_bboxes) as the NMS kernel takes it: float(ratio), float(pad_w), float(pad_h)
   float ratio, pad_w, pad_h;
   int crop_staged;        // K5: whole 32-bit words of the frame's planes can be loaded without leaving them
+  int slot;               // packed network slot (K1 output, network outputs), -1 when the frame is absent
 };
 
 constexpr int FT_COUNTS = 4;
@@ -32,7 +37,7 @@ constexpr size_t K1_SMEM_LIMIT = 200 * 1024;
 constexpr size_t K1_BLOCK_ROW_IMAGE = static_cast<size_t>(AICAM_YOLO_INPUT / 4) * 128;
 
 __host__ __device__ inline size_t frame_table_recs_offset(int capacity) {
-  return (static_cast<size_t>(FT_COUNTS + 2 * capacity) * sizeof(int) + 15) / 16 * 16;
+  return (static_cast<size_t>(FT_COUNTS + 3 * capacity) * sizeof(int) + 15) / 16 * 16;
 }
 __host__ __device__ inline size_t frame_table_bytes(int capacity) {
   return frame_table_recs_offset(capacity) + static_cast<size_t>(capacity) * sizeof(FrameRec);
@@ -45,7 +50,7 @@ int k1_geometry(int h, int w, int* decimate, int* mode, int* new_h, int* new_w, 
 
 struct aicam_frame_table {
   int device, capacity, max_h, max_w;
-  int n;                  // frames set by the last aicam_frame_table_set
+  int n;                  // frames set by the last aicam_frame_table_set[_present], absent ones included
   uint8_t* dev;           // the device block
   uint8_t* host[2];       // pinned staging, used alternately
   cudaEvent_t done[2];    // recorded after the copy out of host[i]
@@ -53,6 +58,7 @@ struct aicam_frame_table {
 
   const int* counts() const { return reinterpret_cast<const int*>(dev); }
   const int* lists() const { return reinterpret_cast<const int*>(dev) + aicam::FT_COUNTS; }
+  const int* present() const { return lists() + 2 * capacity; }
   const aicam::FrameRec* recs() const { return reinterpret_cast<const aicam::FrameRec*>(dev + aicam::frame_table_recs_offset(capacity)); }
   // One row slot of the row-staged K1 ring: the longest staged source row (a BGR row of max_w pixels; an NV12 luma + chroma
   // row is shorter), rounded up to 16 bytes so that every slot, and the format-3 image behind the ring, is a valid 16-byte

@@ -1,5 +1,5 @@
 // The frame table (include/aicam.h, aicam_frame_table_*): per-stream frame descriptors, validated and resolved on the
-// host, read on the device by the ragged K1 / detect / K5 entry points.  See frame_table.cuh for the device layout.
+// host, read on the device by the ragged K1 / detect / K5 entry points and, for presence, by the tracker step.  See frame_table.cuh for the device layout.
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -53,10 +53,20 @@ void aicam_frame_table_destroy(aicam_frame_table* t) {
 }
 
 int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* descs, int n, void* stream) {
-  if (!t || (!descs && n > 0) || n < 0) return fail(AICAM_ERR_INVALID_ARG, "frame_table_set: null table or descriptors");
+  return aicam_frame_table_set_present(t, descs, nullptr, n, stream);
+}
+
+int aicam_frame_table_set_present(aicam_frame_table* t, const aicam_frame_desc* descs, const uint8_t* present_host, int n,
+                                  void* stream) {
+  auto is_present = [&](int i) { return !present_host || present_host[i] != 0; };
+  if (!t || n < 0) return fail(AICAM_ERR_INVALID_ARG, "frame_table_set: null table or descriptors");
+  if (!descs)
+    for (int i = 0; i < n; ++i)
+      if (is_present(i)) return fail(AICAM_ERR_INVALID_ARG, "frame_table_set: null table or descriptors");
   if (n > t->capacity) return fail(AICAM_ERR_CAPACITY, "frame_table_set: more frames than the table's capacity");
-  // validate everything before touching the staging or launching anything
+  // validate every present descriptor before touching the staging or launching anything (absent ones are not read)
   for (int i = 0; i < n; ++i) {
+    if (!is_present(i)) continue;
     const aicam_frame_desc& d = descs[i];
     const std::string at = "frame_table_set: frame " + std::to_string(i) + ": ";
     if (d.kind != 0 && d.kind != 1) return fail(AICAM_ERR_INVALID_ARG, at + "kind must be 0 (BGR) or 1 (NV12)");
@@ -71,9 +81,16 @@ int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* descs, i
   std::vector<FrameRec> recs(n);
   std::vector<int> ring, pix;
   const bool ring_fits = t->ring_fits();
+  int packed = 0;
   for (int i = 0; i < n; ++i) {
-    const aicam_frame_desc& d = descs[i];
     FrameRec& r = recs[i];
+    if (!is_present(i)) {  // nothing of the frame is read: no geometry, no list, no slot
+      r = FrameRec{};
+      r.slot = -1;
+      continue;
+    }
+    const aicam_frame_desc& d = descs[i];
+    r.slot = packed++;
     r.data = d.data; r.chroma = d.kind == 1 ? d.chroma : nullptr;
     r.h = d.h; r.w = d.w; r.pitch = d.pitch; r.kind = d.kind;
     int decimate = 0;
@@ -96,10 +113,12 @@ int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* descs, i
   AICAM_CUDA_OK(cudaEventSynchronize(t->done[slot]));
   uint8_t* h = t->host[slot];
   int* counts = reinterpret_cast<int*>(h);
-  counts[0] = n; counts[1] = static_cast<int>(ring.size()); counts[2] = static_cast<int>(pix.size()); counts[3] = 0;
+  counts[0] = n; counts[1] = static_cast<int>(ring.size()); counts[2] = static_cast<int>(pix.size()); counts[3] = packed;
   int* lists = counts + FT_COUNTS;
   std::copy(ring.begin(), ring.end(), lists);
   std::copy(pix.begin(), pix.end(), lists + t->capacity);
+  int* present = lists + 2 * t->capacity;
+  for (int i = 0; i < t->capacity; ++i) present[i] = i < n && recs[i].slot >= 0 ? 1 : 0;
   if (n) std::memcpy(h + frame_table_recs_offset(t->capacity), recs.data(), n * sizeof(FrameRec));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   AICAM_CUDA_OK(cudaMemcpyAsync(t->dev, h, frame_table_recs_offset(t->capacity) + n * sizeof(FrameRec), cudaMemcpyHostToDevice, st));
@@ -107,6 +126,14 @@ int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* descs, i
   t->next = slot ^ 1;
   t->n = n;
   return AICAM_OK;
+}
+
+const int32_t* aicam_frame_table_present(const aicam_frame_table* t) {
+  if (!t) {
+    fail(AICAM_ERR_INVALID_ARG, "frame_table_present: null table");
+    return nullptr;
+  }
+  return t->present();
 }
 
 }  // extern "C"

@@ -95,7 +95,8 @@ __global__ void __launch_bounds__(256) sppf_pool3_kernel(__nv_bfloat16* __restri
 // nearest-neighbour 2x: one thread per INPUT 16-byte chunk (8 channels of one pixel): one load, four stores
 __global__ void __launch_bounds__(256) upsample2x_kernel(const __nv_bfloat16* __restrict__ in, long long in_img_stride, int in_cstride,
                                                          int in_coff, int h, int w, int c8, __nv_bfloat16* __restrict__ out,
-                                                         long long out_img_stride, int out_cstride, int out_coff, unsigned total) {
+                                                         long long out_img_stride, int out_cstride, int out_coff, unsigned total,
+                                                         const int* __restrict__ n_dev) {
   const unsigned idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= total) return;
   const unsigned g = idx % c8;
@@ -103,6 +104,7 @@ __global__ void __launch_bounds__(256) upsample2x_kernel(const __nv_bfloat16* __
   const unsigned x = p % w; p /= w;
   const unsigned y = p % h;
   const unsigned n = p / h;
+  if (n_dev && static_cast<int>(n) >= __ldg(n_dev)) return;
   const uint4 v = __ldg(reinterpret_cast<const uint4*>(
       in + n * in_img_stride + (static_cast<long long>(y) * w + x) * in_cstride + in_coff + g * 8));
   __nv_bfloat16* o = out + n * out_img_stride + (static_cast<long long>(2 * y) * 2 * w + 2 * x) * out_cstride + out_coff + g * 8;
@@ -169,7 +171,8 @@ __global__ void nchw_to_nhwc4_kernel(const float* __restrict__ in, int hw, __nv_
 
 // [n][h][w][c] -> [n][h/2][w/2][2x2 sub-pixel][c]: one thread per 16-byte (or, for 4 channels, 8-byte) piece
 template <typename V>
-__global__ void space_to_depth_kernel(const V* __restrict__ in, V* __restrict__ out, int h, int w, int pieces, long long total) {
+__global__ void space_to_depth_kernel(const V* __restrict__ in, V* __restrict__ out, int h, int w, int pieces, long long total,
+                                      const int* __restrict__ n_dev) {
   const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
   if (idx >= total) return;
   const int pc = static_cast<int>(idx % pieces);
@@ -177,22 +180,24 @@ __global__ void space_to_depth_kernel(const V* __restrict__ in, V* __restrict__ 
   const int x = static_cast<int>(p % w); p /= w;
   const int y = static_cast<int>(p % h);
   const long long n = p / h;
+  if (n_dev && n >= __ldg(n_dev)) return;
   const long long dst = (((n * (h >> 1) + (y >> 1)) * (w >> 1) + (x >> 1)) * 4 + ((y & 1) << 1) + (x & 1)) * pieces + pc;
   out[dst] = __ldg(in + idx);
 }
 
 }  // namespace
 
-int launch_space_to_depth(const __nv_bfloat16* in, int batch, int h, int w, int c, __nv_bfloat16* out, cudaStream_t stream) {
+int launch_space_to_depth(const __nv_bfloat16* in, int batch, int h, int w, int c, __nv_bfloat16* out, cudaStream_t stream,
+                          const int* n_dev) {
   if ((c != 4 && c % 8) || h % 2 || w % 2) return fail(AICAM_ERR_INVALID_ARG, "space_to_depth: 4 or a multiple of 8 channels, even sizes");
   const int pieces = c == 4 ? 1 : c / 8;
   const long long total = static_cast<long long>(batch) * h * w * pieces;
   if (total == 0) return AICAM_OK;
   const unsigned blocks = static_cast<unsigned>((total + 255) / 256);
   if (c == 4)
-    space_to_depth_kernel<uint2><<<blocks, 256, 0, stream>>>(reinterpret_cast<const uint2*>(in), reinterpret_cast<uint2*>(out), h, w, 1, total);
+    space_to_depth_kernel<uint2><<<blocks, 256, 0, stream>>>(reinterpret_cast<const uint2*>(in), reinterpret_cast<uint2*>(out), h, w, 1, total, n_dev);
   else
-    space_to_depth_kernel<uint4><<<blocks, 256, 0, stream>>>(reinterpret_cast<const uint4*>(in), reinterpret_cast<uint4*>(out), h, w, pieces, total);
+    space_to_depth_kernel<uint4><<<blocks, 256, 0, stream>>>(reinterpret_cast<const uint4*>(in), reinterpret_cast<uint4*>(out), h, w, pieces, total, n_dev);
   count_launch();
   return last_launch("space_to_depth_kernel");
 }
@@ -228,14 +233,14 @@ int try_launch_sppf_pool3(__nv_bfloat16* buf, long long img_stride, int cstride,
 
 int launch_upsample2x(const __nv_bfloat16* in, long long in_img_stride, int in_cstride, int in_coff, int batch, int h,
                       int w, int c, __nv_bfloat16* out, long long out_img_stride, int out_cstride, int out_coff,
-                      cudaStream_t stream) {
+                      cudaStream_t stream, const int* n_dev) {
   if (c % 8 || in_cstride % 8 || in_coff % 8 || out_cstride % 8 || out_coff % 8)
     return fail(AICAM_ERR_INVALID_ARG, "upsample: channel counts/offsets must be multiples of 8");
   const long long total = static_cast<long long>(batch) * h * w * (c / 8);  // input chunks
   if (total == 0) return AICAM_OK;
   if (total >= (1ll << 32)) return fail(AICAM_ERR_CAPACITY, "upsample: tensor too large");
   upsample2x_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, stream>>>(
-      in, in_img_stride, in_cstride, in_coff, h, w, c / 8, out, out_img_stride, out_cstride, out_coff, static_cast<unsigned>(total));
+      in, in_img_stride, in_cstride, in_coff, h, w, c / 8, out, out_img_stride, out_cstride, out_coff, static_cast<unsigned>(total), n_dev);
   count_launch();
   return last_launch("upsample2x_kernel");
 }

@@ -262,7 +262,7 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restri
 }
 
 // The per-pixel path over a frame table: the frames of the table's per-pixel list (frame_table.cuh), any size, pitch and
-// kind.  The grid is sized from the table's capacity and walks the list with a grid-stride loop; the list's length is read
+// kind, each written at its packed slot (absent frames are on no list).  The grid is sized from the table's capacity and walks the list with a grid-stride loop; the list's length is read
 // on the device, so a captured launch stays valid when the table is set to other frames.
 template <int FORMAT>
 __global__ void __launch_bounds__(256) preprocess_table_kernel(const int* __restrict__ counts, const int* __restrict__ list,
@@ -273,12 +273,11 @@ __global__ void __launch_bounds__(256) preprocess_table_kernel(const int* __rest
     const int xg = static_cast<int>(idx % (S / PIX));
     const long long t = idx / (S / PIX);
     const int y = static_cast<int>(t % S);
-    const int n = list[t / S];
-    const FrameRec& r = recs[n];
+    const FrameRec& r = recs[list[t / S]];
     if (r.kind == 0)
-      preprocess_pixels<FORMAT>(FrameSrc<2>{r.data, r.pitch}, r.mode, r.new_h, r.new_w, r.top, r.left, r.tab, out, n, y, xg);
+      preprocess_pixels<FORMAT>(FrameSrc<2>{r.data, r.pitch}, r.mode, r.new_h, r.new_w, r.top, r.left, r.tab, out, r.slot, y, xg);
     else
-      preprocess_pixels<FORMAT>(FrameSrc<3>{r.data, r.chroma, r.pitch}, r.mode, r.new_h, r.new_w, r.top, r.left, r.tab, out, n, y, xg);
+      preprocess_pixels<FORMAT>(FrameSrc<3>{r.data, r.chroma, r.pitch}, r.mode, r.new_h, r.new_w, r.top, r.left, r.tab, out, r.slot, y, xg);
   }
 }
 
@@ -299,8 +298,8 @@ struct PairFrame {
   const int* tab;
 };
 
-// TABLE: the pairs are those of the frames on the table's row-staged list (frame_table.cuh), each with its own geometry, and
-// the count is read on the device; the frame arguments are then unused and a ring stage holds two rows of stage_row bytes.
+// TABLE: the pairs are those of the frames on the table's row-staged list (frame_table.cuh), each with its own geometry and
+// written at its packed slot, and the count is read on the device; the frame arguments are then unused and a ring stage holds two rows of stage_row bytes.
 // Each CTA then walks one contiguous, even-aligned run of pairs, so that its frame - and the geometry it loads from the table,
 // three dependent loads - changes at most a few times per CTA instead of at every pair.
 template <int FORMAT, int SRC, bool TABLE = false>
@@ -325,8 +324,8 @@ __global__ void __launch_bounds__(S / PIX) preprocess_pairs_kernel(const uint8_t
   auto frame_of = [&](int pair) -> PairFrame {
     PairFrame g;
     if (TABLE) {
-      g.n = t_list[pair / (S / 2)];
-      const FrameRec& r = t_recs[g.n];
+      const FrameRec& r = t_recs[t_list[pair / (S / 2)]];
+      g.n = r.slot;  // the packed network slot of the (present) frame
       g.data = r.data; g.chroma = r.chroma; g.pitch = r.pitch; g.w = r.w; g.nv12 = r.kind;
       g.new_h = r.new_h; g.new_w = r.new_w; g.top = r.top; g.left = r.left; g.tab = r.tab;
     } else {

@@ -34,7 +34,8 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
                                                       int max_crops, int* __restrict__ det_index,
                                                       int* __restrict__ det_count, int* __restrict__ crop_slot,
                                                       int* __restrict__ crop_rect, int* __restrict__ crop_count,
-                                                      const FrameRec* __restrict__ recs) {  // frame table: per-frame (w, h); or null
+                                                      const FrameRec* __restrict__ recs) {  // frame table: per-frame (w, h)
+                                                                                            // and presence; or null
   __shared__ int s_scan[32];  // valid crops per frame of the current group of 32 frames, then their exclusive scan
   __shared__ int s_base;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -46,7 +47,8 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
     const int fw = recs && b < batch ? recs[b].w : w, fh = recs && b < batch ? recs[b].h : h;
     int nvalid = 0, nkeep = 0;
     if (b < batch) {
-      const int n = min(num_dets[b], stride_k);
+      // an absent frame of a table keeps no detection whatever num_dets says, so no crop reads its (unset) descriptor
+      const int n = recs && recs[b].slot < 0 ? 0 : min(num_dets[b], stride_k);
       const long long fo = static_cast<long long>(b) * stride_k;
       for (int i0 = 0; i0 < n; i0 += 32) {
         const int i = i0 + lane;

@@ -38,7 +38,8 @@ int appearance_tf32_create(AppearanceTf32** out, int S, int T, int D, int F, int
 void appearance_tf32_destroy(AppearanceTf32* p);
 int launch_appearance_tf32(const AppearanceTf32* p, int S, int T, int D, int F, int G, int min_dets, const int* n_tracks,
                            const int* order, const int* state, const int* gal_count, const int* det_count, const int* crop_slot,
-                           int stride_k, float* app_cost, cudaStream_t stream);
+                           int stride_k, const int* present, float* app_cost,
+                           cudaStream_t stream);
 
 namespace {
 
@@ -412,8 +413,9 @@ __device__ inline LsapMem lsap_carve(uint8_t* p, int n) {
 // detection features -> L2-normalised copies (matching.py:125-130), one block per (det, stream)
 __global__ void __launch_bounds__(128) normalize_kernel(Dev t, const int* __restrict__ det_count,
                                                         const int* __restrict__ crop_slot, int stride_k,
-                                                        const float* __restrict__ feats) {
+                                                        const float* __restrict__ feats, const int* __restrict__ present) {
   const int s = blockIdx.y, d = blockIdx.x;
+  if (present && !present[s]) return;  // an absent stream's crop slots are not this step's
   if (d >= min(det_count[s], t.D)) return;
   const int row = crop_slot[static_cast<long long>(s) * stride_k + d];
   if (row < 0) return;
@@ -588,8 +590,10 @@ constexpr size_t AG_SMEM = (AG_KC * (AG_ROWS + 4) + AG_KC * (AG_DT + 4) + 16 * A
 // One launch, two tilings: frames with at most APP_GEMM_MIN detections take the row kernel (no padding work), busier
 // frames the SGEMM tiling.  The choice is per block from the device-side count.
 __global__ void __launch_bounds__(256) appearance_kernel(Dev t, const int* __restrict__ det_count,
-                                                         const int* __restrict__ crop_slot, int stride_k, int gemm_ok) {
+                                                         const int* __restrict__ crop_slot, int stride_k, int gemm_ok,
+                                                         const int* __restrict__ present) {
   extern __shared__ __align__(16) float sm_f[];
+  if (present && !present[blockIdx.y]) return;  // absent stream: nothing of it is read or written
   const bool crowded = min(det_count[blockIdx.y], t.D) > APP_GEMM_MIN;
   if (crowded && gemm_ok == 2) return;  // appearance_tf32_kernel owns this stream's frame
   if (crowded && gemm_ok == 1) appearance_gemm(t, det_count, crop_slot, stride_k, sm_f);
@@ -604,6 +608,7 @@ struct StepIO {
   long long* trace;  // debug (AICAM_ASSOC_TRACE): clock64 stamps of stream 0's CTA, see aicam_tracker_destroy
   int has_feats;   // 0: the frame carries no features at all (feats == NULL): every appearance cost is INFTY_COST and
                    // nothing is appended to the galleries, as in the reference when every Detection.feature is None
+  const int* present;  // [S] 0: the stream has no frame this step and its state is left as it is; null: all present
 };
 
 // one normalised detection feature (and its TF32 split copies) -> a gallery row, by one warp.  Feature rows are 16-byte
@@ -666,6 +671,12 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
 
 #define ASSOC_STAMP(i) do { if (io.trace && s == 0 && tid == 0) io.trace[i] = clock64(); } while (0)
   ASSOC_STAMP(0);
+  // an absent stream: no predict, no aging, no state change at all - as if its reference process had not been called for
+  // this frame; the whole CTA leaves before the first barrier
+  if (io.present && !io.present[s]) {
+    if (tid == 0) io.out_count[s] = 0;
+    return;
+  }
   const long long sb = static_cast<long long>(s) * T;
   int nt = t.n_tracks[s];
   int nd = io.det_count[s];
@@ -995,8 +1006,10 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
 #undef ASSOC_STAMP
 }
 
-__global__ void reset_kernel(Dev t) {
+// mask: device i32[S], streams with a zero entry are left as they are; null resets every stream
+__global__ void reset_kernel(Dev t, const int* __restrict__ mask) {
   const int s = blockIdx.x;
+  if (mask && !mask[s]) return;
   const long long sb = static_cast<long long>(s) * t.T;
   for (int k = threadIdx.x; k < t.T; k += blockDim.x) {
     t.free_slots[sb + k] = t.T - 1 - k;  // slot 0 is popped first
@@ -1094,8 +1107,8 @@ int dev_alloc(aicam_tracker* t, Tp** p, size_t n) {
 namespace {
 // K8: L2-normalise the frame's detection features, then the appearance cost of every confirmed track
 int launch_appearance(const Dev& d, const AppearanceTf32* tf, const int32_t* det_count, const int32_t* crop_slot, int stride_k,
-                      const float* feats, cudaStream_t st) {
-  normalize_kernel<<<dim3(d.D, d.S), 128, 0, st>>>(d, det_count, crop_slot, stride_k, feats);
+                      const float* feats, const int32_t* present, cudaStream_t st) {
+  normalize_kernel<<<dim3(d.D, d.S), 128, 0, st>>>(d, det_count, crop_slot, stride_k, feats, present);
   count_launch();
   if (int rc = last_launch("normalize_kernel")) return rc;
   static const bool no_gemm = getenv("AICAM_APPEARANCE_ROWS") != nullptr;
@@ -1104,12 +1117,12 @@ int launch_appearance(const Dev& d, const AppearanceTf32* tf, const int32_t* det
   const int gemm_ok = tf ? 2 : ((d.F % AG_KC == 0 && !no_gemm) ? 1 : 0);
   const size_t sm = std::max((APP_DT * d.F + 8 * APP_DT) * sizeof(float), gemm_ok == 1 ? AG_SMEM : size_t(0));
   if (int rc = ensure_dynamic_smem(appearance_kernel, sm)) return rc;
-  appearance_kernel<<<dim3(d.T, d.S), 256, sm, st>>>(d, det_count, crop_slot, stride_k, gemm_ok);
+  appearance_kernel<<<dim3(d.T, d.S), 256, sm, st>>>(d, det_count, crop_slot, stride_k, gemm_ok, present);
   count_launch();
   if (int rc = last_launch("appearance_kernel")) return rc;
   if (tf)
     return launch_appearance_tf32(tf, d.S, d.T, d.D, d.F, d.G, APP_GEMM_MIN, d.n_tracks, d.order, d.state, d.gal_count, det_count,
-                                  crop_slot, stride_k, d.app_cost, st);
+                                  crop_slot, stride_k, present, d.app_cost, st);
   return AICAM_OK;
 }
 }  // namespace
@@ -1195,14 +1208,28 @@ void aicam_tracker_destroy(aicam_tracker* t) {
 
 int aicam_tracker_reset(aicam_tracker* t, void* stream) {
   if (!t) return fail(AICAM_ERR_INVALID_ARG, "tracker_reset: null handle");
-  reset_kernel<<<t->d.S, 128, 0, static_cast<cudaStream_t>(stream)>>>(t->d);
+  reset_kernel<<<t->d.S, 128, 0, static_cast<cudaStream_t>(stream)>>>(t->d, nullptr);
   count_launch();
   return last_launch("reset_kernel");
+}
+
+int aicam_tracker_reset_streams(aicam_tracker* t, const int32_t* mask, void* stream) {
+  if (!t || !mask) return fail(AICAM_ERR_INVALID_ARG, "tracker_reset_streams: null argument");
+  reset_kernel<<<t->d.S, 128, 0, static_cast<cudaStream_t>(stream)>>>(t->d, mask);
+  count_launch();
+  return last_launch("reset_kernel (masked)");
 }
 
 int aicam_tracker_step(aicam_tracker* t, const float* boxes, const float* scores, const int32_t* labels, int stride_k,
                        const int32_t* det_index, const int32_t* det_count, const int32_t* crop_slot, const float* feats,
                        int32_t* out_tracks, float* out_conf, int32_t* out_count, void* stream) {
+  return aicam_tracker_step_present(t, boxes, scores, labels, stride_k, det_index, det_count, crop_slot, feats, nullptr, out_tracks,
+                                    out_conf, out_count, stream);
+}
+
+int aicam_tracker_step_present(aicam_tracker* t, const float* boxes, const float* scores, const int32_t* labels, int stride_k,
+                               const int32_t* det_index, const int32_t* det_count, const int32_t* crop_slot, const float* feats,
+                               const int32_t* present, int32_t* out_tracks, float* out_conf, int32_t* out_count, void* stream) {
   if (!t || !boxes || !scores || !labels || !det_index || !det_count || !crop_slot || !out_tracks || !out_conf || !out_count)
     return fail(AICAM_ERR_INVALID_ARG, "tracker_step: null argument");
   if (stride_k <= 0) return fail(AICAM_ERR_INVALID_ARG, "tracker_step: stride_k must be positive");
@@ -1210,9 +1237,10 @@ int aicam_tracker_step(aicam_tracker* t, const float* boxes, const float* scores
   const Dev& d = t->d;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (feats) {
-    if (int rc = launch_appearance(d, t->tf, det_count, crop_slot, stride_k, feats, st)) return rc;
+    if (int rc = launch_appearance(d, t->tf, det_count, crop_slot, stride_k, feats, present, st)) return rc;
   }
-  StepIO io{boxes, scores, labels, stride_k, det_index, det_count, crop_slot, out_tracks, out_conf, out_count, 0, t->trace, feats ? 1 : 0};
+  StepIO io{boxes, scores, labels, stride_k, det_index, det_count, crop_slot, out_tracks, out_conf, out_count, 0, t->trace, feats ? 1 : 0,
+            present};
   if (t->trace) cudaMemsetAsync(t->trace, 0, sizeof(long long) * 16, st);
   const size_t asm_bytes = assoc_smem(d.T, d.D, &io.cm_in_smem);
   if (int rc = ensure_dynamic_smem(assoc_kernel, asm_bytes)) return rc;
@@ -1230,7 +1258,7 @@ int aicam_tracker_cost_probe(aicam_tracker* t, const float* boxes, int stride_k,
     return fail(AICAM_ERR_INVALID_ARG, "tracker_cost_probe: stride_k must be positive and boxes 16-byte aligned");
   const Dev& d = t->d;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int rc = launch_appearance(d, t->tf, det_count, crop_slot, stride_k, feats, st)) return rc;
+  if (int rc = launch_appearance(d, t->tf, det_count, crop_slot, stride_k, feats, nullptr, st)) return rc;
   cost_probe_kernel<<<dim3(d.T, d.S), 128, 0, st>>>(d, boxes, stride_k, det_index, det_count, app_cost, gate_d2, track_ids, n_tracks);
   count_launch();
   return last_launch("cost_probe_kernel");

@@ -35,7 +35,10 @@ class FrameTable:
     """Owner of an ``aicam_frame_table``: per-stream frames of any size, row pitch and surface format for one batched
     step.  ``set(frames)`` takes a list of uint8 CUDA tensors, each ``[H, W, 3]`` BGR or ``[H*3/2, W]`` NV12, whose rows
     are contiguous (a view into a larger surface is fine: its row stride is the pitch).  The library may read every
-    plane as rows * pitch bytes, so a view's last row must be followed by the rest of its pitch inside the same storage."""
+    plane as rows * pitch bytes, so a view's last row must be followed by the rest of its pitch inside the same storage.
+    A ``None`` entry marks that stream ABSENT for the step (a dropped or late frame, a source that has ended): it is not
+    read, its detection row is empty and its tracker state does not change.  ``present`` is the device i32[capacity] 0/1
+    mask of the last set (a stable pointer that captured steps read)."""
 
     def __init__(self, device, capacity: int, max_frame_hw=(2160, 3840)):
         self.lib = _lib.load()
@@ -45,8 +48,11 @@ class FrameTable:
         _lib.check(self.lib.aicam_frame_table_create(self.device.index or 0, self.capacity, self.max_frame_hw[0],
                                                      self.max_frame_hw[1], C.byref(self._h)))
         self._descs = (_lib.FrameDesc * self.capacity)()
+        self._present = (C.c_uint8 * self.capacity)()
         self.n = 0
+        self.n_present = 0
         self.frames = []
+        self.present_ptr = C.c_void_p(self.lib.aicam_frame_table_present(self._h))
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -70,18 +76,25 @@ class FrameTable:
         if n > self.capacity:
             raise _lib.AicamError(-4, "%d frames exceed the frame table's capacity %d" % (n, self.capacity))
         for i, f in enumerate(frames):
+            d = self._descs[i]
+            self._present[i] = f is not None
+            if f is None:
+                d.data, d.chroma, d.h, d.w, d.pitch, d.kind = None, None, 0, 0, 0, 0
+                continue
             if f.device != self.device:
                 raise _lib.AicamError(-1, "frame %d is not on %s" % (i, self.device))
             h, w, pitch, kind = self.describe(f)
             if f.storage_offset() + f.shape[0] * pitch > f.untyped_storage().nbytes():
                 raise _lib.AicamError(-1, "frame %d: its %d rows of %d bytes (the pitch) run past the end of its storage"
                                       % (i, f.shape[0], pitch))
-            d = self._descs[i]
             d.data, d.h, d.w, d.pitch, d.kind = f.data_ptr(), h, w, pitch, kind
             d.chroma = f.data_ptr() + h * pitch if kind == 1 else None
+        n_present = sum(f is not None for f in frames)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.aicam_frame_table_set(self._h, self._descs, n, _lib.stream_ptr(self.device)))
-        self.n = n
+            _lib.check(self.lib.aicam_frame_table_set_present(self._h, self._descs,
+                                                              self._present if n_present < n else None, n,
+                                                              _lib.stream_ptr(self.device)))
+        self.n, self.n_present = n, n_present
         self.frames = list(frames)  # kept alive while work that reads the table may be in flight
 
     @property
@@ -119,7 +132,8 @@ class BatchDetector:
     def detect(self, frames):
         """frames: uint8 cuda [n<=batch, H, W, 3] BGR, or [n, H*3/2, W] NV12 (Y plane + interleaved UV plane, the
         surface format of hardware decoders: half the bytes), or a list of n such frames ([H_s, W_s, 3] / [H_s*3/2, W_s])
-        of any sizes and kinds.  Returns device tensors (num_dets [n],
+        of any sizes and kinds, where None marks an absent frame (its row reports no detections; the network runs over
+        the present frames only).  Returns device tensors (num_dets [n],
         boxes [n,topk,4] in frame pixels, scores [n,topk], labels [n,topk]); views of internal
         buffers, valid until the next call; asynchronous on the current stream."""
         if is_frame_list(frames):
@@ -208,6 +222,7 @@ class BatchTracker:
         self.out_tracks = torch.zeros((S, max_tracks, 6), **i32)
         self.out_conf = torch.zeros((S, max_tracks), dtype=torch.float32, device=dev)
         self.out_count = torch.zeros(S, **i32)
+        self._reset_mask = torch.zeros(S, **i32)
         self._mask = config.tracked_class_mask()
         # optional running totals (crops, reported tracks) kept on the device, for benchmarks: no host sync
         self.count_stats = False
@@ -224,9 +239,22 @@ class BatchTracker:
         _lib.check(self.lib.aicam_tracker_reset(self._h, _lib.stream_ptr(self.device)))
         self.crop_count.zero_()
 
+    def reset_streams(self, indices):
+        """Reset the given streams to a fresh tracker's state (no tracks, ids from 1), e.g. when a slot is handed to
+        another camera or clip; every other stream keeps its tracks.  One kernel launch on the current stream."""
+        mask = torch.zeros(self.S, dtype=torch.int32)
+        for i in indices:
+            if not 0 <= int(i) < self.S:
+                raise _lib.AicamError(-1, "reset_streams: stream %d out of range" % int(i))
+            mask[int(i)] = 1
+        with torch.cuda.device(self.device):
+            self._reset_mask.copy_(mask)
+            _lib.check(self.lib.aicam_tracker_reset_streams(self._h, _lib.ptr(self._reset_mask), _lib.stream_ptr(self.device)))
+
     def update(self, frames, num_dets, boxes, scores, labels):
         """One frame per stream.  frames uint8 cuda [S,H,W,3] BGR or [S,H*3/2,W] NV12, or a list of S frames of any
-        sizes and kinds (see BatchDetector.detect); detections as BatchDetector
+        sizes and kinds, None for a stream that has no frame this step (see BatchDetector.detect: its state is left as it
+        is and its out_count is 0); detections as BatchDetector
         returns them ([S], [S,K,4], [S,K], [S,K]).  Returns device (out_tracks [S,T,6] int32 =
         x1,y1,x2,y2,id,class, out_conf [S,T], out_count [S]); asynchronous."""
         if is_frame_list(frames):
@@ -246,10 +274,11 @@ class BatchTracker:
                 _lib.ptr(self.det_index),
                 _lib.ptr(self.det_count), _lib.ptr(self.crop_slot), _lib.ptr(self.crop_rect), _lib.ptr(self.crops),
                 _lib.ptr(self.crop_count), st))
-        return self._reid_and_step(boxes, scores, labels)
+        return self._reid_and_step(boxes, scores, labels, None)
 
     def update_table(self, table: FrameTable, num_dets, boxes, scores, labels):
-        """update() on the frames a FrameTable holds (one per stream); capturable."""
+        """update() on the frames a FrameTable holds (one per stream, absent ones included); capturable, and a captured
+        step follows the presence of each later ``table.set``."""
         if table.n != self.S or boxes.shape[1] != self.K:
             raise _lib.AicamError(-4, "update: expected %d streams x %d detections" % (self.S, self.K))
         with torch.cuda.device(self.device):
@@ -258,18 +287,19 @@ class BatchTracker:
                 self.K, self.min_conf, self._mask[0], self._mask[1], 2 if self._nhwc8 else 1, self.max_crops,
                 _lib.ptr(self.det_index), _lib.ptr(self.det_count), _lib.ptr(self.crop_slot), _lib.ptr(self.crop_rect),
                 _lib.ptr(self.crops), _lib.ptr(self.crop_count), _lib.stream_ptr(self.device)))
-        return self._reid_and_step(boxes, scores, labels)
+        return self._reid_and_step(boxes, scores, labels, table.present_ptr)
 
-    def _reid_and_step(self, boxes, scores, labels):
+    def _reid_and_step(self, boxes, scores, labels, present):
         st = _lib.stream_ptr(self.device)
         with torch.cuda.device(self.device):
             fwd = self.lib.aicam_reid_forward_nhwc8 if self._nhwc8 else self.lib.aicam_reid_forward
             _lib.check(fwd(self.reid.handle, _lib.ptr(self.crops), self.max_crops, _lib.ptr(self.crop_count),
                            _lib.ptr(self.feats), st))
-            _lib.check(self.lib.aicam_tracker_step(
+            # present: the frame table's device mask (absent streams keep their state), or None on the tensor path
+            _lib.check(self.lib.aicam_tracker_step_present(
                 self._h, _lib.ptr(boxes), _lib.ptr(scores), _lib.ptr(labels), self.K, _lib.ptr(self.det_index),
-                _lib.ptr(self.det_count), _lib.ptr(self.crop_slot), _lib.ptr(self.feats), _lib.ptr(self.out_tracks),
-                _lib.ptr(self.out_conf), _lib.ptr(self.out_count), st))
+                _lib.ptr(self.det_count), _lib.ptr(self.crop_slot), _lib.ptr(self.feats), present,
+                _lib.ptr(self.out_tracks), _lib.ptr(self.out_conf), _lib.ptr(self.out_count), st))
             if self.count_stats:
                 self.crop_total += self.crop_count[0:1]
                 self.track_total += self.out_count.sum()
@@ -299,7 +329,9 @@ class BatchTracker:
 
 class TrackingPipeline:
     """detect + track for ``n_streams`` streams; one call per time step.  A step takes one stacked tensor of frames of
-    one size, or a list with one frame per stream of any sizes (up to ``max_frame_hw``), pitches and kinds (BGR / NV12)."""
+    one size, or a list with one frame per stream of any sizes (up to ``max_frame_hw``), pitches and kinds (BGR / NV12),
+    where None marks a stream without a frame at this step: its tracks are neither predicted nor aged, and it reports
+    no tracks.  (Aging tracks through a dropped frame is a different policy, not this one.)"""
 
     def __init__(self, yolo_engine_path, reid_engine_path, n_streams: int, device=None, max_tracks: int = 256,
                  max_crops: Optional[int] = None, conf_threshold=config.YOLO_CONF_THRESHOLD, topk=config.YOLO_TOPK,
@@ -325,10 +357,17 @@ class TrackingPipeline:
 
     def step_table(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """One step over the frames ``frame_table`` holds.  Launches depend only on the stream count and the size
-        bound, so a captured step_table() stays valid when ``frame_table.set`` changes the frames between replays."""
+        bound, so a captured step_table() stays valid when ``frame_table.set`` changes the frames, or which of them are
+        present, between replays."""
         num, boxes, scores, labels = self.detector.detect_table(self.frame_table)
         return self.tracker.update_table(self.frame_table, num, boxes, scores, labels)
 
+    def reset_streams(self, indices):
+        """Hand the given stream slots to new sources: their trackers restart (no tracks, ids from 1), the other streams
+        and the captured step are untouched."""
+        self.tracker.reset_streams(indices)
+
     def launches_per_step(self, frame_list=False):
-        """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True)."""
+        """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True), absent frames
+        or not."""
         return self.detector.launches_per_step(frame_list) + self.tracker.launches_per_step()

@@ -249,9 +249,23 @@ typedef struct {
 int aicam_frame_table_create(int device, int capacity, int max_h, int max_w, aicam_frame_table** out);
 void aicam_frame_table_destroy(aicam_frame_table* t);
 int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* host_descs, int n, void* stream);
-/* aicam_preprocess / aicam_preprocess_nv12 over a frame table (formats 0-3): frame n's slice of `out` equals the uniform
- * entry on that frame alone.  Frames whose geometry is a pure decimation (1080p) and whose planes, pitch and row bytes
- * are multiples of 16 take the row-staged path, all others the per-pixel path: at most one launch each. */
+/* Presence: a camera fleet mixes frame rates, drops frames and has streams that end or reconnect, so a step need not
+ * have a frame for every stream.  aicam_frame_table_set_present is aicam_frame_table_set with a host mask:
+ * present_host[i] == 0 marks frame i ABSENT - its descriptor is neither read nor validated (NULL pointers are fine);
+ * present_host == NULL means every frame is present, which is exactly aicam_frame_table_set (same validation, same
+ * error codes, nothing launched on error).  The present frames are packed to the front of the network batch: present
+ * frame i takes packed slot p(i), the number of present frames before it (p(i) = i when all are present).
+ * aicam_frame_table_present: device i32[capacity], 1 for a present frame of the last set, 0 otherwise; the pointer is
+ * stable for the table's lifetime, so a captured aicam_tracker_step_present can read it.  Launch configurations of the
+ * table entry points still depend only on the set's count and the size bound: a captured step stays valid when the
+ * presence pattern changes between replays, and absent frames cost no launch. */
+int aicam_frame_table_set_present(aicam_frame_table* t, const aicam_frame_desc* host_descs, const uint8_t* present_host, int n,
+                                  void* stream);
+const int32_t* aicam_frame_table_present(const aicam_frame_table* t);
+/* aicam_preprocess / aicam_preprocess_nv12 over a frame table (formats 0-3): present frame i's slice of `out` is slice p(i)
+ * (packed, see above; slice i when all frames are present) and equals the uniform entry on that frame alone; slices past
+ * the present count are not written.  Frames whose geometry is a pure decimation (1080p) and whose planes, pitch and row
+ * bytes are multiples of 16 take the row-staged path, all others the per-pixel path: at most one launch each. */
 int aicam_preprocess_table(const aicam_frame_table* t, int format, void* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------
@@ -295,9 +309,11 @@ int aicam_yolo_detect(aicam_engine* e, const void* in, int in_is_s2d, int batch,
                       float* head, int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* scores,
                       int32_t* labels, void* workspace, size_t workspace_bytes, void* stream);
 int aicam_engine_fused_decode(const aicam_engine* e);
-/* aicam_yolo_detect over a frame table (in = aicam_preprocess_table output): the batch is the table's count, and
- * boxes_orig un-letterboxes each frame with its own ratio, pad and size (p->frame_h / frame_w are ignored).  Frame n's
- * results equal aicam_yolo_detect with batch 1 on that frame. */
+/* aicam_yolo_detect over a frame table (in = aicam_preprocess_table output): the outputs have one row per table entry
+ * (the table's count), and boxes_orig un-letterboxes each frame with its own ratio, pad and size (p->frame_h / frame_w
+ * are ignored).  Present frame n's results equal aicam_yolo_detect with batch 1 on that frame.  The network runs over the
+ * packed present frames only, their count read on the device (none present: it launches as usual and does nothing); an
+ * absent frame's row has num_dets = 0 and zero entries. */
 int aicam_yolo_detect_table(aicam_engine* e, const void* in, int in_is_s2d, const aicam_frame_table* t,
                             const aicam_nms_params* p, float* head, int32_t* num_dets, float* boxes_lb, float* boxes_orig,
                             float* scores, int32_t* labels, void* workspace, size_t workspace_bytes, void* stream);
@@ -335,7 +351,8 @@ int aicam_reid_crops_nv12(const uint8_t* frames_nv12, int batch, int h, int w, c
                           int32_t* det_count, int32_t* crop_slot, int32_t* crop_rect, void* crops,
                           int32_t* crop_count, void* stream);
 /* The same over a frame table (any mix of sizes, pitches, BGR and NV12): the batch is the table's count, boxes are
- * clamped to each frame's own size, crop_rect's frame index is the table index.  A crop loads whole 32-bit words of its
+ * clamped to each frame's own size, crop_rect's frame index is the table index.  An absent frame gets det_count 0
+ * whatever num_dets says for it.  A crop loads whole 32-bit words of its
  * rows only when its frame's planes are 4-byte aligned and h * pitch ((h/2) * pitch) is a multiple of 4. */
 int aicam_reid_crops_table(const aicam_frame_table* t, const float* boxes, const float* scores, const int32_t* labels,
                            const int32_t* num_dets, int stride_k, float min_confidence, uint64_t class_mask_lo,
@@ -365,6 +382,10 @@ typedef struct {
 int aicam_tracker_create(const aicam_tracker_config* cfg, aicam_tracker** out);
 void aicam_tracker_destroy(aicam_tracker* t);
 int aicam_tracker_reset(aicam_tracker* t, void* stream);
+/* Reset the streams whose entry of the device mask i32[n_streams] is non-zero: each becomes what a freshly created
+ * tracker's stream is (no tracks, ids from 1, no overflow flags); every other stream is untouched.  One kernel launch,
+ * capturable, so a slot can be handed to another camera or clip while the other streams keep their tracks. */
+int aicam_tracker_reset_streams(aicam_tracker* t, const int32_t* mask, void* stream);
 
 /* One frame for every stream: predict, cascade + IoU matching, update, initiate, prune,
  * format.  Inputs describe, per stream b, the detections of the frame (as returned by
@@ -381,6 +402,15 @@ int aicam_tracker_step(aicam_tracker* t, const float* boxes, const float* scores
                        const int32_t* labels, int stride_k, const int32_t* det_index,
                        const int32_t* det_count, const int32_t* crop_slot, const float* feats,
                        int32_t* out_tracks, float* out_conf, int32_t* out_count, void* stream);
+/* aicam_tracker_step with a device i32[n_streams] presence mask (e.g. aicam_frame_table_present); NULL = every stream is
+ * present, which is exactly aicam_tracker_step.  An absent stream is treated as if its reference process had not been
+ * called for this frame: its state (tracks, Kalman state, age, time_since_update, galleries, free slots, id counter,
+ * overflow flags) does not change bit for bit - no predict, no aging - and out_count is 0 for it; its detection inputs
+ * are not read.  Aging tracks through a dropped frame (predict with no detections) is a different policy, not this one.
+ * The launches are those of aicam_tracker_step whatever the mask, so a captured step follows presence changes. */
+int aicam_tracker_step_present(aicam_tracker* t, const float* boxes, const float* scores, const int32_t* labels, int stride_k,
+                               const int32_t* det_index, const int32_t* det_count, const int32_t* crop_slot, const float* feats,
+                               const int32_t* present, int32_t* out_tracks, float* out_conf, int32_t* out_count, void* stream);
 
 /* Snapshot of the live tracks of one stream in track-list order (host out; synchronises):
  *   ints  [n][7]  = track_id, state(1 tentative, 2 confirmed), hits, age, time_since_update,
