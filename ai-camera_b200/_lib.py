@@ -50,6 +50,16 @@ class FrameDesc(C.Structure):
                 ("kind", C.c_int)]
 
 
+class StreamFilter(C.Structure):
+    _fields_ = [("score_thr", C.c_float), ("iou_thr", C.c_float), ("min_confidence", C.c_float), ("reserved", C.c_int),
+                ("class_mask_lo", C.c_uint64), ("class_mask_hi", C.c_uint64)]
+
+
+class StreamAssoc(C.Structure):
+    _fields_ = [("max_cosine_distance", C.c_double), ("max_iou_distance", C.c_double), ("max_age", C.c_int),
+                ("n_init", C.c_int)]
+
+
 class TrackerConfig(C.Structure):
     _fields_ = [("n_streams", C.c_int), ("max_tracks", C.c_int), ("max_dets", C.c_int),
                 ("feature_dim", C.c_int), ("max_cosine_distance", C.c_double),
@@ -112,6 +122,7 @@ SIGNATURES = {
     "aicam_frame_table_set": (_I, [_P, C.POINTER(FrameDesc), _I, _P]),
     "aicam_frame_table_set_present": (_I, [_P, C.POINTER(FrameDesc), _P, _I, _P]),
     "aicam_frame_table_present": (_P, [_P]),
+    "aicam_frame_table_set_filters": (_I, [_P, C.POINTER(StreamFilter), _I]),
     "aicam_preprocess_table": (_I, [_P, _I, _P, _P]),
     "aicam_yolo_detect_table": (_I, [_P, _P, _I, _P, C.POINTER(NmsParams), _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
     "aicam_reid_crops_table": (_I, [_P, _P, _P, _P, _P, _I, C.c_float, C.c_uint64, C.c_uint64, _I, _I, _P, _P, _P, _P,
@@ -130,6 +141,7 @@ SIGNATURES = {
     "aicam_tracker_destroy": (None, [_P]),
     "aicam_tracker_reset": (_I, [_P, _P]),
     "aicam_tracker_reset_streams": (_I, [_P, _P, _P]),
+    "aicam_tracker_set_stream_assoc": (_I, [_P, _P, C.POINTER(StreamAssoc), _I, _P]),
     "aicam_tracker_step": (_I, [_P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "aicam_tracker_step_present": (_I, [_P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "aicam_tracker_cost_probe": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -20,6 +20,11 @@ Differences, all in the direction of the hardware:
   * batched mode stops when its first input ends; ``--run_all_inputs`` (new) runs every input to its end instead: inputs
     beyond ``--streams`` wait for a slot whose input has ended, an ended slot without a waiting input is absent from
     the steps, track lines carry the input's name and ``--save_video`` writes one file per input.
+  * ``--stream_settings FILE.json`` (new, batched mode) gives each input its own detection and tracking settings (the
+    constructor arguments one reference process per input would take): ``{"default": {...}, "<input file name>": {...}}``
+    with ``pipeline.StreamSettings`` field names.  An input's entry applies over "default", which applies over
+    ``--conf_thresh`` and the config.  Each input runs with its entry from its first frame, also when it takes over a
+    slot under ``--run_all_inputs``.
 """
 import argparse
 import json
@@ -59,10 +64,39 @@ def parse_arguments(argv=None) -> argparse.Namespace:
                         help="Batched mode: run every input to its end, whatever its length; inputs beyond --streams wait "
                              "for a free stream slot (a slot whose input has ended takes the next one with a fresh "
                              "tracker). Track lines carry the input's name and --save_video writes one file per input.")
+    parser.add_argument("--stream_settings", type=str, default=None,
+                        help="Batched mode: JSON file {\"default\": {...}, \"<input file name>\": {...}} of per-input "
+                             "settings (conf_threshold, nms_threshold, classes_to_track, min_detection_confidence, "
+                             "max_cosine_distance, max_iou_distance, max_age, n_init).")
     args = parser.parse_args(argv)
     if args.device == "cpu":
         parser.error("this build has no CPU path (the reference's TensorRT engines do not run on CPU either)")
+    args.settings_for = None
+    if args.stream_settings is not None:
+        if args.streams <= 0:
+            parser.error("--stream_settings needs batched mode (--streams N)")
+        try:
+            args.settings_for = load_stream_settings(args.stream_settings, args.conf_thresh)
+        except (OSError, ValueError, TypeError) as e:
+            parser.error("--stream_settings %s: %s" % (args.stream_settings, e))
     return args
+
+
+def load_stream_settings(path, conf_threshold=config.YOLO_CONF_THRESHOLD):
+    """The --stream_settings file as a function: input file name -> StreamSettings.  An input's entry applies over
+    "default", which applies over ``conf_threshold`` and the config; an input without an entry gets "default"."""
+    from .pipeline import StreamSettings
+    with open(path) as f:
+        spec = json.load(f)
+    if not isinstance(spec, dict) or not all(isinstance(v, dict) for v in spec.values()):
+        raise ValueError("expected a JSON object of objects")
+    default = StreamSettings.from_dict(spec.get("default", {}), StreamSettings(conf_threshold=conf_threshold))
+    entries = {name: StreamSettings.from_dict(v, default) for name, v in spec.items() if name != "default"}
+    return lambda name: entries.get(name, default)
+
+
+def input_name(spec):
+    return Path(spec).name if isinstance(spec, str) else "webcam_%s" % spec
 
 
 class LoopStats:
@@ -288,8 +322,13 @@ def main(argv=None):
         if args.streams > 0:
             from .pipeline import TrackingPipeline
             print("Initializing the batched pipeline (%d streams)..." % args.streams)
+            stream_settings = None
+            if args.settings_for:  # slot s starts with input s (inputs are cycled unless --run_all_inputs is given)
+                first = [sources_spec[s % len(sources_spec)] if not args.run_all_inputs or s < len(sources_spec) else None
+                         for s in range(args.streams)]
+                stream_settings = [args.settings_for(input_name(p) if p is not None else None) for p in first]
             pipe = TrackingPipeline(args.yolo_engine, args.reid_engine, args.streams, device,
-                                    conf_threshold=args.conf_thresh)
+                                    conf_threshold=args.conf_thresh, stream_settings=stream_settings)
             if args.run_all_inputs:
                 stats, frames = _run_all_inputs(args, pipe, sources_spec, writer, out_dir if writer else None,
                                                 stem if writer else None, videos, device)
@@ -365,7 +404,7 @@ def _run_all_inputs(args, pipe, inputs, writer, out_dir, stem, videos, device):
     has ended; every input runs to its end (an ended slot without a waiting input is absent from the steps).  Returns
     (stats, frames processed)."""
     N = args.streams
-    names = [Path(p).name if isinstance(p, str) else "webcam_%s" % p for p in inputs]
+    names = [input_name(p) for p in inputs]
     slot_input = [i if i < len(inputs) else None for i in range(N)]
     frame_idx = [0] * N
     srcs = [video_frames(inputs[i], args.max_frames) if i < len(inputs) else iter(()) for i in range(N)]
@@ -385,6 +424,8 @@ def _run_all_inputs(args, pipe, inputs, writer, out_dir, stem, videos, device):
     def on_refill(slot, k):
         slot_input[slot] = N + k
         frame_idx[slot] = 0
+        if args.settings_for:
+            pipe.configure_streams([slot], args.settings_for(names[N + k]))
 
     def on_step(step, batch, table):
         tabs = [t.numpy() for t in table] if writer else None

@@ -41,11 +41,12 @@ CLASSES = (
 CLASSES_TO_TRACK = {'person', 'car', 'bus', 'truck', 'motorcycle'}
 
 
-def tracked_class_mask():
-    """(lo, hi) 64-bit masks of the COCO ids whose name is in CLASSES_TO_TRACK."""
+def tracked_class_mask(classes=None):
+    """(lo, hi) 64-bit masks of the COCO ids whose name is in ``classes`` (default CLASSES_TO_TRACK)."""
+    classes = CLASSES_TO_TRACK if classes is None else classes
     lo = hi = 0
     for i, n in enumerate(CLASSES):
-        if n in CLASSES_TO_TRACK:
+        if n in classes:
             if i < 64:
                 lo |= 1 << i
             else:

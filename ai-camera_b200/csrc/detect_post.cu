@@ -159,12 +159,15 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(const NmsArgs p) {
     if (tid == 0) p.num_dets[b] = 0;
     return;
   }
+  // thresholds: the entry's own when the table carries settings for it (aicam_frame_table_set_filters)
+  float score_thr = p.score_thr, iou_thr = p.iou_thr;
+  if (p.recs && p.recs[b].filt) { score_thr = p.recs[b].score_thr; iou_thr = p.recs[b].iou_thr; }
   const float* scores = p.scores + static_cast<long long>(slot) * p.anchors;
   if (tid == 0) { s_count = 0; s_kept = 0; }
   __syncthreads();
   for (int a = tid; a < p.anchors; a += NMS_THREADS) {
     const float s = __ldg(scores + a);
-    if (s >= p.score_thr) {
+    if (s >= score_thr) {
       const int pos = atomicAdd(&s_count, 1);
       keys[pos] = (static_cast<unsigned long long>(~__float_as_uint(s)) << 32) | static_cast<unsigned>(a);
     }
@@ -209,7 +212,7 @@ __global__ void __launch_bounds__(NMS_THREADS) nms_kernel(const NmsArgs p) {
       const int jend = min(32, n - j0);
       for (int jj = 0; jj < jend; ++jj) {
         const int j = j0 + jj;
-        if (j > i && clab[j] == li && iou_gt(cbox[j], bi, p.iou_thr)) bits |= 1u << jj;
+        if (j > i && clab[j] == li && iou_gt(cbox[j], bi, iou_thr)) bits |= 1u << jj;
       }
     }
     mask[idx] = bits;

@@ -13,7 +13,10 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <vector>
+
 #include "common.cuh"
+#include "staging.cuh"
 
 namespace aicam {
 
@@ -28,6 +31,11 @@ struct FrameRec {
   float ratio, pad_w, pad_h;
   int crop_staged;        // K5: whole 32-bit words of the frame's planes can be loaded without leaving them
   int slot;               // packed network slot (K1 output, network outputs), -1 when the frame is absent
+  // per-entry detection and filter settings (aicam_frame_table_set_filters): when `filt` is 1 the NMS kernel and K5's filter
+  // read these instead of the thresholds and class mask passed to the entry points
+  int filt;
+  float score_thr, iou_thr, min_conf;
+  unsigned long long mask_lo, mask_hi;
 };
 
 constexpr int FT_COUNTS = 4;
@@ -52,9 +60,8 @@ struct aicam_frame_table {
   int device, capacity, max_h, max_w;
   int n;                  // frames set by the last aicam_frame_table_set[_present], absent ones included
   uint8_t* dev;           // the device block
-  uint8_t* host[2];       // pinned staging, used alternately
-  cudaEvent_t done[2];    // recorded after the copy out of host[i]
-  int next;
+  aicam::PinnedStaging staging;
+  std::vector<aicam_stream_filter> filters;  // of aicam_frame_table_set_filters: entry i < size() carries filters[i]
 
   const int* counts() const { return reinterpret_cast<const int*>(dev); }
   const int* lists() const { return reinterpret_cast<const int*>(dev) + aicam::FT_COUNTS; }

@@ -30,8 +30,7 @@ int aicam_frame_table_create(int device, int capacity, int max_h, int max_w, aic
   t->device = device; t->capacity = capacity; t->max_h = max_h; t->max_w = max_w;
   const size_t bytes = frame_table_bytes(capacity);
   cudaError_t e = cudaMalloc(&t->dev, bytes);
-  for (int i = 0; i < 2 && e == cudaSuccess; ++i) e = cudaMallocHost(&t->host[i], bytes);
-  for (int i = 0; i < 2 && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&t->done[i], cudaEventDisableTiming);
+  if (e == cudaSuccess) e = t->staging.create(bytes);
   if (e == cudaSuccess) e = cudaMemset(t->dev, 0, bytes);  // count 0 until the first set
   if (e != cudaSuccess) {
     aicam_frame_table_destroy(t);
@@ -44,10 +43,7 @@ int aicam_frame_table_create(int device, int capacity, int max_h, int max_w, aic
 void aicam_frame_table_destroy(aicam_frame_table* t) {
   if (!t) return;
   cudaSetDevice(t->device);
-  for (int i = 0; i < 2; ++i) {
-    if (t->done[i]) cudaEventSynchronize(t->done[i]), cudaEventDestroy(t->done[i]);
-    if (t->host[i]) cudaFreeHost(t->host[i]);
-  }
+  t->staging.destroy();
   if (t->dev) cudaFree(t->dev);
   delete t;
 }
@@ -108,10 +104,16 @@ int aicam_frame_table_set_present(aicam_frame_table* t, const aicam_frame_desc* 
     r.crop_staged = aligned(d.data, 4) && (static_cast<long long>(d.h) * d.pitch) % 4 == 0 &&
                     (d.kind == 0 || (aligned(d.chroma, 4) && (static_cast<long long>(d.h / 2) * d.pitch) % 4 == 0));
   }
+  for (int i = 0; i < n && i < static_cast<int>(t->filters.size()); ++i) {  // absent entries carry them too (unread)
+    const aicam_stream_filter& f = t->filters[i];
+    FrameRec& r = recs[i];
+    r.filt = 1;
+    r.score_thr = f.score_thr; r.iou_thr = f.iou_thr; r.min_conf = f.min_confidence;
+    r.mask_lo = f.class_mask_lo; r.mask_hi = f.class_mask_hi;
+  }
   // stage into the pinned buffer whose previous copy has completed
-  const int slot = t->next;
-  AICAM_CUDA_OK(cudaEventSynchronize(t->done[slot]));
-  uint8_t* h = t->host[slot];
+  uint8_t* h = nullptr;
+  AICAM_CUDA_OK(t->staging.acquire(&h));
   int* counts = reinterpret_cast<int*>(h);
   counts[0] = n; counts[1] = static_cast<int>(ring.size()); counts[2] = static_cast<int>(pix.size()); counts[3] = packed;
   int* lists = counts + FT_COUNTS;
@@ -120,11 +122,27 @@ int aicam_frame_table_set_present(aicam_frame_table* t, const aicam_frame_desc* 
   int* present = lists + 2 * t->capacity;
   for (int i = 0; i < t->capacity; ++i) present[i] = i < n && recs[i].slot >= 0 ? 1 : 0;
   if (n) std::memcpy(h + frame_table_recs_offset(t->capacity), recs.data(), n * sizeof(FrameRec));
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  AICAM_CUDA_OK(cudaMemcpyAsync(t->dev, h, frame_table_recs_offset(t->capacity) + n * sizeof(FrameRec), cudaMemcpyHostToDevice, st));
-  AICAM_CUDA_OK(cudaEventRecord(t->done[slot], st));
-  t->next = slot ^ 1;
+  AICAM_CUDA_OK(t->staging.upload(t->dev, frame_table_recs_offset(t->capacity) + n * sizeof(FrameRec),
+                                   static_cast<cudaStream_t>(stream)));
   t->n = n;
+  return AICAM_OK;
+}
+
+int aicam_frame_table_set_filters(aicam_frame_table* t, const aicam_stream_filter* host, int n) {
+  if (!t || n < 0) return fail(AICAM_ERR_INVALID_ARG, "frame_table_set_filters: null table or negative count");
+  if (!host || n == 0) {
+    t->filters.clear();
+    return AICAM_OK;
+  }
+  if (n > t->capacity) return fail(AICAM_ERR_CAPACITY, "frame_table_set_filters: more entries than the table's capacity");
+  for (int i = 0; i < n; ++i) {
+    const aicam_stream_filter& f = host[i];
+    for (float v : {f.score_thr, f.iou_thr, f.min_confidence})
+      if (!(v >= 0.0f && v <= 1.0f))  // (false for NaN)
+        return fail(AICAM_ERR_INVALID_ARG, "frame_table_set_filters: entry " + std::to_string(i) +
+                                               ": thresholds must be finite and in [0, 1]");
+  }
+  t->filters.assign(host, host + n);
   return AICAM_OK;
 }
 

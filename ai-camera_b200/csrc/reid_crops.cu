@@ -50,13 +50,17 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
       // an absent frame of a table keeps no detection whatever num_dets says, so no crop reads its (unset) descriptor
       const int n = recs && recs[b].slot < 0 ? 0 : min(num_dets[b], stride_k);
       const long long fo = static_cast<long long>(b) * stride_k;
+      // the entry's own confidence and class mask when the table carries settings for it
+      float mc = min_conf;
+      unsigned long long mlo = mask_lo, mhi = mask_hi;
+      if (recs && recs[b].filt) { mc = recs[b].min_conf; mlo = recs[b].mask_lo; mhi = recs[b].mask_hi; }
       for (int i0 = 0; i0 < n; i0 += 32) {
         const int i = i0 + lane;
         bool keep = false, ok = false;
         if (i < n) {
           const int cls = labels[fo + i];
-          const bool tracked = cls >= 0 && cls < 128 && (((cls < 64 ? mask_lo >> cls : mask_hi >> (cls - 64)) & 1ull) != 0);
-          keep = scores[fo + i] >= min_conf && tracked;
+          const bool tracked = cls >= 0 && cls < 128 && (((cls < 64 ? mlo >> cls : mhi >> (cls - 64)) & 1ull) != 0);
+          keep = scores[fo + i] >= mc && tracked;
           if (keep) {
             const float4 bx = reinterpret_cast<const float4*>(boxes)[fo + i];
             const int x1 = max(0, static_cast<int>(bx.x)), y1 = max(0, static_cast<int>(bx.y));

@@ -20,11 +20,16 @@
 //   gallery[S][T][G][F] f32 (L2-normalised at insert; ring buffer: head, count)
 //   order[S][T]: slots of the live tracks in creation order (the reference's track list)
 //   free_slots[S][T] stack, next_id[S]
+//   trk_n_init/trk_max_age[S][T] i32: the n_init / max_age a track was created with (track.py keeps them per track)
+//   assoc[S]: each stream's association settings (aicam_tracker_set_stream_assoc), read once per step by its CTA
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
+#include <cstring>
 #include <vector>
 
 #include "common.cuh"
+#include "staging.cuh"
 
 namespace aicam {
 
@@ -48,10 +53,22 @@ constexpr float INFTY_COST = 1e5f;                         // linear_assignment.
 constexpr float CHI2_GATE = 9.487729036781154f;            // kalman_filter.py:16, compared in float32
 constexpr int ASSOC_THREADS = 256;
 
-struct Dev {
-  int S, T, D, F, G;
+// one stream's association settings: the thresholds as the reference compares them (float32 of the Python float) and the
+// clamps of linear_assignment.py:58 (max_distance + 1e-5 rounded from double), the cascade depth and the confirmation count
+struct AssocRec {
   float thr_cos, clamp_cos, thr_iou, clamp_iou;
   int max_age, n_init;
+};
+
+AssocRec resolve_assoc(const aicam_stream_assoc& a) {
+  return AssocRec{static_cast<float>(a.max_cosine_distance), static_cast<float>(a.max_cosine_distance + 1e-5),
+                  static_cast<float>(a.max_iou_distance), static_cast<float>(a.max_iou_distance + 1e-5), a.max_age, a.n_init};
+}
+
+struct Dev {
+  int S, T, D, F, G;
+  const AssocRec* assoc;  // [S]
+  int* trk_n_init; int* trk_max_age;
   float* mean; float* cov;
   int* track_id; int* state; int* hits; int* age; int* tsu; int* cls; float* conf;
   int* gal_count; int* gal_head; float* gallery;
@@ -677,6 +694,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
     if (tid == 0) io.out_count[s] = 0;
     return;
   }
+  const AssocRec cfg = t.assoc[s];  // the stream's settings of this step (register copies: the fewest spills, DESIGN §3.5)
   const long long sb = static_cast<long long>(s) * T;
   int nt = t.n_tracks[s];
   int nd = io.det_count[s];
@@ -728,7 +746,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
       if (st == CONFIRMED) {
         conf_list[nc + __popc(bc & below)] = k;
         const int lv = st_tsu[k];
-        if (lv >= 1 && lv <= t.max_age && lv < 256) lv_bits[lv >> 5] |= 1u << (lv & 31);
+        if (lv >= 1 && lv <= cfg.max_age && lv < 256) lv_bits[lv >> 5] |= 1u << (lv & 31);
       } else if (st == TENTATIVE) {
         tent_list[nn + __popc(bt & below)] = k;
       }
@@ -753,7 +771,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
     const float4 m4 = st_mean4[pos], c4 = st_cov4[pos];
     const float mean4[4] = {m4.x, m4.y, m4.z, m4.w}, cov4[4] = {c4.x, c4.y, c4.z, c4.w};
     if (kf_gating(mean4, cov4, d_xyah + 4 * d, n_meas) > CHI2_GATE) c = INFTY_COST;
-    return c > t.thr_cos ? t.clamp_cos : c;
+    return c > cfg.thr_cos ? cfg.clamp_cos : c;
   };
   // unmatched detections keep their order (linear_assignment.py:64-88): in-place compaction of U by warp 0
   auto compact_U = [&](int nU) {
@@ -788,12 +806,12 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
     if (!small || warp == 0) {
       int level = 0, nU = nd;
       for (;;) {
-        for (++level; level <= t.max_age; ) {  // next level that holds a confirmed track
+        for (++level; level <= cfg.max_age; ) {  // next level that holds a confirmed track
           const unsigned wbits = s_levels[level >> 5] >> (level & 31);
           if (wbits) { level += __ffs(wbits) - 1; break; }
           level = (level | 31) + 1;
         }
-        if (level > t.max_age || nU == 0) break;
+        if (level > cfg.max_age || nU == 0) break;
         if (warp == 0) {  // L = the level's tracks in track-list order
           int n = 0;
           for (int b0 = 0; b0 < nconf; b0 += 32) {
@@ -825,7 +843,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
           const int j = cfr[i];
           if (j < 0) continue;
           const float c = one_col ? colv[i] : cm[L[i] * nd + U[j]];
-          if (c <= t.thr_cos) { match[L[i]] = U[j]; det_used[U[j]] = 1; }
+          if (c <= cfg.thr_cos) { match[L[i]] = U[j]; det_used[U[j]] = 1; }
         }
         csync();
         if (warp == 0) compact_U(nU);
@@ -856,7 +874,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
       float tl[4];
       mean_to_tlwh(mean4, tl);
       const float c = iou_cost(tl, d_tlwh + 4 * U[j]);
-      cm[idx] = c > t.thr_iou ? t.clamp_iou : c;  // linear_assignment.py:58
+      cm[idx] = c > cfg.thr_iou ? cfg.clamp_iou : c;  // linear_assignment.py:58
     }
     __syncthreads();
     const int nw = lsap_warps(nL, nU);
@@ -866,7 +884,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
     if (io.trace && s == 0 && tid == 0) { io.trace[10] += clock64() - c0; io.trace[11] += 1; io.trace[12] += static_cast<long long>(nL) * 1024 + nU; }
     for (int i = tid; i < nL; i += ASSOC_THREADS) {
       const int j = cfr[i];
-      if (j >= 0 && cm[i * nU + j] <= t.thr_iou) { match[L[i]] = U[j]; det_used[U[j]] = 1; }
+      if (j >= 0 && cm[i * nU + j] <= cfg.thr_iou) { match[L[i]] = U[j]; det_used[U[j]] = 1; }
     }
     __syncthreads();
     if (warp == 0) compact_U(nU);
@@ -893,7 +911,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
       st_tsu[k] = 0;
       t.conf[ts] = io.scores[o];
       t.cls[ts] = io.labels[o];
-      if (st_state[k] == TENTATIVE && hits >= t.n_init) { t.state[ts] = CONFIRMED; st_state[k] = CONFIRMED; }
+      if (st_state[k] == TENTATIVE && hits >= t.trk_n_init[ts]) { t.state[ts] = CONFIRMED; st_state[k] = CONFIRMED; }
       // track.py:70-74: the feature is appended to the gallery, FIFO at the budget (rows copied below, one warp each)
       int gp = -1;
       if (io.has_feats && io.crop_slot[static_cast<long long>(s) * io.stride_k + d] >= 0) {
@@ -902,7 +920,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
         if (cnt < t.G) t.gal_count[ts] = cnt + 1; else t.gal_head[ts] = (head + 1) % t.G;
       }
       gpos[k] = gp;
-    } else if (st_state[k] == TENTATIVE || (st_state[k] == CONFIRMED && st_tsu[k] > t.max_age)) {
+    } else if (st_state[k] == TENTATIVE || (st_state[k] == CONFIRMED && st_tsu[k] > t.trk_max_age[ts])) {
       t.state[ts] = DELETED;
       st_state[k] = DELETED;
     }
@@ -945,6 +963,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
       t.state[ts] = TENTATIVE;
       t.hits[ts] = 1; t.age[ts] = 1; t.tsu[ts] = 0;
       t.gal_count[ts] = 0; t.gal_head[ts] = 0;
+      t.trk_n_init[ts] = cfg.n_init; t.trk_max_age[ts] = cfg.max_age;
     }
     t.next_id[s] = next_id;
     t.n_free[s] = nfree;
@@ -1085,6 +1104,9 @@ size_t assoc_smem(int T, int D, int* cm_in_smem = nullptr) {
 struct aicam_tracker {
   aicam::Dev d;
   aicam_tracker_config cfg;
+  std::vector<aicam::AssocRec> assoc;  // host copy of d.assoc
+  aicam::AssocRec* assoc_dev = nullptr;
+  aicam::PinnedStaging staging;        // of aicam_tracker_set_stream_assoc
   std::vector<void*> allocs;
   aicam::AppearanceTf32* tf = nullptr;  // tensor-core appearance path (frames with more than APP_GEMM_MIN detections)
   long long* trace = nullptr;           // AICAM_ASSOC_TRACE: 16 clock64 slots, printed by aicam_tracker_destroy
@@ -1100,6 +1122,25 @@ int dev_alloc(aicam_tracker* t, Tp** p, size_t n) {
   cudaMemset(q, 0, n * sizeof(Tp));
   t->allocs.push_back(q);
   *p = static_cast<Tp*>(q);
+  return AICAM_OK;
+}
+
+// the host copy of the stream table to the device: one copy from pinned staging
+int upload_assoc(aicam_tracker* t, cudaStream_t st) {
+  uint8_t* h = nullptr;
+  AICAM_CUDA_OK(t->staging.acquire(&h));
+  const size_t bytes = t->assoc.size() * sizeof(AssocRec);
+  std::memcpy(h, t->assoc.data(), bytes);
+  AICAM_CUDA_OK(t->staging.upload(t->assoc_dev, bytes, st));
+  return AICAM_OK;
+}
+
+int check_assoc(const aicam_stream_assoc& a, const std::string& at) {
+  if (a.max_age < 1 || a.max_age > 255 || a.n_init < 1)
+    return fail(AICAM_ERR_INVALID_ARG, at + "max_age must be in 1..255 and n_init >= 1");
+  if (!std::isfinite(a.max_cosine_distance) || !std::isfinite(a.max_iou_distance) || a.max_cosine_distance < 0 ||
+      a.max_iou_distance < 0)
+    return fail(AICAM_ERR_INVALID_ARG, at + "distances must be finite and non-negative");
   return AICAM_OK;
 }
 }  // namespace
@@ -1145,11 +1186,8 @@ int aicam_tracker_create(const aicam_tracker_config* cfg, aicam_tracker** out) {
   t->cfg = *cfg;
   Dev& d = t->d;
   d.S = cfg->n_streams; d.T = cfg->max_tracks; d.D = cfg->max_dets; d.F = cfg->feature_dim; d.G = cfg->nn_budget;
-  d.thr_cos = static_cast<float>(cfg->max_cosine_distance);
-  d.clamp_cos = static_cast<float>(cfg->max_cosine_distance + 1e-5);
-  d.thr_iou = static_cast<float>(cfg->max_iou_distance);
-  d.clamp_iou = static_cast<float>(cfg->max_iou_distance + 1e-5);
-  d.max_age = cfg->max_age; d.n_init = cfg->n_init;
+  t->assoc.assign(d.S, resolve_assoc(aicam_stream_assoc{cfg->max_cosine_distance, cfg->max_iou_distance, cfg->max_age,
+                                                         cfg->n_init}));
   const size_t ST = static_cast<size_t>(d.S) * d.T;
   int rc = 0;
   rc |= dev_alloc(t, &d.mean, ST * 8);  rc |= dev_alloc(t, &d.cov, ST * 16);
@@ -1160,6 +1198,9 @@ int aicam_tracker_create(const aicam_tracker_config* cfg, aicam_tracker** out) {
   rc |= dev_alloc(t, &d.order, ST);     rc |= dev_alloc(t, &d.free_slots, ST);
   rc |= dev_alloc(t, &d.n_tracks, d.S); rc |= dev_alloc(t, &d.n_free, d.S); rc |= dev_alloc(t, &d.next_id, d.S);
   rc |= dev_alloc(t, &d.overflow, d.S);
+  rc |= dev_alloc(t, &t->assoc_dev, d.S); d.assoc = t->assoc_dev;
+  rc |= dev_alloc(t, &d.trk_n_init, ST); rc |= dev_alloc(t, &d.trk_max_age, ST);
+  if (t->staging.create(d.S * sizeof(AssocRec)) != cudaSuccess) rc |= 1;
   rc |= dev_alloc(t, &d.app_cost, ST * d.D); rc |= dev_alloc(t, &d.cost_ws, ST * d.D);
   rc |= dev_alloc(t, &d.featn, static_cast<size_t>(d.S) * d.D * d.F);
   d.gal_hi = d.gal_lo = d.featn_hi = d.featn_lo = nullptr;
@@ -1185,6 +1226,7 @@ int aicam_tracker_create(const aicam_tracker_config* cfg, aicam_tracker** out) {
   //  different sizes - or on different GPUs - never lower each other's limit)
   if (getenv("AICAM_ASSOC_TRACE")) { if (dev_alloc(t, &t->trace, 16)) { aicam_tracker_destroy(t); return AICAM_ERR_CUDA; } }
   if (int r2 = aicam_tracker_reset(t, nullptr)) { aicam_tracker_destroy(t); return r2; }
+  if (int r2 = upload_assoc(t, nullptr)) { aicam_tracker_destroy(t); return r2; }
   AICAM_CUDA_OK(cudaDeviceSynchronize());
   *out = t;
   return AICAM_OK;
@@ -1201,6 +1243,7 @@ void aicam_tracker_destroy(aicam_tracker* t) {
               "output %lld total %lld | tracks %lld dets %lld | lsap: %lld cycles in %lld solves (sum rows*1024+cols %lld)\n",
               h[1] - h[0], h[2] - h[1], h[3] - h[2], h[4] - h[3], h[5] - h[4], h[6] - h[5], h[6] - h[0], h[8], h[9], h[10], h[11], h[12]);
   }
+  t->staging.destroy();
   for (void* p : t->allocs) cudaFree(p);
   if (t->tf) appearance_tf32_destroy(t->tf);
   delete t;
@@ -1218,6 +1261,23 @@ int aicam_tracker_reset_streams(aicam_tracker* t, const int32_t* mask, void* str
   reset_kernel<<<t->d.S, 128, 0, static_cast<cudaStream_t>(stream)>>>(t->d, mask);
   count_launch();
   return last_launch("reset_kernel (masked)");
+}
+
+int aicam_tracker_set_stream_assoc(aicam_tracker* t, const int32_t* indices_host, const aicam_stream_assoc* host, int n,
+                                   void* stream) {
+  if (!t || n < 0 || (n > 0 && (!indices_host || !host)))
+    return fail(AICAM_ERR_INVALID_ARG, "tracker_set_stream_assoc: null argument or negative count");
+  std::vector<AssocRec> next = t->assoc;  // validated as a whole before anything is stored or copied
+  for (int i = 0; i < n; ++i) {
+    const std::string at = "tracker_set_stream_assoc: entry " + std::to_string(i) + ": ";
+    if (indices_host[i] < 0 || indices_host[i] >= t->d.S) return fail(AICAM_ERR_INVALID_ARG, at + "stream index out of range");
+    if (int rc = check_assoc(host[i], at)) return rc;
+    next[indices_host[i]] = resolve_assoc(host[i]);
+  }
+  if (n == 0) return AICAM_OK;
+  AICAM_CUDA_OK(cudaSetDevice(t->cfg.device));
+  t->assoc.swap(next);
+  return upload_assoc(t, static_cast<cudaStream_t>(stream));
 }
 
 int aicam_tracker_step(aicam_tracker* t, const float* boxes, const float* scores, const int32_t* labels, int stride_k,

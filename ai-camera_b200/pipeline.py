@@ -8,12 +8,94 @@ buffers.  ``YOLODetector`` / ``DeepSORT`` (the reference-shaped facades) are thi
 wrappers around ``BatchDetector`` / ``BatchTracker``.
 """
 import ctypes as C
-from typing import Optional, Sequence, Tuple, Union
+import math
+from dataclasses import dataclass, fields
+from typing import FrozenSet, Optional, Sequence, Tuple, Union
 
 import torch
 
 from . import _lib, config
 from .trt_engine import TRTEngine
+
+
+def resolve_thresholds(conf_threshold, min_detection_confidence=None):
+    """(NMS score threshold, minimum detection confidence) of a detector confidence threshold, as one reference process
+    applies them: the engine's NMS keeps scores >= min(conf, YOLO_CONF_THRESHOLD) (yolo_detector.py:131 then drops those
+    below conf), and DeepSORT drops those below its own minimum (deepsort_tracker.py:88-95), on the device one comparison
+    whose default is therefore max(DEEPSORT_MIN_CONFIDENCE, conf)."""
+    score = min(conf_threshold, config.YOLO_CONF_THRESHOLD)
+    if min_detection_confidence is None:
+        min_detection_confidence = max(config.DEEPSORT_MIN_CONFIDENCE, conf_threshold)
+    return score, min_detection_confidence
+
+
+@dataclass(frozen=True)
+class StreamSettings:
+    """One stream's detection and tracking settings: what a reference process takes as constructor arguments
+    (``YOLODetector(conf_threshold, nms_threshold)``, ``DeepSORT(max_cosine_distance, max_iou_distance, max_age, n_init,
+    min_detection_confidence)``) and the class names it tracks.  ``min_detection_confidence`` None resolves as
+    ``resolve_thresholds`` does."""
+    conf_threshold: float = config.YOLO_CONF_THRESHOLD
+    nms_threshold: float = config.YOLO_NMS_THRESHOLD
+    classes_to_track: FrozenSet[str] = frozenset(config.CLASSES_TO_TRACK)
+    min_detection_confidence: Optional[float] = None
+    max_cosine_distance: float = config.DEEPSORT_MAX_DIST
+    max_iou_distance: float = config.DEEPSORT_MAX_IOU_DISTANCE
+    max_age: int = config.DEEPSORT_MAX_AGE
+    n_init: int = config.DEEPSORT_N_INIT
+
+    def __post_init__(self):
+        if isinstance(self.classes_to_track, str):
+            raise ValueError("classes_to_track is a set of class names, not one string")
+        classes = frozenset(self.classes_to_track)
+        unknown = classes - set(config.CLASSES)
+        if unknown:
+            raise ValueError("unknown class names: %s" % sorted(unknown))
+        object.__setattr__(self, "classes_to_track", classes)
+        for name in ("conf_threshold", "nms_threshold", "min_detection_confidence"):
+            v = getattr(self, name)
+            if v is not None and not (isinstance(v, (int, float)) and 0.0 <= v <= 1.0):
+                raise ValueError("%s must be a number in [0, 1], got %r" % (name, v))
+        for name in ("max_cosine_distance", "max_iou_distance"):
+            v = getattr(self, name)
+            if not (isinstance(v, (int, float)) and math.isfinite(v) and v >= 0):
+                raise ValueError("%s must be finite and non-negative, got %r" % (name, v))
+        if not (isinstance(self.max_age, int) and 1 <= self.max_age <= 255):
+            raise ValueError("max_age must be an integer in 1..255, got %r" % (self.max_age,))
+        if not (isinstance(self.n_init, int) and self.n_init >= 1):
+            raise ValueError("n_init must be an integer >= 1, got %r" % (self.n_init,))
+
+    @classmethod
+    def from_dict(cls, d, base: Optional["StreamSettings"] = None):
+        """Settings from a dict of field names (e.g. a JSON object), over ``base`` (default: the config defaults)."""
+        names = {f.name for f in fields(cls)}
+        unknown = set(d) - names
+        if unknown:
+            raise ValueError("unknown stream settings: %s" % sorted(unknown))
+        kw = {f.name: getattr(base or cls(), f.name) for f in fields(cls)}
+        kw.update(d)
+        return cls(**kw)
+
+    def resolve(self):
+        """(aicam_stream_filter, aicam_stream_assoc) of these settings."""
+        score, min_conf = resolve_thresholds(self.conf_threshold, self.min_detection_confidence)
+        lo, hi = config.tracked_class_mask(self.classes_to_track)
+        return (_lib.StreamFilter(score, self.nms_threshold, min_conf, 0, lo, hi),
+                _lib.StreamAssoc(float(self.max_cosine_distance), float(self.max_iou_distance), self.max_age, self.n_init))
+
+
+def _filter_key(f):
+    return (f.score_thr, f.iou_thr, f.min_confidence, f.class_mask_lo, f.class_mask_hi)
+
+
+def _as_settings_list(indices, settings):
+    indices = [int(i) for i in indices]
+    if isinstance(settings, StreamSettings):
+        settings = [settings] * len(indices)
+    settings = list(settings)
+    if len(settings) != len(indices) or not all(isinstance(s, StreamSettings) for s in settings):
+        raise ValueError("configure_streams: one StreamSettings per index")
+    return indices, settings
 
 
 def frame_geometry(frames: torch.Tensor):
@@ -53,6 +135,16 @@ class FrameTable:
         self.n_present = 0
         self.frames = []
         self.present_ptr = C.c_void_p(self.lib.aicam_frame_table_present(self._h))
+        self.filters = None
+
+    def set_filters(self, filters: Optional[Sequence["_lib.StreamFilter"]]):
+        """Per-entry detection and filter settings (aicam_frame_table_set_filters): entry i < len(filters) is detected
+        and filtered with filters[i] from the next ``set`` on; None clears them (every entry uses the entry points'
+        arguments again)."""
+        n = len(filters) if filters else 0
+        arr = (_lib.StreamFilter * n)(*filters) if n else None
+        _lib.check(self.lib.aicam_frame_table_set_filters(self._h, arr, n))
+        self.filters = list(filters) if n else None
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -111,7 +203,7 @@ class BatchDetector:
         self.max_frame_hw = tuple(max_frame_hw)
         self.frame_table = None  # created on the first list of frames
         self.engine = TRTEngine(engine_path, device, max_batch=batch, topk=topk,
-                                score_threshold=min(conf_threshold, config.YOLO_CONF_THRESHOLD),
+                                score_threshold=resolve_thresholds(conf_threshold)[0],
                                 nms_threshold=nms_threshold, max_candidates=max_candidates)
         if self.engine.kind != _lib.KIND_YOLOV8:
             raise RuntimeError("BatchDetector needs a yolov8 weight blob")
@@ -188,7 +280,7 @@ class BatchTracker:
                  max_cosine_distance=config.DEEPSORT_MAX_DIST, nn_budget=config.DEEPSORT_NN_BUDGET,
                  max_iou_distance=config.DEEPSORT_MAX_IOU_DISTANCE, max_age=config.DEEPSORT_MAX_AGE,
                  n_init=config.DEEPSORT_N_INIT, min_detection_confidence=config.DEEPSORT_MIN_CONFIDENCE,
-                 max_frame_hw=(2160, 3840)):
+                 max_frame_hw=(2160, 3840), classes_to_track=config.CLASSES_TO_TRACK):
         self.max_frame_hw = tuple(max_frame_hw)
         self.frame_table = None  # created on the first list of frames
         self.max_crops = int(max_crops if max_crops is not None else min(n_streams * max_dets, 4096))
@@ -201,6 +293,9 @@ class BatchTracker:
         self.device = dev = self.reid.device
         self.S, self.K, self.T = n_streams, max_dets, max_tracks
         self.min_conf = float(min_detection_confidence)
+        self.classes_to_track = frozenset(classes_to_track)
+        self.assoc_defaults = dict(max_cosine_distance=float(max_cosine_distance), max_iou_distance=float(max_iou_distance),
+                                   max_age=int(max_age), n_init=int(n_init))
         self.F = self.reid.feature_dim
         cfg = _lib.TrackerConfig(n_streams, max_tracks, max_dets, self.F, float(max_cosine_distance),
                                  float(max_iou_distance), int(max_age), int(n_init), int(nn_budget), dev.index)
@@ -223,7 +318,11 @@ class BatchTracker:
         self.out_conf = torch.zeros((S, max_tracks), dtype=torch.float32, device=dev)
         self.out_count = torch.zeros(S, **i32)
         self._reset_mask = torch.zeros(S, **i32)
-        self._mask = config.tracked_class_mask()
+        self._mask = config.tracked_class_mask(self.classes_to_track)
+        # per-stream confidence and class mask of configure_streams (None: every stream uses the constructor's); a list
+        # step hands them to the frame table, a stacked step whose streams differ goes through the table
+        self._filters = None
+        self._routed = False
         # optional running totals (crops, reported tracks) kept on the device, for benchmarks: no host sync
         self.count_stats = False
         self.crop_total = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -251,15 +350,39 @@ class BatchTracker:
             self._reset_mask.copy_(mask)
             _lib.check(self.lib.aicam_tracker_reset_streams(self._h, _lib.ptr(self._reset_mask), _lib.stream_ptr(self.device)))
 
+    def configure_streams(self, indices, settings):
+        """Give the streams ``indices`` their own association settings (max_cosine_distance, max_iou_distance, max_age,
+        n_init) and crop filter (minimum confidence, tracked classes), from the next step on.  The other streams, and
+        the tracks of these, are untouched; a track keeps the n_init and max_age it was created with, as in the
+        reference.  ``settings``: one StreamSettings per index, or one for all."""
+        indices, settings = _as_settings_list(indices, settings)
+        resolved = [s.resolve() for s in settings]
+        assoc = (_lib.StreamAssoc * len(indices))(*[a for _, a in resolved])
+        idx = (C.c_int32 * len(indices))(*indices)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_tracker_set_stream_assoc(self._h, idx, assoc, len(indices), _lib.stream_ptr(self.device)))
+        base = _lib.StreamFilter(0.0, 0.0, self.min_conf, 0, self._mask[0], self._mask[1])
+        filters = self._filters or [base] * self.S
+        for i, (f, _) in zip(indices, resolved):
+            filters[i] = f
+        self._filters = filters
+        key = _filter_key(base)[2:]
+        self._routed = any(_filter_key(f)[2:] != key for f in filters)
+
     def update(self, frames, num_dets, boxes, scores, labels):
         """One frame per stream.  frames uint8 cuda [S,H,W,3] BGR or [S,H*3/2,W] NV12, or a list of S frames of any
         sizes and kinds, None for a stream that has no frame this step (see BatchDetector.detect: its state is left as it
         is and its out_count is 0); detections as BatchDetector
         returns them ([S], [S,K,4], [S,K], [S,K]).  Returns device (out_tracks [S,T,6] int32 =
         x1,y1,x2,y2,id,class, out_conf [S,T], out_count [S]); asynchronous."""
+        if not is_frame_list(frames) and self._routed:
+            frame_geometry(frames)
+            frames = list(frames.unbind(0))  # streams filter differently: one table entry per stream
         if is_frame_list(frames):
             if self.frame_table is None:
                 self.frame_table = FrameTable(self.device, self.S, self.max_frame_hw)
+            if self._filters is not None:
+                self.frame_table.set_filters(self._filters)
             self.frame_table.set(frames)
             return self.update_table(self.frame_table, num_dets, boxes, scores, labels)
         S, h, w, nv12 = frame_geometry(frames)
@@ -335,20 +458,51 @@ class TrackingPipeline:
 
     def __init__(self, yolo_engine_path, reid_engine_path, n_streams: int, device=None, max_tracks: int = 256,
                  max_crops: Optional[int] = None, conf_threshold=config.YOLO_CONF_THRESHOLD, topk=config.YOLO_TOPK,
-                 max_candidates=config.YOLO_MAX_CANDIDATES, max_frame_hw=(2160, 3840), **tracker_kw):
-        self.detector = BatchDetector(yolo_engine_path, n_streams, device, conf_threshold=conf_threshold, topk=topk,
-                                      max_candidates=max_candidates, max_frame_hw=max_frame_hw)
+                 max_candidates=config.YOLO_MAX_CANDIDATES, max_frame_hw=(2160, 3840),
+                 nms_threshold=config.YOLO_NMS_THRESHOLD, stream_settings: Optional[Sequence[StreamSettings]] = None,
+                 **tracker_kw):
+        self.detector = BatchDetector(yolo_engine_path, n_streams, device, conf_threshold=conf_threshold,
+                                      nms_threshold=nms_threshold, topk=topk, max_candidates=max_candidates,
+                                      max_frame_hw=max_frame_hw)
         # detect() drops detections below conf_threshold before update() sees them (yolo_detector.py:131); on the
         # device that filter and DeepSORT's own (deepsort_tracker.py:88-95) are one comparison
-        tracker_kw.setdefault("min_detection_confidence", max(config.DEEPSORT_MIN_CONFIDENCE, conf_threshold))
+        tracker_kw["min_detection_confidence"] = resolve_thresholds(conf_threshold,
+                                                                    tracker_kw.get("min_detection_confidence"))[1]
         self.tracker = BatchTracker(reid_engine_path, n_streams, self.detector.device, max_dets=self.detector.topk,
                                     max_tracks=max_tracks, max_crops=max_crops, **tracker_kw)
         self.device = self.detector.device
         self.n_streams = n_streams
         # the frames of a list step: set once, read by the detector and the tracker
         self.frame_table = FrameTable(self.device, n_streams, max_frame_hw)
+        # the settings the constructor's arguments amount to, and each stream's current ones
+        self.default_settings = StreamSettings(conf_threshold, nms_threshold, self.tracker.classes_to_track,
+                                               self.tracker.min_conf, **self.tracker.assoc_defaults)
+        self.settings = [self.default_settings] * n_streams
+        self._routed = False  # some stream detects or filters differently: stacked steps go through the frame table
+        if stream_settings is not None:
+            self.configure_streams(range(n_streams), stream_settings)
+
+    def configure_streams(self, indices, settings):
+        """Give the streams ``indices`` their own StreamSettings (one per index, or one for all) from the next step on,
+        with or without a reset, whether the step runs eager or from a captured graph (call it between replays, like
+        ``frame_table.set``).  The other streams are untouched; a stream's existing tracks keep the n_init and max_age
+        they were created with, as in the reference."""
+        indices, settings = _as_settings_list(indices, settings)
+        for i in indices:
+            if not 0 <= i < self.n_streams:
+                raise _lib.AicamError(-1, "configure_streams: stream %d out of range" % i)
+        self.tracker.configure_streams(indices, settings)
+        for i, st in zip(indices, settings):
+            self.settings[i] = st
+        filters = [st.resolve()[0] for st in self.settings]
+        self.frame_table.set_filters(filters)
+        base = _filter_key(self.default_settings.resolve()[0])
+        self._routed = any(_filter_key(f) != base for f in filters)
 
     def step(self, frames: Union[torch.Tensor, Sequence[torch.Tensor]]) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        if not is_frame_list(frames) and self._routed:
+            frame_geometry(frames)
+            frames = list(frames.unbind(0))  # streams detect or filter differently: one table entry per stream
         if is_frame_list(frames):
             self.frame_table.set(frames)
             return self.step_table()
@@ -362,12 +516,14 @@ class TrackingPipeline:
         num, boxes, scores, labels = self.detector.detect_table(self.frame_table)
         return self.tracker.update_table(self.frame_table, num, boxes, scores, labels)
 
-    def reset_streams(self, indices):
+    def reset_streams(self, indices, settings=None):
         """Hand the given stream slots to new sources: their trackers restart (no tracks, ids from 1), the other streams
-        and the captured step are untouched."""
+        and the captured step are untouched.  The slots keep their settings, or take ``settings`` (as configure_streams)."""
+        if settings is not None:
+            self.configure_streams(indices, settings)
         self.tracker.reset_streams(indices)
 
     def launches_per_step(self, frame_list=False):
         """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True), absent frames
-        or not."""
-        return self.detector.launches_per_step(frame_list) + self.tracker.launches_per_step()
+        or not.  A stacked tensor runs as a list while streams detect or filter differently."""
+        return self.detector.launches_per_step(frame_list or self._routed) + self.tracker.launches_per_step()

@@ -262,6 +262,24 @@ int aicam_frame_table_set(aicam_frame_table* t, const aicam_frame_desc* host_des
 int aicam_frame_table_set_present(aicam_frame_table* t, const aicam_frame_desc* host_descs, const uint8_t* present_host, int n,
                                   void* stream);
 const int32_t* aicam_frame_table_present(const aicam_frame_table* t);
+/* Per-stream detection and filter settings: a camera fleet mixes scenes that want different thresholds and tracked
+ * classes (a parking camera tracks vehicles, a corridor camera people; a far-field camera needs a lower confidence
+ * threshold), so each table entry may carry its own:
+ *   score_thr, iou_thr   : aicam_yolo_detect_table's NMS score and IoU thresholds (aicam_nms_params) for the entry
+ *   min_confidence       : aicam_reid_crops_table's confidence filter for the entry
+ *   class_mask_lo / hi   : its class mask (bit c = COCO class c is tracked)
+ * aicam_frame_table_set_filters (host only, launches nothing) stores host[0 .. n) in the table; every following
+ * aicam_frame_table_set[_present] resolves entry i < n into its device record, in that set's single copy, so the settings
+ * take effect with the next set and a captured step follows them.  Entries at or beyond n, and every entry after a call
+ * with host == NULL or n == 0 (which clears the settings), use the arguments passed to the entry points, as before.
+ * Entry i's results then equal the uniform entry points (batch 1) called with its settings.  AICAM_ERR_CAPACITY when
+ * n > capacity; AICAM_ERR_INVALID_ARG for a threshold that is not finite or not in [0, 1]; on an error nothing is stored. */
+typedef struct {
+  float score_thr, iou_thr, min_confidence;
+  int reserved;
+  uint64_t class_mask_lo, class_mask_hi;
+} aicam_stream_filter;
+int aicam_frame_table_set_filters(aicam_frame_table* t, const aicam_stream_filter* host, int n);
 /* aicam_preprocess / aicam_preprocess_nv12 over a frame table (formats 0-3): present frame i's slice of `out` is slice p(i)
  * (packed, see above; slice i when all frames are present) and equals the uniform entry on that frame alone; slices past
  * the present count are not written.  Frames whose geometry is a pure decimation (1080p) and whose planes, pitch and row
@@ -386,6 +404,21 @@ int aicam_tracker_reset(aicam_tracker* t, void* stream);
  * tracker's stream is (no tracks, ids from 1, no overflow flags); every other stream is untouched.  One kernel launch,
  * capturable, so a slot can be handed to another camera or clip while the other streams keep their tracks. */
 int aicam_tracker_reset_streams(aicam_tracker* t, const int32_t* mask, void* stream);
+/* Per-stream association settings (DeepSORT's max_cosine_distance, max_iou_distance, max_age, n_init; the doubles are
+ * kept for the reason given in aicam_tracker_config).  aicam_tracker_create gives every stream the values of its config;
+ * aicam_tracker_set_stream_assoc gives stream indices_host[i] the values host[i] (i < n, host arrays) and copies the
+ * stream table to the device with one asynchronous copy on `stream` from pinned staging.  Not capturable; captured steps
+ * read the table, so they follow its changes from the next step on.  As in the reference, where these are attributes of
+ * one process's tracker: the cascade depth is the stream's current max_age, while each track keeps the n_init and
+ * max_age that applied when it was created, for its confirmation and its deletion.  A reset keeps the settings.
+ * AICAM_ERR_INVALID_ARG (nothing copied) for max_age outside 1..255, n_init < 1, a distance that is negative or not
+ * finite, or an index outside 0..n_streams-1. */
+typedef struct {
+  double max_cosine_distance, max_iou_distance;
+  int max_age, n_init;
+} aicam_stream_assoc;
+int aicam_tracker_set_stream_assoc(aicam_tracker* t, const int32_t* indices_host, const aicam_stream_assoc* host, int n,
+                                   void* stream);
 
 /* One frame for every stream: predict, cascade + IoU matching, update, initiate, prune,
  * format.  Inputs describe, per stream b, the detections of the frame (as returned by
