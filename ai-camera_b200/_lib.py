@@ -25,17 +25,6 @@ class ConvDesc(C.Structure):
                                        "res_mode", "out_f32")]
 
 
-class ChainStage(C.Structure):
-    _fields_ = [("cin", C.c_int), ("cout", C.c_int), ("ksize", C.c_int), ("act", C.c_int), ("nsrc", C.c_int),
-                ("src_buf", C.c_int * 2), ("src_coff", C.c_int * 2), ("src_c", C.c_int * 2),
-                ("res_buf", C.c_int), ("res_coff", C.c_int), ("res_mode", C.c_int)]
-
-
-class ChainDesc(C.Structure):
-    _fields_ = [("batch", C.c_int), ("h", C.c_int), ("w", C.c_int), ("in_c", C.c_int), ("nstages", C.c_int),
-                ("st", ChainStage * 5), ("out_f32", C.c_int)]
-
-
 class Letterbox(C.Structure):
     _fields_ = [("ratio", C.c_double), ("pad_w", C.c_double), ("pad_h", C.c_double)]
 
@@ -109,8 +98,6 @@ SIGNATURES = {
     "aicam_nchw_to_nhwc4": (_I, [_P, _I, _I, _I, _P, _P]),
     "aicam_conv2d": (_I, [C.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P]),
     "aicam_conv2d_padded": (_I, [C.POINTER(ConvDesc), _P, _P, _P, _P, _P, _I, _I, _P]),
-    "aicam_conv_chain": (_I, [C.POINTER(ChainDesc), _P, C.POINTER(_P), C.POINTER(_P), _P, _P]),
-    "aicam_conv_chain_bench": (_I, [C.POINTER(ChainDesc), _I, C.POINTER(C.c_double), _P]),
     "aicam_conv2d_bench": (_I, [C.POINTER(ConvDesc), _I, C.POINTER(C.c_double), _P]),
     "aicam_reid_stem_pool": (_I, [_P, _I, _I, _I, _P, _P, _P, _P]),
     "aicam_letterbox_params": (_I, [_I, _I, C.POINTER(Letterbox)]),

@@ -64,7 +64,6 @@ bool profile_begin(cudaStream_t st, size_t* slot) {
   cudaEventRecord(g_events[*slot].first, st);
   return true;
 }
-bool profile_enabled() { return g_profile; }
 
 // Step timeline (debug): while enabled, every conv_win launch is handed the next 4-slot record of a device buffer and
 // its CTA 0 stamps %globaltimer there at entry, when its dependency on the previous kernel has resolved, and at exit;

@@ -561,15 +561,13 @@ int pack_pair_weights(PackedConv* pc) {
 // Returns 1 when launched on the pair kernel, 0 when the layer is not eligible, negative on error.
 int try_launch_conv_pair(const PackedConv& pc, const ConvLaunch& L, cudaStream_t stream) {
   static const bool enabled = getenv("AICAM_NO_PAIR") == nullptr;
-  static const int force_mt = getenv("AICAM_PAIR_MT") ? atoi(getenv("AICAM_PAIR_MT")) : 0;
   if (!enabled || !pc.w_pair || !L.in_pad || !L.out_pad || L.out_f32 || L.out_s2d || encode_tiled_fn() == nullptr) return 0;
   const int cout_pad = (pc.cout + 15) / 16 * 16;
   // Measured on B200 (1024 crops, same box, conv_win.cu mode 4 -> pairs): 128 channels 146 -> 135 us; 64 channels
   // 203 -> 190..224 us (the epilogue's shared-memory traffic competes with an operand fetch that now keeps the port 95 %
   // busy); 256 / 512 channels 148 -> 158 us and 197 -> 198 us (the 256-column single-CTA tile is already tensor-bound).
-  // So the 128- and 512-channel layers run on pairs by default; AICAM_PAIR_ALL=1 sends every eligible layer here.
-  static const bool pair_all = getenv("AICAM_PAIR_ALL") != nullptr;
-  if (cout_pad != 128 && cout_pad != 512 && !pair_all) return 0;  // (512 channels: 204 -> 195 us with the deeper weight ring)
+  // So only the 128- and 512-channel layers run on pairs.
+  if (cout_pad != 128 && cout_pad != 512) return 0;  // (512 channels: 204 -> 195 us with the deeper weight ring)
   const int n_tile = std::min(cout_pad, 256), n_half = n_tile / 2, n_tiles = cout_pad / n_tile;
   const int tps = n_tile == 256 ? 1 : 3;
   const int res_mode = L.res ? L.res_mode : 0;
@@ -590,7 +588,6 @@ int try_launch_conv_pair(const PackedConv& pc, const ConvLaunch& L, cudaStream_t
   // tiling: MT accumulators per CTA; staging = the TMA-epilogue tile (residual finished in place)
   int best_mt = 0, best_sa = 0, best_sb = 0, best_nstage = 0, best_bh = 0;
   for (int mt = 2; mt >= 1; --mt) {
-    if (force_mt && mt != force_mt) continue;
     if (2 * mt * n_tile > 512) continue;
     const int tm = 128 * mt;
     const int bh = ((tm + 2 * wp + 2 + mt - 1) / mt + 7) / 8 * 8;

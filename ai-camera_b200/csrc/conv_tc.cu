@@ -26,8 +26,6 @@
 // epilogue overlaps another's main loop); the tile count may come from a device-side batch count.
 #include "conv_tc.cuh"
 
-#include <cuda.h>
-
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -73,9 +71,6 @@ struct ConvKernelArgs {
   uint32_t tmem_cols;
   const int* batch_dev;  // optional: images actually present (device), m_total is the capacity
   int staged;            // 1: epilogue goes through the coalescing shared-memory staging path
-  int tma;               // 1: A tiles come from TMA im2col loads (one instruction per 128-pixel slab)
-  int slab;              // channels per TMA load: 16 / 32 / 64 (32 / 64 / 128-byte swizzled rows)
-  int slabs_per_tap, sub_per_kb, n_sub_total;
   int out_dense, res_dense;  // 1: pixel address = m * cstride (images are contiguous in the buffer)
   int res_stage_off;     // byte offset of the residual staging area in shared memory (0: none)
   long long* trace;      // optional debug buffer: clock64 stamps of CTA 0 (conv2d_bench with AICAM_CONV_TRACE)
@@ -136,16 +131,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                "l"(src), "r"(bytes), "r"(bar)
                : "memory");
 }
-// 4-D im2col TMA load: [c, w, h, n] base coordinates + filter offsets (s, r); writes
-// pixelsPerColumn rows of channelsPerPixel elements, swizzled, and completes tx bytes on `bar`.
-__device__ __forceinline__ void tma_im2col_4d(uint32_t dst, const CUtensorMap* tmap, uint32_t bar, int c, int w, int h,
-                                              int n, uint16_t off_w, uint16_t off_h) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.im2col.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h)
-      : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_commit(uint32_t bar) {
@@ -171,10 +156,8 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[16]) {
 }
 
 // K-major: start >> 4 | LBO >> 4 (bits 16..29) | SBO >> 4 (bits 32..45) | version 1 (bit 46)
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes,
-                                                   uint32_t layout_type = 0) {
-  uint64_t d = static_cast<uint64_t>(layout_type & 7u) << 61;  // 0 none, 2 SWIZZLE_128B, 4 SWIZZLE_64B, 6 SWIZZLE_32B
-  d |= static_cast<uint64_t>((addr >> 4) & 0x3FFF);
+__device__ __forceinline__ uint64_t make_smem_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
+  uint64_t d = static_cast<uint64_t>((addr >> 4) & 0x3FFF);
   d |= static_cast<uint64_t>((lbo_bytes >> 4) & 0x3FFF) << 16;
   d |= static_cast<uint64_t>((sbo_bytes >> 4) & 0x3FFF) << 32;
   d |= 1ull << 46;
@@ -187,20 +170,17 @@ __device__ __forceinline__ float apply_act(float x, int act) {
   return x;
 }
 
-__global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKernelArgs a,
-                                                                       const __grid_constant__ CUtensorMap tmap) {
+__global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKernelArgs a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t smem_base = smem_u32(smem);
   const uint32_t bar_full = smem_base;            // STAGES x 8 B
   const uint32_t bar_empty = smem_base + 64;      // STAGES x 8 B
   const uint32_t bar_tmem_full = smem_base + 128;
   const uint32_t bar_tmem_empty = smem_base + 136;
-  const uint32_t bar_stage_free = smem_base + 144;  // TMA mode: epilogue staging (aliases the A stages) is free
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(smem + 160);
   const uint32_t smem_a = smem_base + SMEM_HEADER;
   const uint32_t b_stage_bytes = static_cast<uint32_t>(a.n_tile) * 16u * CHUNKS_PER_STAGE;
-  const uint32_t a_stage_bytes = a.tma ? TILE_M * 128u : A_STAGE_BYTES;  // TMA stages are 1024-byte aligned
-  const uint32_t smem_b = smem_a + STAGES * a_stage_bytes;
+  const uint32_t smem_b = smem_a + STAGES * A_STAGE_BYTES;
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -213,13 +193,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKerne
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) {
-      // gather mode: 128 gather threads + the weight loader's expect_tx; TMA mode: the loader alone
-      mbar_init(bar_full + 8 * s, a.tma ? 1 : TILE_M + 1);
+      mbar_init(bar_full + 8 * s, TILE_M + 1);  // 128 gather threads + the weight loader's expect_tx
       mbar_init(bar_empty + 8 * s, 1);          // one tcgen05.commit
     }
     mbar_init(bar_tmem_full, 1);
     mbar_init(bar_tmem_empty, TILE_M);          // the 128 epilogue threads
-    mbar_init(bar_stage_free, TILE_M);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 4) {
@@ -264,85 +242,81 @@ __global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKerne
       // warp read the 8 consecutive 16-byte channel chunks of ONE pixel (one 128-byte line).
       // Per row: a byte pointer to tap (0,0) and a 9-bit mask of the taps that are inside the
       // image, so that one copy costs an add, a bit test and two selects.
-      if (!a.tma) {
-        const uint8_t* rowptr[8];
-        uint32_t tmask[8];
-        {
-          int m = m0 + r0;
-          int n_img = m / a.howo;
-          int rem = m - n_img * a.howo;
-          int oy = rem / a.wo;
-          int ox = rem - oy * a.wo;
+      const uint8_t* rowptr[8];
+      uint32_t tmask[8];
+      {
+        int m = m0 + r0;
+        int n_img = m / a.howo;
+        int rem = m - n_img * a.howo;
+        int oy = rem / a.wo;
+        int ox = rem - oy * a.wo;
   #pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int iy0 = oy * a.stride - a.pad, ix0 = ox * a.stride - a.pad;
-            // taps inside the image: 3-bit column mask replicated into the valid filter rows
-            uint32_t mk = 0;
-            if (m < m_total) {
-              uint32_t xm = 0;
+        for (int i = 0; i < 8; ++i) {
+          const int iy0 = oy * a.stride - a.pad, ix0 = ox * a.stride - a.pad;
+          // taps inside the image: 3-bit column mask replicated into the valid filter rows
+          uint32_t mk = 0;
+          if (m < m_total) {
+            uint32_t xm = 0;
   #pragma unroll
-              for (int tc = 0; tc < 3; ++tc)
-                if (tc < a.ksize && static_cast<unsigned>(ix0 + tc) < static_cast<unsigned>(a.w)) xm |= 1u << tc;
+            for (int tc = 0; tc < 3; ++tc)
+              if (tc < a.ksize && static_cast<unsigned>(ix0 + tc) < static_cast<unsigned>(a.w)) xm |= 1u << tc;
   #pragma unroll
-              for (int tr = 0; tr < 3; ++tr)
-                if (tr < a.ksize && static_cast<unsigned>(iy0 + tr) < static_cast<unsigned>(a.h)) mk |= xm << (tr * a.ksize);
-            }
-            tmask[i] = mk;
-            rowptr[i] = reinterpret_cast<const uint8_t*>(a.in + a.in_coff) +
-                        (static_cast<long long>(n_img) * a.h * a.w + static_cast<long long>(iy0) * a.w + ix0) * cs_bytes;
-            // advance 16 output pixels
-            m += 16;
-            ox += 16;
-            while (ox >= a.wo) { ox -= a.wo; if (++oy == a.ho) { oy = 0; ++n_img; } }
+            for (int tr = 0; tr < 3; ++tr)
+              if (tr < a.ksize && static_cast<unsigned>(iy0 + tr) < static_cast<unsigned>(a.h)) mk |= xm << (tr * a.ksize);
           }
+          tmask[i] = mk;
+          rowptr[i] = reinterpret_cast<const uint8_t*>(a.in + a.in_coff) +
+                      (static_cast<long long>(n_img) * a.h * a.w + static_cast<long long>(iy0) * a.w + ix0) * cs_bytes;
+          // advance 16 output pixels
+          m += 16;
+          ox += 16;
+          while (ox >= a.wo) { ox -= a.wo; if (++oy == a.ho) { oy = 0; ++n_img; } }
         }
-        // running position of chunk q = kb * 8 + j in (tap, channel chunk) space
-        int tap = 0, tr = 0, tc = 0, c8 = 0;
-        if (!a.stem) {
-          c8 = j;
-          while (c8 >= a.cin_chunks) { c8 -= a.cin_chunks; ++tap; if (++tc == a.ksize) { tc = 0; ++tr; } }
-        }
-        for (int kb = 0; kb < num_kb; ++kb, ++g_kb) {
-          const int s = g_kb % STAGES;
-          const int it = g_kb / STAGES;
-          mbar_wait(bar_empty + 8 * s, (it & 1) ^ 1);
-          if (a.trace && blockIdx.x == 0 && threadIdx.x == 0 && g_kb < 60) a.trace[g_kb * 4 + 0] = clock64();
-          const uint32_t dst = smem_a + s * A_STAGE_BYTES + dst_thread;
-          const int q = kb * CHUNKS_PER_STAGE + j;
-          if (q < a.q_pad) {
-            if (!a.stem) {
-              const uint32_t bit = (q < a.q) ? (1u << tap) : 0u;
-              const int delta = (tr * a.w + tc) * cs_bytes + c8 * 16;
+      }
+      // running position of chunk q = kb * 8 + j in (tap, channel chunk) space
+      int tap = 0, tr = 0, tc = 0, c8 = 0;
+      if (!a.stem) {
+        c8 = j;
+        while (c8 >= a.cin_chunks) { c8 -= a.cin_chunks; ++tap; if (++tc == a.ksize) { tc = 0; ++tr; } }
+      }
+      for (int kb = 0; kb < num_kb; ++kb, ++g_kb) {
+        const int s = g_kb % STAGES;
+        const int it = g_kb / STAGES;
+        mbar_wait(bar_empty + 8 * s, (it & 1) ^ 1);
+        if (a.trace && blockIdx.x == 0 && threadIdx.x == 0 && g_kb < 60) a.trace[g_kb * 4 + 0] = clock64();
+        const uint32_t dst = smem_a + s * A_STAGE_BYTES + dst_thread;
+        const int q = kb * CHUNKS_PER_STAGE + j;
+        if (q < a.q_pad) {
+          if (!a.stem) {
+            const uint32_t bit = (q < a.q) ? (1u << tap) : 0u;
+            const int delta = (tr * a.w + tc) * cs_bytes + c8 * 16;
+  #pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              const bool ok = (tmask[i] & bit) != 0;
+              const uint8_t* src = ok ? rowptr[i] + delta : reinterpret_cast<const uint8_t*>(a.in);
+              cp_async_16(dst + i * 256, src, ok ? 16u : 0u);
+            }
+            c8 += CHUNKS_PER_STAGE;
+            while (c8 >= a.cin_chunks) { c8 -= a.cin_chunks; ++tap; if (++tc == a.ksize) { tc = 0; ++tr; } }
+          } else {
+  #pragma unroll
+            for (int half = 0; half < 2; ++half) {
+              const int tp = 2 * q + half;
+              const int ttr = tp / 3, ttc = tp - ttr * 3;  // the stem is always 3x3
+              const uint32_t bit = (tp < a.taps) ? (1u << tp) : 0u;
+              const int delta = (ttr * a.w + ttc) * cs_bytes;
   #pragma unroll
               for (int i = 0; i < 8; ++i) {
                 const bool ok = (tmask[i] & bit) != 0;
                 const uint8_t* src = ok ? rowptr[i] + delta : reinterpret_cast<const uint8_t*>(a.in);
-                cp_async_16(dst + i * 256, src, ok ? 16u : 0u);
-              }
-              c8 += CHUNKS_PER_STAGE;
-              while (c8 >= a.cin_chunks) { c8 -= a.cin_chunks; ++tap; if (++tc == a.ksize) { tc = 0; ++tr; } }
-            } else {
-  #pragma unroll
-              for (int half = 0; half < 2; ++half) {
-                const int tp = 2 * q + half;
-                const int ttr = tp / 3, ttc = tp - ttr * 3;  // the stem is always 3x3
-                const uint32_t bit = (tp < a.taps) ? (1u << tp) : 0u;
-                const int delta = (ttr * a.w + ttc) * cs_bytes;
-  #pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                  const bool ok = (tmask[i] & bit) != 0;
-                  const uint8_t* src = ok ? rowptr[i] + delta : reinterpret_cast<const uint8_t*>(a.in);
-                  cp_async_8(dst + i * 256 + half * 8, src, ok ? 8u : 0u);
-                }
+                cp_async_8(dst + i * 256 + half * 8, src, ok ? 8u : 0u);
               }
             }
           }
-          // Arrive on the stage's full barrier when this thread's copies have landed (asynchronous).
-          cp_async_arrive_noinc(bar_full + 8 * s);
-          if (a.trace && blockIdx.x == 0 && threadIdx.x == 0 && g_kb < 60) a.trace[g_kb * 4 + 1] = clock64();
         }
-      } else {
-        g_kb += num_kb;  // TMA mode: the loader warp fills the stages
+        // Arrive on the stage's full barrier when this thread's copies have landed (asynchronous).
+        cp_async_arrive_noinc(bar_full + 8 * s);
+        if (a.trace && blockIdx.x == 0 && threadIdx.x == 0 && g_kb < 60) a.trace[g_kb * 4 + 1] = clock64();
       }
       const int ncols = min(a.n_tile, a.cout - n0);  // valid output channels of this tile
       // ---------------------------------------------------------------- epilogue
@@ -478,7 +452,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKerne
       }
       // staging rows alias the A stages, bias_s / res_stage are rewritten by the next tile
       asm volatile("bar.sync 1, 128;" ::: "memory");
-      if (a.tma) mbar_arrive(bar_stage_free);  // the loader may overwrite the A stages now
       if (a.trace && blockIdx.x == 0 && threadIdx.x == 0 && t_iter < 8) a.trace[240 + t_iter * 4 + 2] = clock64();
     }
   } else if (warp == 4) {
@@ -496,26 +469,12 @@ __global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKerne
         if (a.trace && blockIdx.x == 0 && lane == 0 && g_kb < 60) a.trace[g_kb * 4 + 2] = clock64();
         if (lane == 0) {
           const int nchunks = min(CHUNKS_PER_STAGE, a.q_pad - kb * CHUNKS_PER_STAGE);
-          const uint32_t a_stage = smem_a + s * a_stage_bytes;
+          const uint32_t a_stage = smem_a + s * A_STAGE_BYTES;
           const uint32_t b_stage = smem_b + s * b_stage_bytes;
-          if (!a.tma) {
-            for (int kk = 0; kk < nchunks / 2; ++kk) {
-              const uint64_t da = make_smem_desc(a_stage + kk * 2 * A_CHUNK_BYTES, A_CHUNK_BYTES, 128);
-              const uint64_t db = make_smem_desc(b_stage + kk * 2 * b_chunk_bytes, b_chunk_bytes, 128);
-              tc_mma_bf16(tmem_base, da, db, a.idesc, (kb | kk) != 0 ? 1u : 0u);
-            }
-          } else {
-            // A: sub-tiles of 128 rows x slab channels, rows slab*2 bytes apart, hardware swizzle
-            // (SWIZZLE_32B/64B/128B as written by the TMA), 8-row atoms SBO = 8 * row bytes
-            const uint32_t row_bytes = a.slab * 2;
-            const uint32_t ltype = a.slab == 64 ? 2u : (a.slab == 32 ? 4u : 6u);
-            const int k16_per_sub = a.slab / 16;
-            for (int kk = 0; kk < nchunks / 2; ++kk) {
-              const int u = kk / k16_per_sub, k16 = kk - u * k16_per_sub;
-              const uint64_t da = make_smem_desc(a_stage + u * (TILE_M * row_bytes) + k16 * 32, 16, 8 * row_bytes, ltype);
-              const uint64_t db = make_smem_desc(b_stage + kk * 2 * b_chunk_bytes, b_chunk_bytes, 128);
-              tc_mma_bf16(tmem_base, da, db, a.idesc, (kb | kk) != 0 ? 1u : 0u);
-            }
+          for (int kk = 0; kk < nchunks / 2; ++kk) {
+            const uint64_t da = make_smem_desc(a_stage + kk * 2 * A_CHUNK_BYTES, A_CHUNK_BYTES, 128);
+            const uint64_t db = make_smem_desc(b_stage + kk * 2 * b_chunk_bytes, b_chunk_bytes, 128);
+            tc_mma_bf16(tmem_base, da, db, a.idesc, (kb | kk) != 0 ? 1u : 0u);
           }
           tc_commit(bar_empty + 8 * s);
           if (kb == num_kb - 1) tc_commit(bar_tmem_full);
@@ -529,18 +488,9 @@ __global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKerne
     // ------------------------------------------------------------------ weight loader
     if (lane == 0) {
       const uint32_t b_chunk_bytes = static_cast<uint32_t>(a.n_tile) * 16u;
-      int g_kb = 0, lt_iter = 0;
+      int g_kb = 0;
       for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
         const int n0 = (tile % n_tiles) * a.n_tile;
-        // base pixel of the tile in im2col coordinates: (q * stride - pad, p * stride - pad, n)
-        const int m0 = (tile / n_tiles) * TILE_M;
-        const int cn = m0 / a.howo;
-        const int remp = m0 - cn * a.howo;
-        const int p0 = remp / a.wo;
-        const int cw = (remp - p0 * a.wo) * a.stride - a.pad;
-        const int chh = p0 * a.stride - a.pad;
-        if (a.tma) mbar_wait(bar_stage_free, (lt_iter & 1) ^ 1);  // previous tile's epilogue is off the A stages
-        ++lt_iter;
         for (int kb = 0; kb < num_kb; ++kb, ++g_kb) {
           const int s = g_kb % STAGES;
           const int it = g_kb / STAGES;
@@ -548,21 +498,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 3) conv_tc_kernel(const ConvKerne
           const int nchunks = min(CHUNKS_PER_STAGE, a.q_pad - kb * CHUNKS_PER_STAGE);
           const uint32_t bar = bar_full + 8 * s;
           const uint32_t dst = smem_b + s * b_stage_bytes;
-          if (!a.tma) {
-            mbar_arrive_expect_tx(bar, nchunks * b_chunk_bytes);
-          } else {
-            const int nsub = min(a.sub_per_kb, a.n_sub_total - kb * a.sub_per_kb);
-            const uint32_t sub_bytes = TILE_M * a.slab * 2;
-            mbar_arrive_expect_tx(bar, nchunks * b_chunk_bytes + nsub * sub_bytes);
-            for (int u = 0; u < nsub; ++u) {
-              const int U = kb * a.sub_per_kb + u;
-              const int tap = U / a.slabs_per_tap;
-              const int c0 = (U - tap * a.slabs_per_tap) * a.slab;
-              const int tr = tap / a.ksize, tc = tap - tr * a.ksize;
-              tma_im2col_4d(smem_a + s * a_stage_bytes + u * sub_bytes, &tmap, bar, c0, cw, chh, cn,
-                            static_cast<uint16_t>(tc), static_cast<uint16_t>(tr));
-            }
-          }
+          mbar_arrive_expect_tx(bar, nchunks * b_chunk_bytes);
           const __nv_bfloat16* src = a.wgt + (static_cast<long long>(kb) * CHUNKS_PER_STAGE * a.cout_pad + n0) * 8;
           if (a.n_tile == a.cout_pad) {
             bulk_g2s(dst, src, nchunks * b_chunk_bytes, bar);
@@ -587,25 +523,6 @@ inline uint16_t f32_to_bf16_bits(float f) {
   if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<uint16_t>((u >> 16) | 0x40);
   u += 0x7fffu + ((u >> 16) & 1u);
   return static_cast<uint16_t>(u >> 16);
-}
-
-typedef CUresult (*EncodeIm2colFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const int*, const int*, cuuint32_t, cuuint32_t, const cuuint32_t*,
-                                   CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                   CUtensorMapFloatOOBfill);
-
-EncodeIm2colFn get_encode_im2col() {
-  static EncodeIm2colFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeIm2colFn>(p);
-  }
-  return fn;
 }
 
 int pick_n_tile(int cout_pad, bool out_f32) {
@@ -782,36 +699,7 @@ int launch_conv(const PackedConv& pc, const ConvLaunch& L, cudaStream_t stream) 
     if (L.out_s2d) return fail(AICAM_ERR_UNSUPPORTED, "launch_conv: space-to-depth output needs the window kernel");
     if (L.decode) return fail(AICAM_ERR_UNSUPPORTED, "launch_conv: the fused Detect decode needs the window kernel");
   }
-  // TMA im2col path: whole 128-pixel x slab-channel tiles per instruction (all layers but the stems)
-  alignas(64) CUtensorMap tmap;
-  std::memset(&tmap, 0, sizeof(tmap));
-  a.tma = 0; a.slab = 0; a.slabs_per_tap = 0; a.sub_per_kb = 0; a.n_sub_total = 0;
-  static const bool no_tma = getenv("AICAM_TMA_IM2COL") == nullptr;  // opt-in: the cached gather is faster on B200
-  if (!a.stem && !no_tma && pc.cin_pad % 16 == 0 && get_encode_im2col() != nullptr) {
-    a.slab = pc.cin_pad % 64 == 0 ? 64 : (pc.cin_pad % 32 == 0 ? 32 : 16);
-    a.slabs_per_tap = pc.cin_pad / a.slab;
-    a.sub_per_kb = 64 / a.slab;
-    a.n_sub_total = a.taps * a.slabs_per_tap;
-    const cuuint64_t dims[4] = {static_cast<cuuint64_t>(pc.cin_pad), static_cast<cuuint64_t>(L.w),
-                                static_cast<cuuint64_t>(L.h), static_cast<cuuint64_t>(L.batch)};
-    const cuuint64_t strides[3] = {static_cast<cuuint64_t>(L.in_cstride) * 2, static_cast<cuuint64_t>(L.w) * L.in_cstride * 2,
-                                   static_cast<cuuint64_t>(L.h) * L.w * L.in_cstride * 2};
-    const int lower[2] = {-a.pad, -a.pad};
-    const int upper[2] = {a.pad - (a.ksize - 1), a.pad - (a.ksize - 1)};
-    const cuuint32_t estr[4] = {1, static_cast<cuuint32_t>(a.stride), static_cast<cuuint32_t>(a.stride), 1};
-    const CUtensorMapSwizzle sw = a.slab == 64 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                               : (a.slab == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-    void* base = const_cast<__nv_bfloat16*>(L.in) + L.in_coff;
-    const CUresult cr = get_encode_im2col()(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, lower, upper,
-                                            static_cast<cuuint32_t>(a.slab), TILE_M, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                            sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (cr == CUDA_SUCCESS) a.tma = 1;
-    else if (getenv("AICAM_REQUIRE_TMA"))
-      return fail(AICAM_ERR_CUDA, "launch_conv: cuTensorMapEncodeIm2col failed with " + std::to_string(static_cast<int>(cr)));
-  }
-  const size_t a_stage = a.tma ? static_cast<size_t>(TILE_M) * 128 : A_STAGE_BYTES;
-  if (a.staged && 128 * (a.n_tile * (L.out_f32 ? 4 : 2) + 16) > static_cast<long long>(STAGES * a_stage)) a.staged = 0;
-  size_t smem = SMEM_HEADER + STAGES * (a_stage + static_cast<size_t>(a.n_tile) * 16 * CHUNKS_PER_STAGE);
+  size_t smem = SMEM_HEADER + STAGES * (A_STAGE_BYTES + static_cast<size_t>(a.n_tile) * 16 * CHUNKS_PER_STAGE);
   a.res_stage_off = 0;
   if (int rc = ensure_dynamic_smem(conv_tc_kernel, 160 * 1024)) return rc;
   // persistent CTAs: at most 3 resident per SM (registers / shared memory), each loops over tiles
@@ -821,7 +709,7 @@ int launch_conv(const PackedConv& pc, const ConvLaunch& L, cudaStream_t stream) 
   dim3 grid(static_cast<unsigned>(std::min<long long>(tiles, static_cast<long long>(num_sms) * std::max(1, per_sm))));
   size_t slot = 0;
   const bool prof = profile_begin(stream, &slot);
-  conv_tc_kernel<<<grid, NUM_THREADS, smem, stream>>>(a, tmap);
+  conv_tc_kernel<<<grid, NUM_THREADS, smem, stream>>>(a);
   if (prof) profile_end(stream, slot);
   count_launch();
   return last_launch("conv_tc_kernel");

@@ -1149,7 +1149,6 @@ int try_launch_conv_win(const PackedConv& pc, const ConvLaunch& L, cudaStream_t 
     if (prc != 0) return prc;
   }
   static const bool disabled = getenv("AICAM_NO_WIN") != nullptr;
-  static const int force_mt = getenv("AICAM_WIN_MT") ? atoi(getenv("AICAM_WIN_MT")) : 0;
   if (disabled || get_encode_tiled() == nullptr) return 0;
   static const bool no_im2col = getenv("AICAM_WIN_NO_IM2COL") != nullptr;
   const bool s2d = pc.s2d_c0 != 0;  // 3x3 stride-2 layer packed as a 2x2 window over 2x2 input blocks
@@ -1264,17 +1263,15 @@ plan:
                        (!res_mode || L.res_img_stride == static_cast<long long>(L.ho) * L.wo * L.res_cstride);
   // measured: the TMA epilogue pays off where the epilogue bounds the tile (window modes, small K); deep
   // im2col / flat layers are L2-bound and need the shared memory for deeper operand rings instead
-  static const bool epi_everywhere = getenv("AICAM_WIN_TMA_EPI_ALL") != nullptr;
   // (1x1 layers with few input channels are all epilogue: measured 70 -> 50 us on 32 -> 32 @160x160)
-  static const int epi_flat_cin = getenv("AICAM_WIN_EPI_FLAT_CIN") ? atoi(getenv("AICAM_WIN_EPI_FLAT_CIN")) : 128;
-  const bool epi_flat = mode == 1 && flat_io && resident && pc.cin_pad <= epi_flat_cin;
+  const bool epi_flat = mode == 1 && flat_io && resident && pc.cin_pad <= 128;
   // im2col layers storing into zero-bordered images (the stride-2 entry layers of the ReID trunk and their 1x1 partners): TMA epilogue
   // when the tiles can be whole rows of an image or whole images (checked per tile height below)
   static const bool no_pad_store = getenv("AICAM_WIN_NO_PAD_STORE") != nullptr;
   // (measured in the step: the 1x1 stride-2 partners 59 / 38 / 23 -> 58 / 33 / 19 us; the 3x3 entry layers are bound by operand ingest and
   //  lose a little to the smaller operand ring, so they keep the generic epilogue)
   const bool epi_pad2 = mode == 2 && opd && !res_mode && pc.ksize == 1 && !no_pad_store && !pad2_failed && epi_pad2_ok;
-  if (!window && !(epi_everywhere && flat_io) && !epi_flat && !epi_pad2) epi = false;
+  if (!window && !epi_flat && !epi_pad2) epi = false;
   if (mode == 4) epi = epi4 && piece_ch[0] != 0;  // flat TMA epilogue: border positions are stored as zeros
   else if (opd && !epi_pad2) epi = false;           // (un-padded raster -> padded image: row-by-row offsets, generic epilogue)
   fixed_base = (epi ? OFF_RING_A_EPI : OFF_RING_A) + fixed_tail;
@@ -1283,7 +1280,6 @@ plan:
   static const bool no_ws = getenv("AICAM_WIN_NO_WS") != nullptr;
   const bool ws_ok = !no_ws && epi && slab == 64 && n_tile == 64 && (mode == 0 || mode == 4);
   for (int mt = 1; mt <= 2; ++mt) {
-    if (force_mt && mt != force_mt) continue;
     const int tm = 128 * mt;
     if (2 * mt * n_tile > 512) continue;
     if (epi && epi_pad2) {  // tiles = whole output rows of one image, or whole images

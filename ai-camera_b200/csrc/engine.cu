@@ -16,7 +16,6 @@
 #include <map>
 #include <vector>
 
-#include "conv_chain.cuh"
 #include "conv_tc.cuh"
 #include "frame_table.cuh"
 #include "layers.cuh"
@@ -24,7 +23,6 @@
 
 namespace aicam {
 
-bool profile_enabled();
 int nms_impl(const float* boxes, const float* scores, const int32_t* labels, int batch, int anchors, const aicam_nms_params* p,
              int32_t* num_dets, float* boxes_lb, float* boxes_orig, float* out_scores, int32_t* out_labels, int32_t* keep_index,
              void* workspace, size_t workspace_bytes, void* stream, const FrameRec* recs);
@@ -53,22 +51,8 @@ struct View {
   long long eoff = 0;  // extra element offset (Detect levels inside the head tensor)
 };
 
-// A run of consecutive CONV ops that conv_chain.cu can execute as ONE launch (the op list keeps the single layers
-// right behind the CHAIN op: they run when the chain kernel declines the geometry or is switched off)
-struct ChainOp {
-  int nstages = 0;
-  int conv[CHAIN_MAX_STAGES];  // indices into the engine's convs
-  int act[CHAIN_MAX_STAGES];
-  int nsrc[CHAIN_MAX_STAGES];
-  int src_buf[CHAIN_MAX_STAGES][2], src_coff[CHAIN_MAX_STAGES][2], src_c[CHAIN_MAX_STAGES][2];
-  int res_buf[CHAIN_MAX_STAGES], res_coff[CHAIN_MAX_STAGES], res_mode[CHAIN_MAX_STAGES];
-  int in_c = 0;   // channels of the input view loaded as buffer 0
-  int covers = 0; // CONV ops that follow and are skipped when the chain has been launched
-};
-
 struct Op {
-  enum Type { CONV, MAXPOOL, UPSAMPLE, AVGL2, STEMPOOL, SPPF3, CHAIN } type;
-  int chain = -1;
+  enum Type { CONV, MAXPOOL, UPSAMPLE, AVGL2, STEMPOOL, SPPF3 } type;
   int conv = -1;
   View in, out, res;
   int h = 0, w = 0, c = 0;  // input spatial size / channels moved (pool, upsample)
@@ -77,7 +61,6 @@ struct Op {
   int s2d_c0 = 0;   // conv reads its input space-to-depth (h, w are the space-to-depth sizes), c0 channels per pixel
   int out_s2d = 0;  // conv stores its output space-to-depth (for the next stride-2 layer)
   int only_fmt = 0; // 0: always; 2: only when the input is NOT format 3; 3: only when the input is format 3 (the two stems of yolov8n)
-  int lane = 0;     // 0: the caller's stream; 1, 2: the engine's side streams (independent tail chains, joined at the end)
 };
 
 }  // namespace
@@ -95,7 +78,6 @@ struct aicam_engine {
   std::map<std::string, int> conv_by_name;
   std::vector<aicam::Buffer> buffers;
   std::vector<aicam::Op> ops;
-  std::vector<aicam::ChainOp> chains;
   double macs_per_item = 0.0;
   // external tensor geometry
   int in_h = 0, in_w = 0;
@@ -103,11 +85,6 @@ struct aicam_engine {
   long long out_img_stride = 0;
   int num_anchors = 0;
   int feat_buf = -1;           // reid: buffer feeding the average pool
-  // The six chains of the Detect head (3 levels x {box, class}) are independent of each other: they run on the
-  // caller's stream and two side streams, forked after the neck and joined before run_ops returns, so that the
-  // small late layers fill each other's launch gaps and idle SMs (also inside a CUDA-graph capture).
-  cudaStream_t side[2] = {nullptr, nullptr};
-  cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
 };
 
 namespace aicam {
@@ -248,81 +225,19 @@ struct Builder {
 
   static View V(int b, int coff = 0, long long eoff = 0) { View v; v.buf = b; v.coff = coff; v.eoff = eoff; return v; }
 
-  // ---- fused chains (conv_chain.cu).  begin_chain() goes BEFORE the conv() calls of the layers it covers; stage() names
-  // each of them in order with its sources (buffer 0 = the chain's input view, i = the output of stage i - 1)
-  // Measured on B200 (profiles/r2_chain_bench.txt): the fused kernel is bit-for-bit as good as the single layers but NOT
-  // faster - halo recomputation in shared-memory-limited tiles costs more tensor-pipe time than the launches it saves -
-  // so the engines keep the single layers unless AICAM_CHAIN=1 asks for the chains (AICAM_CHAIN=pair,head,tail,full
-  // picks kinds).
-  static bool chains_enabled(const char* what) {
-    const char* on = getenv("AICAM_CHAIN");
-    if (on == nullptr || on[0] == '0') return false;
-    return on[0] == '1' || strstr(on, what) != nullptr;
-  }
-  int begin_chain(View in, int in_c, View out, int h, int w, int out_f32) {
-    Op op; op.type = Op::CHAIN; op.in = in; op.out = out; op.h = h; op.w = w; op.out_f32 = out_f32;
-    ChainOp c; c.in_c = in_c;
-    e->chains.push_back(c);
-    op.chain = static_cast<int>(e->chains.size()) - 1;
-    e->ops.push_back(op);
-    return op.chain;
-  }
-  void chain_stage(int chain, const std::string& conv_name, int act, int b0, int coff0, int c0, int b1 = -1, int coff1 = 0, int c1 = 0,
-                   int res_buf = -1, int res_coff = 0, int res_mode = 0) {
-    if (err) return;
-    ChainOp& c = e->chains[chain];
-    const int s = c.nstages++;
-    c.conv[s] = e->conv_by_name[conv_name];
-    c.act[s] = act;
-    c.nsrc[s] = b1 >= 0 ? 2 : 1;
-    c.src_buf[s][0] = b0; c.src_coff[s][0] = coff0; c.src_c[s][0] = c0;
-    c.src_buf[s][1] = std::max(b1, 0); c.src_coff[s][1] = coff1; c.src_c[s][1] = c1;
-    c.res_buf[s] = res_buf; c.res_coff[s] = res_coff; c.res_mode[s] = res_mode;
-    c.covers = c.nstages;
-  }
-
   // Ultralytics C2f: cv1 -> split -> n chained Bottlenecks (3x3, 3x3, optional shortcut) -> cv2 on the concat
   void c2f(const std::string& name, View in, int cin, View out, int cout, int n, bool shortcut, int h, int w) {
     const int c = cout / 2;
     const int cat = buf(h, w, (2 + n) * c);
     const int tmp = buf(h, w, c);
-    const std::string m0 = name + ".m.0", ml = name + ".m." + std::to_string(n - 1);
-    // Fusion plan (conv_chain.cu): narrow blocks (c <= 32) keep everything after cv1 - or, with few input channels, the
-    // whole block - in shared memory; wide blocks fuse each Bottleneck pair only (their operands fill shared memory)
-    const bool full = n == 1 && c <= 16 && cin <= 32 && c % 16 == 0 && chains_enabled("full");
-    const bool tail = !full && c <= 32 && c % 16 == 0 && chains_enabled("tail");
-    const bool pairs = c % 16 == 0 && chains_enabled("pair");
-    int ch_full = -1;
-    if (full) ch_full = begin_chain(in, cin, out, h, w, 0);
     conv(name + ".cv1.conv", in, h, w, V(cat, 0), cin, 2 * c, 1, 1, 1);
-    int ch_tail = -1;
     for (int j = 0; j < n; ++j) {
       const std::string m = name + ".m." + std::to_string(j);
-      int ch_pair = -1;
-      if (!full) {
-        if (tail && j == n - 1) ch_tail = begin_chain(V(cat, 0), (2 + j) * c, out, h, w, 0);
-        else if (pairs) ch_pair = begin_chain(V(cat, (1 + j) * c), c, V(cat, (2 + j) * c), h, w, 0);
-      }
       conv(m + ".cv1.conv", V(cat, (1 + j) * c), h, w, V(tmp, 0), c, c, 3, 1, 1);
       conv(m + ".cv2.conv", V(tmp, 0), h, w, V(cat, (2 + j) * c), c, c, 3, 1, 1,
            shortcut ? V(cat, (1 + j) * c) : View(), shortcut ? 1 : 0);
-      if (ch_pair >= 0) {
-        chain_stage(ch_pair, m + ".cv1.conv", 1, 0, 0, c);
-        chain_stage(ch_pair, m + ".cv2.conv", 1, 1, 0, c, -1, 0, 0, shortcut ? 0 : -1, 0, shortcut ? 1 : 0);
-      }
     }
     conv(name + ".cv2.conv", V(cat, 0), h, w, out, (2 + n) * c, cout, 1, 1, 1);
-    if (ch_full >= 0) {
-      chain_stage(ch_full, name + ".cv1.conv", 1, 0, 0, cin);
-      chain_stage(ch_full, m0 + ".cv1.conv", 1, 1, c, c);
-      chain_stage(ch_full, m0 + ".cv2.conv", 1, 2, 0, c, -1, 0, 0, shortcut ? 1 : -1, c, shortcut ? 1 : 0);
-      chain_stage(ch_full, name + ".cv2.conv", 1, 1, 0, 2 * c, 3, 0, c);
-    }
-    if (ch_tail >= 0) {  // buffer 0 = the concatenation so far: [cv1 out (2c) | m.0 .. m.(n-2) outputs]
-      chain_stage(ch_tail, ml + ".cv1.conv", 1, 0, n * c, c);
-      chain_stage(ch_tail, ml + ".cv2.conv", 1, 1, 0, c, -1, 0, 0, shortcut ? 0 : -1, n * c, shortcut ? 1 : 0);
-      chain_stage(ch_tail, name + ".cv2.conv", 1, 0, 0, (1 + n) * c, 2, 0, c);
-    }
   }
 
   void build_yolov8() {
@@ -394,42 +309,17 @@ struct Builder {
     const int lvl_c[3] = {c3, c4, c5};
     const int lvl_h[3] = {h8, h16, h32};
     long long anchor_base = 0;
-    // opt-in: measured on B200 the persistent one-CTA-per-SM kernels of different chains only delay each other
-    // (5.68 ms per step on one stream, 5.74 with three)
-    static const bool no_lanes = getenv("AICAM_HEAD_STREAMS") == nullptr;
-    int chain = 0;
-    auto set_lane = [&](size_t first_op, int lane) {
-      for (size_t i = first_op; i < e->ops.size(); ++i) e->ops[i].lane = no_lanes ? 0 : lane;
-    };
     for (int l = 0; l < 3; ++l) {
       const int hh = lvl_h[l];
       const int b1 = buf(hh, hh, cb), b2 = buf(hh, hh, cb), k1 = buf(hh, hh, cc), k2 = buf(hh, hh, cc);
       const std::string p2 = "model.22.cv2." + std::to_string(l), p3 = "model.22.cv3." + std::to_string(l);
       const long long eoff = anchor_base * e->out_cstride;
-      // each branch (3x3 -> 3x3 -> 1x1 into the fp32 head tensor) is one fused launch when conv_chain.cu takes it
-      const bool fuse = no_lanes && chains_enabled("head");
-      size_t first = e->ops.size();
-      const int ch2 = fuse && cb % 16 == 0 ? begin_chain(V(lvl_in[l]), lvl_c[l], V(-2, 0, eoff), hh, hh, 1) : -1;
       conv(p2 + ".0.conv", V(lvl_in[l]), hh, hh, V(b1), lvl_c[l], cb, 3, 1, 1);
       conv(p2 + ".1.conv", V(b1), hh, hh, V(b2), cb, cb, 3, 1, 1);
       conv(p2 + ".2", V(b2), hh, hh, V(-2, 0, eoff), cb, AICAM_HEAD_DFL, 1, 1, 0, View(), 0, 1);
-      if (ch2 >= 0) {
-        chain_stage(ch2, p2 + ".0.conv", 1, 0, 0, lvl_c[l]);
-        chain_stage(ch2, p2 + ".1.conv", 1, 1, 0, cb);
-        chain_stage(ch2, p2 + ".2", 0, 2, 0, cb);
-      }
-      set_lane(first, chain++ % 3);
-      first = e->ops.size();
-      const int ch3 = fuse && cc % 16 == 0 && nc % 16 == 0 ? begin_chain(V(lvl_in[l]), lvl_c[l], V(-2, AICAM_HEAD_DFL, eoff), hh, hh, 1) : -1;
       conv(p3 + ".0.conv", V(lvl_in[l]), hh, hh, V(k1), lvl_c[l], cc, 3, 1, 1);
       conv(p3 + ".1.conv", V(k1), hh, hh, V(k2), cc, cc, 3, 1, 1);
       conv(p3 + ".2", V(k2), hh, hh, V(-2, AICAM_HEAD_DFL, eoff), cc, nc, 1, 1, 0, View(), 0, 1);
-      if (ch3 >= 0) {
-        chain_stage(ch3, p3 + ".0.conv", 1, 0, 0, lvl_c[l]);
-        chain_stage(ch3, p3 + ".1.conv", 1, 1, 0, cc);
-        chain_stage(ch3, p3 + ".2", 0, 2, 0, cc);
-      }
-      set_lane(first, chain++ % 3);
       anchor_base += static_cast<long long>(hh) * hh;
     }
   }
@@ -442,8 +332,7 @@ struct Builder {
     static const bool unfused = getenv("AICAM_NO_STEM_FUSION") != nullptr;
     static const bool no_pad = getenv("AICAM_NO_PADDED_REID") != nullptr;
     static const bool no_pad1 = getenv("AICAM_NO_PADDED_L1") != nullptr;
-    // border kind of the trunk's activations: 2 = shared border (default), 1 = symmetric border (AICAM_REID_PAD=1)
-    static const int pad_kind = getenv("AICAM_REID_PAD") ? std::max(1, std::min(2, atoi(getenv("AICAM_REID_PAD")))) : 2;
+    const int pad_kind = 2;  // border kind of the trunk's activations: the shared border (conv_tc.cuh)
     auto wi = tensors->find("conv.0.weight");
     auto bi = tensors->find("conv.0.bias");
     if (!unfused && wi != tensors->end() && bi != tensors->end() && wi->second.dims.size() == 4 && wi->second.dims[0] == 64 &&
@@ -517,33 +406,9 @@ int run_ops(aicam_engine* e, const void* input, int batch, void* output, cudaStr
   } else if (e->kind == AICAM_KIND_REID && input_is_s2d && e->stem_in8 < 0) {
     return fail(AICAM_ERR_UNSUPPORTED, "engine: this engine was built without the fused NHWC8 stem");
   }
-  cudaStream_t main_stream = stream;
-  bool forked = false, used[2] = {false, false};
-  auto join = [&]() -> int {
-    for (int i = 0; i < 2; ++i)
-      if (used[i]) {
-        AICAM_CUDA_OK(cudaEventRecord(e->ev_join[i], e->side[i]));
-        AICAM_CUDA_OK(cudaStreamWaitEvent(main_stream, e->ev_join[i], 0));
-      }
-    return AICAM_OK;
-  };
-  int skip = 0;  // single-layer ops covered by a chain that has just been launched
   for (const Op& op : e->ops) {
-    if (skip > 0) { --skip; continue; }
     if (op.only_fmt == 3 && input_is_s2d != 2) continue;
     if (op.only_fmt == 2 && input_is_s2d == 2) continue;
-    stream = main_stream;
-    if (op.lane > 0 && e->side[op.lane - 1] && !profile_enabled()) {  // (per-launch timing: one kernel at a time)
-      if (!forked) {
-        AICAM_CUDA_OK(cudaEventRecord(e->ev_fork, main_stream));
-        forked = true;
-      }
-      if (!used[op.lane - 1]) {
-        AICAM_CUDA_OK(cudaStreamWaitEvent(e->side[op.lane - 1], e->ev_fork, 0));
-        used[op.lane - 1] = true;
-      }
-      stream = e->side[op.lane - 1];
-    }
     auto geom = [&](const View& v, int fallback_c, const __nv_bfloat16** ptr, long long* img_stride, int* cstride) {
       if (v.buf >= 0) {
         const Buffer& b = e->buffers[v.buf];
@@ -605,31 +470,6 @@ int run_ops(aicam_engine* e, const void* input, int batch, void* output, cudaStr
         rc = launch_conv(pc, L, stream);
         break;
       }
-      case Op::CHAIN: {
-        const ChainOp& c = e->chains[op.chain];
-        if (n_dev) break;  // (device-side batch counts: single layers)
-        if (dec && op.out.buf == -2) break;  // (fused decode: the single layers carry it)
-        geom(op.out, 0, &op_, &os, &oc);
-        ChainSpec sp;
-        sp.nstages = c.nstages;
-        for (int s = 0; s < c.nstages; ++s) {
-          ChainStageSpec& T = sp.st[s];
-          T.pc = &e->convs[c.conv[s]];
-          T.act = c.act[s]; T.nsrc = c.nsrc[s];
-          for (int j = 0; j < 2; ++j) { T.src_buf[j] = c.src_buf[s][j]; T.src_coff[j] = c.src_coff[s][j]; T.src_c[j] = c.src_c[s][j]; }
-          T.res_buf = c.res_buf[s]; T.res_coff = c.res_coff[s]; T.res_mode = c.res_mode[s];
-        }
-        if (op.in.buf < 0 || (op.in.buf >= 0 && e->buffers[op.in.buf].pad) || (op.out.buf >= 0 && e->buffers[op.out.buf].pad)) break;
-        sp.in = ip; sp.in_img_stride = is; sp.in_cstride = ic; sp.in_coff = op.in.coff; sp.in_c = c.in_c;
-        sp.batch = batch; sp.h = op.h; sp.w = op.w;
-        if (op.out.buf == -2) sp.out = static_cast<float*>(output) + op.out.eoff;
-        else sp.out = const_cast<__nv_bfloat16*>(op_) + op.out.eoff;
-        sp.out_img_stride = os; sp.out_cstride = oc; sp.out_coff = op.out.coff; sp.out_f32 = op.out_f32;
-        const int crc = try_launch_conv_chain(sp, stream);
-        if (crc < 0) rc = crc;
-        else if (crc == 1) skip = c.covers;
-        break;
-      }
       case Op::MAXPOOL:
         geom(op.out, 0, &op_, &os, &oc);
         rc = launch_maxpool(ip, is, ic, op.in.coff, batch, op.h, op.w, op.c, op.k, op.stride,
@@ -670,12 +510,9 @@ int run_ops(aicam_engine* e, const void* input, int batch, void* output, cudaStr
         break;
       }
     }
-    if (rc) {
-      join();  // never leave a side stream un-joined (an open graph capture would be invalidated)
-      return rc;
-    }
+    if (rc) return rc;
   }
-  return join();
+  return AICAM_OK;
 }
 
 }  // namespace
@@ -753,15 +590,6 @@ int aicam_engine_create(const char* blob_path, int device, int max_batch, aicam_
     aicam_engine_destroy(e);
     return b.err;
   }
-  bool lanes = false;
-  for (const auto& op : e->ops) lanes = lanes || op.lane > 0;
-  if (lanes) {
-    for (int i = 0; i < 2; ++i) {
-      AICAM_CUDA_OK(cudaStreamCreateWithFlags(&e->side[i], cudaStreamNonBlocking));
-      AICAM_CUDA_OK(cudaEventCreateWithFlags(&e->ev_join[i], cudaEventDisableTiming));
-    }
-    AICAM_CUDA_OK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-  }
   AICAM_CUDA_OK(cudaDeviceSynchronize());
   *out = e;
   return AICAM_OK;
@@ -774,11 +602,6 @@ void aicam_engine_destroy(aicam_engine* e) {
   free_stem_pool(&e->stem);
   for (auto& b : e->buffers)
     if (b.ptr) cudaFree(b.ptr);
-  for (int i = 0; i < 2; ++i) {
-    if (e->side[i]) cudaStreamDestroy(e->side[i]);
-    if (e->ev_join[i]) cudaEventDestroy(e->ev_join[i]);
-  }
-  if (e->ev_fork) cudaEventDestroy(e->ev_fork);
   delete e;
 }
 
@@ -795,8 +618,8 @@ int aicam_engine_num_launches(const aicam_engine* e) {
   int n = 0;
   for (const auto& op : e->ops) {
     if (op.only_fmt == 2) continue;  // (the stem exists twice, one of the two runs)
-    n += op.type == aicam::Op::STEMPOOL ? 2 : (op.type == aicam::Op::CHAIN ? 0 : 1);
-  }  // upper bound: NHWC8 repack + fused stem; chains replace layers
+    n += op.type == aicam::Op::STEMPOOL ? 2 : 1;
+  }  // upper bound: NHWC8 repack + fused stem
   return n;
 }
 

@@ -593,19 +593,15 @@ int preprocess_impl(const uint8_t* frames, int batch, int h, int w, int format, 
   if (g.decimate && !no_fast && row_bytes % 16 == 0 && reinterpret_cast<uintptr_t>(frames) % 16 == 0 &&
       FrameSrc<SRC>::frame_bytes(h, w) % 16 == 0 && (static_cast<long long>(h) * w) % 16 == 0 && 2 * stage_bytes <= 200 * 1024) {
     const int n_pairs = batch * (S / 2);
-    static const int env_stages = getenv("AICAM_K1_STAGES") ? atoi(getenv("AICAM_K1_STAGES")) : 0;
-    static const int env_ctas = getenv("AICAM_K1_CTAS") ? atoi(getenv("AICAM_K1_CTAS")) : 0;
     int stages = K1_STAGES * stage_bytes <= 100 * 1024 ? K1_STAGES : 2;
     if (format == 3) stages = 2;  // with the 20 KB block-row image, two stages keep four CTAs per SM: measured 63 us per 64 frames against 70 with four
-    if (env_stages >= 2 && env_stages <= K1_STAGES && env_stages * stage_bytes <= 200 * 1024) stages = env_stages;
     const size_t smem = stages * stage_bytes + (format == 3 ? static_cast<size_t>(S / 4) * 128 : 0);  // + the block-row image of format 3
     auto kernel = format == 0 ? preprocess_pairs_kernel<0, SRC>
                               : (format == 1 ? preprocess_pairs_kernel<1, SRC> : (format == 2 ? preprocess_pairs_kernel<2, SRC> : preprocess_pairs_kernel<3, SRC>));
     if (smem > 48 * 1024) {
       if (int rc = ensure_dynamic_smem(kernel, 200 * 1024)) return rc;
     }
-    int per_sm = static_cast<int>(std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024))));
-    if (env_ctas > 0) per_sm = std::min(per_sm, env_ctas);
+    const int per_sm = static_cast<int>(std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (smem + 1024))));
     const unsigned grid = static_cast<unsigned>(std::min<long long>(n_pairs / 2, static_cast<long long>(current_num_sms()) * per_sm));
     kernel<<<grid, S / PIX, smem, st>>>(frames, h, w, g.new_h, g.new_w, g.top, g.left, g.tab, out, n_pairs, stages, nullptr, nullptr,
                                         nullptr, 0);

@@ -1152,10 +1152,9 @@ int launch_appearance(const Dev& d, const AppearanceTf32* tf, const int32_t* det
   normalize_kernel<<<dim3(d.D, d.S), 128, 0, st>>>(d, det_count, crop_slot, stride_k, feats, present);
   count_launch();
   if (int rc = last_launch("normalize_kernel")) return rc;
-  static const bool no_gemm = getenv("AICAM_APPEARANCE_ROWS") != nullptr;
   // 0: row kernel for every frame; 1: fp32 FFMA tiling for crowded frames; 2: crowded frames are left to the
   // tensor-core kernel launched below (their blocks return at once here)
-  const int gemm_ok = tf ? 2 : ((d.F % AG_KC == 0 && !no_gemm) ? 1 : 0);
+  const int gemm_ok = tf ? 2 : (d.F % AG_KC == 0 ? 1 : 0);
   const size_t sm = std::max((APP_DT * d.F + 8 * APP_DT) * sizeof(float), gemm_ok == 1 ? AG_SMEM : size_t(0));
   if (int rc = ensure_dynamic_smem(appearance_kernel, sm)) return rc;
   appearance_kernel<<<dim3(d.T, d.S), 256, sm, st>>>(d, det_count, crop_slot, stride_k, gemm_ok, present);

@@ -153,33 +153,6 @@ int aicam_conv2d_padded(const aicam_conv_desc* d, const void* in_nhwc, const flo
 /* Micro-benchmark of the same operator on device-resident random data: `iters` launches
  * bracketed by CUDA events on `stream`; returns the mean kernel time in milliseconds. */
 int aicam_conv2d_bench(const aicam_conv_desc* d, int iters, double* mean_ms, void* stream);
-/* A chain of 2-5 stride-1 convolutions (1x1 / 3x3, pad k/2) fused into ONE kernel launch (csrc/conv_chain.cu): the
- * Bottleneck pairs and C2f tails of the detector's backbone / neck and the 3x3 -> 3x3 -> 1x1 branches of its Detect
- * head, which the reference's TensorRT engine also fuses behind src/detector/yolo_detector.py:97.  Intermediate
- * activations stay in shared memory; only the last stage's output is stored.  Exposed for parity tests.
- *   buffer 0 = the input tensor (bf16 NHWC [batch][h][w][in_c]); buffer i >= 1 = the output of stage i - 1.
- *   A stage reads the concatenation of nsrc (1 or 2) channel ranges [src_coff, src_coff + src_c) of earlier
- *   buffers (multiples of 16 channels; cin = their sum) and may add a residual: channels
- *   [res_coff, res_coff + cout) of buffer res_buf at the same pixel (res_mode as in aicam_conv_desc).
- *   weights_oihw[s] / bias[s]: HOST fp32 [cout][cin][k][k] / [cout].   out: bf16 or fp32 NHWC [batch][h][w][cout_last].
- * Returns AICAM_ERR_UNSUPPORTED when the chain does not fit the kernel (the engine then runs the layers one by one). */
-typedef struct {
-  int cin, cout, ksize;
-  int act;        /* 0 none, 1 SiLU, 2 ReLU */
-  int nsrc;
-  int src_buf[2], src_coff[2], src_c[2];
-  int res_buf, res_coff, res_mode;
-} aicam_chain_stage;
-typedef struct {
-  int batch, h, w, in_c;
-  int nstages;
-  aicam_chain_stage st[5];
-  int out_f32;
-} aicam_chain_desc;
-int aicam_conv_chain(const aicam_chain_desc* d, const void* in_nhwc, const float* const* weights_oihw,
-                     const float* const* bias, void* out_nhwc, void* stream);
-/* Micro-benchmark of one such chain on device-resident pseudo-random data (like aicam_conv2d_bench). */
-int aicam_conv_chain_bench(const aicam_chain_desc* d, int iters, double* mean_ms, void* stream);
 /* The fused ReID stem on its own (test entry): Conv3x3(3->64, s1, p1) + bias + ReLU + MaxPool(3, s2, p1),
  * the first two layers of the ReID engine (reid_model.py:115).
  *   in_nhwc4 : bf16 [n][h][w][4] (h, w even)   weights_oihw : fp32 host [64][3][3][3]   bias : fp32 host [64]

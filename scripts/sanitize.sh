@@ -2,7 +2,7 @@
 # compute-sanitizer over the kernel parity tests (memcheck, then racecheck); summaries -> gpurun_out/sanitizer_*.txt
 # (copied to profiles/ by hand).  Each tool gets its own process per test file and a wall-clock limit.
 mkdir -p gpurun_out
-FILES=${FILES:-"tests/test_gpu_conv.py tests/test_gpu_chain.py tests/test_gpu_preprocess.py tests/test_gpu_crops.py tests/test_gpu_detect_post.py tests/test_gpu_tracker.py tests/test_gpu_engine.py"}
+FILES=${FILES:-"tests/test_gpu_conv.py tests/test_gpu_preprocess.py tests/test_gpu_crops.py tests/test_gpu_detect_post.py tests/test_gpu_tracker.py tests/test_gpu_engine.py"}
 for tool in ${TOOLS:-memcheck racecheck}; do
   out=gpurun_out/sanitizer_$tool.txt
   echo "# compute-sanitizer --tool $tool over the -m gpu parity tests ($(nvidia-smi --query-gpu=name --format=csv,noheader | head -1), $(compute-sanitizer --version | head -2 | tail -1))" > $out

@@ -88,7 +88,7 @@ def traffic(path, json_out=None, crops=None):
         print("%3d %-24s %-18s grid %-14s %8.1f us  rd %8.1f MB  wr %8.1f MB  tensor %5.1f%%" % (
             i, r["name"][:24], ("<" + tp.group(1).replace("unnamed", "").strip() + ">") if tp and "conv_win" in r["name"] else "", r["grid"], r.get("us", 0),
             r.get("rd", 0) / 1e6, r.get("wr", 0) / 1e6, r.get("tensor", 0)))
-    conv = [r for r in rows if any(k in r["name"] for k in ("conv_win", "conv_pair", "stem_pool", "conv_tc", "conv_chain"))]
+    conv = [r for r in rows if any(k in r["name"] for k in ("conv_win", "conv_pair", "stem_pool", "conv_tc"))]
     out = {"dram_read_bytes": sum(r.get("rd", 0) for r in conv), "dram_write_bytes": sum(r.get("wr", 0) for r in conv),
            "launches": len(conv), "kernel_time_us": sum(r.get("us", 0) for r in conv), "crops_in_step": crops,
            "source": "ncu --metrics dram__bytes_read.sum,dram__bytes_write.sum over scripts/profile_step.py (64 streams), summed over "

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Hardware probe for the window kernel: max error of a few layer shapes against torch fp32.
-Run once per descriptor rule:  AICAM_WIN_BASE_OFFSET=0|1 python scripts/win_probe.py"""
+   python scripts/win_probe.py"""
 import os
 import sys
 
@@ -15,7 +15,6 @@ import gpu_util as G  # noqa: E402
 
 CASES = [("c64", 2, 20, 20, 64, 64, 3), ("c32", 2, 20, 20, 32, 32, 3), ("c16", 2, 20, 20, 16, 16, 3),
          ("c128s", 2, 20, 20, 128, 128, 3), ("1x1_64", 2, 20, 20, 64, 64, 1), ("1x1_48", 2, 20, 20, 48, 32, 1)]
-print("base_offset mode", os.environ.get("AICAM_WIN_BASE_OFFSET", "0"), "mt", os.environ.get("AICAM_WIN_MT", "auto"))
 for name, B, H, W, cin, cout, k in CASES:
     rng = np.random.default_rng(1)
     x = G.bf16_round_np(rng.normal(0, 1, (B, H, W, cin)))
