@@ -56,6 +56,20 @@ class TrackerConfig(C.Structure):
                 ("nn_budget", C.c_int), ("device", C.c_int)]
 
 
+COUNT_MAX_LINES, COUNT_MAX_ZONES, COUNT_MAX_VERTICES, COUNT_CLASSES, COUNT_MAX_COORD = 16, 16, 32, 80, 1 << 20
+
+
+class StreamCounting(C.Structure):
+    _fields_ = [("n_lines", C.c_int32), ("n_zones", C.c_int32), ("line", (C.c_int32 * 4) * COUNT_MAX_LINES),
+                ("line_class_mask", (C.c_uint64 * 2) * COUNT_MAX_LINES), ("zone_n", C.c_int32 * COUNT_MAX_ZONES),
+                ("zone_xy", ((C.c_int32 * 2) * COUNT_MAX_VERTICES) * COUNT_MAX_ZONES),
+                ("zone_class_mask", (C.c_uint64 * 2) * COUNT_MAX_ZONES)]
+
+
+class CounterOutput(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("line_counts", "zone_counts", "occupancy", "row_zones", "events", "event_count")]
+
+
 class OverlayItem(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("type", "x1", "y1", "x2", "y2", "color", "slot", "reserved")]
 
@@ -134,6 +148,14 @@ SIGNATURES = {
     "aicam_tracker_cost_probe": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "aicam_tracker_snapshot": (_I, [_P, _I, _P, _P, _I]),
     "aicam_tracker_overflow": (_I, [_P, _P]),
+    "aicam_tracker_row_slots": (_P, [_P]),
+    "aicam_counter_create": (_I, [_I, _I, _I, _I, C.POINTER(_P)]),
+    "aicam_counter_destroy": (None, [_P]),
+    "aicam_counter_set_streams": (_I, [_P, _P, C.POINTER(StreamCounting), _I, _P]),
+    "aicam_counter_step": (_I, [_P, _P, _P, _P, _P, _P]),
+    "aicam_counter_reset_streams": (_I, [_P, _P, _P]),
+    "aicam_counter_outputs": (_I, [_P, C.POINTER(CounterOutput)]),
+    "aicam_counter_overflow": (_I, [_P, _P]),
     "aicam_lsap": (_I, [_P, _I, _I, _I, _P, _P]),
     "aicam_kf_gating": (_I, [_P, _P, _I, _I, _P, _P]),
     "aicam_overlay_draw": (_I, [_P, _I, _I, _I, _P, _P, _P, _I, _I, _P]),

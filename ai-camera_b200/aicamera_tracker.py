@@ -25,6 +25,11 @@ Differences, all in the direction of the hardware:
     with ``pipeline.StreamSettings`` field names.  An input's entry applies over "default", which applies over
     ``--conf_thresh`` and the config.  Each input runs with its entry from its first frame, also when it takes over a
     slot under ``--run_all_inputs``.
+  * ``--counting FILE.json`` (new, batched mode) counts line crossings and zone entries per input on the device, in the
+    same ``{"default": {...}, "<input file name>": {...}}`` shape (values: ``pipeline.StreamCounting.from_dict``
+    objects; an input's "lines" / "zones" replace those of "default").  Each track line of ``.tracks.jsonl`` then
+    carries the step's ``"events"``, ``<stem>.counts.json`` holds each input's totals (summed from the events), and
+    ``--save_video`` adds one panel line per counting line or zone.
 """
 import argparse
 import json
@@ -68,6 +73,10 @@ def parse_arguments(argv=None) -> argparse.Namespace:
                         help="Batched mode: JSON file {\"default\": {...}, \"<input file name>\": {...}} of per-input "
                              "settings (conf_threshold, nms_threshold, classes_to_track, min_detection_confidence, "
                              "max_cosine_distance, max_iou_distance, max_age, n_init).")
+    parser.add_argument("--counting", type=str, default=None,
+                        help="Batched mode: JSON file {\"default\": {...}, \"<input file name>\": {...}} of per-input "
+                             "counting lines and zones ({\"lines\": [{\"a\": [x, y], \"b\": [x, y], \"name\": .., "
+                             "\"classes\": [..]}], \"zones\": [{\"points\": [[x, y], ...], ...}]}).")
     args = parser.parse_args(argv)
     if args.device == "cpu":
         parser.error("this build has no CPU path (the reference's TensorRT engines do not run on CPU either)")
@@ -79,7 +88,71 @@ def parse_arguments(argv=None) -> argparse.Namespace:
             args.settings_for = load_stream_settings(args.stream_settings, args.conf_thresh)
         except (OSError, ValueError, TypeError) as e:
             parser.error("--stream_settings %s: %s" % (args.stream_settings, e))
+    args.counting_for = None
+    if args.counting is not None:
+        if args.streams <= 0:
+            parser.error("--counting needs batched mode (--streams N)")
+        try:
+            args.counting_for = load_counting(args.counting)
+        except (OSError, ValueError, TypeError) as e:
+            parser.error("--counting %s: %s" % (args.counting, e))
     return args
+
+
+def load_counting(path):
+    """The --counting file as a function: input file name -> StreamCounting.  An input's "lines" / "zones" replace those
+    of "default"; an input without an entry gets "default" (no lines and zones if there is none)."""
+    from .pipeline import StreamCounting
+    with open(path) as f:
+        spec = json.load(f)
+    if not isinstance(spec, dict) or not all(isinstance(v, dict) for v in spec.values()):
+        raise ValueError("expected a JSON object of objects")
+    base = spec.get("default", {})
+    default = StreamCounting.from_dict(base)
+    entries = {name: StreamCounting.from_dict({**base, **v}) for name, v in spec.items() if name != "default"}
+    return lambda name: entries.get(name, default)
+
+
+EVENT_KINDS = ("in", "out", "entered", "exited")
+# the pipeline's track capacity; the counter gets room for every event a step can make (each reported row crosses each
+# line and enters or leaves each zone at most once), so the totals summed from the events are exact
+MAX_TRACKS = 256
+COUNT_MAX_LINES = COUNT_MAX_ZONES = 16
+
+
+class CountTotals:
+    """One input's counts summed on the host from its events (no read of the device counters, so a slot handed to the
+    next input needs no synchronisation before its reset)."""
+
+    def __init__(self, counting):
+        self.counting = counting
+        self.lines = {x.name: {"in": {}, "out": {}} for x in counting.lines}
+        self.zones = {x.name: {"entered": {}, "exited": {}} for x in counting.zones}
+
+    def add(self, events):
+        for e in events:
+            d = (self.lines if e["kind"] in ("in", "out") else self.zones)[e["name"]][e["kind"]]
+            d[e["class"]] = d.get(e["class"], 0) + 1
+
+    def as_dict(self):
+        return {"lines": self.lines, "zones": self.zones}
+
+    def panel_lines(self):
+        return (["%s: in %d out %d" % (n, sum(v["in"].values()), sum(v["out"].values())) for n, v in self.lines.items()] +
+                ["%s: entered %d exited %d" % (n, sum(v["entered"].values()), sum(v["exited"].values()))
+                 for n, v in self.zones.items()])
+
+
+def step_events(pipe):
+    """Per stream, the events of the step that has just completed, with the names of their lines and zones."""
+    counter = pipe.counter
+    out = []
+    for s, n in enumerate(counter.event_count.cpu().tolist()):
+        c = pipe.counting[s]
+        evs = counter.events[s, :n].cpu().tolist() if n and c is not None else []
+        out.append([{"kind": EVENT_KINDS[k], "name": (c.lines if k < 2 else c.zones)[i].name, "id": tid,
+                     "class": config.CLASSES[cls]} for k, i, tid, cls in evs])
+    return out
 
 
 def load_stream_settings(path, conf_threshold=config.YOLO_CONF_THRESHOLD):
@@ -322,13 +395,17 @@ def main(argv=None):
         if args.streams > 0:
             from .pipeline import TrackingPipeline
             print("Initializing the batched pipeline (%d streams)..." % args.streams)
-            stream_settings = None
-            if args.settings_for:  # slot s starts with input s (inputs are cycled unless --run_all_inputs is given)
-                first = [sources_spec[s % len(sources_spec)] if not args.run_all_inputs or s < len(sources_spec) else None
-                         for s in range(args.streams)]
+            # slot s starts with input s (inputs are cycled unless --run_all_inputs is given)
+            first = [sources_spec[s % len(sources_spec)] if not args.run_all_inputs or s < len(sources_spec) else None
+                     for s in range(args.streams)]
+            stream_settings = counting = None
+            if args.settings_for:
                 stream_settings = [args.settings_for(input_name(p) if p is not None else None) for p in first]
-            pipe = TrackingPipeline(args.yolo_engine, args.reid_engine, args.streams, device,
-                                    conf_threshold=args.conf_thresh, stream_settings=stream_settings)
+            if args.counting_for:
+                counting = [args.counting_for(input_name(p)) if p is not None else None for p in first]
+            pipe = TrackingPipeline(args.yolo_engine, args.reid_engine, args.streams, device, max_tracks=MAX_TRACKS,
+                                    conf_threshold=args.conf_thresh, stream_settings=stream_settings, counting=counting,
+                                    max_events=MAX_TRACKS * (COUNT_MAX_LINES + COUNT_MAX_ZONES))
             if args.run_all_inputs:
                 stats, frames = _run_all_inputs(args, pipe, sources_spec, writer, out_dir if writer else None,
                                                 stem if writer else None, videos, device)
@@ -345,20 +422,32 @@ def main(argv=None):
                 return pipe_step(frames_dev, *a, **k)
             pipe.step = step_and_keep
             stats_ref = []
+            totals = [CountTotals(c) for c in counting] if counting else None
 
             def on_step(step, batch, table):
                 if writer:
                     tabs = [t.numpy() for t in table]
                     fps = stats_ref[0].fps() * args.streams if stats_ref else 0.0
+                    events = step_events(pipe) if totals else None
                     for s in range(args.streams):
                         rows = tracks_to_rows(tabs, s)
-                        writer.write(json.dumps({"frame": step, "stream": s, "tracks": rows}) + "\n")
+                        line = {"frame": step, "stream": s, "tracks": rows}
+                        panel = ["AICamera: YOLOv8 + DeepSORT", f"Input: {source_name}", "FPS: %.2f" % fps]
+                        if totals:
+                            line["events"] = events[s]
+                            totals[s].add(events[s])
+                            panel += totals[s].panel_lines()
+                        writer.write(json.dumps(line) + "\n")
                         if videos:
-                            videos[s].write(dev_frames["f"][s], rows, ["AICamera: YOLOv8 + DeepSORT", f"Input: {source_name}", "FPS: %.2f" % fps])
+                            videos[s].write(dev_frames["f"][s], rows, panel)
                 if (step + 1) % 100 == 0:
                     print(f"Processed {step + 1} steps.")
             stats = run_batched(srcs, pipe, on_step, stats_out=stats_ref)
             frames = stats.frames * args.streams
+            if writer and totals:
+                _write_counts(out_dir / (stem + ".counts.json"),
+                              [dict(input=input_name(sources_spec[s % len(sources_spec)]), stream=s, **t.as_dict())
+                               for s, t in enumerate(totals)])
         else:
             from .deepsort_tracker import DeepSORT
             from .yolo_detector import YOLODetector
@@ -387,6 +476,12 @@ def main(argv=None):
         for v in videos:
             v.close()
     return _summary(args, stats, frames)
+
+
+def _write_counts(path, entries):
+    with open(path, "w") as f:
+        json.dump(entries, f, indent=1)
+    print(f"Counts saved to: {path}")
 
 
 def _summary(args, stats, frames):
@@ -420,30 +515,44 @@ def _run_all_inputs(args, pipe, inputs, writer, out_dir, stem, videos, device):
         return pipe_step(frames_dev, *a, **k)
     pipe.step = step_and_keep
     stats_ref, counted = [], [0]
+    totals = [CountTotals(args.counting_for(n)) for n in names] if args.counting_for else None
+    ran_in = [None] * len(names)
 
     def on_refill(slot, k):
         slot_input[slot] = N + k
         frame_idx[slot] = 0
         if args.settings_for:
             pipe.configure_streams([slot], args.settings_for(names[N + k]))
+        if totals:
+            pipe.configure_counting([slot], totals[N + k].counting)
 
     def on_step(step, batch, table):
         tabs = [t.numpy() for t in table] if writer else None
+        events = step_events(pipe) if writer and totals else None
         for s, f in enumerate(batch):
             if f is None:
                 continue
             counted[0] += 1
             if writer:
                 i = slot_input[s]
+                ran_in[i] = s
                 rows = tracks_to_rows(tabs, s)
-                writer.write(json.dumps({"frame": frame_idx[s], "stream": s, "input": names[i], "tracks": rows}) + "\n")
+                line = {"frame": frame_idx[s], "stream": s, "input": names[i], "tracks": rows}
+                panel = ["AICamera: YOLOv8 + DeepSORT", f"Input: {names[i]}"]
+                if totals:
+                    line["events"] = events[s]
+                    totals[i].add(events[s])
+                writer.write(json.dumps(line) + "\n")
                 if videos:
                     fps = stats_ref[0].fps() * N if stats_ref else 0.0
-                    videos[i].write(dev_frames["f"][s], rows, ["AICamera: YOLOv8 + DeepSORT", f"Input: {names[i]}", "FPS: %.2f" % fps])
+                    videos[i].write(dev_frames["f"][s], rows, panel + ["FPS: %.2f" % fps] + (totals[i].panel_lines() if totals else []))
             frame_idx[s] += 1
         if (step + 1) % 100 == 0:
             print(f"Processed {step + 1} steps.")
     stats = run_batched(srcs, pipe, on_step, stats_out=stats_ref, until="all", refill=refill, on_refill=on_refill)
+    if writer and totals:
+        _write_counts(out_dir / (stem + ".counts.json"),
+                      [dict(input=n, stream=ran_in[i], **totals[i].as_dict()) for i, n in enumerate(names)])
     return stats, counted[0]
 
 

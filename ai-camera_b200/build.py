@@ -17,7 +17,8 @@ LIB = os.path.join(HERE, "libaicam.so")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall",
           "--expt-relaxed-constexpr"]
-# Files whose float arithmetic must match the reference bit for bit: no FMA contraction.
+# Files whose float arithmetic must match the reference bit for bit: no FMA contraction.  (counting.cu needs no entry: its
+# geometry is integer-only.)
 NO_FMA = {"tracker.cu", "detect_post.cu", "reid_crops.cu", "preprocess.cu"}
 
 

@@ -20,6 +20,7 @@
 //   gallery[S][T][G][F] f32 (L2-normalised at insert; ring buffer: head, count)
 //   order[S][T]: slots of the live tracks in creation order (the reference's track list)
 //   free_slots[S][T] stack, next_id[S]
+//   row_slot[S][T]: the slot behind each row of out_tracks of the last step (what aicam_counter_step keys its state by)
 //   trk_n_init/trk_max_age[S][T] i32: the n_init / max_age a track was created with (track.py keeps them per track)
 //   assoc[S]: each stream's association settings (aicam_tracker_set_stream_assoc), read once per step by its CTA
 #include <algorithm>
@@ -73,6 +74,7 @@ struct Dev {
   int* track_id; int* state; int* hits; int* age; int* tsu; int* cls; float* conf;
   int* gal_count; int* gal_head; float* gallery;
   int* order; int* n_tracks; int* free_slots; int* n_free; int* next_id; int* overflow;
+  int* row_slot;    // [S][T]: tracker slot of each reported row of the last step (aicam_tracker_row_slots)
   float* app_cost;  // [S][T][D] by (slot, det)
   float* cost_ws;   // [S][T*D]
   float* featn;     // [S][D][F]
@@ -1006,7 +1008,8 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
   }
   __syncthreads();
   for (int n = tid; n < s_nL; n += ASSOC_THREADS) {  // ... and their rows, one thread each
-    const long long ts = sb + ord[L[n]];
+    const int slot = ord[L[n]];
+    const long long ts = sb + slot;
     float tl[4];
     mean_to_tlwh(t.mean + ts * 8, tl);
     const float w = tl[2] > 0.0f ? tl[2] : 0.0f, h = tl[3] > 0.0f ? tl[3] : 0.0f;
@@ -1018,6 +1021,7 @@ __global__ void __launch_bounds__(ASSOC_THREADS) assoc_kernel(Dev t, StepIO io) 
     o[4] = t.track_id[ts];
     o[5] = t.cls[ts];
     io.out_conf[sb + n] = t.conf[ts];
+    t.row_slot[sb + n] = slot;
   }
   __syncthreads();
   ASSOC_STAMP(6);
@@ -1196,7 +1200,7 @@ int aicam_tracker_create(const aicam_tracker_config* cfg, aicam_tracker** out) {
   rc |= dev_alloc(t, &d.gallery, ST * d.G * d.F);
   rc |= dev_alloc(t, &d.order, ST);     rc |= dev_alloc(t, &d.free_slots, ST);
   rc |= dev_alloc(t, &d.n_tracks, d.S); rc |= dev_alloc(t, &d.n_free, d.S); rc |= dev_alloc(t, &d.next_id, d.S);
-  rc |= dev_alloc(t, &d.overflow, d.S);
+  rc |= dev_alloc(t, &d.overflow, d.S);     rc |= dev_alloc(t, &d.row_slot, ST);
   rc |= dev_alloc(t, &t->assoc_dev, d.S); d.assoc = t->assoc_dev;
   rc |= dev_alloc(t, &d.trk_n_init, ST); rc |= dev_alloc(t, &d.trk_max_age, ST);
   if (t->staging.create(d.S * sizeof(AssocRec)) != cudaSuccess) rc |= 1;
@@ -1358,6 +1362,8 @@ int aicam_tracker_snapshot(aicam_tracker* t, int stream_index, int32_t* ints, fl
   }
   return n;
 }
+
+const int32_t* aicam_tracker_row_slots(const aicam_tracker* t) { return t ? t->d.row_slot : nullptr; }
 
 int aicam_tracker_overflow(aicam_tracker* t, int32_t* flags_host) {
   if (!t || !flags_host) return fail(AICAM_ERR_INVALID_ARG, "tracker_overflow: null argument");

@@ -9,7 +9,7 @@ wrappers around ``BatchDetector`` / ``BatchTracker``.
 """
 import ctypes as C
 import math
-from dataclasses import dataclass, fields
+from dataclasses import dataclass, fields, replace
 from typing import FrozenSet, Optional, Sequence, Tuple, Union
 
 import torch
@@ -96,6 +96,217 @@ def _as_settings_list(indices, settings):
     if len(settings) != len(indices) or not all(isinstance(s, StreamSettings) for s in settings):
         raise ValueError("configure_streams: one StreamSettings per index")
     return indices, settings
+
+
+def _point(p, what):
+    if not (isinstance(p, (tuple, list)) and len(p) == 2):
+        raise ValueError("%s must be an (x, y) pair, got %r" % (what, p))
+    for v in p:
+        if isinstance(v, bool) or not isinstance(v, int):
+            raise ValueError("%s: coordinates must be integers, got %r" % (what, p))
+        if abs(v) > _lib.COUNT_MAX_COORD:
+            raise ValueError("%s: coordinates are limited to +-2^20, got %r" % (what, p))
+    return (int(p[0]), int(p[1]))
+
+
+def _classes(classes):
+    if classes is None:
+        return None
+    if isinstance(classes, str):
+        raise ValueError("classes is a set of class names, not one string")
+    classes = frozenset(classes)
+    unknown = classes - set(config.CLASSES)
+    if unknown:
+        raise ValueError("unknown class names: %s" % sorted(unknown))
+    return classes
+
+
+def _from_dict(cls, d):
+    if not isinstance(d, dict):
+        raise ValueError("%s: expected an object, got %r" % (cls.__name__, d))
+    unknown = set(d) - {f.name for f in fields(cls)}
+    if unknown:
+        raise ValueError("unknown %s fields: %s" % (cls.__name__, sorted(unknown)))
+    return cls(**d)
+
+
+@dataclass(frozen=True)
+class CountingLine:
+    """A counting line from ``a`` to ``b`` (integer frame pixels).  A track whose bottom-centre anchor passes from the
+    left-hand side of a->b to its right-hand side (on screen, y pointing down) goes "in", the other way "out".
+    ``classes``: the class names counted (None: the pipeline's tracked classes)."""
+    a: Tuple[int, int]
+    b: Tuple[int, int]
+    name: Optional[str] = None
+    classes: Optional[FrozenSet[str]] = None
+
+    def __post_init__(self):
+        object.__setattr__(self, "a", _point(self.a, "line end a"))
+        object.__setattr__(self, "b", _point(self.b, "line end b"))
+        if self.a == self.b:
+            raise ValueError("a counting line needs two distinct ends, got %r twice" % (self.a,))
+        if self.name is not None and not isinstance(self.name, str):
+            raise ValueError("name must be a string, got %r" % (self.name,))
+        object.__setattr__(self, "classes", _classes(self.classes))
+
+    @classmethod
+    def from_dict(cls, d):
+        return _from_dict(cls, d)
+
+
+@dataclass(frozen=True)
+class CountingZone:
+    """A counting zone: a polygon of 3 to 32 integer vertices (even-odd rule; may be concave or self-intersecting).
+    ``classes`` as for CountingLine."""
+    points: Tuple[Tuple[int, int], ...]
+    name: Optional[str] = None
+    classes: Optional[FrozenSet[str]] = None
+
+    def __post_init__(self):
+        if isinstance(self.points, str) or not hasattr(self.points, "__len__"):
+            raise ValueError("points must be a sequence of (x, y) pairs")
+        pts = tuple(_point(p, "zone vertex") for p in self.points)
+        if not 3 <= len(pts) <= _lib.COUNT_MAX_VERTICES:
+            raise ValueError("a zone needs 3 to %d vertices, got %d" % (_lib.COUNT_MAX_VERTICES, len(pts)))
+        object.__setattr__(self, "points", pts)
+        if self.name is not None and not isinstance(self.name, str):
+            raise ValueError("name must be a string, got %r" % (self.name,))
+        object.__setattr__(self, "classes", _classes(self.classes))
+
+    @classmethod
+    def from_dict(cls, d):
+        return _from_dict(cls, d)
+
+
+@dataclass(frozen=True)
+class StreamCounting:
+    """One stream's counting lines and zones (at most 16 of each).  Unnamed ones are called ``line{i}`` / ``zone{i}``
+    after their index; names are unique within the stream."""
+    lines: Tuple[CountingLine, ...] = ()
+    zones: Tuple[CountingZone, ...] = ()
+
+    def __post_init__(self):
+        lines, zones = tuple(self.lines), tuple(self.zones)
+        if not all(isinstance(x, CountingLine) for x in lines) or not all(isinstance(x, CountingZone) for x in zones):
+            raise ValueError("lines must be CountingLine and zones CountingZone objects")
+        if len(lines) > _lib.COUNT_MAX_LINES or len(zones) > _lib.COUNT_MAX_ZONES:
+            raise ValueError("at most %d lines and %d zones per stream" % (_lib.COUNT_MAX_LINES, _lib.COUNT_MAX_ZONES))
+        lines = tuple(x if x.name is not None else replace(x, name="line%d" % i) for i, x in enumerate(lines))
+        zones = tuple(x if x.name is not None else replace(x, name="zone%d" % i) for i, x in enumerate(zones))
+        for kind, items in (("line", lines), ("zone", zones)):
+            names = [x.name for x in items]
+            if len(set(names)) != len(names):
+                raise ValueError("%s names must be unique within a stream: %s" % (kind, names))
+        object.__setattr__(self, "lines", lines)
+        object.__setattr__(self, "zones", zones)
+
+    @classmethod
+    def from_dict(cls, d):
+        """From ``{"lines": [{"a": [x, y], "b": [x, y], "name": .., "classes": [..]}], "zones": [{"points": [[x, y],
+        ..], ..}]}`` (e.g. a JSON object)."""
+        if not isinstance(d, dict):
+            raise ValueError("StreamCounting: expected an object, got %r" % (d,))
+        unknown = set(d) - {"lines", "zones"}
+        if unknown:
+            raise ValueError("unknown counting fields: %s" % sorted(unknown))
+
+        def items(key, kind):
+            v = d.get(key, [])
+            if not isinstance(v, list):
+                raise ValueError("%s must be a list" % key)
+            return tuple(kind.from_dict(x) for x in v)
+        return cls(items("lines", CountingLine), items("zones", CountingZone))
+
+    def resolve(self, default_classes):
+        """The aicam_stream_counting of this geometry; lines and zones without classes count ``default_classes``."""
+        g = _lib.StreamCounting()
+        g.n_lines, g.n_zones = len(self.lines), len(self.zones)
+        for i, x in enumerate(self.lines):
+            g.line[i][:] = [x.a[0], x.a[1], x.b[0], x.b[1]]
+            g.line_class_mask[i][:] = config.tracked_class_mask(x.classes if x.classes is not None else default_classes)
+        for i, x in enumerate(self.zones):
+            g.zone_n[i] = len(x.points)
+            for k, (px, py) in enumerate(x.points):
+                g.zone_xy[i][k][:] = [px, py]
+            g.zone_class_mask[i][:] = config.tracked_class_mask(x.classes if x.classes is not None else default_classes)
+        return g
+
+
+class _DeviceArray:
+    """A library-owned device array as torch sees it (__cuda_array_interface__); holds the handle's owner alive."""
+
+    def __init__(self, owner, ptr, shape, typestr):
+        self.owner = owner
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False),
+                                         "version": 2, "strides": None}
+
+
+class _CounterHandle:
+    def __init__(self, lib, device, n_streams, max_tracks, max_events):
+        self.lib, self.h = lib, C.c_void_p()
+        _lib.check(lib.aicam_counter_create(device.index or 0, n_streams, max_tracks, max_events, C.byref(self.h)))
+
+    def __del__(self):
+        if getattr(self, "h", None):
+            self.lib.aicam_counter_destroy(self.h)
+            self.h = None
+
+
+class StreamCounter:
+    """Owner of an ``aicam_counter``: line crossings and zone entries of ``n_streams`` streams, counted on the device
+    from a tracker's reported rows.  The outputs are device tensors over the library's buffers (stable, so a captured
+    step keeps writing them; they stay valid while any of them or the counter lives):
+      line_counts int64 [S, 16, 2, 80] (in, out per class), zone_counts int64 [S, 16, 2, 80] (entries, exits),
+      occupancy int32 [S, 16, 80], row_zones int32 [S, T] (zone bits of row n of out_tracks), events int32
+      [S, max_events, 4] (kind 0 line in, 1 line out, 2 zone entry, 3 zone exit; index; track id; class) and
+      event_count int32 [S] of the last step."""
+
+    def __init__(self, device, n_streams: int, max_tracks: int, max_events: int = 1024):
+        self.lib = _lib.load()
+        self.device = torch.device(device)
+        self.S, self.T, self.E = int(n_streams), int(max_tracks), int(max_events)
+        self._handle = _CounterHandle(self.lib, self.device, self.S, self.T, self.E)
+        o = _lib.CounterOutput()
+        _lib.check(self.lib.aicam_counter_outputs(self._handle.h, C.byref(o)))
+        L, Z, K = _lib.COUNT_MAX_LINES, _lib.COUNT_MAX_ZONES, _lib.COUNT_CLASSES
+
+        def view(ptr, shape, typestr):
+            return torch.as_tensor(_DeviceArray(self._handle, ptr, shape, typestr), device=self.device)
+        self.line_counts = view(o.line_counts, (self.S, L, 2, K), "<i8")
+        self.zone_counts = view(o.zone_counts, (self.S, Z, 2, K), "<i8")
+        self.occupancy = view(o.occupancy, (self.S, Z, K), "<i4")
+        self.row_zones = view(o.row_zones, (self.S, self.T), "<i4")  # (bits 0..15: never negative)
+        self.events = view(o.events, (self.S, self.E, 4), "<i4")
+        self.event_count = view(o.event_count, (self.S,), "<i4")
+
+    @property
+    def handle(self):
+        return self._handle.h
+
+    def set_streams(self, indices, geometry: Sequence["_lib.StreamCounting"]):
+        """Streams ``indices`` take ``geometry`` (aicam_stream_counting records); their counts and tracks restart."""
+        n = len(indices)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_counter_set_streams(self.handle, (C.c_int32 * n)(*indices),
+                                                          (_lib.StreamCounting * n)(*geometry), n,
+                                                          _lib.stream_ptr(self.device)))
+
+    def step(self, out_tracks, out_count, row_slot, present=None):
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_counter_step(self.handle, _lib.ptr(out_tracks), _lib.ptr(out_count), row_slot, present,
+                                                   _lib.stream_ptr(self.device)))
+
+    def reset_streams(self, mask):
+        """Restart the streams whose entry of the device int32 [S] mask is non-zero."""
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_counter_reset_streams(self.handle, _lib.ptr(mask), _lib.stream_ptr(self.device)))
+
+    def overflow(self):
+        """Sticky per-stream flags: some step had more events than max_events (the counters stayed exact)."""
+        import numpy as np
+        f = np.zeros(self.S, np.int32)
+        _lib.check(self.lib.aicam_counter_overflow(self.handle, _lib.ptr(f)))
+        return f
 
 
 def frame_geometry(frames: torch.Tensor):
@@ -317,6 +528,7 @@ class BatchTracker:
         self.out_tracks = torch.zeros((S, max_tracks, 6), **i32)
         self.out_conf = torch.zeros((S, max_tracks), dtype=torch.float32, device=dev)
         self.out_count = torch.zeros(S, **i32)
+        self.row_slots = C.c_void_p(self.lib.aicam_tracker_row_slots(self._h))  # device i32 [S, T]: slot of each row
         self._reset_mask = torch.zeros(S, **i32)
         self._mask = config.tracked_class_mask(self.classes_to_track)
         # per-stream confidence and class mask of configure_streams (None: every stream uses the constructor's); a list
@@ -460,7 +672,7 @@ class TrackingPipeline:
                  max_crops: Optional[int] = None, conf_threshold=config.YOLO_CONF_THRESHOLD, topk=config.YOLO_TOPK,
                  max_candidates=config.YOLO_MAX_CANDIDATES, max_frame_hw=(2160, 3840),
                  nms_threshold=config.YOLO_NMS_THRESHOLD, stream_settings: Optional[Sequence[StreamSettings]] = None,
-                 **tracker_kw):
+                 counting: Optional[Sequence[Optional[StreamCounting]]] = None, max_events: int = 1024, **tracker_kw):
         self.detector = BatchDetector(yolo_engine_path, n_streams, device, conf_threshold=conf_threshold,
                                       nms_threshold=nms_threshold, topk=topk, max_candidates=max_candidates,
                                       max_frame_hw=max_frame_hw)
@@ -481,6 +693,12 @@ class TrackingPipeline:
         self._routed = False  # some stream detects or filters differently: stacked steps go through the frame table
         if stream_settings is not None:
             self.configure_streams(range(n_streams), stream_settings)
+        # line and zone counting: the counter exists (and each step launches it) once some stream has counting
+        self.counter: Optional[StreamCounter] = None
+        self.counting = [None] * n_streams
+        self.max_events = int(max_events)
+        if counting is not None:
+            self.configure_counting(range(n_streams), counting)
 
     def configure_streams(self, indices, settings):
         """Give the streams ``indices`` their own StreamSettings (one per index, or one for all) from the next step on,
@@ -499,6 +717,31 @@ class TrackingPipeline:
         base = _filter_key(self.default_settings.resolve()[0])
         self._routed = any(_filter_key(f) != base for f in filters)
 
+    def configure_counting(self, indices, counting):
+        """Give the streams ``indices`` their counting lines and zones (one StreamCounting or None per index, or one for
+        all; None: no counting) from the next step on, eager or from a captured graph (call it between replays, like
+        ``frame_table.set``).  Their counters and occupancy restart at zero and their tracks are counted from their next
+        report on, as first reports; the other streams are untouched.  The first call that gives a stream counting
+        creates the counter: from then on every step launches it once after the tracker.  A step captured before that
+        does not include the counter, so capture again after turning counting on."""
+        indices = [int(i) for i in indices]
+        if counting is None or isinstance(counting, StreamCounting):
+            counting = [counting] * len(indices)
+        counting = list(counting)
+        if len(counting) != len(indices) or not all(c is None or isinstance(c, StreamCounting) for c in counting):
+            raise ValueError("configure_counting: one StreamCounting (or None) per index")
+        for i in indices:
+            if not 0 <= i < self.n_streams:
+                raise _lib.AicamError(-1, "configure_counting: stream %d out of range" % i)
+        if self.counter is None:
+            if all(c is None for c in counting):
+                return
+            self.counter = StreamCounter(self.device, self.n_streams, self.tracker.T, self.max_events)
+        geometry = [(c or StreamCounting()).resolve(self.tracker.classes_to_track) for c in counting]
+        self.counter.set_streams(indices, geometry)
+        for i, c in zip(indices, counting):
+            self.counting[i] = c
+
     def step(self, frames: Union[torch.Tensor, Sequence[torch.Tensor]]) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         if not is_frame_list(frames) and self._routed:
             frame_geometry(frames)
@@ -507,23 +750,53 @@ class TrackingPipeline:
             self.frame_table.set(frames)
             return self.step_table()
         num, boxes, scores, labels = self.detector.detect(frames)
-        return self.tracker.update(frames, num, boxes, scores, labels)
+        return self._count(self.tracker.update(frames, num, boxes, scores, labels), None)
 
     def step_table(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """One step over the frames ``frame_table`` holds.  Launches depend only on the stream count and the size
         bound, so a captured step_table() stays valid when ``frame_table.set`` changes the frames, or which of them are
         present, between replays."""
         num, boxes, scores, labels = self.detector.detect_table(self.frame_table)
-        return self.tracker.update_table(self.frame_table, num, boxes, scores, labels)
+        return self._count(self.tracker.update_table(self.frame_table, num, boxes, scores, labels),
+                           self.frame_table.present_ptr)
+
+    def _count(self, tables, present):
+        if self.counter is not None:
+            out_tracks, _, out_count = tables
+            self.counter.step(out_tracks, out_count, self.tracker.row_slots, present)
+        return tables
+
+    def counts(self):
+        """Per stream, the cumulative counts since the stream's counting was last set or reset, and the occupancy of
+        its last step: ``{"lines": {name: {"in": {class: n}, "out": {...}}}, "zones": {name: {"entered": {...},
+        "exited": {...}, "occupancy": {...}}}}``, zeros omitted ({} for a stream without counting).  Synchronises."""
+        out = [{} for _ in range(self.n_streams)]
+        if self.counter is None:
+            return out
+        lc, zc, occ = (x.cpu().numpy() for x in (self.counter.line_counts, self.counter.zone_counts, self.counter.occupancy))
+
+        def by_class(v):
+            return {config.CLASSES[k]: int(v[k]) for k in range(len(v)) if v[k]}
+        for s, c in enumerate(self.counting):
+            if c is None:
+                continue
+            out[s] = {"lines": {x.name: {"in": by_class(lc[s, i, 0]), "out": by_class(lc[s, i, 1])} for i, x in enumerate(c.lines)},
+                      "zones": {x.name: {"entered": by_class(zc[s, i, 0]), "exited": by_class(zc[s, i, 1]),
+                                         "occupancy": by_class(occ[s, i])} for i, x in enumerate(c.zones)}}
+        return out
 
     def reset_streams(self, indices, settings=None):
-        """Hand the given stream slots to new sources: their trackers restart (no tracks, ids from 1), the other streams
-        and the captured step are untouched.  The slots keep their settings, or take ``settings`` (as configure_streams)."""
+        """Hand the given stream slots to new sources: their trackers restart (no tracks, ids from 1) and so do their
+        counts, the other streams and the captured step are untouched.  The slots keep their settings and counting
+        geometry, or take ``settings`` (as configure_streams)."""
         if settings is not None:
             self.configure_streams(indices, settings)
         self.tracker.reset_streams(indices)
+        if self.counter is not None:  # (ids restart at 1: a new track must not continue an old one's counting state)
+            self.counter.reset_streams(self.tracker._reset_mask)
 
     def launches_per_step(self, frame_list=False):
         """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True), absent frames
-        or not.  A stacked tensor runs as a list while streams detect or filter differently."""
-        return self.detector.launches_per_step(frame_list or self._routed) + self.tracker.launches_per_step()
+        or not.  A stacked tensor runs as a list while streams detect or filter differently; the counter adds one."""
+        return (self.detector.launches_per_step(frame_list or self._routed) + self.tracker.launches_per_step() +
+                (1 if self.counter is not None else 0))

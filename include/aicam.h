@@ -440,6 +440,86 @@ int aicam_tracker_cost_probe(aicam_tracker* t, const float* boxes, int stride_k,
 /* Sticky per-stream overflow flags since the last reset (host out i32[n_streams]):
  * bit 0 = track capacity exceeded, bit 1 = detection capacity exceeded. */
 int aicam_tracker_overflow(aicam_tracker* t, int32_t* flags_host);
+/* Device i32[n_streams][max_tracks]: row n < out_count[s] of the last step's out_tracks came from tracker slot
+ * row_slots[s][n].  A live track keeps its slot; live tracks of a stream have distinct slots.  Stable for the tracker's
+ * lifetime (aicam_counter_step reads it). */
+const int32_t* aicam_tracker_row_slots(const aicam_tracker* t);
+
+/* ------------------------------------------------------------------------------------------
+ * Counting: line crossings and zone entries per stream, on the tracker's reported rows, in one capturable launch after
+ * the tracker step (what a camera-fleet operator does with the tracks: people through a door, cars over a stop line,
+ * objects in a loading bay).  All geometry is exact integer arithmetic:
+ *   anchor   the bottom centre of a row x1,y1,x2,y2 held doubled, P = (x1 + x2, 2 * y2), each coordinate clamped to
+ *            [-2^24, 2^24]; line and zone coordinates are integer frame pixels, |v| <= 2^20, doubled to match
+ *   state    per (stream, tracker slot): track id, last reported anchor, bit set of the zones the track is in; a row whose
+ *            id differs from its slot's stored id is the track's first report
+ *   line A->B: side(P) = +1 if (Bx-Ax)*(Py-Ay) - (By-Ay)*(Px-Ax) > 0, else -1 (a point on the line is on the -1 side).
+ *            A report moving a track from P0 (its last reported anchor) to P1 crosses when side(P0) != side(P1) and A, B
+ *            are not strictly on the same side of the line P0P1.  -1 -> +1 is "in" (on screen, y down: from the left of
+ *            A->B to its right), +1 -> -1 "out".  Every crossing counts; a first report never crosses.
+ *   zone     a polygon of 3..AICAM_COUNT_MAX_VERTICES vertices, even-odd rule with half-open edges: edge (xi,yi)->(xj,yj)
+ *            counts when (yi > Py) != (yj > Py) and P is strictly left of the edge at Py (int64, no division).  A report
+ *            inside a zone the track was not in is an entry (a first report inside included), a report outside a zone
+ *            it was in an exit.  A track deleted inside a zone makes no exit; a track not reported at a step (missed,
+ *            tentative) keeps its bits.
+ *   classes  each line and zone counts only rows whose class is in its 80-bit mask (lo, hi as aicam_stream_filter);
+ *            membership bits are kept for every row.
+ * ---------------------------------------------------------------------------------------- */
+#define AICAM_COUNT_MAX_LINES 16
+#define AICAM_COUNT_MAX_ZONES 16
+#define AICAM_COUNT_MAX_VERTICES 32
+#define AICAM_COUNT_CLASSES 80
+#define AICAM_COUNT_MAX_COORD (1 << 20)
+typedef struct aicam_counter aicam_counter;
+typedef struct {
+  int32_t n_lines, n_zones;
+  int32_t line[AICAM_COUNT_MAX_LINES][4];                          /* ax, ay, bx, by */
+  uint64_t line_class_mask[AICAM_COUNT_MAX_LINES][2];              /* lo, hi */
+  int32_t zone_n[AICAM_COUNT_MAX_ZONES];                           /* vertex count */
+  int32_t zone_xy[AICAM_COUNT_MAX_ZONES][AICAM_COUNT_MAX_VERTICES][2];
+  uint64_t zone_class_mask[AICAM_COUNT_MAX_ZONES][2];
+} aicam_stream_counting;
+/* Device outputs, stable for the counter's lifetime; entries of streams present at the last step:
+ *   line_counts i64 [S][MAX_LINES][2][80]  cumulative in / out per class     zone_counts i64 [S][MAX_ZONES][2][80]
+ *   occupancy   i32 [S][MAX_ZONES][80]     rows of the last step inside      cumulative entries / exits per class
+ *   row_zones   u32 [S][max_tracks]        zone bits of row n of out_tracks (bit z = zone z)
+ *   events      i32 [S][max_events][4]     (kind, index, track id, class): kind 0 line in, 1 line out, 2 zone entry,
+ *               3 zone exit; one per counted crossing, entry or exit of the last step, ordered by row, then lines by
+ *               index, then zones by index
+ *   event_count i32 [S]                    events of the last step (at most max_events) */
+typedef struct {
+  int64_t* line_counts;
+  int64_t* zone_counts;
+  int32_t* occupancy;
+  uint32_t* row_zones;
+  int32_t* events;
+  int32_t* event_count;
+} aicam_counter_output;
+/* n_streams and max_tracks as the tracker whose rows it counts; max_events >= 1 per stream and step.  Every stream starts
+ * with no lines and zones and no state. */
+int aicam_counter_create(int device, int n_streams, int max_tracks, int max_events, aicam_counter** out);
+void aicam_counter_destroy(aicam_counter* c);
+/* Stream indices_host[i] takes the geometry host[i] (host arrays, i < n): validated as a whole first - counts over the
+ * maxima, a zone of fewer than 3 vertices, a zero-length line, a coordinate beyond AICAM_COUNT_MAX_COORD, an index outside
+ * 0..n_streams-1 are AICAM_ERR_INVALID_ARG and nothing is copied or launched.  Then one asynchronous copy on `stream` from
+ * pinned staging and the masked reset of those streams (as aicam_counter_reset_streams).  Not capturable; captured steps
+ * read the table, so they follow its changes. */
+int aicam_counter_set_streams(aicam_counter* c, const int32_t* indices_host, const aicam_stream_counting* host, int n,
+                              void* stream);
+/* One launch, capturable, no host synchronisation: counts the rows out_tracks i32 [S][max_tracks][6] / out_count i32 [S]
+ * of a tracker step whose slots are row_slot (aicam_tracker_row_slots).  present: device i32[S] as for
+ * aicam_tracker_step_present, NULL = every stream; an absent stream changes no state, counter, occupancy or row_zones
+ * entry, and its event_count is 0.  Counters are integer atomics: the result does not depend on the order of the rows.
+ * Events beyond max_events are dropped and set the stream's sticky overflow flag; the counters stay exact. */
+int aicam_counter_step(aicam_counter* c, const int32_t* out_tracks, const int32_t* out_count, const int32_t* row_slot,
+                       const int32_t* present, void* stream);
+/* Zero the counters, occupancy and overflow flag of the streams whose entry of the device mask i32[S] is non-zero and
+ * forget their tracks (each track's next report is a first report); one launch, capturable.  It must accompany every
+ * aicam_tracker_reset_streams of a stream: ids restart at 1 there, and a new track could otherwise continue an old one. */
+int aicam_counter_reset_streams(aicam_counter* c, const int32_t* mask, void* stream);
+int aicam_counter_outputs(const aicam_counter* c, aicam_counter_output* out);
+/* Sticky per-stream event-overflow flags since the stream's last reset (host out i32[S]); synchronises. */
+int aicam_counter_overflow(aicam_counter* c, int32_t* flags_host);
 
 /* Stand-alone pieces of the association, exposed for bit-exact parity tests. */
 /* scipy.optimize.linear_sum_assignment (linear_assignment.py:62) on `count` fp32 cost
