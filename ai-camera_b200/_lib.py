@@ -22,7 +22,7 @@ class AicamError(RuntimeError):
 
 class ConvDesc(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("batch", "h", "w", "cin", "cout", "ksize", "stride", "act",
-                                       "res_mode", "out_f32")]
+                                       "res_mode", "out_f32")] + [("n_dev", C.c_void_p)]  # (NULL unless given)
 
 
 class Letterbox(C.Structure):

@@ -802,7 +802,7 @@ int aicam_conv2d(const aicam_conv_desc* d, const void* in, const float* w, const
       free_packed_conv(&pc);
       return fail(AICAM_ERR_CUDA, "conv2d: cudaMalloc failed");
     }
-    int rc = launch_space_to_depth(static_cast<const __nv_bfloat16*>(in), d->batch, d->h, d->w, c0, s2, st);
+    int rc = launch_space_to_depth(static_cast<const __nv_bfloat16*>(in), d->batch, d->h, d->w, c0, s2, st, d->n_dev);
     ConvLaunch L;
     L.in = s2; L.in_cstride = 4 * c0; L.in_coff = 0;
     L.batch = d->batch; L.h = d->h / 2; L.w = d->w / 2; L.ho = L.h; L.wo = L.w;
@@ -812,6 +812,7 @@ int aicam_conv2d(const aicam_conv_desc* d, const void* in, const float* w, const
     L.res = static_cast<const __nv_bfloat16*>(res); L.res_img_stride = L.out_img_stride; L.res_cstride = d->cout;
     L.res_coff = 0; L.res_mode = res ? d->res_mode : 0;
     L.act = d->act;
+    L.batch_dev = d->n_dev;
     if (!rc) rc = launch_conv(pc, L, st);
     cudaError_t se = cudaStreamSynchronize(st);
     cudaFree(s2);
@@ -843,6 +844,7 @@ int aicam_conv2d_padded(const aicam_conv_desc* d, const void* in, const float* w
   L.res_coff = 0; L.res_mode = res ? d->res_mode : 0;
   L.act = d->act;
   L.in_pad = ip; L.out_pad = opd;
+  L.batch_dev = d->n_dev;
   if (ip && opd) pack_pair_weights(&pc);
   int rc = launch_conv(pc, L, static_cast<cudaStream_t>(stream));
   cudaError_t se = cudaStreamSynchronize(static_cast<cudaStream_t>(stream));

@@ -134,6 +134,11 @@ typedef struct {
   int act;        /* 0 none, 1 SiLU, 2 ReLU */
   int res_mode;   /* 0 none, 1 act(conv)+res, 2 act(conv+res) */
   int out_f32;    /* 0: bf16 output, 1: fp32 output */
+  /* optional device i32[1], as the engines pass it to every layer: when not NULL, aicam_conv2d[_padded] read the
+   * number of images on the device (clamped to batch, which then is the capacity the launch is planned for); the
+   * images below that count neither read nor write the images at or past it.  NULL: all batch images.
+   * aicam_conv2d_bench ignores it. */
+  const int32_t* n_dev;
 } aicam_conv_desc;
 int aicam_conv2d(const aicam_conv_desc* d, const void* in_nhwc, const float* weights_oihw,
                  const float* bias, const void* res_nhwc, void* out_nhwc, void* stream);

@@ -22,14 +22,17 @@ def bf16_round_np(x):
     return torch.from_numpy(np.ascontiguousarray(x, dtype=np.float32)).to(torch.bfloat16).float().numpy()
 
 
-def conv2d(x_nhwc, w_oihw, bias, ksize, stride, act=0, res=None, res_mode=0, out_f32=False):
-    """x_nhwc: torch bf16 cuda [B,H,W,Cpad]; w_oihw/bias numpy fp32 (host)."""
+def conv2d(x_nhwc, w_oihw, bias, ksize, stride, act=0, res=None, res_mode=0, out_f32=False, n_dev=None, out=None):
+    """x_nhwc: torch bf16 cuda [B,H,W,Cpad]; w_oihw/bias numpy fp32 (host).  n_dev: optional device int32 [1], the image
+    count (B is then the capacity); out: optional output tensor to store into (kept as it is for images >= the count)."""
     B, H, W, _ = x_nhwc.shape
     cout, cin = w_oihw.shape[:2]
     ho = (H + 2 * (ksize // 2) - ksize) // stride + 1
     wo = (W + 2 * (ksize // 2) - ksize) // stride + 1
-    out = torch.empty((B, ho, wo, cout), dtype=torch.float32 if out_f32 else torch.bfloat16, device=DEV)
-    d = ConvDesc(B, H, W, cin, cout, ksize, stride, act, res_mode, 1 if out_f32 else 0)
+    if out is None:
+        out = torch.empty((B, ho, wo, cout), dtype=torch.float32 if out_f32 else torch.bfloat16, device=DEV)
+    d = ConvDesc(B, H, W, cin, cout, ksize, stride, act, res_mode, 1 if out_f32 else 0,
+                 n_dev.data_ptr() if n_dev is not None else None)
     w = np.ascontiguousarray(w_oihw, np.float32)
     b = np.ascontiguousarray(bias, np.float32)
     check(lib().aicam_conv2d(C.byref(d), ptr(x_nhwc), ptr(w), ptr(b), ptr(res), ptr(out), None))
