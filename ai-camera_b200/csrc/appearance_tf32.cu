@@ -3,7 +3,7 @@
 //   cost[track][det] = min over the track's gallery of max(0, 1 - <g, f_det>)
 //   (/root/reference/src/tracker/core/matching.py:109-217: a float32 sgemm per track, then a min over rows)
 //
-// The reference multiplies float32 features, and parity on the cost is held to 1e-5 (tests/test_gpu_tracker.py), so
+// The reference multiplies float32 features, and parity on the cost is held to 1e-5 (tests/test_gpu_appearance.py), so
 // bf16 operands are out.  Every normalised feature x is kept as x = hi + lo with hi = x rounded to the 10-bit TF32
 // mantissa (exactly representable, so whatever the tensor core does with the 13 low bits, it reads hi) and
 // lo = x - hi (exact in float32); <g, f> ~ <g_hi, f_hi> + <g_hi, f_lo> + <g_lo, f_hi> accumulated in fp32 by three

@@ -468,6 +468,9 @@ __global__ void __launch_bounds__(128) normalize_kernel(Dev t, const int* __rest
 // on the usual ~17-detection frames (97 vs 70 us per 64 streams: three times the shared memory, a third of the blocks).
 constexpr int APP_DT = 16;
 constexpr int APP_GEMM_MIN = 48;
+// dynamic shared memory of the row kernel: the detection tile and the per-warp minima.  aicam_tracker_create rejects a
+// feature_dim for which this exceeds what a block can opt in to.
+constexpr size_t appearance_rows_smem(int F) { return (static_cast<size_t>(APP_DT) * F + 8 * APP_DT) * sizeof(float); }
 __device__ __forceinline__ void appearance_rows(const Dev& t, const int* __restrict__ det_count,
                                                 const int* __restrict__ crop_slot, int stride_k, float* sm_f) {
   // sm_f: [APP_DT][F] detection tile, then [8][APP_DT] per-warp minima
@@ -1159,7 +1162,7 @@ int launch_appearance(const Dev& d, const AppearanceTf32* tf, const int32_t* det
   // 0: row kernel for every frame; 1: fp32 FFMA tiling for crowded frames; 2: crowded frames are left to the
   // tensor-core kernel launched below (their blocks return at once here)
   const int gemm_ok = tf ? 2 : (d.F % AG_KC == 0 ? 1 : 0);
-  const size_t sm = std::max((APP_DT * d.F + 8 * APP_DT) * sizeof(float), gemm_ok == 1 ? AG_SMEM : size_t(0));
+  const size_t sm = std::max(appearance_rows_smem(d.F), gemm_ok == 1 ? AG_SMEM : size_t(0));
   if (int rc = ensure_dynamic_smem(appearance_kernel, sm)) return rc;
   appearance_kernel<<<dim3(d.T, d.S), 256, sm, st>>>(d, det_count, crop_slot, stride_k, gemm_ok, present);
   count_launch();
@@ -1185,6 +1188,13 @@ int aicam_tracker_create(const aicam_tracker_config* cfg, aicam_tracker** out) {
   if (cfg->max_age < 1 || cfg->max_age > 255 || cfg->n_init < 1)
     return fail(AICAM_ERR_INVALID_ARG, "tracker_create: max_age must be in 1..255 and n_init >= 1");
   AICAM_CUDA_OK(cudaSetDevice(cfg->device));
+  int smem_optin = 0;
+  AICAM_CUDA_OK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device));
+  if (appearance_rows_smem(cfg->feature_dim) > static_cast<size_t>(smem_optin))
+    return fail(AICAM_ERR_CAPACITY, "tracker_create: feature_dim " + std::to_string(cfg->feature_dim) + " needs " +
+                                        std::to_string(appearance_rows_smem(cfg->feature_dim)) +
+                                        " bytes of shared memory in the appearance kernel, more than the " +
+                                        std::to_string(smem_optin) + " a block can use");
   aicam_tracker* t = new aicam_tracker();
   t->cfg = *cfg;
   Dev& d = t->d;

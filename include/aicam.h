@@ -366,7 +366,8 @@ typedef struct {
   int n_streams;
   int max_tracks;          /* live tracks per stream (capacity) */
   int max_dets;            /* filtered detections per frame per stream (capacity) */
-  int feature_dim;         /* 512 */
+  int feature_dim;         /* 512; AICAM_ERR_CAPACITY when the appearance kernel's 16 * feature_dim + 128 floats of
+                              shared memory exceed what a block may opt in to (feature_dim <= 3624 at 227 KB) */
   double max_cosine_distance; /* src/config.py:23 (a Python float: kept as double so that
                                  max_distance + 1e-5 rounds as in linear_assignment.py:58) */
   double max_iou_distance;    /* src/config.py:26 */

@@ -136,7 +136,8 @@ class Tracker:
     def step(self, frames, probe=False, feats_null=False):
         """frames: list (one per stream) of dicts boxes/scores/classes/feats (numpy).  Returns, per
         stream, (out [n,6] int64, conf [n] float64).  probe=True: no step; returns, per stream,
-        (track_ids [T], app_cost [T,D], gate_d2 [T,D]) from aicam_tracker_cost_probe."""
+        (track_ids [T], app_cost [T,D], gate_d2 [T,D]) from aicam_tracker_cost_probe, and sets
+        self.probe_launches to the number of kernels that call launched."""
         from ai_camera_b200.config import tracked_class_mask
         S, K = self.S, self.K
         b = np.zeros((S, K, 4), np.float32)
@@ -170,9 +171,11 @@ class Tracker:
             d2 = torch.zeros((S, self.T, Dm), dtype=torch.float32, device=DEV)
             ids = torch.zeros((S, self.T), dtype=torch.int32, device=DEV)
             nt = torch.zeros(S, dtype=torch.int32, device=DEV)
+            launches = lib().aicam_launch_count()
             check(lib().aicam_tracker_cost_probe(self.h, ptr(self.boxes), K, ptr(self.det_index), ptr(self.det_count),
                                                  ptr(self.crop_slot), ptr(self.feats), ptr(app), ptr(d2), ptr(ids),
                                                  ptr(nt), None))
+            self.probe_launches = lib().aicam_launch_count() - launches
             sync()
             app, d2, ids, nt = app.cpu().numpy(), d2.cpu().numpy(), ids.cpu().numpy(), nt.cpu().numpy()
             return [(ids[s, :nt[s]].astype(np.int64), app[s, :nt[s], :dc[s]], d2[s, :nt[s], :dc[s]]) for s in range(S)]

@@ -130,75 +130,6 @@ def test_tracker_empty_frames_and_capacity_flag():
         trk.close()
 
 
-def _long_lived(seed, n_frames, n_objects, feat_dim=512):
-    """Objects that are seen in EVERY frame, so that their galleries reach the budget (100) and the ring wraps."""
-    rng = np.random.default_rng(seed)
-    base = rng.normal(size=(n_objects, feat_dim)).astype(np.float32)
-    base /= np.linalg.norm(base, axis=1, keepdims=True)
-    cx = rng.uniform(300, 1600, n_objects); cy = rng.uniform(200, 900, n_objects)
-    vx = rng.normal(0, 2.0, n_objects); vy = rng.normal(0, 1.0, n_objects)
-    h = rng.uniform(80, 200, n_objects); w = h * rng.uniform(0.3, 0.6, n_objects)
-    frames = []
-    for t in range(n_frames):
-        x, y = cx + vx * t + rng.normal(0, 1, n_objects), cy + vy * t + rng.normal(0, 1, n_objects)
-        order = rng.permutation(n_objects)
-        frames.append(dict(
-            boxes=np.stack([x - w / 2, y - h / 2, x + w / 2, y + h / 2], 1).astype(np.float32)[order],
-            scores=rng.uniform(0.4, 0.95, n_objects).astype(np.float32)[order],
-            classes=np.zeros(n_objects, np.int32),
-            feats=(base * rng.uniform(0.5, 2.0, (n_objects, 1)) + 0.05 * rng.normal(size=(n_objects, feat_dim))).astype(np.float32)[order]))
-    return frames
-
-
-@pytest.mark.parametrize("seed,n_objects,n_frames,kw", [
-    (301, 12, 40, {}),                                         # row tiling (<= 48 detections per frame)
-    (302, 70, 14, dict(size_range=(25.0, 90.0))),               # SGEMM tiling (> 48 detections per frame)
-    (303, 5, 125, "long_lived"),                                # galleries past the budget: the ring wraps at G = 100
-])
-def test_appearance_cost_and_gate_match_oracle(seed, n_objects, n_frames, kw):
-    """K8 / K9 as VALUES (not only through the ids they lead to): before every frame, the appearance cost of
-    every live track against every filtered detection (|diff| <= 1e-5: the reference's own value goes through a
-    BLAS sgemm) and the squared Mahalanobis distance (bit-exact) equal the oracle's; the minimum margins to
-    the 0.2 cosine threshold and the 9.4877 gate are reported."""
-    import gpu_util as G
-    from oracle.tracker import DeepSORT
-    from oracle.constants import INFTY_COST
-    frames = (_long_lived(seed, n_frames, n_objects) if kw == "long_lived" else
-              make_scenario(seed=seed, n_frames=n_frames, n_objects=n_objects, **kw))
-    kmax = max(8, max(len(f["boxes"]) for f in frames))
-    trk = G.Tracker(1, max_tracks=256, max_dets=kmax, stride_k=kmax)
-    ora = DeepSORT()
-    worst, margin_cos, margin_gate, compared, wrapped = 0.0, 1e9, 1e9, 0, False
-    try:
-        for f in frames:
-            ids, app, d2 = trk.step([f], probe=True)[0]
-            wid, wapp, wd2 = ora.probe_costs(f["boxes"], f["scores"], f["classes"], frame_hw=(1080, 1920),
-                                             planted_features=f["feats"])
-            assert np.array_equal(ids, wid)
-            assert app.shape == wapp.shape
-            if app.size:
-                inf_g, inf_w = app >= INFTY_COST, wapp >= INFTY_COST
-                assert np.array_equal(inf_g, inf_w)
-                fin = ~inf_w
-                if fin.any():
-                    worst = max(worst, float(np.abs(app[fin] - wapp[fin]).max()))
-                    margin_cos = min(margin_cos, float(np.abs(wapp[fin] - 0.2).min()))
-                    compared += int(fin.sum())
-                assert np.array_equal(d2.view(np.uint32), wd2.view(np.uint32)), "gating distance differs"
-                margin_gate = min(margin_gate, float(np.abs(wd2 - 9.487729036781154).min()))
-            o, c = trk.step([f])[0]
-            want = ora.update(f["boxes"], f["scores"], f["classes"], frame_hw=(1080, 1920), planted_features=f["feats"])
-            assert [tuple(r[:5]) for r in o.tolist()] == [w[:5] for w in want]
-            wrapped = wrapped or (any(len(t.features) >= 100 for t in ora.tracker_core.tracks) and len(frames) > 110)
-    finally:
-        trk.close()
-    print("appearance cost: %d values, max |diff| %.2e, min margin to 0.2: %.3e, to the gate: %.3e" %
-          (compared, worst, margin_cos, margin_gate))
-    assert compared > 0 and worst <= 1e-5
-    if seed == 303:
-        assert wrapped, "the scenario was meant to fill a gallery to its budget"
-
-
 def test_tracker_without_features_matches_reference_semantics():
     """feats == NULL: every appearance cost is INFTY_COST and the galleries stay as they were (the reference with
     every Detection.feature None); the same frames through the oracle with all crops invalid."""
