@@ -66,6 +66,15 @@ class StreamCounting(C.Structure):
                 ("zone_class_mask", (C.c_uint64 * 2) * COUNT_MAX_ZONES)]
 
 
+REGION_MAX_POLYGONS = 8
+
+
+class StreamRegion(C.Structure):
+    _fields_ = [("n_polygons", C.c_int32), ("kind", C.c_int32 * REGION_MAX_POLYGONS),
+                ("n_vertices", C.c_int32 * REGION_MAX_POLYGONS),
+                ("xy", ((C.c_int32 * 2) * COUNT_MAX_VERTICES) * REGION_MAX_POLYGONS)]
+
+
 class CounterOutput(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("line_counts", "zone_counts", "occupancy", "row_zones", "events", "event_count")]
 
@@ -124,6 +133,7 @@ SIGNATURES = {
     "aicam_frame_table_set_present": (_I, [_P, C.POINTER(FrameDesc), _P, _I, _P]),
     "aicam_frame_table_present": (_P, [_P]),
     "aicam_frame_table_set_filters": (_I, [_P, C.POINTER(StreamFilter), _I]),
+    "aicam_frame_table_set_regions": (_I, [_P, _P, C.POINTER(StreamRegion), _I, _P]),
     "aicam_preprocess_table": (_I, [_P, _I, _P, _P]),
     "aicam_yolo_detect_table": (_I, [_P, _P, _I, _P, C.POINTER(NmsParams), _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _P]),
     "aicam_reid_crops_table": (_I, [_P, _P, _P, _P, _P, _I, C.c_float, C.c_uint64, C.c_uint64, _I, _I, _P, _P, _P, _P,

@@ -72,7 +72,8 @@ def parse_arguments(argv=None) -> argparse.Namespace:
     parser.add_argument("--stream_settings", type=str, default=None,
                         help="Batched mode: JSON file {\"default\": {...}, \"<input file name>\": {...}} of per-input "
                              "settings (conf_threshold, nms_threshold, classes_to_track, min_detection_confidence, "
-                             "max_cosine_distance, max_iou_distance, max_age, n_init).")
+                             "max_cosine_distance, max_iou_distance, max_age, n_init, include_regions, exclude_regions: lists of "
+                             "polygons [[x, y], ...] in frame pixels).")
     parser.add_argument("--counting", type=str, default=None,
                         help="Batched mode: JSON file {\"default\": {...}, \"<input file name>\": {...}} of per-input "
                              "counting lines and zones ({\"lines\": [{\"a\": [x, y], \"b\": [x, y], \"name\": .., "

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "polygon.cuh"
 #include "staging.cuh"
 
 namespace aicam {
@@ -21,7 +22,6 @@ namespace {
 constexpr int COUNT_THREADS = 256;
 constexpr int NL = AICAM_COUNT_MAX_LINES, NZ = AICAM_COUNT_MAX_ZONES, NV = AICAM_COUNT_MAX_VERTICES;
 constexpr int NCLS = AICAM_COUNT_CLASSES;
-constexpr long long ANCHOR_LIMIT = 1ll << 24;  // |anchor coordinate| after clamping: every cross product fits in int64
 constexpr int MAX_EVENTS = 1 << 20;
 
 struct CounterDev {
@@ -41,26 +41,9 @@ __device__ __forceinline__ bool class_in(const uint64_t* mask, int cls) {
   return cls >= 0 && cls < NCLS && ((cls < 64 ? mask[0] >> cls : mask[1] >> (cls - 64)) & 1ull);
 }
 
-__device__ __forceinline__ long long clamp_anchor(long long v) {
-  return v < -ANCHOR_LIMIT ? -ANCHOR_LIMIT : (v > ANCHOR_LIMIT ? ANCHOR_LIMIT : v);
-}
-
 // +1 when P is strictly on the positive side of A->B (a point on the line belongs to the -1 side)
 __device__ __forceinline__ int line_side(long long ax, long long ay, long long bx, long long by, long long px, long long py) {
   return (bx - ax) * (py - ay) - (by - ay) * (px - ax) > 0 ? 1 : -1;
-}
-
-// even-odd rule, half-open edges, doubled coordinates; "strictly left of the edge at py" without division
-__device__ bool in_zone(const int32_t (*xy)[2], int n, long long px, long long py) {
-  bool inside = false;
-  for (int i = 0, j = n - 1; i < n; j = i++) {
-    const long long xi = 2ll * xy[i][0], yi = 2ll * xy[i][1], xj = 2ll * xy[j][0], yj = 2ll * xy[j][1];
-    if ((yi > py) != (yj > py)) {
-      const long long dy = yj - yi, lhs = (px - xi) * dy, rhs = (py - yi) * (xj - xi);
-      if (dy > 0 ? lhs < rhs : lhs > rhs) inside = !inside;
-    }
-  }
-  return inside;
 }
 
 __global__ void __launch_bounds__(COUNT_THREADS) count_kernel(CounterDev c, const int* __restrict__ out_tracks,

@@ -62,6 +62,14 @@ struct aicam_frame_table {
   uint8_t* dev;           // the device block
   aicam::PinnedStaging staging;
   std::vector<aicam_stream_filter> filters;  // of aicam_frame_table_set_filters: entry i < size() carries filters[i]
+  // aicam_frame_table_set_regions, allocated by its first call: the host copy of the region block, the device block
+  // (capacity records), its own staging (the block is ~2 KB per entry, far larger than the records), and K5's scratch of
+  // the region test, one keep bit per detection (capacity x 1024 bits)
+  std::vector<aicam_stream_region> regions;
+  aicam_stream_region* regions_dev = nullptr;
+  unsigned* region_keep = nullptr;
+  aicam::PinnedStaging region_staging;
+  bool region_test = false;  // some entry has had polygons: aicam_reid_crops_table launches the region test
 
   const int* counts() const { return reinterpret_cast<const int*>(dev); }
   const int* lists() const { return reinterpret_cast<const int*>(dev) + aicam::FT_COUNTS; }

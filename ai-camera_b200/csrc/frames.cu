@@ -2,6 +2,7 @@
 // host, read on the device by the ragged K1 / detect / K5 entry points and, for presence, by the tracker step.  See frame_table.cuh for the device layout.
 #include <algorithm>
 #include <cstring>
+#include <string>
 #include <vector>
 
 #include "frame_table.cuh"
@@ -44,7 +45,10 @@ void aicam_frame_table_destroy(aicam_frame_table* t) {
   if (!t) return;
   cudaSetDevice(t->device);
   t->staging.destroy();
+  t->region_staging.destroy();
   if (t->dev) cudaFree(t->dev);
+  if (t->regions_dev) cudaFree(t->regions_dev);
+  if (t->region_keep) cudaFree(t->region_keep);
   delete t;
 }
 
@@ -143,6 +147,60 @@ int aicam_frame_table_set_filters(aicam_frame_table* t, const aicam_stream_filte
                                                ": thresholds must be finite and in [0, 1]");
   }
   t->filters.assign(host, host + n);
+  return AICAM_OK;
+}
+
+int aicam_frame_table_set_regions(aicam_frame_table* t, const int32_t* indices_host, const aicam_stream_region* host, int n,
+                                  void* stream) {
+  if (!t || n < 0 || (n > 0 && (!indices_host || !host)))
+    return fail(AICAM_ERR_INVALID_ARG, "frame_table_set_regions: null argument or negative count");
+  // validated as a whole before anything is stored, allocated or copied
+  for (int i = 0; i < n; ++i) {
+    const aicam_stream_region& r = host[i];
+    const std::string at = "frame_table_set_regions: entry " + std::to_string(i) + ": ";
+    if (indices_host[i] < 0 || indices_host[i] >= t->capacity) return fail(AICAM_ERR_INVALID_ARG, at + "index out of range");
+    if (r.n_polygons < 0 || r.n_polygons > AICAM_REGION_MAX_POLYGONS)
+      return fail(AICAM_ERR_INVALID_ARG, at + "n_polygons must be in 0..8");
+    for (int p = 0; p < r.n_polygons; ++p) {
+      const std::string pa = at + "polygon " + std::to_string(p) + ": ";
+      if (r.kind[p] != 0 && r.kind[p] != 1) return fail(AICAM_ERR_INVALID_ARG, pa + "kind must be 0 (include) or 1 (exclude)");
+      if (r.n_vertices[p] < 3 || r.n_vertices[p] > AICAM_COUNT_MAX_VERTICES)
+        return fail(AICAM_ERR_INVALID_ARG, pa + "must have 3..32 vertices");
+      for (int v = 0; v < r.n_vertices[p]; ++v)
+        for (int c = 0; c < 2; ++c)
+          if (r.xy[p][v][c] < -AICAM_COUNT_MAX_COORD || r.xy[p][v][c] > AICAM_COUNT_MAX_COORD)
+            return fail(AICAM_ERR_INVALID_ARG, pa + "coordinate beyond 2^20");
+    }
+  }
+  if (n == 0) return AICAM_OK;
+  AICAM_CUDA_OK(cudaSetDevice(t->device));
+  const size_t bytes = static_cast<size_t>(t->capacity) * sizeof(aicam_stream_region);
+  if (!t->regions_dev) {
+    const size_t keep_bytes = static_cast<size_t>(t->capacity) * (1024 / 8);
+    cudaError_t e = cudaMalloc(&t->regions_dev, bytes);
+    if (e == cudaSuccess) e = cudaMalloc(&t->region_keep, keep_bytes);
+    if (e == cudaSuccess) e = t->region_staging.create(bytes);
+    if (e != cudaSuccess) {
+      t->region_staging.destroy();
+      if (t->regions_dev) cudaFree(t->regions_dev);
+      if (t->region_keep) cudaFree(t->region_keep);
+      t->regions_dev = nullptr; t->region_keep = nullptr;
+      return fail(AICAM_ERR_CUDA, std::string("frame_table_set_regions: ") + cudaGetErrorString(e));
+    }
+    t->regions.assign(t->capacity, aicam_stream_region{});
+  }
+  std::vector<aicam_stream_region> next = t->regions;
+  bool any = false;
+  for (int i = 0; i < n; ++i) {
+    next[indices_host[i]] = host[i];
+    any |= host[i].n_polygons > 0;
+  }
+  uint8_t* h = nullptr;
+  AICAM_CUDA_OK(t->region_staging.acquire(&h));
+  std::memcpy(h, next.data(), bytes);
+  AICAM_CUDA_OK(t->region_staging.upload(t->regions_dev, bytes, static_cast<cudaStream_t>(stream)));
+  t->regions.swap(next);
+  t->region_test |= any;
   return AICAM_OK;
 }
 

@@ -16,6 +16,7 @@
 #include "common.cuh"
 #include "frame_src.cuh"
 #include "frame_table.cuh"
+#include "polygon.cuh"
 
 namespace aicam {
 
@@ -34,8 +35,10 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
                                                       int max_crops, int* __restrict__ det_index,
                                                       int* __restrict__ det_count, int* __restrict__ crop_slot,
                                                       int* __restrict__ crop_rect, int* __restrict__ crop_count,
-                                                      const FrameRec* __restrict__ recs) {  // frame table: per-frame (w, h)
-                                                                                            // and presence; or null
+                                                      const FrameRec* __restrict__ recs,  // frame table: per-frame (w, h)
+                                                                                          // and presence; or null
+                                                      const unsigned* __restrict__ region_keep,  // region_kernel's bits,
+                                                      const aicam_stream_region* __restrict__ regions) {  // or null
   __shared__ int s_scan[32];  // valid crops per frame of the current group of 32 frames, then their exclusive scan
   __shared__ int s_base;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -54,13 +57,15 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
       float mc = min_conf;
       unsigned long long mlo = mask_lo, mhi = mask_hi;
       if (recs && recs[b].filt) { mc = recs[b].min_conf; mlo = recs[b].mask_lo; mhi = recs[b].mask_hi; }
+      // the entry's region test (region_kernel) when it has polygons
+      const unsigned* rk = region_keep && regions[b].n_polygons > 0 ? region_keep + static_cast<long long>(b) * 32 : nullptr;
       for (int i0 = 0; i0 < n; i0 += 32) {
         const int i = i0 + lane;
         bool keep = false, ok = false;
         if (i < n) {
           const int cls = labels[fo + i];
           const bool tracked = cls >= 0 && cls < 128 && (((cls < 64 ? mlo >> cls : mhi >> (cls - 64)) & 1ull) != 0);
-          keep = scores[fo + i] >= mc && tracked;
+          keep = scores[fo + i] >= mc && tracked && (!rk || ((rk[i >> 5] >> (i & 31)) & 1u));
           if (keep) {
             const float4 bx = reinterpret_cast<const float4*>(boxes)[fo + i];
             const int x1 = max(0, static_cast<int>(bx.x)), y1 = max(0, static_cast<int>(bx.y));
@@ -121,6 +126,51 @@ __global__ void __launch_bounds__(1024) filter_kernel(const float* __restrict__ 
     // high-water mark of the crops WANTED (un-clamped): > max_crops means detections lost their feature to the
     // capacity (the reference always extracts one); sticky until the caller zeroes it
     if (s_base > crop_count[1]) crop_count[1] = s_base;
+  }
+}
+
+// The per-entry region test of aicam_frame_table_set_regions: one CTA per table entry, the entry's polygons in shared
+// memory, threads over its (detection, polygon) pairs.  Writes one keep bit per detection (bit i of word i / 32 of the
+// entry's 32 words); filter_kernel reads them for entries with polygons only, so absent entries and entries without
+// polygons leave at once.  The anchor is the only float arithmetic: one float32 sum (no contraction: --fmad=false) and
+// two floors; the test itself is counting's exact integer in_zone (polygon.cuh).
+constexpr int REGION_THREADS = 256;
+
+__global__ void __launch_bounds__(REGION_THREADS) region_kernel(const FrameRec* __restrict__ recs,
+                                                                const aicam_stream_region* __restrict__ regions,
+                                                                const float* __restrict__ boxes,
+                                                                const int* __restrict__ num_dets, int stride_k,
+                                                                unsigned* __restrict__ keep) {
+  __shared__ __align__(16) aicam_stream_region g;
+  __shared__ unsigned hits[1024];  // per detection: bit p = inside polygon p
+  const int b = blockIdx.x, tid = threadIdx.x;
+  if (recs[b].slot < 0 || regions[b].n_polygons <= 0) return;
+  {
+    const int* src = reinterpret_cast<const int*>(regions + b);
+    int* dst = reinterpret_cast<int*>(&g);
+    for (int i = tid; i < static_cast<int>(sizeof(aicam_stream_region) / 4); i += REGION_THREADS) dst[i] = src[i];
+  }
+  const int n = min(num_dets[b], stride_k);
+  for (int i = tid; i < n; i += REGION_THREADS) hits[i] = 0u;
+  __syncthreads();
+  const int np = g.n_polygons;
+  const long long fo = static_cast<long long>(b) * stride_k;
+  for (int q = tid; q < n * np; q += REGION_THREADS) {
+    const int i = q / np, p = q - i * np;
+    const float4 bx = reinterpret_cast<const float4*>(boxes)[fo + i];
+    const long long px = clamp_anchor(__float2ll_rd(__fadd_rn(bx.x, bx.z)));
+    const long long py = clamp_anchor(__float2ll_rd(__fmul_rn(2.0f, bx.w)));
+    if (in_zone(g.xy[p], g.n_vertices[p], px, py)) atomicOr(&hits[i], 1u << p);
+  }
+  __syncthreads();
+  unsigned inc = 0u, exc = 0u;
+  for (int p = 0; p < np; ++p) (g.kind[p] ? exc : inc) |= 1u << p;
+  for (int i0 = tid & ~31; i0 < n; i0 += REGION_THREADS) {  // whole warps: one ballot per 32 detections
+    const int i = i0 + (tid & 31);
+    const unsigned h = i < n ? hits[i] : 0u;
+    const bool k = i < n && (inc == 0u || (h & inc) != 0u) && (h & exc) == 0u;
+    const unsigned w = __ballot_sync(0xffffffffu, k);
+    if ((tid & 31) == 0) keep[static_cast<long long>(b) * 32 + (i0 >> 5)] = w;
   }
 }
 
@@ -397,7 +447,7 @@ int reid_crops_impl(const uint8_t* frames, int batch, int h, int w, const float*
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   filter_kernel<<<1, 1024, 0, st>>>(boxes, scores, labels, num_dets, batch, stride_k, h, w, min_confidence,
                                     class_mask_lo, class_mask_hi, max_crops, det_index, det_count, crop_slot, crop_rect,
-                                    crop_count, nullptr);
+                                    crop_count, nullptr, nullptr, nullptr);
   count_launch();
   if (int rc = last_launch("filter_kernel")) return rc;
   if (max_crops == 0 || !frames || !crops) return AICAM_OK;  // filter only
@@ -441,9 +491,18 @@ extern "C" int aicam_reid_crops_table(const aicam_frame_table* t, const float* b
   if (stride_k <= 0 || max_crops < 0 || (format < 0 || format > 2))
     return fail(AICAM_ERR_INVALID_ARG, "reid_crops_table: bad shape arguments");
   if (reinterpret_cast<uintptr_t>(boxes) % 16) return fail(AICAM_ERR_INVALID_ARG, "reid_crops_table: boxes must be 16-byte aligned");
+  if (t->region_test && stride_k > 1024)
+    return fail(AICAM_ERR_CAPACITY, "reid_crops_table: the region test takes at most 1024 detections per frame (stride_k)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (t->region_test && t->n > 0) {
+    region_kernel<<<t->n, REGION_THREADS, 0, st>>>(t->recs(), t->regions_dev, boxes, num_dets, stride_k, t->region_keep);
+    count_launch();
+    if (int rc = last_launch("region_kernel")) return rc;
+  }
+  const bool regions = t->region_test && t->n > 0;
   filter_kernel<<<1, 1024, 0, st>>>(boxes, scores, labels, num_dets, t->n, stride_k, 0, 0, min_confidence, class_mask_lo,
-                                    class_mask_hi, max_crops, det_index, det_count, crop_slot, crop_rect, crop_count, t->recs());
+                                    class_mask_hi, max_crops, det_index, det_count, crop_slot, crop_rect, crop_count, t->recs(),
+                                    regions ? t->region_keep : nullptr, regions ? t->regions_dev : nullptr);
   count_launch();
   if (int rc = last_launch("filter_kernel (table)")) return rc;
   if (max_crops == 0 || !crops) return AICAM_OK;  // filter only

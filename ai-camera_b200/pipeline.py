@@ -34,7 +34,10 @@ class StreamSettings:
     """One stream's detection and tracking settings: what a reference process takes as constructor arguments
     (``YOLODetector(conf_threshold, nms_threshold)``, ``DeepSORT(max_cosine_distance, max_iou_distance, max_age, n_init,
     min_detection_confidence)``) and the class names it tracks.  ``min_detection_confidence`` None resolves as
-    ``resolve_thresholds`` does."""
+    ``resolve_thresholds`` does.  ``include_regions`` / ``exclude_regions``: where in its frame the stream tracks, polygons of
+    3 to 32 integer frame-pixel (x, y) vertices, at most 8 in all; a detection is tracked when the bottom centre of its box
+    is inside some include polygon (or there is none) and inside no exclude polygon (include/aicam.h,
+    aicam_frame_table_set_regions)."""
     conf_threshold: float = config.YOLO_CONF_THRESHOLD
     nms_threshold: float = config.YOLO_NMS_THRESHOLD
     classes_to_track: FrozenSet[str] = frozenset(config.CLASSES_TO_TRACK)
@@ -43,6 +46,8 @@ class StreamSettings:
     max_iou_distance: float = config.DEEPSORT_MAX_IOU_DISTANCE
     max_age: int = config.DEEPSORT_MAX_AGE
     n_init: int = config.DEEPSORT_N_INIT
+    include_regions: Tuple[Tuple[Tuple[int, int], ...], ...] = ()
+    exclude_regions: Tuple[Tuple[Tuple[int, int], ...], ...] = ()
 
     def __post_init__(self):
         if isinstance(self.classes_to_track, str):
@@ -64,6 +69,11 @@ class StreamSettings:
             raise ValueError("max_age must be an integer in 1..255, got %r" % (self.max_age,))
         if not (isinstance(self.n_init, int) and self.n_init >= 1):
             raise ValueError("n_init must be an integer >= 1, got %r" % (self.n_init,))
+        for name in ("include_regions", "exclude_regions"):
+            object.__setattr__(self, name, _polygons(getattr(self, name), name))
+        if len(self.include_regions) + len(self.exclude_regions) > _lib.REGION_MAX_POLYGONS:
+            raise ValueError("at most %d include and exclude polygons per stream, got %d"
+                             % (_lib.REGION_MAX_POLYGONS, len(self.include_regions) + len(self.exclude_regions)))
 
     @classmethod
     def from_dict(cls, d, base: Optional["StreamSettings"] = None):
@@ -82,6 +92,20 @@ class StreamSettings:
         lo, hi = config.tracked_class_mask(self.classes_to_track)
         return (_lib.StreamFilter(score, self.nms_threshold, min_conf, 0, lo, hi),
                 _lib.StreamAssoc(float(self.max_cosine_distance), float(self.max_iou_distance), self.max_age, self.n_init))
+
+    def has_regions(self):
+        return bool(self.include_regions or self.exclude_regions)
+
+    def resolve_region(self):
+        """The aicam_stream_region of these settings' include and exclude polygons."""
+        r = _lib.StreamRegion()
+        polygons = [(0, p) for p in self.include_regions] + [(1, p) for p in self.exclude_regions]
+        r.n_polygons = len(polygons)
+        for i, (kind, pts) in enumerate(polygons):
+            r.kind[i], r.n_vertices[i] = kind, len(pts)
+            for k, (x, y) in enumerate(pts):
+                r.xy[i][k][:] = [x, y]
+        return r
 
 
 def _filter_key(f):
@@ -107,6 +131,21 @@ def _point(p, what):
         if abs(v) > _lib.COUNT_MAX_COORD:
             raise ValueError("%s: coordinates are limited to +-2^20, got %r" % (what, p))
     return (int(p[0]), int(p[1]))
+
+
+def _polygons(v, what):
+    """A tuple of polygons (tuples of 3 to 32 integer (x, y) vertices) from a sequence of them."""
+    if isinstance(v, str) or not isinstance(v, (tuple, list)):
+        raise ValueError("%s must be a list of polygons, got %r" % (what, v))
+    out = []
+    for poly in v:
+        if isinstance(poly, str) or not isinstance(poly, (tuple, list)):
+            raise ValueError("%s: a polygon is a list of (x, y) vertices, got %r" % (what, poly))
+        pts = tuple(_point(p, what + " vertex") for p in poly)
+        if not 3 <= len(pts) <= _lib.COUNT_MAX_VERTICES:
+            raise ValueError("%s: a polygon needs 3 to %d vertices, got %d" % (what, _lib.COUNT_MAX_VERTICES, len(pts)))
+        out.append(pts)
+    return tuple(out)
 
 
 def _classes(classes):
@@ -347,6 +386,7 @@ class FrameTable:
         self.frames = []
         self.present_ptr = C.c_void_p(self.lib.aicam_frame_table_present(self._h))
         self.filters = None
+        self.region_test = False  # some entry has had polygons: each table crop step launches the region test
 
     def set_filters(self, filters: Optional[Sequence["_lib.StreamFilter"]]):
         """Per-entry detection and filter settings (aicam_frame_table_set_filters): entry i < len(filters) is detected
@@ -356,6 +396,19 @@ class FrameTable:
         arr = (_lib.StreamFilter * n)(*filters) if n else None
         _lib.check(self.lib.aicam_frame_table_set_filters(self._h, arr, n))
         self.filters = list(filters) if n else None
+
+    def set_regions(self, indices, regions: Sequence["_lib.StreamRegion"]):
+        """Entries ``indices`` take ``regions`` (aicam_stream_region records; n_polygons 0 clears one) from the next
+        step on, eager or captured; the other entries keep theirs.  One copy on the current stream."""
+        indices = [int(i) for i in indices]
+        n = len(indices)
+        if len(regions) != n:
+            raise ValueError("set_regions: one region per index")
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_frame_table_set_regions(self._h, (C.c_int32 * n)(*indices),
+                                                              (_lib.StreamRegion * n)(*regions), n,
+                                                              _lib.stream_ptr(self.device)))
+        self.region_test |= any(r.n_polygons > 0 for r in regions)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -535,6 +588,8 @@ class BatchTracker:
         # step hands them to the frame table, a stacked step whose streams differ goes through the table
         self._filters = None
         self._routed = False
+        # per-stream regions of configure_streams (None until some stream has had polygons), handed to the frame table
+        self._regions = None
         # optional running totals (crops, reported tracks) kept on the device, for benchmarks: no host sync
         self.count_stats = False
         self.crop_total = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -578,8 +633,16 @@ class BatchTracker:
         for i, (f, _) in zip(indices, resolved):
             filters[i] = f
         self._filters = filters
+        if self._regions is not None or any(s.has_regions() for s in settings):
+            if self._regions is None:
+                self._regions = [_lib.StreamRegion() for _ in range(self.S)]
+            for i, s in zip(indices, settings):
+                self._regions[i] = s.resolve_region()
+            if self.frame_table is not None:
+                self.frame_table.set_regions(indices, [self._regions[i] for i in indices])
         key = _filter_key(base)[2:]
-        self._routed = any(_filter_key(f)[2:] != key for f in filters)
+        # (once some stream has had a region, every step runs the region test over the table)
+        self._routed = any(_filter_key(f)[2:] != key for f in filters) or self._regions is not None
 
     def update(self, frames, num_dets, boxes, scores, labels):
         """One frame per stream.  frames uint8 cuda [S,H,W,3] BGR or [S,H*3/2,W] NV12, or a list of S frames of any
@@ -593,6 +656,8 @@ class BatchTracker:
         if is_frame_list(frames):
             if self.frame_table is None:
                 self.frame_table = FrameTable(self.device, self.S, self.max_frame_hw)
+                if self._regions is not None:
+                    self.frame_table.set_regions(range(self.S), self._regions)
             if self._filters is not None:
                 self.frame_table.set_filters(self._filters)
             self.frame_table.set(frames)
@@ -659,7 +724,9 @@ class BatchTracker:
         return ints[:n], floats[:n]
 
     def launches_per_step(self):
-        return 2 + self.reid.launches_per_forward() - (1 if self._nhwc8 else 0) + 3  # no NHWC8 repack kernel
+        # (no NHWC8 repack kernel; the region test once some stream has had a region)
+        return (2 + self.reid.launches_per_forward() - (1 if self._nhwc8 else 0) + 3 +
+                (1 if self._regions is not None else 0))
 
 
 class TrackingPipeline:
@@ -704,7 +771,8 @@ class TrackingPipeline:
         """Give the streams ``indices`` their own StreamSettings (one per index, or one for all) from the next step on,
         with or without a reset, whether the step runs eager or from a captured graph (call it between replays, like
         ``frame_table.set``).  The other streams are untouched; a stream's existing tracks keep the n_init and max_age
-        they were created with, as in the reference."""
+        they were created with, as in the reference.  The first settings with regions add the region test to every step
+        from then on; a step captured before that does not include it, so capture again after the first region."""
         indices, settings = _as_settings_list(indices, settings)
         for i in indices:
             if not 0 <= i < self.n_streams:
@@ -714,8 +782,10 @@ class TrackingPipeline:
             self.settings[i] = st
         filters = [st.resolve()[0] for st in self.settings]
         self.frame_table.set_filters(filters)
+        if self.frame_table.region_test or any(st.has_regions() for st in settings):
+            self.frame_table.set_regions(indices, [st.resolve_region() for st in settings])
         base = _filter_key(self.default_settings.resolve()[0])
-        self._routed = any(_filter_key(f) != base for f in filters)
+        self._routed = any(_filter_key(f) != base for f in filters) or self.frame_table.region_test
 
     def configure_counting(self, indices, counting):
         """Give the streams ``indices`` their counting lines and zones (one StreamCounting or None per index, or one for
@@ -797,6 +867,7 @@ class TrackingPipeline:
 
     def launches_per_step(self, frame_list=False):
         """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True), absent frames
-        or not.  A stacked tensor runs as a list while streams detect or filter differently; the counter adds one."""
+        or not.  A stacked tensor runs as a list while streams detect or filter differently or once some stream has had a
+        region; the region test adds one from then on, the counter one."""
         return (self.detector.launches_per_step(frame_list or self._routed) + self.tracker.launches_per_step() +
                 (1 if self.counter is not None else 0))

@@ -258,6 +258,34 @@ typedef struct {
   uint64_t class_mask_lo, class_mask_hi;
 } aicam_stream_filter;
 int aicam_frame_table_set_filters(aicam_frame_table* t, const aicam_stream_filter* host, int n);
+/* Per-stream regions: where in its frame a stream tracks (a door camera whose top third shows a street, a parking camera
+ * facing a screen or a poster).  Each entry may carry up to AICAM_REGION_MAX_POLYGONS polygons of 3 to
+ * AICAM_COUNT_MAX_VERTICES integer frame-pixel vertices (|v| <= AICAM_COUNT_MAX_COORD), each an include (kind 0) or an
+ * exclude (kind 1) polygon.  aicam_reid_crops_table then keeps a detection only when, besides passing the entry's
+ * confidence and class filter, its anchor is inside at least one include polygon (or the entry has none) and inside no
+ * exclude polygon.  A detection that fails is treated as if detect() had not returned it: no det_index entry, no crop,
+ * no part in tracking; the crop rows of the others stay in scan order.
+ *   anchor  the bottom centre of boxes_orig's (x1, y1, x2, y2), doubled: PX = floor(x1 + x2) with the sum rounded to
+ *           float32, PY = floor(2 * y2), each clamped to +-2^24 (as counting's anchor)
+ *   inside  counting's zone test: even-odd rule, half-open edges, exact int64 arithmetic on doubled vertices
+ * aicam_frame_table_set_regions: entry indices_host[i] takes host[i] (i < n, host arrays); the other entries keep
+ *   theirs and n_polygons == 0 clears an entry.  The whole call is validated first; AICAM_ERR_INVALID_ARG (nothing
+ *   stored, copied or launched) for an index outside 0..capacity-1, n_polygons outside 0..8, a kind other than 0 / 1, a
+ *   vertex count outside 3..32 or a coordinate beyond AICAM_COUNT_MAX_COORD.  On success it copies the table's region
+ *   block (capacity records) to the device with one asynchronous copy on `stream` from pinned staging.  Not capturable;
+ *   captured steps read the block, so they follow its changes, absent or not.
+ * Once any entry of the table has had polygons, aicam_reid_crops_table makes one more launch (the region test, one CTA
+ * per entry) before its filter, whatever the regions are later; a step captured before that does not include it, so
+ * capture again after the first region.  With regions, stride_k is limited to 1024 (AICAM_ERR_CAPACITY). */
+#define AICAM_REGION_MAX_POLYGONS 8
+typedef struct {
+  int32_t n_polygons;
+  int32_t kind[AICAM_REGION_MAX_POLYGONS];        /* 0 include, 1 exclude */
+  int32_t n_vertices[AICAM_REGION_MAX_POLYGONS];
+  int32_t xy[AICAM_REGION_MAX_POLYGONS][32][2];   /* 32 = AICAM_COUNT_MAX_VERTICES */
+} aicam_stream_region;
+int aicam_frame_table_set_regions(aicam_frame_table* t, const int32_t* indices_host, const aicam_stream_region* host, int n,
+                                  void* stream);
 /* aicam_preprocess / aicam_preprocess_nv12 over a frame table (formats 0-3): present frame i's slice of `out` is slice p(i)
  * (packed, see above; slice i when all frames are present) and equals the uniform entry on that frame alone; slices past
  * the present count are not written.  Frames whose geometry is a pure decimation (1080p) and whose planes, pitch and row
