@@ -79,6 +79,17 @@ class CounterOutput(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("line_counts", "zone_counts", "occupancy", "row_zones", "events", "event_count")]
 
 
+DWELL_MAX_LOITER = 1 << 30
+
+
+class StreamDwell(C.Structure):
+    _fields_ = [("enabled", C.c_int32), ("loiter_frames", C.c_int32 * COUNT_MAX_ZONES)]
+
+
+class CounterDwellOutput(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("visits", "frames_total", "frames_max", "row_dwell", "events", "event_count")]
+
+
 class OverlayItem(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("type", "x1", "y1", "x2", "y2", "color", "slot", "reserved")]
 
@@ -166,6 +177,10 @@ SIGNATURES = {
     "aicam_counter_reset_streams": (_I, [_P, _P, _P]),
     "aicam_counter_outputs": (_I, [_P, C.POINTER(CounterOutput)]),
     "aicam_counter_overflow": (_I, [_P, _P]),
+    "aicam_counter_set_dwell": (_I, [_P, _P, C.POINTER(StreamDwell), _I, _P]),
+    "aicam_counter_dwell_step": (_I, [_P, _P, _P, _P, _P, _P]),
+    "aicam_counter_dwell_outputs": (_I, [_P, C.POINTER(CounterDwellOutput)]),
+    "aicam_counter_dwell_overflow": (_I, [_P, _P]),
     "aicam_lsap": (_I, [_P, _I, _I, _I, _P, _P]),
     "aicam_kf_gating": (_I, [_P, _P, _I, _I, _P, _P]),
     "aicam_overlay_draw": (_I, [_P, _I, _I, _I, _P, _P, _P, _I, _I, _P]),

@@ -29,7 +29,10 @@ Differences, all in the direction of the hardware:
     same ``{"default": {...}, "<input file name>": {...}}`` shape (values: ``pipeline.StreamCounting.from_dict``
     objects; an input's "lines" / "zones" replace those of "default").  Each track line of ``.tracks.jsonl`` then
     carries the step's ``"events"``, ``<stem>.counts.json`` holds each input's totals (summed from the events), and
-    ``--save_video`` adds one panel line per counting line or zone.
+    ``--save_video`` adds one panel line per counting line or zone.  An input object with ``"dwell": true``, or a zone
+    with ``"loiter_frames"``, also measures how long tracks stay in its zones: track lines carry the step's
+    ``"dwell_events"`` (completed visits and loiter alerts, in the stream's frames) and each zone of ``counts.json`` its
+    ``visits``, ``frames_total`` and ``frames_max`` per class, summed from them.
 """
 import argparse
 import json
@@ -77,7 +80,8 @@ def parse_arguments(argv=None) -> argparse.Namespace:
     parser.add_argument("--counting", type=str, default=None,
                         help="Batched mode: JSON file {\"default\": {...}, \"<input file name>\": {...}} of per-input "
                              "counting lines and zones ({\"lines\": [{\"a\": [x, y], \"b\": [x, y], \"name\": .., "
-                             "\"classes\": [..]}], \"zones\": [{\"points\": [[x, y], ...], ...}]}).")
+                             "\"classes\": [..]}], \"zones\": [{\"points\": [[x, y], ...], \"loiter_frames\": n, ...}], "
+                             "\"dwell\": true}).")
     args = parser.parse_args(argv)
     if args.device == "cpu":
         parser.error("this build has no CPU path (the reference's TensorRT engines do not run on CPU either)")
@@ -129,11 +133,23 @@ class CountTotals:
         self.counting = counting
         self.lines = {x.name: {"in": {}, "out": {}} for x in counting.lines}
         self.zones = {x.name: {"entered": {}, "exited": {}} for x in counting.zones}
+        if counting.dwell:
+            for z in self.zones.values():
+                z.update(visits={}, frames_total={}, frames_max={})
 
     def add(self, events):
         for e in events:
             d = (self.lines if e["kind"] in ("in", "out") else self.zones)[e["name"]][e["kind"]]
             d[e["class"]] = d.get(e["class"], 0) + 1
+
+    def add_dwell(self, events):
+        for e in events:
+            if e["kind"] != "visit":
+                continue
+            z, c = self.zones[e["name"]], e["class"]
+            z["visits"][c] = z["visits"].get(c, 0) + 1
+            z["frames_total"][c] = z["frames_total"].get(c, 0) + e["frames"]
+            z["frames_max"][c] = max(z["frames_max"].get(c, 0), e["frames"])
 
     def as_dict(self):
         return {"lines": self.lines, "zones": self.zones}
@@ -153,6 +169,23 @@ def step_events(pipe):
         evs = counter.events[s, :n].cpu().tolist() if n and c is not None else []
         out.append([{"kind": EVENT_KINDS[k], "name": (c.lines if k < 2 else c.zones)[i].name, "id": tid,
                      "class": config.CLASSES[cls]} for k, i, tid, cls in evs])
+    return out
+
+
+DWELL_KINDS = ("visit", "loiter")
+
+
+def step_dwell_events(pipe):
+    """Per stream, the dwell events of the step that has just completed, with the names of their zones."""
+    counter = pipe.counter
+    if not counter.has_dwell:
+        return [[] for _ in range(pipe.n_streams)]
+    out = []
+    for s, n in enumerate(counter.dwell_event_count.cpu().tolist()):
+        c = pipe.counting[s]
+        evs = counter.dwell_events[s, :n].cpu().tolist() if n and c is not None else []
+        out.append([{"kind": DWELL_KINDS[k], "name": c.zones[z].name, "id": tid, "class": config.CLASSES[cls], "frames": fr}
+                    for k, z, tid, cls, fr in evs])
     return out
 
 
@@ -430,6 +463,7 @@ def main(argv=None):
                     tabs = [t.numpy() for t in table]
                     fps = stats_ref[0].fps() * args.streams if stats_ref else 0.0
                     events = step_events(pipe) if totals else None
+                    dwell = step_dwell_events(pipe) if totals else None
                     for s in range(args.streams):
                         rows = tracks_to_rows(tabs, s)
                         line = {"frame": step, "stream": s, "tracks": rows}
@@ -437,6 +471,9 @@ def main(argv=None):
                         if totals:
                             line["events"] = events[s]
                             totals[s].add(events[s])
+                            if totals[s].counting.dwell:
+                                line["dwell_events"] = dwell[s]
+                                totals[s].add_dwell(dwell[s])
                             panel += totals[s].panel_lines()
                         writer.write(json.dumps(line) + "\n")
                         if videos:
@@ -530,6 +567,7 @@ def _run_all_inputs(args, pipe, inputs, writer, out_dir, stem, videos, device):
     def on_step(step, batch, table):
         tabs = [t.numpy() for t in table] if writer else None
         events = step_events(pipe) if writer and totals else None
+        dwell = step_dwell_events(pipe) if writer and totals else None
         for s, f in enumerate(batch):
             if f is None:
                 continue
@@ -543,6 +581,9 @@ def _run_all_inputs(args, pipe, inputs, writer, out_dir, stem, videos, device):
                 if totals:
                     line["events"] = events[s]
                     totals[i].add(events[s])
+                    if totals[i].counting.dwell:
+                        line["dwell_events"] = dwell[s]
+                        totals[i].add_dwell(dwell[s])
                 writer.write(json.dumps(line) + "\n")
                 if videos:
                     fps = stats_ref[0].fps() * N if stats_ref else 0.0

@@ -37,6 +37,19 @@ struct CounterDev {
   int* event_count; int* overflow;    // [S]
 };
 
+// Dwell (include/aicam.h, "Dwell"): every pointer null until the first aicam_counter_set_dwell.
+struct DwellDev {
+  const aicam_stream_dwell* cfg;      // [S]
+  const int* restart;                 // [S], right after cfg in one allocation: the streams the last set call enabled
+  int* clock;                         // [S]
+  int* st_id; unsigned* st_bits;      // [S][T]: bits 0..15 open visits, 16..31 alerted visits
+  int* st_entry;                      // [S][T][NZ]
+  int64_t* visits; int64_t* frames_total; int64_t* frames_max;  // [S][NZ][NCLS]
+  int* row_dwell;                     // [S][T][NZ]
+  int* events;                        // [S][E][5]
+  int* event_count; int* overflow;    // [S]
+};
+
 __device__ __forceinline__ bool class_in(const uint64_t* mask, int cls) {
   return cls >= 0 && cls < NCLS && ((cls < 64 ? mask[0] >> cls : mask[1] >> (cls - 64)) & 1ull);
 }
@@ -165,6 +178,143 @@ __global__ void counter_reset_kernel(CounterDev c, const int* __restrict__ mask)
   if (threadIdx.x == 0) { c.event_count[s] = 0; c.overflow[s] = 0; }
 }
 
+// One CTA per stream, one thread per row, after count_kernel of the same step: reads its row_zones and the zone class
+// masks.  Per row the open and alerted bits and entry[16] live in registers (loops over zones fully unrolled); durations
+// are added with integer atomics, events laid out in row order by the same block scan as count_kernel.
+__global__ void __launch_bounds__(COUNT_THREADS) dwell_kernel(CounterDev c, DwellDev w, const int* __restrict__ out_tracks,
+                                                              const int* __restrict__ out_count,
+                                                              const int* __restrict__ row_slot,
+                                                              const int* __restrict__ present) {
+  __shared__ uint64_t zmask[NZ][2];
+  __shared__ int loiter[NZ];
+  __shared__ int warp_sum[COUNT_THREADS / 32];
+  __shared__ int clock_s, nz_s;
+  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if ((present && !present[s]) || !w.cfg[s].enabled) {  // nothing of the stream changes, its clock included
+    if (tid == 0) w.event_count[s] = 0;
+    return;
+  }
+  if (tid < NZ) {
+    zmask[tid][0] = c.geom[s].zone_class_mask[tid][0];
+    zmask[tid][1] = c.geom[s].zone_class_mask[tid][1];
+    loiter[tid] = w.cfg[s].loiter_frames[tid];
+  }
+  if (tid == 0) {
+    clock_s = w.clock[s] + 1;
+    w.clock[s] = clock_s;
+    nz_s = c.geom[s].n_zones;
+  }
+  __syncthreads();
+  const int f = clock_s, nz = nz_s;
+  const long long sT = static_cast<long long>(s) * c.T;
+  const int n = max(0, min(out_count[s], c.T));
+  const long long sz = static_cast<long long>(s) * NZ * NCLS;
+  int* ev = w.events + static_cast<long long>(s) * c.E * 5;
+  int base = 0;
+  for (int r0 = 0; r0 < n; r0 += COUNT_THREADS) {
+    const int r = r0 + tid;
+    unsigned closed = 0, alert = 0;  // bit z: a visit of zone z completed / alerted at this row
+    int id = 0, cls = 0;
+    int val[NZ];  // frames since entry (the duration, for a completed visit)
+    if (r < n) {
+      const int* row = out_tracks + (sT + r) * 6;
+      id = row[4];
+      cls = row[5];
+      const unsigned zb = c.row_zones[sT + r];
+      const int slot = row_slot[sT + r];
+      const bool valid = slot >= 0 && slot < c.T;  // (a row without a slot is a first report and keeps no state)
+      const long long ss = sT + (valid ? slot : 0);
+      const bool first = !valid || w.st_id[ss] != id;
+      unsigned bits = first ? 0u : w.st_bits[ss];
+      int4* ep = reinterpret_cast<int4*>(w.st_entry + ss * NZ);
+      int entry[NZ];
+#pragma unroll
+      for (int q = 0; q < NZ / 4; ++q) {
+        const int4 e = first ? make_int4(0, 0, 0, 0) : ep[q];
+        entry[4 * q] = e.x; entry[4 * q + 1] = e.y; entry[4 * q + 2] = e.z; entry[4 * q + 3] = e.w;
+      }
+      unsigned shown = 0;  // zones whose row_dwell entry is val
+#pragma unroll
+      for (int z = 0; z < NZ; ++z) {
+        val[z] = -1;
+        if (z >= nz || !class_in(zmask[z], cls)) continue;
+        const unsigned ob = 1u << z, ab = 1u << (16 + z);
+        if ((zb >> z) & 1u) {
+          if (!(bits & ob)) { bits = (bits | ob) & ~ab; entry[z] = f; }
+          val[z] = f - entry[z];
+          shown |= ob;
+          if (loiter[z] > 0 && val[z] >= loiter[z] && !(bits & ab)) { bits |= ab; alert |= ob; }
+        } else if (bits & ob) {
+          val[z] = f - entry[z];
+          bits &= ~(ob | ab);
+          closed |= ob;
+          const long long k = sz + z * NCLS + cls;
+          atomicAdd(reinterpret_cast<unsigned long long*>(w.visits + k), 1ull);
+          atomicAdd(reinterpret_cast<unsigned long long*>(w.frames_total + k), static_cast<unsigned long long>(val[z]));
+          atomicMax(reinterpret_cast<long long*>(w.frames_max + k), static_cast<long long>(val[z]));
+        }
+      }
+      int4* rd = reinterpret_cast<int4*>(w.row_dwell + (sT + r) * NZ);
+#pragma unroll
+      for (int q = 0; q < NZ / 4; ++q) {
+        int o[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) o[k] = (shown >> (4 * q + k)) & 1u ? val[4 * q + k] : -1;
+        rd[q] = make_int4(o[0], o[1], o[2], o[3]);
+      }
+      if (valid) {
+        w.st_id[ss] = id;
+        w.st_bits[ss] = bits;
+#pragma unroll
+        for (int q = 0; q < NZ / 4; ++q)
+          ep[q] = make_int4(entry[4 * q], entry[4 * q + 1], entry[4 * q + 2], entry[4 * q + 3]);
+      }
+    }
+    const int nev = __popc(closed | alert);
+    int incl = nev;
+    for (int o = 1; o < 32; o <<= 1) {
+      const int v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += v;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    int before = 0, total = 0;
+    for (int q = 0; q < COUNT_THREADS / 32; ++q) {
+      const int v = warp_sum[q];
+      if (q < warp) before += v;
+      total += v;
+    }
+    int at = base + before + incl - nev;
+#pragma unroll
+    for (int z = 0; z < NZ; ++z) {
+      if (!(((closed | alert) >> z) & 1u) || at >= c.E) continue;
+      int* e = ev + 5ll * at;
+      e[0] = (closed >> z) & 1u ? 0 : 1; e[1] = z; e[2] = id; e[3] = cls; e[4] = val[z];
+      ++at;
+    }
+    base += total;
+    __syncthreads();  // (warp_sum is rewritten by the next tile)
+  }
+  if (tid == 0) {
+    w.event_count[s] = min(base, c.E);
+    if (base > c.E) w.overflow[s] = 1;
+  }
+}
+
+// Restart the dwell state of the streams whose mask entry is non-zero (null: every stream); settings are kept.
+__global__ void dwell_reset_kernel(CounterDev c, DwellDev w, const int* __restrict__ mask) {
+  const int s = blockIdx.x;
+  if (mask && !mask[s]) return;
+  const long long sT = static_cast<long long>(s) * c.T;
+  for (int k = threadIdx.x; k < c.T; k += blockDim.x) { w.st_id[sT + k] = 0; w.st_bits[sT + k] = 0u; }
+  for (int k = threadIdx.x; k < c.T * NZ; k += blockDim.x) w.row_dwell[sT * NZ + k] = -1;
+  for (int i = threadIdx.x; i < NZ * NCLS; i += blockDim.x) {
+    const long long k = static_cast<long long>(s) * NZ * NCLS + i;
+    w.visits[k] = 0; w.frames_total[k] = 0; w.frames_max[k] = 0;
+  }
+  if (threadIdx.x == 0) { w.clock[s] = 0; w.event_count[s] = 0; w.overflow[s] = 0; }
+}
+
 bool coord_ok(int32_t v) { return v >= -AICAM_COUNT_MAX_COORD && v <= AICAM_COUNT_MAX_COORD; }
 bool mask_ok(const uint64_t* m) { return (m[1] >> (NCLS - 64)) == 0; }
 
@@ -199,6 +349,10 @@ struct aicam_counter {
   uint8_t* upload = nullptr;                // device: geom [S] then the set mask i32 [S]
   aicam::PinnedStaging staging;             // of aicam_counter_set_streams
   std::vector<void*> allocs;
+  aicam::DwellDev w{};                      // dwell: allocated by the first aicam_counter_set_dwell
+  std::vector<aicam_stream_dwell> dwell;    // host copy of w.cfg (empty until then)
+  uint8_t* dwell_upload = nullptr;          // device: cfg [S] then the restart mask i32 [S]
+  aicam::PinnedStaging dwell_staging;       // of aicam_counter_set_dwell
 };
 
 using namespace aicam;
@@ -216,10 +370,48 @@ int counter_alloc(aicam_counter* c, Tp** p, size_t n) {
   return AICAM_OK;
 }
 
+size_t dwell_upload_bytes(int S) { return static_cast<size_t>(S) * (sizeof(aicam_stream_dwell) + sizeof(int32_t)); }
+
+int launch_dwell_reset(aicam_counter* c, const int32_t* mask, cudaStream_t st) {
+  dwell_reset_kernel<<<c->d.S, 256, 0, st>>>(c->d, c->w, mask);
+  count_launch();
+  return last_launch("dwell_reset_kernel");
+}
+
+// (the dwell restart is a launch of its own, made only once dwell is set, so that counting alone launches as before)
 int launch_reset(aicam_counter* c, const int32_t* mask, cudaStream_t st) {
   counter_reset_kernel<<<c->d.S, 256, 0, st>>>(c->d, mask);
   count_launch();
-  return last_launch("counter_reset_kernel");
+  if (int rc = last_launch("counter_reset_kernel")) return rc;
+  return c->w.cfg ? launch_dwell_reset(c, mask, st) : AICAM_OK;
+}
+
+int dwell_alloc(aicam_counter* c) {
+  DwellDev w{};
+  const int S = c->d.S;
+  const size_t ST = static_cast<size_t>(S) * c->d.T, SZK = static_cast<size_t>(S) * NZ * NCLS;
+  int rc = 0;
+  rc |= counter_alloc(c, &c->dwell_upload, dwell_upload_bytes(S));
+  rc |= counter_alloc(c, &w.clock, S);
+  rc |= counter_alloc(c, &w.st_id, ST); rc |= counter_alloc(c, &w.st_bits, ST); rc |= counter_alloc(c, &w.st_entry, ST * NZ);
+  rc |= counter_alloc(c, &w.visits, SZK); rc |= counter_alloc(c, &w.frames_total, SZK); rc |= counter_alloc(c, &w.frames_max, SZK);
+  rc |= counter_alloc(c, &w.row_dwell, ST * NZ);
+  rc |= counter_alloc(c, &w.events, static_cast<size_t>(S) * c->d.E * 5);
+  rc |= counter_alloc(c, &w.event_count, S); rc |= counter_alloc(c, &w.overflow, S);
+  if (rc) return AICAM_ERR_CUDA;
+  if (cudaMemset(w.row_dwell, 0xff, ST * NZ * sizeof(int)) != cudaSuccess)
+    return fail(AICAM_ERR_CUDA, "counter_set_dwell: cudaMemset failed");
+  if (c->dwell_staging.create(dwell_upload_bytes(S)) != cudaSuccess) {
+    c->dwell_staging.destroy();
+    return fail(AICAM_ERR_CUDA, "counter_set_dwell: pinned staging failed");
+  }
+  // (the zeroing above runs on the legacy stream: finish it before work on the caller's stream reads the buffers)
+  if (cudaDeviceSynchronize() != cudaSuccess) return fail(AICAM_ERR_CUDA, "counter_set_dwell: synchronise failed");
+  w.cfg = reinterpret_cast<const aicam_stream_dwell*>(c->dwell_upload);
+  w.restart = reinterpret_cast<const int*>(c->dwell_upload + static_cast<size_t>(S) * sizeof(aicam_stream_dwell));
+  c->w = w;
+  c->dwell.assign(S, aicam_stream_dwell{});
+  return AICAM_OK;
 }
 }  // namespace
 
@@ -261,6 +453,7 @@ void aicam_counter_destroy(aicam_counter* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   c->staging.destroy();
+  c->dwell_staging.destroy();
   for (void* p : c->allocs) cudaFree(p);
   delete c;
 }
@@ -316,6 +509,73 @@ int aicam_counter_overflow(aicam_counter* c, int32_t* flags_host) {
   AICAM_CUDA_OK(cudaSetDevice(c->device));
   AICAM_CUDA_OK(cudaDeviceSynchronize());
   AICAM_CUDA_OK(cudaMemcpy(flags_host, c->d.overflow, sizeof(int32_t) * c->d.S, cudaMemcpyDeviceToHost));
+  return AICAM_OK;
+}
+
+int aicam_counter_set_dwell(aicam_counter* c, const int32_t* indices_host, const aicam_stream_dwell* host, int n,
+                            void* stream) {
+  if (!c || n < 0 || (n > 0 && (!indices_host || !host)))
+    return fail(AICAM_ERR_INVALID_ARG, "counter_set_dwell: null argument or negative count");
+  const int S = c->d.S;
+  // validated as a whole before anything is allocated, stored or copied
+  std::vector<aicam_stream_dwell> next = c->dwell.empty() ? std::vector<aicam_stream_dwell>(S, aicam_stream_dwell{}) : c->dwell;
+  for (int i = 0; i < n; ++i) {
+    const std::string at = "counter_set_dwell: entry " + std::to_string(i) + ": ";
+    if (indices_host[i] < 0 || indices_host[i] >= S) return fail(AICAM_ERR_INVALID_ARG, at + "stream index out of range");
+    if (host[i].enabled != 0 && host[i].enabled != 1) return fail(AICAM_ERR_INVALID_ARG, at + "enabled must be 0 or 1");
+    for (int z = 0; z < NZ; ++z)
+      if (host[i].loiter_frames[z] < 0 || host[i].loiter_frames[z] > AICAM_DWELL_MAX_LOITER)
+        return fail(AICAM_ERR_INVALID_ARG, at + "loiter_frames[" + std::to_string(z) + "] must be in 0..2^30");
+    next[indices_host[i]] = host[i];
+  }
+  if (n == 0) return AICAM_OK;
+  AICAM_CUDA_OK(cudaSetDevice(c->device));
+  if (!c->w.cfg)
+    if (int rc = dwell_alloc(c)) return rc;
+  std::vector<int32_t> restart(S, 0);  // disabled -> enabled: the stream's dwell state starts
+  bool any = false;
+  for (int k = 0; k < S; ++k) {
+    restart[k] = next[k].enabled && !c->dwell[k].enabled;
+    any |= restart[k] != 0;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  uint8_t* h = nullptr;
+  AICAM_CUDA_OK(c->dwell_staging.acquire(&h));
+  const size_t cbytes = next.size() * sizeof(aicam_stream_dwell);
+  std::memcpy(h, next.data(), cbytes);
+  std::memcpy(h + cbytes, restart.data(), restart.size() * sizeof(int32_t));
+  AICAM_CUDA_OK(c->dwell_staging.upload(c->dwell_upload, dwell_upload_bytes(S), st));
+  c->dwell.swap(next);
+  return any ? launch_dwell_reset(c, c->w.restart, st) : AICAM_OK;
+}
+
+int aicam_counter_dwell_step(aicam_counter* c, const int32_t* out_tracks, const int32_t* out_count, const int32_t* row_slot,
+                             const int32_t* present, void* stream) {
+  if (!c || !out_tracks || !out_count || !row_slot) return fail(AICAM_ERR_INVALID_ARG, "counter_dwell_step: null argument");
+  if (!c->w.cfg) return fail(AICAM_ERR_INVALID_ARG, "counter_dwell_step: dwell is not set (aicam_counter_set_dwell)");
+  dwell_kernel<<<c->d.S, COUNT_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(c->d, c->w, out_tracks, out_count, row_slot,
+                                                                                present);
+  count_launch();
+  return last_launch("dwell_kernel");
+}
+
+int aicam_counter_dwell_outputs(const aicam_counter* c, aicam_counter_dwell_output* out) {
+  if (!c || !out) return fail(AICAM_ERR_INVALID_ARG, "counter_dwell_outputs: null argument");
+  if (!c->w.cfg) return fail(AICAM_ERR_INVALID_ARG, "counter_dwell_outputs: dwell is not set (aicam_counter_set_dwell)");
+  const DwellDev& w = c->w;
+  *out = aicam_counter_dwell_output{w.visits, w.frames_total, w.frames_max, w.row_dwell, w.events, w.event_count};
+  return AICAM_OK;
+}
+
+int aicam_counter_dwell_overflow(aicam_counter* c, int32_t* flags_host) {
+  if (!c || !flags_host) return fail(AICAM_ERR_INVALID_ARG, "counter_dwell_overflow: null argument");
+  if (!c->w.cfg) {
+    std::memset(flags_host, 0, sizeof(int32_t) * c->d.S);
+    return AICAM_OK;
+  }
+  AICAM_CUDA_OK(cudaSetDevice(c->device));
+  AICAM_CUDA_OK(cudaDeviceSynchronize());
+  AICAM_CUDA_OK(cudaMemcpy(flags_host, c->w.overflow, sizeof(int32_t) * c->d.S, cudaMemcpyDeviceToHost));
   return AICAM_OK;
 }
 

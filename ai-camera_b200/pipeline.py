@@ -196,10 +196,12 @@ class CountingLine:
 @dataclass(frozen=True)
 class CountingZone:
     """A counting zone: a polygon of 3 to 32 integer vertices (even-odd rule; may be concave or self-intersecting).
-    ``classes`` as for CountingLine."""
+    ``classes`` as for CountingLine.  ``loiter_frames``: a track that stays in the zone for that many of its stream's
+    frames raises one loiter event per visit (0: none); setting it turns dwell on for the stream (StreamCounting)."""
     points: Tuple[Tuple[int, int], ...]
     name: Optional[str] = None
     classes: Optional[FrozenSet[str]] = None
+    loiter_frames: Optional[int] = None
 
     def __post_init__(self):
         if isinstance(self.points, str) or not hasattr(self.points, "__len__"):
@@ -211,6 +213,9 @@ class CountingZone:
         if self.name is not None and not isinstance(self.name, str):
             raise ValueError("name must be a string, got %r" % (self.name,))
         object.__setattr__(self, "classes", _classes(self.classes))
+        v = self.loiter_frames
+        if v is not None and (isinstance(v, bool) or not isinstance(v, int) or not 0 <= v <= _lib.DWELL_MAX_LOITER):
+            raise ValueError("loiter_frames must be an integer in 0..2^30, got %r" % (v,))
 
     @classmethod
     def from_dict(cls, d):
@@ -220,14 +225,20 @@ class CountingZone:
 @dataclass(frozen=True)
 class StreamCounting:
     """One stream's counting lines and zones (at most 16 of each).  Unnamed ones are called ``line{i}`` / ``zone{i}``
-    after their index; names are unique within the stream."""
+    after their index; names are unique within the stream.  ``dwell``: also measure how long tracks stay in the zones
+    (include/aicam.h, "Dwell"); a zone with ``loiter_frames`` turns it on."""
     lines: Tuple[CountingLine, ...] = ()
     zones: Tuple[CountingZone, ...] = ()
+    dwell: bool = False
 
     def __post_init__(self):
         lines, zones = tuple(self.lines), tuple(self.zones)
         if not all(isinstance(x, CountingLine) for x in lines) or not all(isinstance(x, CountingZone) for x in zones):
             raise ValueError("lines must be CountingLine and zones CountingZone objects")
+        if not isinstance(self.dwell, bool):
+            raise ValueError("dwell must be true or false, got %r" % (self.dwell,))
+        if any(x.loiter_frames is not None for x in zones):
+            object.__setattr__(self, "dwell", True)
         if len(lines) > _lib.COUNT_MAX_LINES or len(zones) > _lib.COUNT_MAX_ZONES:
             raise ValueError("at most %d lines and %d zones per stream" % (_lib.COUNT_MAX_LINES, _lib.COUNT_MAX_ZONES))
         lines = tuple(x if x.name is not None else replace(x, name="line%d" % i) for i, x in enumerate(lines))
@@ -242,10 +253,10 @@ class StreamCounting:
     @classmethod
     def from_dict(cls, d):
         """From ``{"lines": [{"a": [x, y], "b": [x, y], "name": .., "classes": [..]}], "zones": [{"points": [[x, y],
-        ..], ..}]}`` (e.g. a JSON object)."""
+        ..], "loiter_frames": n, ..}], "dwell": true}`` (e.g. a JSON object)."""
         if not isinstance(d, dict):
             raise ValueError("StreamCounting: expected an object, got %r" % (d,))
-        unknown = set(d) - {"lines", "zones"}
+        unknown = set(d) - {"lines", "zones", "dwell"}
         if unknown:
             raise ValueError("unknown counting fields: %s" % sorted(unknown))
 
@@ -254,7 +265,7 @@ class StreamCounting:
             if not isinstance(v, list):
                 raise ValueError("%s must be a list" % key)
             return tuple(kind.from_dict(x) for x in v)
-        return cls(items("lines", CountingLine), items("zones", CountingZone))
+        return cls(items("lines", CountingLine), items("zones", CountingZone), d.get("dwell", False))
 
     def resolve(self, default_classes):
         """The aicam_stream_counting of this geometry; lines and zones without classes count ``default_classes``."""
@@ -269,6 +280,14 @@ class StreamCounting:
                 g.zone_xy[i][k][:] = [px, py]
             g.zone_class_mask[i][:] = config.tracked_class_mask(x.classes if x.classes is not None else default_classes)
         return g
+
+    def resolve_dwell(self):
+        """The aicam_stream_dwell of these settings."""
+        d = _lib.StreamDwell()
+        d.enabled = int(self.dwell)
+        for i, x in enumerate(self.zones):
+            d.loiter_frames[i] = x.loiter_frames or 0
+        return d
 
 
 class _DeviceArray:
@@ -298,7 +317,11 @@ class StreamCounter:
       line_counts int64 [S, 16, 2, 80] (in, out per class), zone_counts int64 [S, 16, 2, 80] (entries, exits),
       occupancy int32 [S, 16, 80], row_zones int32 [S, T] (zone bits of row n of out_tracks), events int32
       [S, max_events, 4] (kind 0 line in, 1 line out, 2 zone entry, 3 zone exit; index; track id; class) and
-      event_count int32 [S] of the last step."""
+      event_count int32 [S] of the last step.
+    Dwell (after the first ``set_dwell``; None before): visits, frames_total, frames_max int64 [S, 16, 80] (completed
+    visits per zone and class, their summed and largest durations in frames), row_dwell int32 [S, T, 16] (frames since
+    entry of row n's open visit in each zone, -1 for none), dwell_events int32 [S, max_events, 5] (kind 0 visit
+    completed, 1 loiter; zone; track id; class; frames) and dwell_event_count int32 [S] of the last step."""
 
     def __init__(self, device, n_streams: int, max_tracks: int, max_events: int = 1024):
         self.lib = _lib.load()
@@ -317,10 +340,51 @@ class StreamCounter:
         self.row_zones = view(o.row_zones, (self.S, self.T), "<i4")  # (bits 0..15: never negative)
         self.events = view(o.events, (self.S, self.E, 4), "<i4")
         self.event_count = view(o.event_count, (self.S,), "<i4")
+        self.visits = self.frames_total = self.frames_max = self.row_dwell = None
+        self.dwell_events = self.dwell_event_count = None
 
     @property
     def handle(self):
         return self._handle.h
+
+    @property
+    def has_dwell(self):
+        """Dwell is set up (some set_dwell call has succeeded): the dwell buffers exist."""
+        return self.visits is not None
+
+    def set_dwell(self, indices, settings: Sequence["_lib.StreamDwell"]):
+        """Streams ``indices`` take the dwell ``settings`` (aicam_stream_dwell records); a stream that was disabled and
+        is enabled starts its dwell state, an enabled one whose thresholds change keeps it."""
+        n = len(indices)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_counter_set_dwell(self.handle, (C.c_int32 * n)(*indices), (_lib.StreamDwell * n)(*settings),
+                                                        n, _lib.stream_ptr(self.device)))
+        if self.visits is None and n:
+            o = _lib.CounterDwellOutput()
+            _lib.check(self.lib.aicam_counter_dwell_outputs(self.handle, C.byref(o)))
+            Z, K = _lib.COUNT_MAX_ZONES, _lib.COUNT_CLASSES
+
+            def view(ptr, shape, typestr):
+                return torch.as_tensor(_DeviceArray(self._handle, ptr, shape, typestr), device=self.device)
+            self.visits = view(o.visits, (self.S, Z, K), "<i8")
+            self.frames_total = view(o.frames_total, (self.S, Z, K), "<i8")
+            self.frames_max = view(o.frames_max, (self.S, Z, K), "<i8")
+            self.row_dwell = view(o.row_dwell, (self.S, self.T, Z), "<i4")
+            self.dwell_events = view(o.events, (self.S, self.E, 5), "<i4")
+            self.dwell_event_count = view(o.event_count, (self.S,), "<i4")
+
+    def dwell_step(self, out_tracks, out_count, row_slot, present=None):
+        """The dwell step of the rows ``step`` has just counted (same arguments, after it)."""
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.aicam_counter_dwell_step(self.handle, _lib.ptr(out_tracks), _lib.ptr(out_count), row_slot,
+                                                         present, _lib.stream_ptr(self.device)))
+
+    def dwell_overflow(self):
+        """Sticky per-stream flags: some dwell step had more events than max_events (the dwell counters stayed exact)."""
+        import numpy as np
+        f = np.zeros(self.S, np.int32)
+        _lib.check(self.lib.aicam_counter_dwell_overflow(self.handle, _lib.ptr(f)))
+        return f
 
     def set_streams(self, indices, geometry: Sequence["_lib.StreamCounting"]):
         """Streams ``indices`` take ``geometry`` (aicam_stream_counting records); their counts and tracks restart."""
@@ -793,7 +857,9 @@ class TrackingPipeline:
         ``frame_table.set``).  Their counters and occupancy restart at zero and their tracks are counted from their next
         report on, as first reports; the other streams are untouched.  The first call that gives a stream counting
         creates the counter: from then on every step launches it once after the tracker.  A step captured before that
-        does not include the counter, so capture again after turning counting on."""
+        does not include the counter, so capture again after turning counting on.  Dwell (StreamCounting.dwell, or a zone
+        with loiter_frames) is set or cleared with the geometry; the first stream with dwell adds the dwell launch to
+        every step from then on, and likewise a step captured before it does not include it."""
         indices = [int(i) for i in indices]
         if counting is None or isinstance(counting, StreamCounting):
             counting = [counting] * len(indices)
@@ -809,6 +875,8 @@ class TrackingPipeline:
             self.counter = StreamCounter(self.device, self.n_streams, self.tracker.T, self.max_events)
         geometry = [(c or StreamCounting()).resolve(self.tracker.classes_to_track) for c in counting]
         self.counter.set_streams(indices, geometry)
+        if self.counter.has_dwell or any(c is not None and c.dwell for c in counting):
+            self.counter.set_dwell(indices, [(c or StreamCounting()).resolve_dwell() for c in counting])
         for i, c in zip(indices, counting):
             self.counting[i] = c
 
@@ -834,6 +902,8 @@ class TrackingPipeline:
         if self.counter is not None:
             out_tracks, _, out_count = tables
             self.counter.step(out_tracks, out_count, self.tracker.row_slots, present)
+            if self.counter.has_dwell:
+                self.counter.dwell_step(out_tracks, out_count, self.tracker.row_slots, present)
         return tables
 
     def counts(self):
@@ -855,9 +925,27 @@ class TrackingPipeline:
                                          "occupancy": by_class(occ[s, i])} for i, x in enumerate(c.zones)}}
         return out
 
+    def dwell(self):
+        """Per stream with dwell, the visits completed since the stream's dwell state last started (its counting was set
+        or reset, or dwell turned on), per zone and class: ``{zone name: {"visits": {class: n}, "frames_total": {...},
+        "frames_max": {...}}}``, durations in the stream's own frames, zeros omitted ({} for a stream without dwell).
+        Synchronises."""
+        out = [{} for _ in range(self.n_streams)]
+        if self.counter is None or not self.counter.has_dwell:
+            return out
+        v, ft, fm = (x.cpu().numpy() for x in (self.counter.visits, self.counter.frames_total, self.counter.frames_max))
+
+        def by_class(a):
+            return {config.CLASSES[k]: int(a[k]) for k in range(len(a)) if a[k]}
+        for s, c in enumerate(self.counting):
+            if c is not None and c.dwell:
+                out[s] = {x.name: {"visits": by_class(v[s, i]), "frames_total": by_class(ft[s, i]),
+                                   "frames_max": by_class(fm[s, i])} for i, x in enumerate(c.zones)}
+        return out
+
     def reset_streams(self, indices, settings=None):
         """Hand the given stream slots to new sources: their trackers restart (no tracks, ids from 1) and so do their
-        counts, the other streams and the captured step are untouched.  The slots keep their settings and counting
+        counts and dwell, the other streams and the captured step are untouched.  The slots keep their settings and counting
         geometry, or take ``settings`` (as configure_streams)."""
         if settings is not None:
             self.configure_streams(indices, settings)
@@ -868,6 +956,6 @@ class TrackingPipeline:
     def launches_per_step(self, frame_list=False):
         """Kernel launches of one step: of a stacked tensor, or of a list of frames (frame_list=True), absent frames
         or not.  A stacked tensor runs as a list while streams detect or filter differently or once some stream has had a
-        region; the region test adds one from then on, the counter one."""
+        region; the region test adds one from then on, the counter one, dwell one more."""
         return (self.detector.launches_per_step(frame_list or self._routed) + self.tracker.launches_per_step() +
-                (1 if self.counter is not None else 0))
+                (1 if self.counter is not None else 0) + (1 if self.counter is not None and self.counter.has_dwell else 0))

@@ -537,7 +537,8 @@ void aicam_counter_destroy(aicam_counter* c);
  * maxima, a zone of fewer than 3 vertices, a zero-length line, a coordinate beyond AICAM_COUNT_MAX_COORD, an index outside
  * 0..n_streams-1 are AICAM_ERR_INVALID_ARG and nothing is copied or launched.  Then one asynchronous copy on `stream` from
  * pinned staging and the masked reset of those streams (as aicam_counter_reset_streams).  Not capturable; captured steps
- * read the table, so they follow its changes. */
+ * read the table, so they follow its changes.  Once dwell is set, the reset restarts their dwell state too (one more
+ * launch; their dwell settings are kept). */
 int aicam_counter_set_streams(aicam_counter* c, const int32_t* indices_host, const aicam_stream_counting* host, int n,
                               void* stream);
 /* One launch, capturable, no host synchronisation: counts the rows out_tracks i32 [S][max_tracks][6] / out_count i32 [S]
@@ -549,11 +550,80 @@ int aicam_counter_step(aicam_counter* c, const int32_t* out_tracks, const int32_
                        const int32_t* present, void* stream);
 /* Zero the counters, occupancy and overflow flag of the streams whose entry of the device mask i32[S] is non-zero and
  * forget their tracks (each track's next report is a first report); one launch, capturable.  It must accompany every
- * aicam_tracker_reset_streams of a stream: ids restart at 1 there, and a new track could otherwise continue an old one. */
+ * aicam_tracker_reset_streams of a stream: ids restart at 1 there, and a new track could otherwise continue an old one.
+ * Once dwell is set, a second launch restarts the dwell state of those streams (clock, visits, counters, overflow flag;
+ * their dwell settings are kept). */
 int aicam_counter_reset_streams(aicam_counter* c, const int32_t* mask, void* stream);
 int aicam_counter_outputs(const aicam_counter* c, aicam_counter_output* out);
 /* Sticky per-stream event-overflow flags since the stream's last reset (host out i32[S]); synchronises. */
 int aicam_counter_overflow(aicam_counter* c, int32_t* flags_host);
+
+/* ------------------------------------------------------------------------------------------
+ * Dwell: how long tracks stay in the counting zones of a stream, and loitering alerts, in one more capturable launch
+ * after aicam_counter_step (queue wait at a checkout, a vehicle's time in a loading bay, someone staying too long by a
+ * door).  Integer rules, on counting's zone membership and class masks:
+ *   clock    each stream with dwell enabled has a frame clock f: the number of present steps of the stream since its
+ *            dwell state last started, this step included (1 at the first).  The state starts when dwell is enabled for
+ *            the stream and again at aicam_counter_set_streams / aicam_counter_reset_streams of it.  An absent step does
+ *            not advance the clock and changes nothing.  All times are in the stream's own frames (a stream present at
+ *            every other step of a 30 fps fleet counts 15 per second); int32: 2^31 present steps.
+ *   state    per (stream, tracker slot): track id, a bit set of the zones with an open visit, a bit set of the visits
+ *            already alerted, entry[16] (the clock at each open visit's entry).  A row whose id differs from its slot's
+ *            stored id is a first report: the visits still open from the slot's previous occupant are dropped without
+ *            being counted (as counting makes no exit for a track deleted inside a zone).  A row without a valid slot is
+ *            a first report and keeps no state.
+ *   per row and zone z < n_zones, with in = bit z of the row's row_zones entry:
+ *            class not in the zone's class mask: the visit state of z is left as it is; the row reports -1 for z.
+ *            in, no open visit: a visit opens, entry = f.
+ *            not in, open visit: it closes with duration d = f - entry (>= 1): visits[z][cls] += 1,
+ *              frames_total[z][cls] += d, frames_max[z][cls] = max(.., d), and a visit event.
+ *            in, open visit, loiter_frames[z] = L > 0, f - entry >= L, not yet alerted: a loiter event, and the visit is
+ *              alerted (once per visit, at its first report at or past L; L = 0: no alerts).
+ *   A track not reported at a step (missed, tentative) keeps its open visits, and their clock keeps running.
+ * ---------------------------------------------------------------------------------------- */
+#define AICAM_DWELL_MAX_LOITER (1 << 30)
+typedef struct {
+  int32_t enabled;                                  /* 0 or 1 */
+  int32_t loiter_frames[AICAM_COUNT_MAX_ZONES];     /* 0..AICAM_DWELL_MAX_LOITER; 0 = no alerts */
+} aicam_stream_dwell;
+/* Device outputs, stable for the counter's lifetime once dwell is set; entries of enabled streams present at the last
+ * dwell step:
+ *   visits, frames_total, frames_max  i64 [S][MAX_ZONES][80]  completed visits per zone and class since the stream's
+ *                                                             dwell state last started, their summed and largest
+ *                                                             durations in frames
+ *   row_dwell         i32 [S][max_tracks][MAX_ZONES]  frames since entry of row n's open visit in zone z (0 at the
+ *                                                     entry step), -1 otherwise; aligned with out_tracks
+ *   events            i32 [S][max_events][5]  (kind, zone, track id, class, frames): kind 0 visit completed (frames =
+ *                                             its duration), 1 loiter (frames = f - entry); ordered by row, then zone
+ *   event_count       i32 [S]                 events of the last step (at most max_events; 0 for a disabled or absent
+ *                                             stream) */
+typedef struct {
+  int64_t* visits;
+  int64_t* frames_total;
+  int64_t* frames_max;
+  int32_t* row_dwell;
+  int32_t* events;
+  int32_t* event_count;
+} aicam_counter_dwell_output;
+/* Stream indices_host[i] takes the dwell settings host[i] (host arrays, i < n): validated as a whole first - enabled
+ * not 0 or 1, loiter_frames outside 0..AICAM_DWELL_MAX_LOITER, an index outside 0..n_streams-1 are AICAM_ERR_INVALID_ARG
+ * and nothing is allocated, copied or launched.  The first valid call allocates the dwell buffers (a counter that never
+ * sets dwell allocates and launches nothing more).  Then one asynchronous copy on `stream` from pinned staging; a stream
+ * that goes from disabled to enabled starts its dwell state (one launch), an enabled stream whose thresholds change keeps
+ * it.  Not capturable; captured dwell steps read the settings, so they follow their changes. */
+int aicam_counter_set_dwell(aicam_counter* c, const int32_t* indices_host, const aicam_stream_dwell* host, int n,
+                            void* stream);
+/* One launch, capturable, no host synchronisation: the dwell step of the rows aicam_counter_step has just counted, with
+ * the same out_tracks, out_count, row_slot and present, on the same stream after it (it reads the counter's row_zones
+ * and zone class masks).  Disabled and absent streams change nothing.  Events beyond max_events are dropped and set the
+ * stream's sticky dwell-overflow flag; the counters stay exact.  AICAM_ERR_INVALID_ARG before aicam_counter_set_dwell. */
+int aicam_counter_dwell_step(aicam_counter* c, const int32_t* out_tracks, const int32_t* out_count, const int32_t* row_slot,
+                             const int32_t* present, void* stream);
+/* AICAM_ERR_INVALID_ARG before aicam_counter_set_dwell. */
+int aicam_counter_dwell_outputs(const aicam_counter* c, aicam_counter_dwell_output* out);
+/* Sticky per-stream dwell event-overflow flags since the stream's dwell state last started (host out i32[S], all 0
+ * before aicam_counter_set_dwell); synchronises. */
+int aicam_counter_dwell_overflow(aicam_counter* c, int32_t* flags_host);
 
 /* Stand-alone pieces of the association, exposed for bit-exact parity tests. */
 /* scipy.optimize.linear_sum_assignment (linear_assignment.py:62) on `count` fp32 cost
