@@ -34,6 +34,9 @@ constexpr int MAX_SORT = 16384;
 // class logits; a warp reads 8 consecutive head rows (8 x 576 B, every sector fully used).  The softmax
 // expectation is a register loop (no shuffles); two shuffle rounds merge the class argmax
 // (lowest index on ties) and gather the four distances.
+// VEC: every head row starts on a 16-byte boundary (64 + nc a multiple of 4, head 16-byte aligned) and the logits are
+// read as float4; otherwise (nc = 1, 2, 3, 601, ...) every logit is a scalar load.
+template <bool VEC>
 __global__ void __launch_bounds__(256) decode_kernel(const float* __restrict__ head, int anchors, int nc, int total,
                                                      float* __restrict__ boxes, float* __restrict__ scores,
                                                      int* __restrict__ labels) {
@@ -44,10 +47,15 @@ __global__ void __launch_bounds__(256) decode_kernel(const float* __restrict__ h
   const int gw = live ? gw_raw : total - 1;  // tail lanes recompute the last anchor (the shuffles need a full warp)
   const float* row = head + static_cast<long long>(gw) * (AICAM_HEAD_DFL + nc);
   float v[16];
+  if (VEC) {
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float4 q = __ldg(reinterpret_cast<const float4*>(row + 16 * k) + i);
-    v[4 * i] = q.x; v[4 * i + 1] = q.y; v[4 * i + 2] = q.z; v[4 * i + 3] = q.w;
+    for (int i = 0; i < 4; ++i) {
+      const float4 q = __ldg(reinterpret_cast<const float4*>(row + 16 * k) + i);
+      v[4 * i] = q.x; v[4 * i + 1] = q.y; v[4 * i + 2] = q.z; v[4 * i + 3] = q.w;
+    }
+  } else {
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = __ldg(row + 16 * k + i);
   }
   float m = v[0];
 #pragma unroll
@@ -66,7 +74,7 @@ __global__ void __launch_bounds__(256) decode_kernel(const float* __restrict__ h
   float best = -INFINITY;
   int bi = 0x7fffffff;
   const float* cls = row + AICAM_HEAD_DFL;
-  if ((nc & 3) == 0) {
+  if (VEC) {
     for (int c = c_lo; c < c_hi; c += 4) {
       const float4 q = __ldg(reinterpret_cast<const float4*>(cls + c));
       if (q.x > best) { best = q.x; bi = c; }
@@ -354,14 +362,14 @@ size_t aicam_decode_nms_workspace(int batch, int anchors, const aicam_nms_params
 
 int aicam_decode(const float* head, int batch, int anchors, int nc, float* boxes, float* scores, int32_t* labels,
                  void* stream) {
-  if (!head || !boxes || !scores || !labels || batch < 0) return fail(AICAM_ERR_INVALID_ARG, "decode: bad arguments");
+  if (!head || !boxes || !scores || !labels || batch < 0 || nc < 1) return fail(AICAM_ERR_INVALID_ARG, "decode: bad arguments");
   if (anchors != 8400) return fail(AICAM_ERR_UNSUPPORTED, "decode: only the 640x640 anchor grid (8400) is supported");
   if (batch == 0) return AICAM_OK;
   const int total = batch * anchors;
-  if ((AICAM_HEAD_DFL + nc) % 4 != 0 || reinterpret_cast<uintptr_t>(head) % 16 != 0)
-    return fail(AICAM_ERR_INVALID_ARG, "decode: head rows must be 16-byte aligned");
-  decode_kernel<<<cdiv(total * 4, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(head, anchors, nc, total, boxes,
-                                                                                    scores, labels);
+  const bool vec = (AICAM_HEAD_DFL + nc) % 4 == 0 && reinterpret_cast<uintptr_t>(head) % 16 == 0;
+  const int grid = cdiv(total * 4, 256);
+  if (vec) decode_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(head, anchors, nc, total, boxes, scores, labels);
+  else decode_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(head, anchors, nc, total, boxes, scores, labels);
   count_launch();
   return last_launch("decode_kernel");
 }

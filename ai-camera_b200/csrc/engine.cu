@@ -308,10 +308,13 @@ struct Builder {
     const int lvl_in[3] = {o3, o4, o5};
     const int lvl_c[3] = {c3, c4, c5};
     const int lvl_h[3] = {h8, h16, h32};
+    // the class branch's buffers: a convolution reads channels in groups of 8, so their channel stride is cc rounded up to 8
+    // (cc = 100 for nc >= 100 on yolov8n); the pad channels stay zero (buf) and meet zero weights
+    const int ccs = (cc + 7) / 8 * 8;
     long long anchor_base = 0;
     for (int l = 0; l < 3; ++l) {
       const int hh = lvl_h[l];
-      const int b1 = buf(hh, hh, cb), b2 = buf(hh, hh, cb), k1 = buf(hh, hh, cc), k2 = buf(hh, hh, cc);
+      const int b1 = buf(hh, hh, cb), b2 = buf(hh, hh, cb), k1 = buf(hh, hh, ccs), k2 = buf(hh, hh, ccs);
       const std::string p2 = "model.22.cv2." + std::to_string(l), p3 = "model.22.cv3." + std::to_string(l);
       const long long eoff = anchor_base * e->out_cstride;
       conv(p2 + ".0.conv", V(lvl_in[l]), hh, hh, V(b1), lvl_c[l], cb, 3, 1, 1);

@@ -297,7 +297,7 @@ int aicam_preprocess_table(const aicam_frame_table* t, int format, void* out, vo
  * num_dets/bboxes/scores/labels, yolo_detector.py:49-54,108-112) and the part of
  * YOLODetector.detect after the engine (yolo_detector.py:107-149, scale_bboxes
  * image_processing.py:141-183).
- *   head        : fp32 [batch][anchors][64+nc]
+ *   head        : fp32 [batch][anchors][64+nc], any nc >= 1 (rows need not be 16-byte aligned)
  *   num_dets    : i32 [batch]
  *   boxes_lb    : fp32 [batch][topk][4] xyxy in letterbox pixels (engine output)
  *   boxes_orig  : fp32 [batch][topk][4] xyxy in frame pixels, clipped (detect() output), may be NULL

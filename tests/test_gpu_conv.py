@@ -24,6 +24,15 @@ CASES = [
     ("bigk_512", 4, 8, 4, 512, 512, 3, 1, 2, 0, False),
     ("1x1s2_down", 2, 16, 8, 64, 128, 1, 2, 0, 0, False),
     ("yolo_160_c32", 2, 160, 160, 32, 32, 3, 1, 1, 0, False),
+    # unstaged epilogue: rows that are not a multiple of 16 bytes (Detect heads at class counts other than 80), stored
+    # and, with a residual, read one channel at a time
+    ("rows40B_3x3_20", 2, 20, 20, 32, 20, 3, 1, 1, 0, False),
+    ("rows40B_1x1_20_res1", 2, 20, 20, 64, 20, 1, 1, 1, 1, False),
+    ("rows200B_3x3_100_res1", 1, 20, 20, 100, 100, 3, 1, 1, 1, False),
+    ("rows200B_1x1_100", 2, 20, 20, 100, 100, 1, 1, 1, 0, False),
+    ("rows40B_3x3s2_20", 2, 33, 31, 32, 20, 3, 2, 1, 0, False),
+    ("f32_rows4B_1x1_1", 2, 40, 40, 64, 1, 1, 1, 0, 0, True),
+    ("f32_rows12B_1x1_3", 2, 20, 20, 100, 3, 1, 1, 0, 0, True),
     # window kernel (conv_win.cu): patch rasters with strips, every swizzle width, resident and
     # streamed weights, one and two accumulators per tile, residual modes, fp32 output
     ("win_reid_l1", 3, 64, 32, 64, 64, 3, 1, 2, 2, False),

@@ -57,16 +57,43 @@ def test_nms_keep_set_bit_exact(A, n_hot, topk, max_cand):
 
 
 def test_decode_matches_oracle():
+    _check_decode(80)
+
+
+@pytest.mark.parametrize("nc", [1, 3, 4, 12, 100, 601])
+def test_decode_matches_oracle_at_class_count(nc):
+    _check_decode(nc)
+
+
+def _check_decode(nc):
+    """decode_kernel at any class count: float4 loads when 64 + nc is a multiple of 4, scalar loads otherwise (head
+    rows of 65, 67 or 665 floats).  Each thread of an anchor scans a quarter of the classes (`per` classes each);
+    exact ties planted across the quarter boundaries must go to the lowest index."""
     import gpu_util as G
     from oracle import detect_post
-    rng = np.random.default_rng(5)
-    head = rng.normal(0, 2.0, (2, 8400, 144)).astype(np.float32)
+    rng = np.random.default_rng(5 + nc)
+    head = rng.normal(0, 2.0, (2, 8400, 64 + nc)).astype(np.float32)
     head[0, :, 64:] -= 3.0
-    head[1, 5, 64 + 7] = head[1, 5, 64 + 3] = 9.0  # class tie -> lowest index
+    per = ((nc + 3) // 4 + 3) // 4 * 4
+    starts = [q * per for q in range(1, 4) if q * per < nc]
+    # class lists; the lowest of each must win
+    ties = [[min(3, nc - 1), min(7, nc - 1)], [0, nc - 1], [0] + starts, starts, [nc - 1, nc // 2]]
+    ties += [[s - 1, s] for s in starts] + [[s, min(nc - 1, s + per)] for s in starts]
+    ties = [sorted(set(t)) for t in ties if len(set(t)) > 1]
+    planted = []
+    anchors = rng.choice(np.arange(6, 8400), len(ties), replace=False)
+    for t, a in zip(ties, [5] + list(anchors[1:])):
+        for b in range(2):
+            head[b, a, 64:] = np.minimum(head[b, a, 64:], 8.0)
+            head[b, a, [64 + c for c in t]] = 12.0
+            planted.append((b, a, t[0]))
     boxes, scores, labels = G.decode(torch.from_numpy(head).to(G.DEV))
     for b in range(2):
         wb, ws, wl = detect_post.decode(head[b])
         assert np.array_equal(labels[b].cpu().numpy(), wl)
         assert np.allclose(scores[b].cpu().numpy(), ws, rtol=1e-5, atol=1e-6)
         assert np.allclose(boxes[b].cpu().numpy(), wb, rtol=1e-4, atol=1e-3)
-    assert labels[1, 5].item() == 3
+    assert labels.min().item() >= 0 and labels.max().item() < nc
+    assert planted or nc == 1
+    for b, a, want in planted:
+        assert labels[b, a].item() == want, (b, a, want)

@@ -3,9 +3,10 @@
 ReID: one engine of capacity 4 096 (64 streams) through aicam_reid_forward_nhwc8, the call of a batched step, with the
 crop count changing on the same buffers, eagerly and from a CUDA graph whose own kernel writes the count right before
 the network (as the crop kernel writes crop_count inside a captured step).  YOLOv8n: a 64-entry frame table of 1080p
-frames through aicam_preprocess_table format 3 and aicam_yolo_detect_table (4x4-block stem, fused decode) with 64, 37,
-1 and 64 present frames.  Everything past the count is poisoned with NaN; what lies below it must be bit-identical with
-the full run, and samples must match the fp32 oracle nets."""
+frames through aicam_preprocess_table format 3 and aicam_yolo_detect_table (4x4-block stem; fused decode at 80 classes,
+the fp32 head tensor and decode_kernel at 20) with 64, 37, 1 and 64 present frames.  Everything past the count is
+poisoned with NaN; what lies below it must be bit-identical with the full run, and samples must match the fp32 oracle
+nets."""
 import ctypes as C
 
 import numpy as np
@@ -142,18 +143,31 @@ def test_reid_at_product_capacity_under_changing_counts(blobs):
 
 
 def test_yolov8n_frame_table_of_64_1080p_frames_under_present_counts(blobs):
+    """80 classes: the decode runs inside the Detect-head epilogues."""
+    _frame_table_under_present_counts(blobs[0], 80)
+
+
+def test_yolov8n_frame_table_without_fused_decode(tmp_path):
+    """20 classes: no fused decode, so the network writes the fp32 head tensor and decode_kernel reads it.  The dense
+    arrays sit in the same workspace layout, so the checks are those of the 80-class run."""
+    from ai_camera_b200 import weights as W
+    yolo = str(tmp_path / "yolov8n_nc20.aicw")
+    W.write_blob(yolo, *W.synth_yolov8_weights("n", nc=20, seed=0))
+    _frame_table_under_present_counts(yolo, 20)
+
+
+def _frame_table_under_present_counts(yolo, nc):
     from ai_camera_b200 import synth
     from ai_camera_b200.pipeline import BatchDetector, FrameTable
     from oracle import detect_post, image_ops
     from oracle.pipeline import Detector
-    yolo, _ = blobs
     S, A = 64, 8400
     lib = _lib()
     det = BatchDetector(yolo, S)
     bias = synth.shifted_class_bias(yolo, -0.6)
     synth.apply_class_bias(det.engine, bias)
     e = det.engine
-    assert det._s2d == 2 and e.fused_decode
+    assert det._s2d == 2 and e.fused_decode == (nc == 80) and (e._head is None) == (nc == 80)
     video = synth.SynthVideo(S, (1080, 1920), n_frames=1, device=DEV, seed=808)
     frames = [video.ring[0, s] for s in range(S)]
     table = FrameTable(DEV, S, (1080, 1920))
@@ -170,7 +184,7 @@ def test_yolov8n_frame_table_of_64_1080p_frames_under_present_counts(blobs):
         e._nhwc.view(torch.int16).view(S, -1)[count:] = 0x7FC0  # bf16 NaN in the input slots past the present count
         e._ws.fill_(0)
         det.num_dets.fill_(-1)
-        _check(lib.aicam_yolo_detect_table(e.handle, _ptr(e._nhwc), 2, table.handle, C.byref(det._nms), None,
+        _check(lib.aicam_yolo_detect_table(e.handle, _ptr(e._nhwc), 2, table.handle, C.byref(det._nms), _ptr(e._head),
                                            _ptr(det.num_dets), _ptr(det.boxes_lb), _ptr(det.boxes), _ptr(det.scores),
                                            _ptr(det.labels), _ptr(e._ws), e._ws.numel(), None))
         torch.cuda.synchronize()
@@ -181,6 +195,7 @@ def test_yolov8n_frame_table_of_64_1080p_frames_under_present_counts(blobs):
         runs.append((present, dense, rows))
     (_, dense0, rows0) = runs[0]
     assert int((rows0[0] > 0).sum()) >= S // 2, "too few frames with detections to compare"
+    assert int(dense0[2].min()) >= 0 and int(dense0[2].max()) < nc and int(rows0[4].max()) < nc
     for present, dense, rows in runs[1:]:
         slots = np.nonzero(present)[0]
         for j, b in enumerate(slots):

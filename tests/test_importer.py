@@ -87,6 +87,34 @@ def test_yolov8_onnx_import_named_and_unfused(tmp_path, scale):
     assert np.array_equal(back["model.22.cv3.1.2.bias"], ck["model.22.cv3.1.2.bias"])
 
 
+@pytest.mark.parametrize("nc", [1, 20, 601])
+def test_yolov8_state_dict_import_at_class_count(tmp_path, nc):
+    """A fine-tuned checkpoint carries its class count in model.22.cv3.0.2.weight: the blob header says nc, the class
+    branch is cc = max(c3, min(nc, 100)) wide, and the oracle net gives (B, 8400, 64 + nc) head rows."""
+    from oracle import nets
+    specs = W.yolov8_conv_specs("n", nc)
+    ck = _unfused(specs, W.KIND_YOLOV8, 11, 1e-3)
+    path = tmp_path / "best.pt"
+    torch.save({"model": {k: torch.from_numpy(np.asarray(v)) for k, v in ck.items()}}, path)
+    blob = tmp_path / "yolo.aicw"
+    kind, params, out = importer.import_file(str(path), str(blob))
+    k2, p2, back = W.read_blob(str(blob))
+    assert kind == k2 == W.KIND_YOLOV8 and p2 == params and params[7] == nc
+    D = W.yolov8_dims("n", nc)
+    cc = max(D["c"][2], min(nc, 100))  # c3 = 64: 64, 64, 100
+    assert D["cc"] == cc
+    for l, c in enumerate(D["c"][2:5]):
+        assert back["model.22.cv3.%d.0.conv.weight" % l].shape == (cc, c, 3, 3)
+        assert back["model.22.cv3.%d.1.conv.weight" % l].shape == (cc, cc, 3, 3)
+        assert back["model.22.cv3.%d.2.weight" % l].shape == (nc, cc, 1, 1)
+        assert back["model.22.cv3.%d.2.bias" % l].shape == (nc,)
+        assert back["model.22.cv2.%d.2.weight" % l].shape == (64, D["cb"], 1, 1)
+        assert np.array_equal(back["model.22.cv3.%d.2.weight" % l], ck["model.22.cv3.%d.2.weight" % l])
+    x = torch.from_numpy(np.random.default_rng(2).normal(0, 1, (2, 3, 640, 640)).astype(np.float32))
+    head = nets.load_net(str(blob)).head_flat(x)
+    assert head.shape == (2, 8400, 64 + nc) and bool(torch.isfinite(head).all())
+
+
 def test_fused_anonymous_onnx_is_matched_by_order(tmp_path):
     """Exports with Conv+BN fused rename the initialisers (onnx::Conv_<n>): layers are matched by order and shape."""
     kind, params, tensors = W.synth_yolov8_weights("n", seed=3)
